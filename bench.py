@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--rays-per-step R] [--precision exact|fast]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...     # the reference's CPU algorithm (restated oracle) on the host cores
+  python bench.py ... --dump-outputs DIR   # also writes the last timed step's image and counters as DIR/<name>.npy
 
 Workload (config.workload): BASELINE config "CAST magnet + LLNL telescope, detector chain active
 (Si3N4/Al window + Ar), 1e9 rays" — the largest single-GPU configuration of the setup the north-star target is
@@ -20,6 +21,7 @@ import argparse
 import ctypes as C
 import json
 import os
+import signal
 import statistics
 import subprocess
 import sys
@@ -52,7 +54,13 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-presampled", action="store_true", help="skip the tier-(a) pre-sampled kernel measurement")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configurations (2, 4, 5)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (image, w^2 image, counters) "
+                         "as DIR/<name>.npy in float64, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm sizes its steps by its own speed)")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -184,9 +192,12 @@ class ClockSampler:
         self.p = None
 
     def start(self):
+        # PR_SET_PDEATHSIG: the sampler gets SIGTERM when bench.py exits, also when it dies before stop()
+        libc = C.CDLL(None, use_errno=True)
         try:
             self.p = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.QUERY}", "--format=csv,noheader,nounits",
-                                       "-lms", "100", "-i", str(self.index)], stdout=self.f, stderr=subprocess.DEVNULL)
+                                       "-lms", "100", "-i", str(self.index)], stdout=self.f, stderr=subprocess.DEVNULL,
+                                      preexec_fn=lambda: libc.prctl(1, signal.SIGTERM))
         except OSError:
             self.p = None
 
@@ -526,6 +537,21 @@ def passed_leg(tr, torch, n: int = 1 << 26, reps: int = 3):
             "retraced_fp64_fraction": cnt["n_retraced"] / n}
 
 
+def dump_outputs(res, out_dir: str):
+    """Writes a step's outputs as out_dir/<name>.npy, float64: `image` and `image_w2` [M, 256, 256], every counter per
+    mass [M] and `n_exit` [M, 13] (columns in abi.EXIT_NAMES order), M = number of axion masses. n_retraced and
+    n_unresolved are left out: they tell how the FP32 pipeline reached its result, not what the result is."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    arrays = {"image": res.image, "image_w2": res.image_w2, "n_exit": [list(c["n_exit"].values()) for c in res.counters]}
+    for name in res.counters[0]:
+        if name not in ("n_exit", "n_retraced", "n_unresolved"):
+            arrays[name] = [c[name] for c in res.counters]
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", np.asarray(a, dtype=np.float64))
+
+
 def ncu_traffic(kernel: str):
     """DRAM bytes per launch of `kernel` from the committed ncu --set full capture (profiles/ncu_traffic.json), or None."""
     try:
@@ -619,6 +645,16 @@ def run_ours(args):
         ms_total = e0.elapsed_time(e1)
         kernel_ms = [a.elapsed_time(b) for a, b in kev]
     res = tr.read_merged() if dist is not None else tr.read_image()
+    if args.dump_outputs:
+        # the image accumulates over the timed steps: trace the last one again into a cleared image. These are the same
+        # rays (Philox is keyed on the global ray index), and the timed window stays free of host reads.
+        with torch.cuda.stream(stream):
+            tr.reset_image()
+            step(W + K - 1)
+        barrier()
+        last = tr.read_merged() if dist is not None else tr.read_image()
+        if rank == 0:
+            dump_outputs(last, args.dump_outputs)
     # per-rank kernel times: a straggler rank must be visible
     t_k = torch.tensor(kernel_ms, dtype=torch.float64, device=f"cuda:{local}")
     all_k = [torch.empty_like(t_k) for _ in range(world)]
