@@ -359,6 +359,20 @@ int sart_reset_image(sart_handle_t* h);
  * nbins = 0 switches it off (default). sum_w / counts are host arrays [nbins] (either may be NULL). */
 int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max);
 int sart_read_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
+/* Optional weighted spectra of the rays that PASS (weight != 0, rt:2220) in sart_trace_mc, single axion mass — the
+ * reductions generateResultPlots (rt:2246-2635) makes over energiesAx, shellNumber and weights, without per-ray records:
+ * energy bin i < nEnergies = tabulated energy i (a Monte Carlo ray's energy is a table value, rt:470), bin nEnergies = the
+ * X-ray test source's energy; shell bin j = shellNumber (rt:2198). Accumulated (+=) like the image and cleared by
+ * sart_reset_image; filled in every precision mode, by the FP32 kernel and by the FP64 re-trace of its uncertain rays
+ * alike, so precision 2 has the counts of precision 0. With spectra on, precision modes 1 and 2 run the generic kernel
+ * variant (as with the radial histogram) and sart_trace_mc with more than one axion mass fails with SART_ERR_CONFIG.
+ * sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev) and sart_trace_words leave
+ * them untouched. on != 0 synchronises, then (re)allocates and zeroes them; on = 0 switches them off (default). */
+int sart_enable_spectra(sart_handle_t* h, int on);
+/* Synchronises and copies out; host arrays, any may be NULL: energy_* [nEnergies + 1], shell_* [SART_MAX_SHELLS].
+ * SART_ERR_ARG when the spectra are off. */
+int sart_read_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
+                      double* shell_sum_w, uint64_t* shell_counts);
 /* Device pointers for collectives (ncclAllReduce / torch.distributed on the caller's side). */
 double* sart_image_dev(sart_handle_t* h);       /* [M][256][256] Σw  */
 double* sart_image_w2_dev(sart_handle_t* h);    /* [M][256][256] Σw² */

@@ -3,7 +3,8 @@
 
   python -m solaraxionraytracing_b200 [--ignoreDetWindow] [--ignoreGasAbs] [--ignoreConvProb] [--ignoreReflection]
       [--xrayTest] [--detectorInstall] [--magnet] [--angularScanMin A --angularScanMax B --numAngularScanPoints N]
-      [--noPlots] [--config FILE | --configPath DIR] [--nRays N] [--precision f32|fast|exact] [--device D]
+      [--noPlots] [--config FILE | --configPath DIR] [--nRays N] [--precision f32|fast|exact] [--writeSpectra]
+      [--device D]
 
 Inputs the reference reads from `resources/` and that are not shipped with it (solar_model_dataframe.csv, the two
 reflectivity HDF5 files) are taken from [Resources] when present, else generated: Primakoff emission rates from AGSS09
@@ -33,6 +34,9 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--precision", choices=["f32", "fast", "exact"], default=None)
     ap.add_argument("--sampler", choices=["inverse_cdf", "alias"], default=None,
                     help="alias: emission shell / energy from alias tables of the same distributions (f32, single mass)")
+    ap.add_argument("--writeSpectra", action="store_true",
+                    help="also write the energy spectrum and the per-shell flux of the detected rays as CSV files next to "
+                         "the image (single-mass runs; the run then takes the generic kernel variant)")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--outputPath", default="", help="overrides [Resources].outputPath")
     ap.add_argument("--allowSynthetic", action="store_true",
@@ -130,8 +134,13 @@ def main(argv=None) -> int:
             tr.set_axion_masses(run.mAxion)
         if a.angularScanMin == a.angularScanMax:
             print("start")
+            spectra = a.writeSpectra and len(run.mAxion) <= 1
+            if a.writeSpectra and not spectra:
+                print("--writeSpectra: spectra are written for single-mass runs only", file=sys.stderr)
             if len(run.mAxion) <= 1:
                 tr.enable_radial_hist()
+            if spectra:
+                tr.enable_spectra()
             tr.reset_image()
             tr.trace_mc(n, a.seed)
             result = tr.read_image()
@@ -140,6 +149,9 @@ def main(argv=None) -> int:
                 path = output.generateResultPlots(result, setup.detector.windowYear, outpath, radii=radii,
                                                   chipXMax=setup.consts.chipXMax, chipYMax=setup.consts.chipYMax)
                 print("wrote", path)
+                if spectra:
+                    for p in output.write_spectra_csvs(tr.read_spectra(), setup.detector.windowYear, outpath):
+                        print("wrote", p)
             else:   # mass scan: one image per mass, total flux per mass on stdout
                 Path(outpath).mkdir(parents=True, exist_ok=True)
                 for m, c in zip(run.mAxion, result.counters):

@@ -202,6 +202,8 @@ SIGNATURES = {
     "sart_reset_image": (C.c_int, [H]),
     "sart_enable_radial_hist": (C.c_int, [H, C.c_int, C.c_double]),
     "sart_read_radial_hist": (C.c_int, [H, c_double_p, C.POINTER(C.c_uint64)]),
+    "sart_enable_spectra": (C.c_int, [H, C.c_int]),
+    "sart_read_spectra": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64), c_double_p, C.POINTER(C.c_uint64)]),
     "sart_image_dev": (C.c_void_p, [H]),
     "sart_image_w2_dev": (C.c_void_p, [H]),
     "sart_counters_dev": (C.c_void_p, [H]),

@@ -501,6 +501,24 @@ static int ensure_stage(sart_handle* h, size_t bytes) {
   return SART_OK;
 }
 
+// One allocation of spectra (device_params.h: Spectra), 8-byte words: eW | eW2 | eN, each eRep x eStride | sW | sN, each
+// sRep x SART_MAX_SHELLS.
+static size_t spectra_bytes(int eStride, int eRep, int sRep) {
+  return 3 * align256(size_t(eRep) * eStride * 8) + 2 * align256(size_t(sRep) * SART_MAX_SHELLS * 8);
+}
+static Spectra carve_spectra(void* base, int eStride, int eRep, int sRep) {
+  unsigned char* p = static_cast<unsigned char*>(base);
+  const size_t e = align256(size_t(eRep) * eStride * 8), s = align256(size_t(sRep) * SART_MAX_SHELLS * 8);
+  Spectra r{};
+  r.eW = reinterpret_cast<double*>(p);
+  r.eW2 = reinterpret_cast<double*>(p + e);
+  r.eN = reinterpret_cast<unsigned long long*>(p + 2 * e);
+  r.sW = reinterpret_cast<double*>(p + 3 * e);
+  r.sN = reinterpret_cast<unsigned long long*>(p + 3 * e + s);
+  r.eStride = uint32_t(eStride); r.eRepMask = uint32_t(eRep - 1); r.sRepMask = uint32_t(sRep - 1);
+  return r;
+}
+
 // Parameter block of `s` for a live handle: setup-derived fields recomputed, table-derived fields kept.
 static void rederive_params(const sart_handle* h, const sart_setup_t& s, Params* p) {
   const Params old = h->params;
@@ -638,7 +656,7 @@ void sart_destroy(sart_handle_t* h) {
   sart_comm_destroy(h);
   cudaFree(h->table_blob); cudaFree(h->fast_blob); cudaFree(h->d_masses); cudaFree(h->d_image); cudaFree(h->d_merged);
   cudaFree(h->d_counters); cudaFree(h->d_stage); cudaFree(h->d_rad_w); cudaFree(h->d_rad_n); cudaFree(h->d_rep); cudaFree(h->d_mass_acc);
-  cudaFree(h->d_queue);
+  cudaFree(h->d_queue); cudaFree(h->d_spec); cudaFree(h->d_spec_rep);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->stream_in) cudaStreamDestroy(h->stream_in);
   if (h->stream_out) cudaStreamDestroy(h->stream_out);
@@ -1132,6 +1150,7 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   DeviceGuard dg(h->device);
   if (h->sampler == SART_SAMPLER_ALIAS && (h->precision != 2 || h->n_masses > 1))
     return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2 and a single axion mass");
+  if (h->spec.eW && h->n_masses > 1) return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass");
   // Precision 2: launches of at most 2^31 rays, each followed on the same stream by the exact pipeline's pass over the
   // rays the FP32 kernel queued as uncertain (it adds them to the same image and counters). Not with the alias sampler,
   // whose ray <-> index mapping is not the exact pipeline's.
@@ -1167,6 +1186,7 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
     if (rc) return rc;
     const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
     fast::FastTables ft = h->ftables;
+    ft.spec = h->spec_rep;   // the spectra replicas, or off
     double *img = h->d_image, *img2 = h->d_image_w2;
     if (h->n_rep > 1) {
       ft.nImgRep = h->n_rep; ft.imgRepStride = h->rep_stride;
@@ -1181,6 +1201,7 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
         if (ft.rq.cap) {
           Tables et = h->tables;
           if (!ft.rad.w) et.rad = RadialHist{};
+          et.spec = h->spec;   // the re-traced rays belong in the spectra as much as in the image
           SART_CUDA(launch_retrace_mc_image(h->params, et, 1, h->d_masses, first_ray + done, seed, ft.rq, h->d_image,
                                             h->d_image_w2, h->d_counters, h->sm_count, h->stream));
         }
@@ -1191,9 +1212,12 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
     }
     if (h->n_rep > 1)
       SART_CUDA(launch_fold_replicas(img, img2, h->n_rep, h->rep_stride, plane, h->d_image, h->d_image_w2, h->stream));
+    if (h->spec.eW) SART_CUDA(launch_fold_spectra(h->spec_rep, h->spec_e1, h->spec, h->stream));
     return SART_OK;
   }
-  SART_CUDA(launch_mc_image_exact(h->params, h->tables, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
+  Tables et = h->tables;
+  et.spec = h->spec;
+  SART_CUDA(launch_mc_image_exact(h->params, et, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
                                   h->d_image_w2, h->d_counters, h->sm_count, h->stream));
   return SART_OK;
 }
@@ -1208,6 +1232,53 @@ int sart_reset_image(sart_handle_t* h) {
     SART_CUDA(cudaMemsetAsync(h->d_rad_w, 0, size_t(h->rad_bins) * sizeof(double), h->stream));
     SART_CUDA(cudaMemsetAsync(h->d_rad_n, 0, size_t(h->rad_bins) * sizeof(unsigned long long), h->stream));
   }
+  if (h->spec.eW) SART_CUDA(cudaMemsetAsync(h->d_spec, 0, spectra_bytes(h->spec_e1, 1, 1), h->stream));
+  return SART_OK;
+}
+
+int sart_enable_spectra(sart_handle_t* h, int on) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  DeviceGuard dg(h->device);
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  cudaFree(h->d_spec); cudaFree(h->d_spec_rep);
+  h->d_spec = nullptr; h->d_spec_rep = nullptr; h->spec = Spectra{}; h->spec_rep = Spectra{}; h->spec_e1 = 0;
+  if (!on) return SART_OK;
+  const int nE1 = h->params.nEnergies + 1;
+  // Replicas of the throughput kernels (powers of two; SART_SPEC_E_REPLICAS / SART_SPEC_S_REPLICAS override them for
+  // measurements). The energy bins spread the passed rays over hundreds of addresses, like the focal spot the image
+  // replicas serve: one replica per block residue. The shell bins are a handful of addresses (4 for LLNL): one per warp.
+  auto pow2 = [](const char* env, int dflt) {
+    int n = dflt;
+    if (const char* e = std::getenv(env)) n = std::max(1, std::min(1 << 16, std::atoi(e)));
+    int p = 1;
+    while (p * 2 <= n) p *= 2;
+    return p;
+  };
+  const int eRep = pow2("SART_SPEC_E_REPLICAS", 32), sRep = pow2("SART_SPEC_S_REPLICAS", 1024);
+  const uint32_t eStride = uint32_t((nE1 + 31) & ~31);
+  SART_CUDA(cudaMalloc(&h->d_spec, spectra_bytes(nE1, 1, 1)));
+  SART_CUDA(cudaMalloc(&h->d_spec_rep, spectra_bytes(int(eStride), eRep, sRep)));
+  SART_CUDA(cudaMemsetAsync(h->d_spec, 0, spectra_bytes(nE1, 1, 1), h->stream));
+  SART_CUDA(cudaMemsetAsync(h->d_spec_rep, 0, spectra_bytes(int(eStride), eRep, sRep), h->stream));
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  h->spec = carve_spectra(h->d_spec, nE1, 1, 1);
+  h->spec_rep = carve_spectra(h->d_spec_rep, int(eStride), eRep, sRep);
+  h->spec_e1 = nE1;
+  return SART_OK;
+}
+
+int sart_read_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
+                      double* shell_sum_w, uint64_t* shell_counts) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (!h->spec.eW) return fail(SART_ERR_ARG, "sart_read_spectra: no spectra enabled (sart_enable_spectra)");
+  DeviceGuard dg(h->device);
+  const size_t e = size_t(h->spec_e1) * 8, s = size_t(SART_MAX_SHELLS) * 8;
+  if (energy_sum_w) SART_CUDA(cudaMemcpyAsync(energy_sum_w, h->spec.eW, e, cudaMemcpyDeviceToHost, h->stream));
+  if (energy_sum_w2) SART_CUDA(cudaMemcpyAsync(energy_sum_w2, h->spec.eW2, e, cudaMemcpyDeviceToHost, h->stream));
+  if (energy_counts) SART_CUDA(cudaMemcpyAsync(energy_counts, h->spec.eN, e, cudaMemcpyDeviceToHost, h->stream));
+  if (shell_sum_w) SART_CUDA(cudaMemcpyAsync(shell_sum_w, h->spec.sW, s, cudaMemcpyDeviceToHost, h->stream));
+  if (shell_counts) SART_CUDA(cudaMemcpyAsync(shell_counts, h->spec.sN, s, cudaMemcpyDeviceToHost, h->stream));
+  SART_CUDA(cudaStreamSynchronize(h->stream));
   return SART_OK;
 }
 

@@ -72,6 +72,34 @@ struct RadialHist {
   int32_t nbins, pad;
 };
 
+// Optional spectra of the passed rays (sart_enable_spectra): Σw, Σw² and the ray count per energy bin (the index of the
+// ray's tabulated energy, rt:470; bin nEnergies = the X-ray source), Σw and the ray count per mirror shell (shellNumber
+// rt:2198). eW == nullptr: off. Replica r of the energy arrays starts r * eStride elements in, replica r of the shell
+// arrays r * SART_MAX_SHELLS; a block adds into energy replica (block & eRepMask) and a warp into shell replica
+// (global warp & sRepMask). Masks 0 = the arrays themselves (the exact kernels; the throughput kernels get replicas that a
+// fold kernel adds up after the launch). 64 bytes: the kernel parameters behind a table block keep their 16-byte alignment.
+struct Spectra {
+  double* eW;
+  double* eW2;
+  unsigned long long* eN;
+  double* sW;
+  unsigned long long* sN;
+  uint32_t eStride, eRepMask, sRepMask, pad[3];
+};
+static_assert(sizeof(Spectra) == 64, "Spectra: 64 bytes");
+
+#if defined(__CUDACC__)
+__device__ __forceinline__ void spec_add(const Spectra& s, int eBin, int shell, double w) {
+  const uint32_t e = (blockIdx.x & s.eRepMask) * s.eStride + uint32_t(eBin);
+  atomicAdd(s.eW + e, w);
+  atomicAdd(s.eW2 + e, w * w);
+  atomicAdd(s.eN + e, 1ull);
+  const uint32_t k = ((blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) & s.sRepMask) * uint32_t(SART_MAX_SHELLS) + uint32_t(shell);
+  atomicAdd(s.sW + k, w);
+  atomicAdd(s.sN + k, 1ull);
+}
+#endif
+
 // Table pointers (device memory).
 struct Tables {
   const double* energies;
@@ -92,6 +120,7 @@ struct Tables {
   // contraction on either side => the same bits). A Monte Carlo ray's energy is a table value (rt:470), so its three
   // 10-step binary searches with dependent loads become one 32-byte record.
   const struct EnergyFactors* energyFactors;   // [nEnergies]
+  Spectra spec;   // optional (last member: the offsets of the fields above stay those of the kernels built without it)
 };
 struct EnergyFactors {
   double window, strongback, gas;

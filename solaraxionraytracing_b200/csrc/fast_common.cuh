@@ -135,6 +135,25 @@ __device__ __forceinline__ void rad_add(const RadialHist& h, double r, double w)
   atomicAdd(h.n + b, 1ull);
 }
 
+// Spectra of the throughput kernels (device_params.h: Spectra, spec_add). The energy bins spread the lanes of a warp over
+// hundreds of addresses; the shell bins are a handful (4 for LLNL), so the lanes of a warp that hit the same shell first
+// sum their weights through the warp and one of them adds (measured on CAST+LLNL, 1e9 rays: one add per lane made the
+// spectra cost 73 % of the kernel, the same-address adds of a warp being serialised in L2).
+__device__ __forceinline__ void spec_add_warp(const Spectra& s, int eBin, int shell, double w) {
+  const uint32_t e = (blockIdx.x & s.eRepMask) * s.eStride + uint32_t(eBin);
+  atomicAdd(s.eW + e, w);
+  atomicAdd(s.eW2 + e, w * w);
+  atomicAdd(s.eN + e, 1ull);
+  const unsigned peers = __match_any_sync(__activemask(), shell);
+  double sum = 0.0;
+  for (unsigned m = peers; m; m &= m - 1u) sum += __shfl_sync(peers, w, __ffs(m) - 1);
+  if ((threadIdx.x & 31u) == unsigned(__ffs(peers) - 1)) {
+    const uint32_t k = ((blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) & s.sRepMask) * uint32_t(SART_MAX_SHELLS) + uint32_t(shell);
+    atomicAdd(s.sW + k, sum);
+    atomicAdd(s.sN + k, (unsigned long long)__popc(peers));
+  }
+}
+
 // ---- shared memory layout -----------------------------------------------------------------------------------
 struct WarpCounters { unsigned int n_exit[16]; unsigned int n_clamped; unsigned int n_unresolved; unsigned int pad[2]; };
 
@@ -330,8 +349,10 @@ struct RecordSink {
 // applied where the ray's outcome becomes known. Sums live in the caller's registers, exit counts in the warp's
 // shared-memory counters.
 // kRadial = false compiles the optional radial histogram out (the plain-run kernel variants; the launcher takes the generic
-// variant when sart_enable_radial_hist is on).
-template <bool kRadial>
+// variant when sart_enable_radial_hist is on). kSpectra = false compiles the spectra out: the FP32 launcher has generic
+// variants with and without them, so that a run without spectra runs the code it ran before they existed (measured on
+// BabyIAXO+XMM: the spectra code compiled in but off made the compacting kernel 4 % slower).
+template <bool kRadial, bool kSpectra = kRadial>
 struct ImageSinkT {
   static constexpr bool kFold = true;
   static constexpr bool kRecord = false;
@@ -366,6 +387,7 @@ struct ImageSinkT {
       }
 #endif
       if (kRadial && T.rad.w) rad_add(T.rad, h.r, wd);
+      if (kSpectra && T.spec.eW) spec_add_warp(T.spec, h.eIdx, h.shell, wd);
     } else {
       atomicAdd(&wc.n_exit[SART_EXIT_ZERO_WEIGHT], 1u);
     }

@@ -201,6 +201,9 @@ struct FastTables {
   int32_t nImgRep, pad_;
   uint64_t imgRepStride;
   RetraceQueue rq;            // cap == 0: re-tracing off
+  // optional spectra of the passed rays (device_params.h: Spectra; the generic kernel variants only). Last member, so that
+  // the plain-run kernels, which compile them out, read every other field at the offset they always had.
+  Spectra spec;
 };
 
 }  // namespace fast

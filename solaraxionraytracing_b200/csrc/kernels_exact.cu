@@ -275,6 +275,8 @@ __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, i
       atomicAdd(T.rad.w + b, f.w);
       atomicAdd(T.rad.n + b, 1ull);
     }
+    // spectra (sart_enable_spectra, single mass): the X-ray source's rays carry no table index and go to bin nEnergies
+    if (T.spec.eW && m == 0) spec_add(T.spec, g.eIdx >= 0 ? g.eIdx : P.nEnergies, g.shell, f.w);
   }
 }
 

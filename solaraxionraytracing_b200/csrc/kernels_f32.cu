@@ -26,7 +26,8 @@ namespace fast {
 // ---- fused kernel ---------------------------------------------------------------------------------------------
 // A ray of stage A that is uncertain (rec.unc) goes to the re-trace queue whatever its code; stage B does the same at its
 // own exits. The launcher keeps nRays below 2^32, so the queue entry (ray index - first) fits 32 bits.
-template <bool kWolter, bool kPlain, bool kAlias, bool kMargins>
+// kSpectra: the generic variant that also fills the spectra (sart_enable_spectra; fast_common.cuh: ImageSinkT).
+template <bool kWolter, bool kPlain, bool kAlias, bool kMargins, bool kSpectra = false>
 __global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
 k_trace_mc_f32(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G, const __grid_constant__ FastTables T,
                double mAxion2, uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image,
@@ -44,7 +45,7 @@ k_trace_mc_f32(const __grid_constant__ FastParams P, const __grid_constant__ Geo
   unsigned int nPassed = 0, nTill = 0, nIter = 0;
   double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
   const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
-  ImageSinkT<!kPlain> sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
+  ImageSinkT<!kPlain, kSpectra> sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
   const uint64_t stride = uint64_t(gridDim.x) * kBlock32;
   // 32-bit trip count + running 64-bit ray index: 5 loop instructions per ray instead of 12 (the launcher keeps
   // nRays <= kMaxRaysPerLaunch, so the count fits)
@@ -84,7 +85,7 @@ struct WarpQueue32 {
   uint32_t id[kQueue32];   // ray index - first ray of the launch
 };
 
-template <bool kWolter, bool kPlain, bool kAlias, bool kMargins>
+template <bool kWolter, bool kPlain, bool kAlias, bool kMargins, bool kSpectra = false>
 __global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
 k_trace_mc_f32_compact(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G,
                        const __grid_constant__ FastTables T, double mAxion2, uint64_t first, uint64_t nRays,
@@ -105,7 +106,7 @@ k_trace_mc_f32_compact(const __grid_constant__ FastParams P, const __grid_consta
   unsigned int nPassed = 0, nTill = 0, nIter = 0;
   double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
   const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
-  ImageSinkT<!kPlain> sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
+  ImageSinkT<!kPlain, kSpectra> sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
   const uint64_t stride = uint64_t(gridDim.x) * kBlock32;
   uint64_t base = uint64_t(blockIdx.x) * kBlock32 + (threadIdx.x & ~31);
   const bool solar = kPlain || !P.testXray;
@@ -217,20 +218,21 @@ cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G,
   // alias sampler: solar source only (the X-ray test source draws no table values)
   const bool alias = T.sampler == SART_SAMPLER_ALIAS && !P.testXray && T.radiusAlias && T.energyAlias;
   const size_t smem = fast::smem_bytes32(P, fast::kWarps32, alias) + (compact ? fast::kWarps32 * sizeof(fast::WarpQueue32) : 0);
-  const bool plain = !P.testXray && P.stage == SART_SK_VACUUM && !P.rotated && P.flags == 0 && P.reflKind != SART_RK_EFFECTIVE_AREA && !T.rad.w;
+  const bool plain = !P.testXray && P.stage == SART_SK_VACUUM && !P.rotated && P.flags == 0 && P.reflKind != SART_RK_EFFECTIVE_AREA && !T.rad.w && !T.spec.eW;
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, uint64_t, uint64_t, PhiloxKeys, double*, double*,
                         sart_counters_t*);
-  // [compact][wolter][plain][variant]; variant 0: inverse-CDF sampler, pure FP32; 1: inverse-CDF sampler with the margin tests
-  // (re-trace queue attached); 2: alias sampler (no re-trace: its ray <-> index mapping is not the exact pipeline's)
-#define SART_ROW(K, W, PL) {fast::K<W, PL, false, false>, fast::K<W, PL, false, true>, fast::K<W, PL, true, false>}
-  static const Kern table[2][2][2][3] = {
-      {{SART_ROW(k_trace_mc_f32, false, false), SART_ROW(k_trace_mc_f32, false, true)},
-       {SART_ROW(k_trace_mc_f32, true, false), SART_ROW(k_trace_mc_f32, true, true)}},
-      {{SART_ROW(k_trace_mc_f32_compact, false, false), SART_ROW(k_trace_mc_f32_compact, false, true)},
-       {SART_ROW(k_trace_mc_f32_compact, true, false), SART_ROW(k_trace_mc_f32_compact, true, true)}}};
+  // [compact][wolter][kind][variant]; kind 0: generic, 1: plain, 2: generic with the spectra; variant 0: inverse-CDF sampler,
+  // pure FP32; 1: inverse-CDF sampler with the margin tests (re-trace queue attached); 2: alias sampler (no re-trace: its
+  // ray <-> index mapping is not the exact pipeline's)
+#define SART_ROW(K, W, PL, SP) {fast::K<W, PL, false, false, SP>, fast::K<W, PL, false, true, SP>, fast::K<W, PL, true, false, SP>}
+#define SART_KINDS(K, W) {SART_ROW(K, W, false, false), SART_ROW(K, W, true, false), SART_ROW(K, W, false, true)}
+  static const Kern table[2][2][3][3] = {{SART_KINDS(k_trace_mc_f32, false), SART_KINDS(k_trace_mc_f32, true)},
+                                         {SART_KINDS(k_trace_mc_f32_compact, false), SART_KINDS(k_trace_mc_f32_compact, true)}};
+#undef SART_KINDS
 #undef SART_ROW
   const bool margins = !alias && T.rq.cap != 0u;
-  const Kern kern = table[compact ? 1 : 0][wolter ? 1 : 0][plain ? 1 : 0][alias ? 2 : (margins ? 1 : 0)];
+  const int kind = plain ? 1 : (T.spec.eW ? 2 : 0);
+  const Kern kern = table[compact ? 1 : 0][wolter ? 1 : 0][kind][alias ? 2 : (margins ? 1 : 0)];
   if (getenv("SART_DEBUG"))
     fprintf(stderr, "[sart] k_trace_mc_f32 compact=%d wolter=%d plain=%d alias=%d (sampler=%d ra=%p ea=%p) smem=%zu\n", int(compact),
             int(wolter), int(plain), int(alias), T.sampler, (const void*)T.radiusAlias, (const void*)T.energyAlias, smem);

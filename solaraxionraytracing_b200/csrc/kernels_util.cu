@@ -29,6 +29,44 @@ cudaError_t launch_fold_replicas(double* rep, double* rep2, int nRep, size_t str
   return cudaGetLastError();
 }
 
+// Folds the spectra replicas of a launch (device_params.h: Spectra) into the handle's spectra and clears them. One block per
+// element of the five arrays (eW, eW2, eN [nE1] | sW, sN [SART_MAX_SHELLS]); its threads split the replicas, so that the
+// 1024 shell replicas cost 4 loads per thread instead of one thread's 1024 dependent ones.
+__global__ void __launch_bounds__(256) k_fold_spectra(const __grid_constant__ Spectra rep, int nE1, const __grid_constant__ Spectra dst) {
+  const int b = blockIdx.x;
+  const bool energy = b < 3 * nE1;
+  const int arr = energy ? b / nE1 : 3 + (b - 3 * nE1) / SART_MAX_SHELLS;
+  const int k = energy ? b % nE1 : (b - 3 * nE1) % SART_MAX_SHELLS;
+  const bool isCount = arr == 2 || arr == 4;
+  unsigned long long* const src[5] = {reinterpret_cast<unsigned long long*>(rep.eW), reinterpret_cast<unsigned long long*>(rep.eW2),
+                                      rep.eN, reinterpret_cast<unsigned long long*>(rep.sW), rep.sN};
+  unsigned long long* const out[5] = {reinterpret_cast<unsigned long long*>(dst.eW), reinterpret_cast<unsigned long long*>(dst.eW2),
+                                      dst.eN, reinterpret_cast<unsigned long long*>(dst.sW), dst.sN};
+  const uint32_t nRep = (energy ? rep.eRepMask : rep.sRepMask) + 1u;
+  const size_t stride = energy ? size_t(rep.eStride) : size_t(SART_MAX_SHELLS);
+  double a = 0.0;
+  unsigned long long n = 0ull;
+  for (uint32_t r = threadIdx.x; r < nRep; r += blockDim.x) {
+    unsigned long long* p = src[arr] + size_t(r) * stride + k;
+    const unsigned long long v = *p;
+    if (v) { *p = 0ull; if (isCount) n += v; else a += __longlong_as_double(v); }
+  }
+  for (int o = 16; o > 0; o >>= 1) { a += __shfl_down_sync(0xffffffffu, a, o); n += __shfl_down_sync(0xffffffffu, n, o); }
+  __shared__ double sa[8];
+  __shared__ unsigned long long sn[8];
+  if ((threadIdx.x & 31) == 0) { sa[threadIdx.x >> 5] = a; sn[threadIdx.x >> 5] = n; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < int(blockDim.x >> 5); ++w) { a += sa[w]; n += sn[w]; }
+    if (isCount) { if (n) out[arr][k] += n; }
+    else if (a != 0.0) reinterpret_cast<double*>(out[arr])[k] += a;
+  }
+}
+cudaError_t launch_fold_spectra(const Spectra& rep, int nE1, const Spectra& dst, cudaStream_t s) {
+  k_fold_spectra<<<unsigned(3 * nE1 + 2 * SART_MAX_SHELLS), 256, 0, s>>>(rep, nE1, dst);
+  return cudaGetLastError();
+}
+
 // Mass scan: adds the mass-major accumulators acc[bin][SART_MAX_MASSES] of a launch to the images [mass][bin] and clears them.
 __global__ void __launch_bounds__(256) k_fold_mass_acc(double* __restrict__ acc, double* __restrict__ acc2, int nMasses,
                                                        size_t plane, double* __restrict__ image, double* __restrict__ imageW2) {

@@ -109,6 +109,13 @@ struct sart_handle {
   unsigned long long* d_rad_n = nullptr;
   int rad_bins = 0;
   double rad_rmax = 0.0;
+  // optional spectra of the passed rays (sart_enable_spectra), one allocation each: the handle's arrays (the exact kernels
+  // and the re-trace add into them directly) and the replicas of the throughput kernels (device_params.h: Spectra), which
+  // the fold after every launch adds up and clears. Only sart_trace_mc hands them to a kernel.
+  void* d_spec = nullptr;
+  void* d_spec_rep = nullptr;
+  sart::Spectra spec{}, spec_rep{};   // spec.eW == nullptr: off
+  int spec_e1 = 0;                    // energy bins: nEnergies + 1 (the last one is the X-ray source's)
   // staging for the host-pointer entry points
   void* d_stage = nullptr;
   size_t stage_bytes = 0;

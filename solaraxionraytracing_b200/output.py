@@ -152,6 +152,97 @@ def result_summary(counters: dict, radii: ContainmentRadii | None = None, image:
     return "\n".join(lines)
 
 
+@dataclass
+class Spectra:
+    """Weighted spectra of the passed rays of a run: per energy bin (bin i < nE = tabulated energy i, bin nE = the X-ray
+    source's energy) and per mirror shell (shellNumber rt:2198) the sum of weights, of squared weights and the ray count."""
+    energies_keV: np.ndarray   # [nE + 1]: the tabulated energies, then the source energy (NaN without an X-ray source)
+    sum_w: np.ndarray          # [nE + 1]
+    sum_w2: np.ndarray         # [nE + 1]
+    counts: np.ndarray         # [nE + 1] uint64
+    shell_sum_w: np.ndarray    # [nShells]
+    shell_counts: np.ndarray   # [nShells] uint64
+
+
+def spectra_from_records(energy_keV, shell, weights, energies, source_energy: float | None = None,
+                         n_shells: int = abi.MAX_SHELLS) -> Spectra:
+    """The spectra of per-ray records (traceAxionWrapper output), the host-side counterpart of the fused run's
+    (RayTracer.read_spectra). Rays with weight != 0 are the passed ones (rt:2220). Bins are energy INDICES: a record
+    reports fmax(energies[i], 0.03) keV (rt:470-471), so the index is recovered from the value; table energies below
+    0.03 keV all report 0.03 and are credited to the first of them. With `source_energy` (an X-ray source run, which draws no
+    table energies) every ray goes to bin nE."""
+    E = np.asarray(energy_keV, dtype=np.float64)
+    S = np.asarray(shell, dtype=np.int64)
+    W = np.asarray(weights, dtype=np.float64)
+    en = np.asarray(energies, dtype=np.float64)
+    nE = en.size
+    sel = W != 0.0
+    E, S, W = E[sel], S[sel], W[sel]
+    if source_energy is not None:
+        idx = np.full(E.size, nE, dtype=np.int64)
+    else:
+        reported = np.maximum(en, 0.03)
+        idx = np.searchsorted(reported, E, side="left")
+        ok = (idx < nE) & (reported[np.minimum(idx, nE - 1)] == E)
+        if not ok.all():
+            raise ValueError(f"{int((~ok).sum())} record energies are not tabulated energies")
+    if S.size and (S.min() < 0 or S.max() >= n_shells):
+        raise ValueError("shell numbers of passed rays outside [0, n_shells)")
+    src = np.nan if source_energy is None else float(source_energy)
+    return Spectra(energies_keV=np.append(en, src),
+                   sum_w=np.bincount(idx, weights=W, minlength=nE + 1),
+                   sum_w2=np.bincount(idx, weights=W * W, minlength=nE + 1),
+                   counts=np.bincount(idx, minlength=nE + 1).astype(np.uint64),
+                   shell_sum_w=np.bincount(S, weights=W, minlength=n_shells),
+                   shell_counts=np.bincount(S, minlength=n_shells).astype(np.uint64))
+
+
+SPECTRUM_COLUMNS = ["Energy [keV]", "flux", "flux error", "rays"]
+SHELL_FLUX_COLUMNS = ["shell", "flux", "rays"]
+
+
+def _write_columns(path: str | Path, header: list[str], cols: list[np.ndarray], ints: set[int], precision: int) -> Path:
+    path = Path(path)
+    path.parent.mkdir(parents=True, exist_ok=True)
+    fmt = f"%.{precision}g"
+    with open(path, "w") as f:
+        f.write(",".join(header) + "\n")
+        for k in range(cols[0].size):
+            f.write(",".join(str(int(c[k])) if j in ints else fmt % c[k] for j, c in enumerate(cols)) + "\n")
+    return path
+
+
+def write_energy_spectrum_csv(path: str | Path, spectra: Spectra, precision: int = 17) -> Path:
+    """The energy spectrum of the detected flux: one row per energy bin with a known energy (the source bin is left out
+    without an X-ray source), columns `Energy [keV]`, `flux` (Σw), `flux error` (√Σw²) and `rays`."""
+    keep = np.isfinite(spectra.energies_keV)
+    return _write_columns(path, SPECTRUM_COLUMNS, [spectra.energies_keV[keep], spectra.sum_w[keep],
+                                                   np.sqrt(spectra.sum_w2[keep]), spectra.counts[keep]], {3}, precision)
+
+
+def write_shell_flux_csv(path: str | Path, spectra: Spectra, precision: int = 17) -> Path:
+    """The detected flux per mirror shell: columns `shell`, `flux` (Σw) and `rays`."""
+    n = spectra.shell_sum_w.size
+    return _write_columns(path, SHELL_FLUX_COLUMNS, [np.arange(n), spectra.shell_sum_w, spectra.shell_counts], {0, 2},
+                          precision)
+
+
+def read_columns_csv(path: str | Path) -> dict[str, np.ndarray]:
+    """Reads a CSV written by write_energy_spectrum_csv / write_shell_flux_csv back into its columns."""
+    with open(path) as f:
+        header = f.readline().rstrip("\n").split(",")
+    data = np.loadtxt(path, delimiter=",", skiprows=1, ndmin=2)
+    return {name: data[:, i] for i, name in enumerate(header)}
+
+
+def write_spectra_csvs(spectra: Spectra, windowYear: int, outpath: str | Path, suffix: str = "",
+                       precision: int = 17) -> tuple[Path, Path]:
+    """`axion_energy_spectrum_{year}{suffix}.csv` and `axion_shell_flux_{year}{suffix}.csv` next to the image CSV."""
+    year = WINDOW_YEAR_NAMES.get(windowYear, str(windowYear))
+    return (write_energy_spectrum_csv(Path(outpath) / f"axion_energy_spectrum_{year}{suffix}.csv", spectra, precision),
+            write_shell_flux_csv(Path(outpath) / f"axion_shell_flux_{year}{suffix}.csv", spectra, precision))
+
+
 def generateResultPlots(result, windowYear: int, outpath: str | Path, suffix: str = "",
                         radii: ContainmentRadii | None = None, chipXMax: float = 14.0, chipYMax: float = 14.0,
                         precision: int = 17, echo=print) -> Path:

@@ -15,6 +15,7 @@ import numpy as np
 
 from . import abi, tables as _tables
 from ._lib import SartError, check, lib  # noqa: F401  (re-exported)
+from .output import Spectra
 
 
 def _dp(a: np.ndarray):
@@ -296,6 +297,26 @@ class RayTracer:
         n = np.empty(nbins, dtype=np.uint64)
         check(lib.sart_read_radial_hist(self._h, _dp(w), n.ctypes.data_as(C.POINTER(C.c_uint64))))
         return np.linspace(0.0, r_max, nbins + 1), w, n
+
+    def enable_spectra(self, on: bool = True):
+        """Energy spectrum and per-shell flux of the rays that pass in trace_mc (single axion mass; sart_enable_spectra).
+        Switching them on clears them; precision modes 1 and 2 then run their generic kernel variant."""
+        check(lib.sart_enable_spectra(self._h, int(bool(on))))
+
+    def read_spectra(self) -> Spectra:
+        """The spectra accumulated since enable_spectra / reset_image (raises SartError while they are off)."""
+        en = np.asarray(self.fullSetup.tables.energies if self.fullSetup.tables.energies is not None else [], dtype=np.float64)
+        nE1 = en.size + 1
+        w, w2 = np.empty(nE1), np.empty(nE1)
+        n = np.empty(nE1, dtype=np.uint64)
+        sw = np.empty(abi.MAX_SHELLS)
+        sn = np.empty(abi.MAX_SHELLS, dtype=np.uint64)
+        u64 = C.POINTER(C.c_uint64)
+        check(lib.sart_read_spectra(self._h, _dp(w), _dp(w2), n.ctypes.data_as(u64), _dp(sw), sn.ctypes.data_as(u64)))
+        s = self.fullSetup.expSetup
+        src = s.testSource.energy if s.testSource.active else np.nan
+        ns = s.telescope.nShells
+        return Spectra(np.append(en, src), w, w2, n, sw[:ns].copy(), sn[:ns].copy())
 
     def synchronize(self):
         check(lib.sart_synchronize(self._h))
