@@ -27,7 +27,6 @@ UNITS = [
     ("kernels_fast.cu", []),
     ("kernels_f32.cu", []),
     ("kernels_f32_rays.cu", []),
-    ("kernels_f32x2.cu", []),
     ("kernels_util.cu", []),
     ("kernels_emission.cu", []),
     ("api.cu", []),

@@ -430,7 +430,6 @@ static int ensure_stage(sart_handle* h, size_t bytes);
 
 // Re-trace queue for a launch of n rays of the FP32 pipeline: room for 6 % of them (measured: 0.01 - 0.3 % are
 // uncertain), cleared on the stream. Returns a queue with cap = 0 when re-tracing is off.
-constexpr uint64_t kRetraceChunk = uint64_t(1) << 31;   // rays per launch: queue entries are 32-bit offsets
 static int begin_queue(sart_handle* h, uint64_t n, fast::RetraceQueue* q) {
   *q = fast::RetraceQueue{nullptr, nullptr, 0u, 0u};
   if (!h->retrace || n == 0) return SART_OK;
@@ -447,6 +446,25 @@ static int begin_queue(sart_handle* h, uint64_t n, fast::RetraceQueue* q) {
   return SART_OK;
 }
 
+// A run of the FP32 pipeline: launches of at most fast::kMaxRaysPerLaunch rays, each followed on the same stream by the
+// exact pipeline's pass over the rays it queued as uncertain. f32(done, m, q) launches rays [done, done + m) of the run with
+// queue q attached (cap 0: none), retrace(done, m, q) traces the rays in q. `queue`: whether the run may be re-traced at all
+// (begin_queue attaches no queue either while re-tracing is switched off).
+template <class F32, class Retrace>
+static int f32_then_retrace(sart_handle* h, uint64_t n, bool queue, F32&& f32, Retrace&& retrace) {
+  for (uint64_t done = 0; done < n; done += fast::kMaxRaysPerLaunch) {
+    const uint64_t m = std::min<uint64_t>(n - done, fast::kMaxRaysPerLaunch);
+    fast::RetraceQueue q{};
+    if (queue) {
+      const int rc = begin_queue(h, m, &q);
+      if (rc) return rc;
+    }
+    SART_CUDA(f32(done, m, q));
+    if (q.cap) SART_CUDA(retrace(done, m, q));
+  }
+  return SART_OK;
+}
+
 // Replica buffers for the single-mass throughput kernels. SART_IMG_REPLICAS overrides the count (1 = off).
 static int ensure_replicas(sart_handle* h) {
   if (h->n_rep > 0) return SART_OK;
@@ -454,7 +472,6 @@ static int ensure_replicas(sart_handle* h) {
   if (const char* e = std::getenv("SART_IMG_REPLICAS")) n = std::max(1, std::min(256, std::atoi(e)));
   h->n_rep = n;
   h->rep_stride = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
-  if (const char* e = std::getenv("SART_IMG_REP_SKEW")) h->rep_stride += size_t(std::max(0, std::atoi(e)));   // experiment: replicas not 512 KiB apart
   if (n > 1) {
     const size_t bytes = size_t(2) * n * h->rep_stride * sizeof(double);
     SART_CUDA(cudaMalloc(&h->d_rep, bytes));
@@ -862,16 +879,18 @@ static int check_out(const sart_ray_out_t* out) {
 static int launch_presampled(sart_handle* h, size_t m, const double* dO, const double* dX, const double* dE,
                              const sart_ray_out_t& dev) {
   if (h->precision == 2 && h->ftables.energies) {
-    if (m > kRetraceChunk) return fail(SART_ERR_ARG, "sart_trace_presampled: at most 2^31 rays per call in precision mode 2");
+    if (m > fast::kMaxRaysPerLaunch) return fail(SART_ERR_ARG, "sart_trace_presampled: at most 2^31 rays per call in precision mode 2");
     fast::FastTables ft = h->ftables;
-    int rc = begin_queue(h, m, &ft.rq);
-    if (rc) return rc;
-    SART_CUDA(launch_presampled_f32(h->fparams, h->geo32, ft, h->masses[0], m, dO, dX, dE, dev, h->sm_count, h->stream));
-    if (ft.rq.cap)
-      SART_CUDA(launch_retrace_presampled(h->params, h->tables, h->masses[0], m, dO, dX, dE, ft.rq, dev, h->sm_count, h->stream));
-  } else {
-    SART_CUDA(launch_presampled_exact(h->params, h->tables, h->masses[0], m, dO, dX, dE, dev, h->stream));
+    return f32_then_retrace(h, m, true,   // one launch
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          ft.rq = q;
+          return launch_presampled_f32(h->fparams, h->geo32, ft, h->masses[0], m, dO, dX, dE, dev, h->sm_count, h->stream);
+        },
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          return launch_retrace_presampled(h->params, h->tables, h->masses[0], m, dO, dX, dE, q, dev, h->sm_count, h->stream);
+        });
   }
+  SART_CUDA(launch_presampled_exact(h->params, h->tables, h->masses[0], m, dO, dX, dE, dev, h->stream));
   return SART_OK;
 }
 
@@ -1004,13 +1023,18 @@ int sart_trace_mc_rays(sart_handle_t* h, uint64_t first_ray, size_t n, uint64_t 
   sart_ray_out_t dev;
   carve_out(static_cast<unsigned char*>(h->d_stage), n, *out, &dev);
   if (h->precision == 2) {
-    if (n > kRetraceChunk) return fail(SART_ERR_ARG, "sart_trace_mc_rays: at most 2^31 rays per call");
+    if (n > fast::kMaxRaysPerLaunch) return fail(SART_ERR_ARG, "sart_trace_mc_rays: at most 2^31 rays per call");
     fast::FastTables ft = h->ftables;
-    const bool alias = h->sampler == SART_SAMPLER_ALIAS;   // another ray <-> index mapping than the exact pipeline's: no re-trace
-    if (!alias && (rc = begin_queue(h, n, &ft.rq))) return rc;
-    SART_CUDA(launch_mc_rays_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray, n, seed, dev, h->sm_count, h->stream));
-    if (ft.rq.cap)
-      SART_CUDA(launch_retrace_mc_rays(h->params, h->tables, h->masses[0], first_ray, n, seed, nullptr, ft.rq, dev, h->sm_count, h->stream));
+    // the alias sampler has another ray <-> index mapping than the exact pipeline's: no re-trace
+    rc = f32_then_retrace(h, n, h->sampler != SART_SAMPLER_ALIAS,   // one launch
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          ft.rq = q;
+          return launch_mc_rays_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray, n, seed, dev, h->sm_count, h->stream);
+        },
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          return launch_retrace_mc_rays(h->params, h->tables, h->masses[0], first_ray, n, seed, nullptr, q, dev, h->sm_count, h->stream);
+        });
+    if (rc) return rc;
   } else if (h->precision == 1) {
     SART_CUDA(launch_mc_rays_fast(h->fparams, h->ftables, h->masses[0], first_ray, n, seed, dev, h->sm_count, h->stream));
   } else {
@@ -1088,13 +1112,18 @@ int sart_trace_mc_passed(sart_handle_t* h, uint64_t first_ray, uint64_t n, uint6
     if (k >= 2) SART_CUDA(cudaStreamWaitEvent(h->stream, evCopied(b), 0));   // the records of chunk k - 2 have left this buffer
     SART_CUDA(cudaMemsetAsync(dCount, 0, 256, h->stream));
     fast::FastTables ft = h->ftables;
-    if ((rc = begin_queue(h, m, &ft.rq))) return rc;
     const sart_passed_out_t d = devOut(b);
-    SART_CUDA(launch_mc_passed_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray + done, m, seed, d, dCount, unsigned(chunk),
-                                   uint32_t(done), dCnt, h->sm_count, h->stream));
-    if (ft.rq.cap)
-      SART_CUDA(launch_retrace_mc_passed(h->params, h->tables, h->masses[0], first_ray + done, seed, ft.rq, d, dCount, unsigned(chunk),
-                                         uint32_t(done), dCnt, h->sm_count, h->stream));
+    rc = f32_then_retrace(h, m, true,   // one launch
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          ft.rq = q;
+          return launch_mc_passed_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray + done, m, seed, d, dCount, unsigned(chunk),
+                                      uint32_t(done), dCnt, h->sm_count, h->stream);
+        },
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          return launch_retrace_mc_passed(h->params, h->tables, h->masses[0], first_ray + done, seed, q, d, dCount, unsigned(chunk),
+                                          uint32_t(done), dCnt, h->sm_count, h->stream);
+        });
+    if (rc) return rc;
     SART_CUDA(cudaMemcpyAsync(hcount + b, dCount, sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
     SART_CUDA(cudaEventRecord(evDone(b), h->stream));
     if (k >= 1 && (rc = finish(k - 1))) return rc;
@@ -1130,18 +1159,51 @@ int sart_trace_words(sart_handle_t* h, size_t n, const uint32_t* words, int late
   int32_t* dEmit = emission_shell ? reinterpret_cast<int32_t*>(base + outBytes + wBytes) : nullptr;
   SART_CUDA(cudaMemcpyAsync(dW, words, 6 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
   if (h->precision == 2) {
-    if (n > kRetraceChunk) return fail(SART_ERR_ARG, "sart_trace_words: at most 2^31 rays per call");
+    if (n > fast::kMaxRaysPerLaunch) return fail(SART_ERR_ARG, "sart_trace_words: at most 2^31 rays per call");
     fast::FastTables ft = h->ftables;
-    if (h->sampler != SART_SAMPLER_ALIAS && (rc = begin_queue(h, n, &ft.rq))) return rc;
-    SART_CUDA(launch_mc_rays_f32(h->fparams, h->geo32, ft, h->masses[0], 0, n, 0, dev, h->sm_count, h->stream, dW,
-                                 late_energy != 0, dEmit));
-    if (ft.rq.cap)
-      SART_CUDA(launch_retrace_mc_rays(h->params, h->tables, h->masses[0], 0, n, 0, dW, ft.rq, dev, h->sm_count, h->stream));
+    rc = f32_then_retrace(h, n, h->sampler != SART_SAMPLER_ALIAS,   // one launch
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          ft.rq = q;
+          return launch_mc_rays_f32(h->fparams, h->geo32, ft, h->masses[0], 0, n, 0, dev, h->sm_count, h->stream, dW,
+                                    late_energy != 0, dEmit);
+        },
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          return launch_retrace_mc_rays(h->params, h->tables, h->masses[0], 0, n, 0, dW, q, dev, h->sm_count, h->stream);
+        });
+    if (rc) return rc;
   } else {
     SART_CUDA(launch_mc_rays_exact(h->params, h->tables, h->masses[0], 0, n, 0, dev, h->stream, dW, dEmit));
   }
   if (dEmit) SART_CUDA(cudaMemcpyAsync(emission_shell, dEmit, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
   return copy_out(h, n, *out, dev);
+}
+
+// A fused image run of one axion mass in the handle's precision mode, with the parameter blocks and table views the caller
+// prepared (the handle's, or those of a scan point). The throughput kernels add into img / img2, which ft may spread over
+// replicas; the exact kernels (mode 0, and the re-trace of mode 2) add into exImg / exImg2. All add into `counters`.
+static int trace_image(sart_handle* h, const Params& P, const fast::FastParams& F, const fast::Geo32& G, fast::FastTables ft,
+                       const Tables& et, uint64_t first, uint64_t n, uint64_t seed, double* img, double* img2, double* exImg,
+                       double* exImg2, sart_counters_t* counters) {
+  if (h->precision == 0) {
+    SART_CUDA(launch_mc_image_exact(P, et, 1, h->d_masses, first, n, seed, exImg, exImg2, counters, h->sm_count, h->stream));
+    return SART_OK;
+  }
+  if (h->precision == 1) {
+    SART_CUDA(launch_mc_image_fast(F, ft, h->masses[0], first, n, seed, img, img2, counters, h->sm_count, h->compact != 0,
+                                   h->stream));
+    return SART_OK;
+  }
+  // the alias sampler has another ray <-> index mapping than the exact pipeline's: no re-trace
+  return f32_then_retrace(h, n, h->sampler != SART_SAMPLER_ALIAS,
+      [&](uint64_t done, uint64_t m, const fast::RetraceQueue& q) {
+        ft.rq = q;
+        return launch_mc_image_f32(F, G, ft, h->masses[0], first + done, m, seed, img, img2, counters, h->sm_count,
+                                   h->compact != 0, h->stream);
+      },
+      [&](uint64_t done, uint64_t, const fast::RetraceQueue& q) {
+        return launch_retrace_mc_image(P, et, 1, h->d_masses, first + done, seed, q, exImg, exImg2, counters, h->sm_count,
+                                       h->stream);
+      });
 }
 
 int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_t seed) {
@@ -1151,28 +1213,32 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   if (h->sampler == SART_SAMPLER_ALIAS && (h->precision != 2 || h->n_masses > 1))
     return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2 and a single axion mass");
   if (h->spec.eW && h->n_masses > 1) return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass");
-  // Precision 2: launches of at most 2^31 rays, each followed on the same stream by the exact pipeline's pass over the
-  // rays the FP32 kernel queued as uncertain (it adds them to the same image and counters). Not with the alias sampler,
-  // whose ray <-> index mapping is not the exact pipeline's.
-  const bool retrace = h->precision == 2 && h->retrace && h->sampler != SART_SAMPLER_ALIAS;
-  if (h->precision >= 1 && h->n_masses > 1) {
-    const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS, accLen = plane * SART_MAX_MASSES;
+  const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
+  int rc = SART_OK;
+  if (h->n_masses > 1) {
+    if (h->precision == 0) {
+      SART_CUDA(launch_mc_image_exact(h->params, h->tables, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
+                                      h->d_image_w2, h->d_counters, h->sm_count, h->stream));
+      return SART_OK;
+    }
+    const size_t accLen = plane * SART_MAX_MASSES;
     if (!h->d_mass_acc) {
       SART_CUDA(cudaMalloc(&h->d_mass_acc, 2 * accLen * sizeof(double)));
       SART_CUDA(cudaMemsetAsync(h->d_mass_acc, 0, 2 * accLen * sizeof(double), h->stream));
     }
     if (h->precision == 2) {
-      for (uint64_t done = 0; done < n_rays; done += kRetraceChunk) {
-        const uint64_t n = std::min<uint64_t>(n_rays - done, kRetraceChunk);
-        fast::FastTables ft = h->ftables;
-        int rc = retrace ? begin_queue(h, n, &ft.rq) : SART_OK;
-        if (rc) return rc;
-        SART_CUDA(launch_mc_image_f32_masses(h->fparams, h->geo32, ft, h->n_masses, h->d_masses, first_ray + done, n, seed,
-                                             h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream));
-        if (ft.rq.cap)
-          SART_CUDA(launch_retrace_mc_image(h->params, h->tables, h->n_masses, h->d_masses, first_ray + done, seed, ft.rq,
-                                            h->d_image, h->d_image_w2, h->d_counters, h->sm_count, h->stream));
-      }
+      fast::FastTables ft = h->ftables;
+      rc = f32_then_retrace(h, n_rays, true,   // the alias sampler was refused above
+          [&](uint64_t done, uint64_t m, const fast::RetraceQueue& q) {
+            ft.rq = q;
+            return launch_mc_image_f32_masses(h->fparams, h->geo32, ft, h->n_masses, h->d_masses, first_ray + done, m, seed,
+                                              h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream);
+          },
+          [&](uint64_t done, uint64_t, const fast::RetraceQueue& q) {
+            return launch_retrace_mc_image(h->params, h->tables, h->n_masses, h->d_masses, first_ray + done, seed, q, h->d_image,
+                                           h->d_image_w2, h->d_counters, h->sm_count, h->stream);
+          });
+      if (rc) return rc;
     } else {
       SART_CUDA(launch_mc_image_fast_masses(h->fparams, h->ftables, h->n_masses, h->d_masses, first_ray, n_rays, seed,
                                             h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream));
@@ -1181,44 +1247,24 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
                                    h->stream));
     return SART_OK;
   }
+  Tables et = h->tables;
+  et.spec = h->spec;   // mode 0 and the re-trace of mode 2 add into the spectra directly
+  fast::FastTables ft = h->ftables;
+  double *img = h->d_image, *img2 = h->d_image_w2;
   if (h->precision >= 1) {
-    int rc = ensure_replicas(h);
-    if (rc) return rc;
-    const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
-    fast::FastTables ft = h->ftables;
+    if ((rc = ensure_replicas(h))) return rc;
     ft.spec = h->spec_rep;   // the spectra replicas, or off
-    double *img = h->d_image, *img2 = h->d_image_w2;
     if (h->n_rep > 1) {
       ft.nImgRep = h->n_rep; ft.imgRepStride = h->rep_stride;
       img = h->d_rep; img2 = h->d_rep + size_t(h->n_rep) * h->rep_stride;
     }
-    if (h->precision == 2) {
-      for (uint64_t done = 0; done < n_rays; done += kRetraceChunk) {
-        const uint64_t n = std::min<uint64_t>(n_rays - done, kRetraceChunk);
-        if (retrace && (rc = begin_queue(h, n, &ft.rq))) return rc;
-        SART_CUDA(launch_mc_image_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray + done, n, seed, img, img2,
-                                      h->d_counters, h->sm_count, h->compact != 0, h->stream));
-        if (ft.rq.cap) {
-          Tables et = h->tables;
-          if (!ft.rad.w) et.rad = RadialHist{};
-          et.spec = h->spec;   // the re-traced rays belong in the spectra as much as in the image
-          SART_CUDA(launch_retrace_mc_image(h->params, et, 1, h->d_masses, first_ray + done, seed, ft.rq, h->d_image,
-                                            h->d_image_w2, h->d_counters, h->sm_count, h->stream));
-        }
-      }
-    } else {
-      SART_CUDA(launch_mc_image_fast(h->fparams, ft, h->masses[0], first_ray, n_rays, seed, img, img2, h->d_counters,
-                                     h->sm_count, h->compact != 0, h->stream));
-    }
-    if (h->n_rep > 1)
-      SART_CUDA(launch_fold_replicas(img, img2, h->n_rep, h->rep_stride, plane, h->d_image, h->d_image_w2, h->stream));
-    if (h->spec.eW) SART_CUDA(launch_fold_spectra(h->spec_rep, h->spec_e1, h->spec, h->stream));
-    return SART_OK;
   }
-  Tables et = h->tables;
-  et.spec = h->spec;
-  SART_CUDA(launch_mc_image_exact(h->params, et, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
-                                  h->d_image_w2, h->d_counters, h->sm_count, h->stream));
+  rc = trace_image(h, h->params, h->fparams, h->geo32, ft, et, first_ray, n_rays, seed, img, img2, h->d_image, h->d_image_w2,
+                   h->d_counters);
+  if (rc || h->precision == 0) return rc;
+  if (h->n_rep > 1)
+    SART_CUDA(launch_fold_replicas(img, img2, h->n_rep, h->rep_stride, plane, h->d_image, h->d_image_w2, h->stream));
+  if (h->spec.eW) SART_CUDA(launch_fold_spectra(h->spec_rep, h->spec_e1, h->spec, h->stream));
   return SART_OK;
 }
 
@@ -1390,37 +1436,23 @@ int sart_angular_scan(sart_handle_t* h, int n_angles, const double* angles_deg, 
     s.telescope.telescope_turned_y = angles_deg[i];   // rt:2796
     Params P;
     rederive_params(h, s, &P);
-    const uint64_t first = first_ray + uint64_t(i) * n_rays_per_angle;   // every scan point traces its own rays, like the reference
+    fast::FastParams F{};
+    fast::Geo32 G{};
     if (h->precision >= 1) {
-      fast::FastParams F;
       fast::derive_params(s, P, &F);
       F.shellRhoMin = h->fparams.shellRhoMin; F.shellInvStep = h->fparams.shellInvStep; F.nShellGuide = h->fparams.nShellGuide;
-      if (h->precision == 2) {
-        fast::Geo32 G;
-        std::vector<fast::ShellF32> unused(SART_MAX_SHELLS);
-        fast::derive_f32(F, nullptr, 0, &G, unused.data());
-        // error budgets: the handle's (they depend on the shells, which do not turn), doubled where the rotation of the
-        // telescope frame adds rounding steps
-        G.tol = h->geo32.tol;
-        if (F.rotated && !h->fparams.rotated) { G.tol.latA *= 2.0f; G.tol.detA *= 2.0f; }
-        for (uint64_t done = 0; done < n_rays_per_angle; done += kRetraceChunk) {
-          const uint64_t n = std::min<uint64_t>(n_rays_per_angle - done, kRetraceChunk);
-          fast::FastTables fq = ft;
-          if (h->retrace && h->sampler != SART_SAMPLER_ALIAS && (rc = begin_queue(h, n, &fq.rq))) return rc;
-          SART_CUDA(launch_mc_image_f32(F, G, fq, h->masses[0], first + done, n, seed, dImg + size_t(i) * plane,
-                                        dImg2 + size_t(i) * plane, dCnt + i, h->sm_count, h->compact != 0, h->stream));
-          if (fq.rq.cap)
-            SART_CUDA(launch_retrace_mc_image(P, et, 1, h->d_masses, first + done, seed, fq.rq, dImg + size_t(i) * plane,
-                                              dImg2 + size_t(i) * plane, dCnt + i, h->sm_count, h->stream));
-        }
-        continue;
-      }
-      SART_CUDA(launch_mc_image_fast(F, ft, h->masses[0], first, n_rays_per_angle, seed, dImg + size_t(i) * plane,
-                                     dImg2 + size_t(i) * plane, dCnt + i, h->sm_count, h->compact != 0, h->stream));
-    } else {
-      SART_CUDA(launch_mc_image_exact(P, et, 1, h->d_masses, first, n_rays_per_angle, seed, dImg + size_t(i) * plane,
-                                      dImg2 + size_t(i) * plane, dCnt + i, h->sm_count, h->stream));
     }
+    if (h->precision == 2) {
+      std::vector<fast::ShellF32> unused(SART_MAX_SHELLS);
+      fast::derive_f32(F, nullptr, 0, &G, unused.data());
+      // error budgets: the handle's (they depend on the shells, which do not turn), doubled where the rotation of the
+      // telescope frame adds rounding steps
+      G.tol = h->geo32.tol;
+      if (F.rotated && !h->fparams.rotated) { G.tol.latA *= 2.0f; G.tol.detA *= 2.0f; }
+    }
+    const uint64_t first = first_ray + uint64_t(i) * n_rays_per_angle;   // every scan point traces its own rays, like the reference
+    double *img = dImg + size_t(i) * plane, *img2 = dImg2 + size_t(i) * plane;
+    if ((rc = trace_image(h, P, F, G, ft, et, first, n_rays_per_angle, seed, img, img2, img, img2, dCnt + i))) return rc;
   }
   std::vector<sart_counters_t> cnt;
   cnt.resize(size_t(n_angles));

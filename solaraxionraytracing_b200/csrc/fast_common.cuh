@@ -19,13 +19,6 @@ namespace fast {
 #ifndef SART_FAST_MINBLOCKS
 #define SART_FAST_MINBLOCKS 3
 #endif
-#ifndef SART_REFL_ALIGNED
-#define SART_REFL_ALIGNED 0   // measured slower (35.2 -> 37.6 ms): 16 bytes per lane through L1TEX cost more than the request saved
-#endif
-#ifndef SART_LAZY_THR
-#define SART_LAZY_THR 1   // second group of four energy thresholds loaded only by the ~12 % of lanes that need it: one
-                          // divergent 32-line gather less per ray (CAST+LLNL, gather-bound: 35.2 -> 32.8 ms)
-#endif
 constexpr int kBlock = SART_FAST_BLOCK;
 constexpr int kWarps = kBlock / 32;
 
@@ -205,7 +198,7 @@ __device__ __forceinline__ int guide_upper(const uint16_t* __restrict__ guide, u
 // Reflectivity at grazing angle alphaDeg from the row pre-interpolated at the ray's energy: linear in the angle.
 // (Variants measured on B200 and rejected: rows of overlapping 16-byte quads — one load per lookup, but the table grows by
 // a third and CAST+LLNL, whose tables already fill most of one L2 partition, loses 25 %; one aligned 16-byte load plus a
-// conditional second one — no gain over two 4-byte loads.)
+// conditional second one — slower, 35.2 -> 37.6 ms: 16 bytes per lane through L1TEX cost more than the requests saved.)
 __device__ __forceinline__ float refl_lookup(const FastParams& P, const float* __restrict__ row, float alphaDeg, bool& clamped,
                                              uint32_t rowOff = 0u) {   // rowOff: 32-bit element offset of the row in `row`
   const float x = fminf(fmaxf(alphaDeg, P.angleMin), P.angleMax);   // NaN -> angleMin
@@ -213,18 +206,8 @@ __device__ __forceinline__ float refl_lookup(const FastParams& P, const float* _
   const float fx = (x - P.angleMin) * P.invReflDx;
   int i = int(fx);
   if (i > P.nAngles - 2) i = P.nAngles - 2;
-#if SART_REFL_ALIGNED
-  // one aligned 16-byte load holds both nodes of the cell unless the cell straddles two such words (1 lookup in 4):
-  // 1.25 gather requests per lookup instead of 2 (rows start 16-byte aligned: nAngles % 4 == 0, checked at create)
-  const int j = i & 3;
-  const float4 z = __ldg(reinterpret_cast<const float4*>(row + rowOff + (i - j)));
-  const float z0 = j == 0 ? z.x : (j == 1 ? z.y : (j == 2 ? z.z : z.w));
-  float z1 = j == 0 ? z.y : (j == 1 ? z.z : z.w);
-  if (j == 3) z1 = __ldg(row + rowOff + i + 1);
-#else
   const float* cell = row + (rowOff + uint32_t(i));   // one 32-bit add + one wide multiply-add per lookup
   const float z0 = __ldg(cell), z1 = __ldg(cell + 1);
-#endif
   return fmaf(fx - float(i), z1 - z0, z0);
 }
 

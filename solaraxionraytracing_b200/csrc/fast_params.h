@@ -130,6 +130,9 @@ struct RetraceQueue {
   uint32_t* count;
   uint32_t cap, pad;
 };
+// Rays per launch of the FP32 kernels: queue entries (ray index - first ray of the launch) and the fused kernel's per-thread
+// trip count are 32-bit. api.cu cuts longer runs into launches of at most this many rays.
+constexpr uint64_t kMaxRaysPerLaunch = uint64_t(1) << 31;
 
 // Radial lookup of the shell search (rt:1932-1957) for the FP32 kernels: the radial buckets of the shell guide are fine
 // enough to hold at most one boundary (a shell's front radius R1 or the outer edge R1 + thickness of its glass) each,

@@ -8,6 +8,37 @@
 
 namespace sart {
 
+// Run-wide switches of a throughput launch, decided on the host and compiled into the kernel variants as template
+// parameters.
+struct LaunchVariant {
+  bool wolter;    // Wolter-I optic (XMM, ABRIXAS) instead of two cones
+  bool plain;     // solar source, vacuum stage, unturned telescope, no flags, a reflectivity table
+  bool alias;     // alias sampler (solar source only: the X-ray test source draws no table values)
+  bool margins;   // a re-trace queue is attached: the FP32 kernels test their decision margins
+};
+inline LaunchVariant launch_variant(const fast::FastParams& P, const fast::FastTables& T) {
+  LaunchVariant v;
+  v.wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
+  v.plain = !P.testXray && P.stage == SART_SK_VACUUM && !P.rotated && P.flags == 0 && P.reflKind != SART_RK_EFFECTIVE_AREA;
+  v.alias = T.sampler == SART_SAMPLER_ALIAS && !P.testXray && T.radiusAlias && T.energyAlias;
+  v.margins = T.rq.cap != 0u;
+  return v;
+}
+
+// Grid of a grid-stride launch over n rays: one thread per ray, at most perSM blocks on each of smCount SMs. perSM = 0: one
+// resident wave, i.e. the occupancy of `kern` with `smem` bytes of dynamic shared memory (at least one block per SM).
+template <class K>
+inline cudaError_t grid_size(K kern, int block, size_t smem, uint64_t n, int smCount, int perSM, unsigned* grid) {
+  if (perSM == 0) {
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kern, block, smem);
+    if (e != cudaSuccess) return e;
+    if (perSM < 1) perSM = 1;
+  }
+  const uint64_t want = (n + block - 1) / block, cap = uint64_t(smCount) * perSM;
+  *grid = unsigned(want < cap ? want : cap);
+  return cudaSuccess;
+}
+
 // ---- FP64 "exact" pipeline (kernels_exact.cu)
 cudaError_t launch_presampled_exact(const Params& P, const Tables& T, double mAxion, size_t n, const double* origin,
                                     const double* exitxy, const double* energy, const sart_ray_out_t& out,

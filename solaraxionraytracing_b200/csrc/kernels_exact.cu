@@ -440,13 +440,9 @@ cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses,
   if (nRays == 0) return cudaSuccess;
   const int block = 128;
   const size_t smem = sizeof(BlockCounters) + size_t(nMasses) * sizeof(MassCounters);
-  int perSM = 0;
-  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image, block, smem);
+  unsigned grid = 0;   // one resident wave; the grid-stride loop covers the rest
+  const cudaError_t e = grid_size(k_trace_mc_image, block, smem, nRays, smCount, 0, &grid);
   if (e != cudaSuccess) return e;
-  if (perSM < 1) perSM = 1;
-  uint64_t want = (nRays + block - 1) / block;
-  uint64_t cap = uint64_t(smCount) * perSM;  // one resident wave; the grid-stride loop covers the rest
-  const unsigned grid = unsigned(want < cap ? want : cap);
   k_trace_mc_image<<<grid, block, smem, s>>>(P, T, nMasses, masses, first, nRays, seed, nullptr, nullptr, 0u, image, imageW2,
                                              counters);
   return cudaGetLastError();

@@ -16,16 +16,12 @@
 
 #include "trace_f32.cuh"
 
-#ifndef SART_F32_PAIR_DEFAULT
-#define SART_F32_PAIR_DEFAULT 0
-#endif
-
 namespace sart {
 namespace fast {
 
 // ---- fused kernel ---------------------------------------------------------------------------------------------
 // A ray of stage A that is uncertain (rec.unc) goes to the re-trace queue whatever its code; stage B does the same at its
-// own exits. The launcher keeps nRays below 2^32, so the queue entry (ray index - first) fits 32 bits.
+// own exits. A launch has at most kMaxRaysPerLaunch rays (fast_params.h), so the queue entry (ray index - first) fits 32 bits.
 // kSpectra: the generic variant that also fills the spectra (sart_enable_spectra; fast_common.cuh: ImageSinkT).
 template <bool kWolter, bool kPlain, bool kAlias, bool kMargins, bool kSpectra = false>
 __global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
@@ -47,8 +43,8 @@ k_trace_mc_f32(const __grid_constant__ FastParams P, const __grid_constant__ Geo
   const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
   ImageSinkT<!kPlain, kSpectra> sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
   const uint64_t stride = uint64_t(gridDim.x) * kBlock32;
-  // 32-bit trip count + running 64-bit ray index: 5 loop instructions per ray instead of 12 (the launcher keeps
-  // nRays <= kMaxRaysPerLaunch, so the count fits)
+  // 32-bit trip count + running 64-bit ray index: 5 loop instructions per ray instead of 12 (nRays <= kMaxRaysPerLaunch,
+  // so the count fits)
   const uint64_t i0 = uint64_t(blockIdx.x) * kBlock32 + threadIdx.x;
   nIter = i0 < nRays ? unsigned((nRays - 1 - i0) / stride) + 1u : 0u;
   uint64_t ray = first + i0;
@@ -199,26 +195,15 @@ k_trace_mc_f32_masses(const __grid_constant__ FastParams P, const __grid_constan
 }  // namespace fast
 
 #ifndef SART_NO_LAUNCHERS   // tools/micro/one_kernel.cu instantiates single kernels of this file for SASS inspection
-cudaError_t launch_mc_image_f32x2(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T, double mAxion2,
-                                  uint64_t first, uint64_t n, const PhiloxKeys& keys, double* image, double* imageW2,
-                                  sart_counters_t* counters, int smCount, bool margins, cudaStream_t s);   // kernels_f32x2.cu
-
-// Two rays per thread (kernels_f32x2.cu) for the plain run of a cone telescope without compaction. SART_F32_PAIR=0 / 1 in the
-// environment overrides the default for A/B measurements and for the test that compares the two kernels ray set by ray set.
-static bool pair_kernel_wanted() {
-  const char* e = getenv("SART_F32_PAIR");
-  return e ? (e[0] != '0') : (SART_F32_PAIR_DEFAULT != 0);
-}
-
+// One launch of at most fast::kMaxRaysPerLaunch rays (api.cu cuts longer runs).
 cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T, double mAxion,
                                 uint64_t first, uint64_t nRays, uint64_t seed, double* image, double* imageW2,
                                 sart_counters_t* counters, int smCount, bool compact, cudaStream_t s) {
   if (nRays == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
-  // alias sampler: solar source only (the X-ray test source draws no table values)
-  const bool alias = T.sampler == SART_SAMPLER_ALIAS && !P.testXray && T.radiusAlias && T.energyAlias;
-  const size_t smem = fast::smem_bytes32(P, fast::kWarps32, alias) + (compact ? fast::kWarps32 * sizeof(fast::WarpQueue32) : 0);
-  const bool plain = !P.testXray && P.stage == SART_SK_VACUUM && !P.rotated && P.flags == 0 && P.reflKind != SART_RK_EFFECTIVE_AREA && !T.rad.w && !T.spec.eW;
+  const LaunchVariant v = launch_variant(P, T);
+  // the plain-run kernels compile the radial histogram and the spectra out
+  const bool plain = v.plain && !T.rad.w && !T.spec.eW;
+  const size_t smem = fast::smem_bytes32(P, fast::kWarps32, v.alias) + (compact ? fast::kWarps32 * sizeof(fast::WarpQueue32) : 0);
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, uint64_t, uint64_t, PhiloxKeys, double*, double*,
                         sart_counters_t*);
   // [compact][wolter][kind][variant]; kind 0: generic, 1: plain, 2: generic with the spectra; variant 0: inverse-CDF sampler,
@@ -230,60 +215,36 @@ cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G,
                                          {SART_KINDS(k_trace_mc_f32_compact, false), SART_KINDS(k_trace_mc_f32_compact, true)}};
 #undef SART_KINDS
 #undef SART_ROW
-  const bool margins = !alias && T.rq.cap != 0u;
   const int kind = plain ? 1 : (T.spec.eW ? 2 : 0);
-  const Kern kern = table[compact ? 1 : 0][wolter ? 1 : 0][kind][alias ? 2 : (margins ? 1 : 0)];
+  const Kern kern = table[compact ? 1 : 0][v.wolter ? 1 : 0][kind][v.alias ? 2 : (v.margins ? 1 : 0)];
   if (getenv("SART_DEBUG"))
     fprintf(stderr, "[sart] k_trace_mc_f32 compact=%d wolter=%d plain=%d alias=%d (sampler=%d ra=%p ea=%p) smem=%zu\n", int(compact),
-            int(wolter), int(plain), int(alias), T.sampler, (const void*)T.radiusAlias, (const void*)T.energyAlias, smem);
+            int(v.wolter), int(plain), int(v.alias), T.sampler, (const void*)T.radiusAlias, (const void*)T.energyAlias, smem);
   cudaError_t e = fast::set_smem(kern, smem);
   if (e != cudaSuccess) return e;
-  int perSM = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kern, fast::kBlock32, smem);
-  if (e != cudaSuccess) return e;
-  if (perSM < 1) perSM = 1;
-  const uint64_t cap = uint64_t(smCount) * perSM;
-  const PhiloxKeys keys = philox_round_keys(seed);
-  const bool pairs = plain && !wolter && !compact && !alias && pair_kernel_wanted();
-  for (uint64_t done = 0; done < nRays; done += fast::kMaxRaysPerLaunch) {   // one launch for anything below 6.9e10 rays
-    const uint64_t n = nRays - done < fast::kMaxRaysPerLaunch ? nRays - done : fast::kMaxRaysPerLaunch;
-    if (pairs) {
-      e = launch_mc_image_f32x2(P, G, T, mAxion * mAxion, first + done, n, keys, image, imageW2, counters, smCount, margins, s);
-      if (e != cudaSuccess) return e;
-      continue;
-    }
-    const uint64_t want = (n + fast::kBlock32 - 1) / fast::kBlock32;
-    const unsigned grid = unsigned(want < cap ? want : cap);
-    kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, first + done, n, keys, image, imageW2, counters);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-  }
-  return cudaSuccess;
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlock32, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
+  kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, first, nRays, philox_round_keys(seed), image, imageW2, counters);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_mc_image_f32_masses(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T,
                                        int nMasses, const double* dMasses, uint64_t first, uint64_t nRays, uint64_t seed,
                                        double* acc, double* accW2, sart_counters_t* counters, int smCount, cudaStream_t s) {
   if (nRays == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
+  const LaunchVariant v = launch_variant(P, T);
   const size_t smem = fast::smem_bytes32(P, fast::kWarpsM);
-  const bool margins = T.rq.cap != 0u;
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, const double*, int, uint64_t, uint64_t, PhiloxKeys, double*,
                         double*, sart_counters_t*);
   constexpr int kAll = SART_MAX_MASSES / 32;
 #define SART_ROW(W, M) {fast::k_trace_mc_f32_masses<W, M, 1>, fast::k_trace_mc_f32_masses<W, M, 2>, fast::k_trace_mc_f32_masses<W, M, kAll>}
   static const Kern table[2][2][3] = {{SART_ROW(false, false), SART_ROW(false, true)}, {SART_ROW(true, false), SART_ROW(true, true)}};
 #undef SART_ROW
-  const Kern kern = table[wolter ? 1 : 0][margins ? 1 : 0][nMasses <= 32 ? 0 : (nMasses <= 64 ? 1 : 2)];   // masses per lane
+  const Kern kern = table[v.wolter ? 1 : 0][v.margins ? 1 : 0][nMasses <= 32 ? 0 : (nMasses <= 64 ? 1 : 2)];   // masses per lane
   cudaError_t e = fast::set_smem(kern, smem);
   if (e != cudaSuccess) return e;
-  int perSM = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kern, fast::kBlockM, smem);
-  if (e != cudaSuccess) return e;
-  if (perSM < 1) perSM = 1;
-  const uint64_t want = (nRays + fast::kBlockM - 1) / fast::kBlockM;
-  const uint64_t cap = uint64_t(smCount) * perSM;
-  const unsigned grid = unsigned(want < cap ? want : cap);
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlockM, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
   kern<<<grid, fast::kBlockM, smem, s>>>(P, G, T, dMasses, nMasses, first, nRays, philox_round_keys(seed), acc, accW2, counters);
   return cudaGetLastError();
 }

@@ -221,10 +221,8 @@ cudaError_t launch_presampled_f32(const fast::FastParams& P, const fast::Geo32& 
                                   size_t n, const double* origin, const double* exitxy, const double* energy,
                                   const sart_ray_out_t& o, int smCount, cudaStream_t s) {
   if (n == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
+  const LaunchVariant v = launch_variant(P, T);   // pre-sampled rays have no source: the sampler plays no part
   const size_t smem = fast::smem_bytes32(P);
-  // the plain-run variant (run-wide switches as compile-time constants, see k_trace_mc_f32); pre-sampled rays have no source
-  const bool plain = !P.testXray && P.stage == SART_SK_VACUUM && !P.rotated && P.flags == 0 && P.reflKind != SART_RK_EFFECTIVE_AREA;
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, size_t, const double*, const double*, const double*,
                         sart_ray_out_t);
 #define SART_ROW(W, PL) {{fast::k_trace_presampled_f32<W, PL, false, false>, fast::k_trace_presampled_f32<W, PL, false, true>}, \
@@ -234,16 +232,11 @@ cudaError_t launch_presampled_f32(const fast::FastParams& P, const fast::Geo32& 
 #undef SART_ROW
   const bool optional = o.energy || o.reflect || o.transMagnet || o.yaw || o.alpha1 || o.alpha2 || o.pathCB || o.r ||
                         o.deviationDet || o.transProbArgon;
-  const Kern kern = table[wolter ? 1 : 0][plain ? 1 : 0][T.rq.cap != 0u ? 1 : 0][optional ? 1 : 0];
+  const Kern kern = table[v.wolter ? 1 : 0][v.plain ? 1 : 0][v.margins ? 1 : 0][optional ? 1 : 0];
   cudaError_t e = fast::set_smem(kern, smem);
   if (e != cudaSuccess) return e;
-  int perSM = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kern, fast::kBlock32, smem);
-  if (e != cudaSuccess) return e;
-  if (perSM < 1) perSM = 1;
-  const uint64_t want = (n + fast::kBlock32 - 1) / fast::kBlock32;
-  const uint64_t cap = uint64_t(smCount) * perSM;
-  const unsigned grid = unsigned(want < cap ? want : cap);
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlock32, smem, n, smCount, 0, &grid)) != cudaSuccess) return e;
   kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, n, origin, exitxy, energy, o);
   return cudaGetLastError();
 }
@@ -252,15 +245,14 @@ cudaError_t launch_mc_passed_f32(const fast::FastParams& P, const fast::Geo32& G
                                  uint64_t first, uint64_t nRays, uint64_t seed, const sart_passed_out_t& o, unsigned int* count,
                                  unsigned int cap, uint32_t idBase, sart_counters_t* counters, int smCount, cudaStream_t s) {
   if (nRays == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
+  const LaunchVariant v = launch_variant(P, T);
   const size_t smem = fast::smem_bytes32(P);
-  const bool plain = !P.testXray && P.stage == SART_SK_VACUUM && !P.rotated && P.flags == 0 && P.reflKind != SART_RK_EFFECTIVE_AREA;
-  auto kern = wolter ? (plain ? fast::k_trace_mc_passed_f32<true, true> : fast::k_trace_mc_passed_f32<true, false>)
-                     : (plain ? fast::k_trace_mc_passed_f32<false, true> : fast::k_trace_mc_passed_f32<false, false>);
+  auto kern = v.wolter ? (v.plain ? fast::k_trace_mc_passed_f32<true, true> : fast::k_trace_mc_passed_f32<true, false>)
+                       : (v.plain ? fast::k_trace_mc_passed_f32<false, true> : fast::k_trace_mc_passed_f32<false, false>);
   cudaError_t e = fast::set_smem(kern, smem);
   if (e != cudaSuccess) return e;
-  const uint64_t want = (nRays + fast::kBlock32 - 1) / fast::kBlock32;
-  const unsigned grid = unsigned(want < uint64_t(smCount) ? want : uint64_t(smCount));
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlock32, smem, nRays, smCount, 1, &grid)) != cudaSuccess) return e;
   kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, first, nRays, philox_round_keys(seed), o, count, cap, idBase, counters);
   return cudaGetLastError();
 }
@@ -269,10 +261,8 @@ cudaError_t launch_mc_rays_f32(const fast::FastParams& P, const fast::Geo32& G, 
                                uint64_t first, uint64_t nRays, uint64_t seed, const sart_ray_out_t& o, int smCount,
                                cudaStream_t s, const uint32_t* words, bool lateEnergy, int32_t* emit) {
   if (nRays == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
-  const bool alias = T.sampler == SART_SAMPLER_ALIAS && !P.testXray && T.radiusAlias && T.energyAlias;
-  const size_t smem = fast::smem_bytes32(P, fast::kWarps32, alias);
-  const bool plain = !P.testXray && P.stage == SART_SK_VACUUM && !P.rotated && P.flags == 0 && P.reflKind != SART_RK_EFFECTIVE_AREA;
+  const LaunchVariant v = launch_variant(P, T);
+  const size_t smem = fast::smem_bytes32(P, fast::kWarps32, v.alias);
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, uint64_t, uint64_t, PhiloxKeys, const uint32_t*,
                         int32_t*, sart_ray_out_t);
   static const Kern table[2][2][2] = {   // [wolter][plain][alias]
@@ -283,12 +273,11 @@ cudaError_t launch_mc_rays_f32(const fast::FastParams& P, const fast::Geo32& G, 
   static const Kern late[2][2] = {   // [wolter][alias], generic (non-plain) variant: the hook of sart_trace_words
       {fast::k_trace_mc_rays_f32<false, false, false, true>, fast::k_trace_mc_rays_f32<false, false, true, true>},
       {fast::k_trace_mc_rays_f32<true, false, false, true>, fast::k_trace_mc_rays_f32<true, false, true, true>}};
-  const Kern kern = lateEnergy ? late[wolter ? 1 : 0][alias ? 1 : 0] : table[wolter ? 1 : 0][plain ? 1 : 0][alias ? 1 : 0];
+  const Kern kern = lateEnergy ? late[v.wolter ? 1 : 0][v.alias ? 1 : 0] : table[v.wolter ? 1 : 0][v.plain ? 1 : 0][v.alias ? 1 : 0];
   cudaError_t e = fast::set_smem(kern, smem);
   if (e != cudaSuccess) return e;
-  const uint64_t want = (nRays + fast::kBlock32 - 1) / fast::kBlock32;
-  const uint64_t cap = uint64_t(smCount) * 2;
-  const unsigned grid = unsigned(want < cap ? want : cap);
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlock32, smem, nRays, smCount, 2, &grid)) != cudaSuccess) return e;
   kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, first, nRays, philox_round_keys(seed), words, emit, o);
   return cudaGetLastError();
 }

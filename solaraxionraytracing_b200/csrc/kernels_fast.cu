@@ -217,10 +217,6 @@ __device__ __forceinline__ int stage_a(const FastParams& P, const FastTables& T,
   if (!(fma(x0, x0, y0 * y0) < P.rPipe12)) return SART_EXIT_CLIP_PIPE_XRT;  // quirk Q2
   // energy thresholds: 8 entries from the 16-byte aligned entry at or below the guide's start (windows are 1-2 wide)
   uint4 etA = make_uint4(0, 0, 0, 0);
-#if !SART_LAZY_THR
-  uint4 etB = etA;
-  if (eRow) etB = __ldg(reinterpret_cast<const uint4*>(eRow + e0 + 4));
-#endif
   if (eRow) etA = __ldg(reinterpret_cast<const uint4*>(eRow + e0));
 
   // ================= telescope frame rt:1888-1905 (rotation about (0, 0, halfLenTel); identity when not turned)
@@ -298,12 +294,9 @@ __device__ __forceinline__ int stage_a(const FastParams& P, const FastTables& T,
   if (eRow) {
     const uint32_t we = w[5];
     eIdx = e0 + count_le(etA, we);
-    if (eIdx == e0 + 4) {   // ~1 ray in 8: the next four thresholds (loaded only by the lanes that need them)
-#if SART_LAZY_THR
+    if (eIdx == e0 + 4) {   // ~1 ray in 8: the next four thresholds, loaded only by the lanes that need them (one divergent
+                            // gather less per ray than loading them with etA: CAST+LLNL 35.2 -> 32.8 ms)
       eIdx += count_le(__ldg(reinterpret_cast<const uint4*>(eRow + e0 + 4)), we);
-#else
-      eIdx += count_le(etB, we);
-#endif
       if (eIdx == e0 + 8) eIdx = thr_search_tail(eRow, e0 + 8, P.nEnergies, we);
     }
     if (we == 0xffffffffu)   // saturated thresholds: the f64 row decides
@@ -746,19 +739,14 @@ cudaError_t launch_mc_image_fast(const fast::FastParams& P, const fast::FastTabl
                                  uint64_t nRays, uint64_t seed, double* image, double* imageW2,
                                  sart_counters_t* counters, int smCount, bool compact, cudaStream_t s) {
   if (nRays == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
+  const bool wolter = launch_variant(P, T).wolter;
   const size_t smem = fast::smem_bytes(P, fast::kWarpsF) + (compact ? fast::kWarpsF * sizeof(fast::WarpQueue) : 0);
   auto kern = compact ? (wolter ? fast::k_trace_mc_fast_compact<true> : fast::k_trace_mc_fast_compact<false>)
                       : (wolter ? fast::k_trace_mc_fast<true> : fast::k_trace_mc_fast<false>);
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
   if (e != cudaSuccess) return e;
-  int perSM = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kern, fast::kBlockF, smem);
-  if (e != cudaSuccess) return e;
-  if (perSM < 1) perSM = 1;
-  const uint64_t want = (nRays + fast::kBlockF - 1) / fast::kBlockF;
-  const uint64_t cap = uint64_t(smCount) * perSM;
-  const unsigned grid = unsigned(want < cap ? want : cap);
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlockF, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
   kern<<<grid, fast::kBlockF, smem, s>>>(P, T, mAxion * mAxion, first, nRays, seed, image, imageW2, counters);
   return cudaGetLastError();
 }
@@ -768,18 +756,12 @@ cudaError_t launch_mc_image_fast_masses(const fast::FastParams& P, const fast::F
                                         double* image, double* imageW2, sart_counters_t* counters, int smCount,
                                         cudaStream_t s) {
   if (nRays == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
   const size_t smem = fast::smem_bytes(P);
-  auto kern = wolter ? fast::k_trace_mc_fast_masses<true> : fast::k_trace_mc_fast_masses<false>;
+  auto kern = launch_variant(P, T).wolter ? fast::k_trace_mc_fast_masses<true> : fast::k_trace_mc_fast_masses<false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
   if (e != cudaSuccess) return e;
-  int perSM = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kern, fast::kBlock, smem);
-  if (e != cudaSuccess) return e;
-  if (perSM < 1) perSM = 1;
-  const uint64_t want = (nRays + fast::kBlock - 1) / fast::kBlock;
-  const uint64_t cap = uint64_t(smCount) * perSM;
-  const unsigned grid = unsigned(want < cap ? want : cap);
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlock, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
   kern<<<grid, fast::kBlock, smem, s>>>(P, T, dMasses, nMasses, first, nRays, seed, image, imageW2, counters);
   return cudaGetLastError();
 }
@@ -787,14 +769,12 @@ cudaError_t launch_mc_image_fast_masses(const fast::FastParams& P, const fast::F
 cudaError_t launch_mc_rays_fast(const fast::FastParams& P, const fast::FastTables& T, double mAxion, uint64_t first,
                                 uint64_t nRays, uint64_t seed, const sart_ray_out_t& o, int smCount, cudaStream_t s) {
   if (nRays == 0) return cudaSuccess;
-  const bool wolter = P.telKind == SART_TK_XMM || P.telKind == SART_TK_ABRIXAS;
   const size_t smem = fast::smem_bytes(P);
-  auto kern = wolter ? fast::k_trace_mc_rays_fast<true> : fast::k_trace_mc_rays_fast<false>;
+  auto kern = launch_variant(P, T).wolter ? fast::k_trace_mc_rays_fast<true> : fast::k_trace_mc_rays_fast<false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
   if (e != cudaSuccess) return e;
-  const uint64_t want = (nRays + fast::kBlock - 1) / fast::kBlock;
-  const uint64_t cap = uint64_t(smCount) * 2;
-  const unsigned grid = unsigned(want < cap ? want : cap);
+  unsigned grid = 0;
+  if ((e = grid_size(kern, fast::kBlock, smem, nRays, smCount, 2, &grid)) != cudaSuccess) return e;
   kern<<<grid, fast::kBlock, smem, s>>>(P, T, mAxion * mAxion, first, nRays, seed, o);
   return cudaGetLastError();
 }

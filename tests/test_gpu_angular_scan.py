@@ -35,8 +35,15 @@ def _turned(setup, angle):
     return s
 
 
-@pytest.mark.parametrize("mode", [0, 1])
+@pytest.mark.parametrize("mode", [0, 1, 2])
 def test_scan_equals_loop_of_runs(rt, mode):
+    """Mode 2: a scan point keeps the handle's error budgets (latA / detA doubled for a turned frame), sart_update_setup
+    derives them for the turned setup, so a few rays are re-traced in FP64 in one run and kept in FP32 in the other. Their
+    classification is the same either way (DESIGN.md section 3b), so the integer counters are identical. What such a ray
+    adds differs by the FP32 / FP64 agreement of section 3b: weights 99 % within 2e-4 relative, positions ~1e-4 mm, which
+    can move a ray into the neighbouring image bin. At most the 2.4e-3 of the rays that are re-traced on BabyIAXO+XMM
+    differ: 2.4e-3 x 2e-4 ~ 5e-7 of the flux, checked at 1e-5; a ray in another bin counts twice its weight in the L1
+    distance of the images, at most 2 x 2.4e-3 of the image's sum, checked at 5e-3."""
     setup, tb = make_config("babyiaxo_xmm")
     angles = np.array([0.0, 0.02, 0.05, -0.03])
     n = 400_000
@@ -51,8 +58,13 @@ def test_scan_equals_loop_of_runs(rt, mode):
             res = tr.read_image()
             c = res.counters[0]
             assert c["n_exit"] == cnt[i]["n_exit"] and c["n_passed"] == cnt[i]["n_passed"]
-            assert c["sum_w"] == pytest.approx(fl[i], rel=1e-12)
-            assert np.allclose(res.image[0], img[i], rtol=1e-10, atol=0)
+            if mode == 2:
+                assert c["n_passed_till_window"] == cnt[i]["n_passed_till_window"]
+                assert c["sum_w"] == pytest.approx(fl[i], rel=1e-5)
+                assert np.abs(res.image[0] - img[i]).sum() <= 5e-3 * img[i].sum()
+            else:
+                assert c["sum_w"] == pytest.approx(fl[i], rel=1e-12)
+                assert np.allclose(res.image[0], img[i], rtol=1e-10, atol=0)
     assert fl[0] > fl[2] > 0
 
 

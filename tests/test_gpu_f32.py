@@ -362,26 +362,3 @@ def test_alias_sampler_draws_the_same_distributions(rt, cfg):
     assert abs(ca["sum_w"] - cb["sum_w"]) < 5.0 * np.sqrt(ca["sum_w2"] + cb["sum_w2"])
     assert ca["n_rays"] == cb["n_rays"] == m and sum(cb["n_exit"].values()) == m
 
-
-def test_pair_kernel_equals_one_ray_kernel(rt, monkeypatch):
-    """k_trace_mc_f32x2 (two rays per thread, packed FP32 instructions; kernels_f32x2.cu) performs the same IEEE operations
-    per ray as k_trace_mc_f32: every integer counter identical, sums equal up to the order of the f64 additions. Ray counts
-    that are odd and not a multiple of the block size exercise the passenger lane of the last pair. (The pair kernel is
-    opt-in: SART_F32_PAIR=1; DESIGN.md section 5, step 20 has the measurement that keeps it off by default.)"""
-    setup, tb = make_config("cast_llnl")
-    out = {}
-    with rt.RayTracer(rt.FullRaytraceSetup(setup, tb)) as tr:
-        tr.set_precision(2)
-        tr.set_compaction(0)
-        for n in (1, 1_000_001, 6_000_000):
-            for pair in ("0", "1"):
-                monkeypatch.setenv("SART_F32_PAIR", pair)
-                tr.reset_image()
-                tr.trace_mc(n, SEED, first_ray=3)
-                out[pair] = tr.read_image()
-            a, b = out["0"].counters[0], out["1"].counters[0]
-            assert a["n_rays"] == b["n_rays"] == n
-            for k in ("n_exit", "n_passed", "n_passed_till_window", "n_interp_clamped", "n_retraced", "n_unresolved"):
-                assert a[k] == b[k], (n, k, a[k], b[k])
-            assert a["sum_w"] == pytest.approx(b["sum_w"], rel=1e-12)
-            assert np.allclose(out["0"].image, out["1"].image, rtol=1e-9, atol=0)
