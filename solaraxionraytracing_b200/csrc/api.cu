@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include "kernels.h"
@@ -36,7 +37,22 @@ static int cuda_fail(cudaError_t e, const char* what) {
     if (e__ != cudaSuccess) return cuda_fail(e__, #call); \
   } while (0)
 
-static size_t align256(size_t n) { return (n + 255) & ~size_t(255); }
+// Bump allocator over one device buffer: every piece starts on a 256-byte boundary. Over a null base it only measures, so a
+// layout is written once and run twice: over nullptr to size the buffer, then over the allocation to hand out its pointers.
+struct Carve {
+  unsigned char* base;
+  size_t off = 0;
+  explicit Carve(void* b = nullptr) : base(static_cast<unsigned char*>(b)) {}
+  template <class T> void take(T*& p, size_t count) {
+    p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+    off = (off + count * sizeof(T) + 255) & ~size_t(255);
+  }
+};
+
+// Synchronous host -> device copy of n elements into a table the kernels only read.
+template <class T> static cudaError_t put(const T* dst, const T* src, size_t n) {
+  return cudaMemcpy(const_cast<T*>(dst), src, n * sizeof(T), cudaMemcpyHostToDevice);
+}
 
 struct DeviceGuard {
   int prev = -1;
@@ -102,21 +118,6 @@ static void build_thresholds(const double* cdf, int n, uint32_t* out /* [thr_pit
   for (int i = n; i < pitch; ++i) out[i] = 0xffffffffu;
 }
 
-struct Blob {  // bump allocator over one device allocation
-  unsigned char* base = nullptr;
-  size_t off = 0;
-  std::vector<std::pair<size_t, std::vector<unsigned char>>> pending;
-  template <class T> size_t add(const T* src, size_t count) {
-    const size_t bytes = count * sizeof(T);
-    const size_t at = off;
-    std::vector<unsigned char> v(bytes);
-    if (bytes) std::memcpy(v.data(), src, bytes);
-    pending.emplace_back(at, std::move(v));
-    off = align256(off + bytes);
-    return at;
-  }
-};
-
 // numericalnim newLinear1D.eval as the device evaluates it (trace_exact.cuh: eval_linear1d), operation for operation: this
 // translation unit's host code is compiled without contraction, the device code with -fmad=false, so both produce the same
 // bits.
@@ -137,26 +138,13 @@ static double eval_linear1d_host(const sart_interp1d_t& t, double x, int* clampe
 }
 
 static int upload_tables(sart_handle* h, const sart_tables_t* t) {
-  Blob b;
-  size_t oEn = 0, oRC = 0, oDC = 0, oRefl = 0;
   const bool solar = t->nRadii > 0 && t->energies;
-  if (solar) {
-    oEn = b.add(t->energies, t->nEnergies);
-    oRC = b.add(t->fluxRadiusCDF, t->nRadii);
-    oDC = b.add(t->diffFluxCDFs, size_t(t->nRadii) * t->nEnergies);
-  }
   const bool refl = t->reflectivity && t->nCoatings > 0;
-  if (refl) oRefl = b.add(t->reflectivity, size_t(t->nCoatings) * t->nAngles * t->nReflEnergies);
   const sart_interp1d_t* I[4] = {&t->strongbackTransmission, &t->windowTransmission, &t->gasAbsorption, &t->telescopeTransmission};
-  size_t oX[4] = {0, 0, 0, 0}, oY[4] = {0, 0, 0, 0};
-  for (int k = 0; k < 4; ++k)
-    if (I[k]->n > 0 && I[k]->x && I[k]->y) { oX[k] = b.add(I[k]->x, I[k]->n); oY[k] = b.add(I[k]->y, I[k]->n); }
   std::vector<sart::ShellF64> shells(SART_MAX_SHELLS);
   derive_shells(h->setup, shells.data());
-  const size_t oSh = b.add(shells.data(), shells.size());
   // window / strongback / detector-gas factors at each tabulated energy (device_params.h: EnergyFactors)
   std::vector<EnergyFactors> ef;
-  size_t oEf = 0;
   if (solar) {
     ef.resize(size_t(t->nEnergies));
     for (int i = 0; i < t->nEnergies; ++i) {
@@ -168,37 +156,38 @@ static int upload_tables(sart_handle* h, const sart_tables_t* t) {
       ef[size_t(i)].clamped = cw | (cs << 1) | (cg << 2);
       ef[size_t(i)].pad = 0;
     }
-    oEf = b.add(ef.data(), ef.size());
   }
-
-  if (h->table_blob) { cudaFree(h->table_blob); h->table_blob = nullptr; }
-  SART_CUDA(cudaMalloc(&h->table_blob, b.off ? b.off : 256));
-  h->table_bytes = b.off;
-  unsigned char* base = static_cast<unsigned char*>(h->table_blob);
-  for (auto& pr : b.pending)
-    if (!pr.second.empty()) SART_CUDA(cudaMemcpyAsync(base + pr.first, pr.second.data(), pr.second.size(), cudaMemcpyHostToDevice, h->stream));
-  SART_CUDA(cudaStreamSynchronize(h->stream));
 
   Tables& T = h->tables;
   std::memset(&T, 0, sizeof T);
-  if (solar) {
-    T.energies = reinterpret_cast<const double*>(base + oEn);
-    T.fluxRadiusCDF = reinterpret_cast<const double*>(base + oRC);
-    T.diffFluxCDFs = reinterpret_cast<const double*>(base + oDC);
-  }
-  if (refl) T.reflectivity = reinterpret_cast<const double*>(base + oRefl);
   const double** PX[4] = {&T.sbX, &T.wdX, &T.gaX, &T.ttX};
   const double** PY[4] = {&T.sbY, &T.wdY, &T.gaY, &T.ttY};
   int32_t* PN[4] = {&T.sbN, &T.wdN, &T.gaN, &T.ttN};
-  for (int k = 0; k < 4; ++k)
-    if (I[k]->n > 0 && I[k]->x && I[k]->y) {
-      *PX[k] = reinterpret_cast<const double*>(base + oX[k]);
-      *PY[k] = reinterpret_cast<const double*>(base + oY[k]);
-      *PN[k] = I[k]->n;
+  struct Copy { const void* dst; const void* src; size_t bytes; };
+  std::vector<Copy> copies;
+  auto layout = [&](Carve c) {   // every table: its place in table_blob and the host array it is filled from
+    copies.clear();
+    auto add = [&](auto*& dst, const auto* src, size_t n) { c.take(dst, n); copies.push_back({dst, src, n * sizeof *src}); };
+    if (solar) {
+      add(T.energies, t->energies, t->nEnergies);
+      add(T.fluxRadiusCDF, t->fluxRadiusCDF, t->nRadii);
+      add(T.diffFluxCDFs, t->diffFluxCDFs, size_t(t->nRadii) * t->nEnergies);
     }
-  T.shells = reinterpret_cast<const ShellF64*>(base + oSh);
-  if (solar) T.energyFactors = reinterpret_cast<const EnergyFactors*>(base + oEf);
-  h->shell_offset = oSh;
+    if (refl) add(T.reflectivity, t->reflectivity, size_t(t->nCoatings) * t->nAngles * t->nReflEnergies);
+    for (int k = 0; k < 4; ++k)
+      if (I[k]->n > 0 && I[k]->x && I[k]->y) { add(*PX[k], I[k]->x, I[k]->n); add(*PY[k], I[k]->y, I[k]->n); *PN[k] = I[k]->n; }
+    add(T.shells, shells.data(), shells.size());
+    if (solar) add(T.energyFactors, ef.data(), ef.size());
+    return c.off;
+  };
+  const size_t bytes = layout(Carve());
+  if (h->table_blob) { cudaFree(h->table_blob); h->table_blob = nullptr; }
+  SART_CUDA(cudaMalloc(&h->table_blob, bytes));
+  h->table_bytes = bytes;
+  layout(Carve(h->table_blob));
+  for (const Copy& c : copies)
+    if (c.bytes) SART_CUDA(cudaMemcpyAsync(const_cast<void*>(c.dst), c.src, c.bytes, cudaMemcpyHostToDevice, h->stream));
+  SART_CUDA(cudaStreamSynchronize(h->stream));
   h->have_solar = solar ? 1 : 0;
   h->n_refl_coatings = refl ? t->nCoatings : 0;
   h->have_tel_transmission = (I[3]->n >= 2 && I[3]->x && I[3]->y) ? 1 : 0;
@@ -295,33 +284,30 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
       size_t(std::max(P.nRadii, 1)) * kEnGuide >= (size_t(1) << 31) ||
       size_t(std::max(P.nRadii, 1)) * kEnCells >= (size_t(1) << 31))
     return fail(SART_ERR_CONFIG, "tables too large for the throughput pipelines (a table exceeds 2^31 elements)");
-  unsigned char* base = static_cast<unsigned char*>(h->fast_blob);
+  fast::FastTables& F = h->ftables;
   if (t) {
-    // layout: shells | shell guide (4 KiB) | lut | gas lut | radius guide | energy guide | reflE
-    size_t off = 0;
-    h->fast_shell_off = off; off += align256(shf.size() * sizeof(fast::ShellFast));
-    h->fast_shell32_off = off; off += align256(size_t(SART_MAX_SHELLS) * sizeof(fast::ShellF32));
-    h->fast_sguide_off = off; off += 4096;
-    h->fast_stab_off = off; off += 4096 * sizeof(fast::ShellCell);
-    h->fast_lut_off = off; off += align256(lut.size() * sizeof(fast::EnergyLUT));
-    h->fast_glut_off = off; off += align256(glut.size() * sizeof(fast::GasLUT));
-    h->fast_tt_off = off; off += align256(telTrans.size() * sizeof(float));
-    const size_t rgOff = off; off += align256(size_t(kRadGuide) * 2);
-    const size_t egOff = off; off += align256(size_t(std::max(P.nRadii, 1)) * kEnGuide * 2);
-    const size_t rtOff = off; off += align256(size_t(thr_pitch(std::max(P.nRadii, 1))) * 4);
-    const size_t etOff = off; off += align256(size_t(std::max(P.nRadii, 1)) * thr_pitch(std::max(P.nEnergies, 1)) * 4);
-    const size_t rcOff = off; off += align256(size_t(kRadCells) * sizeof(fast::SampleCell));
-    const size_t ecOff = off; off += align256(size_t(std::max(P.nRadii, 1)) * kEnCells * sizeof(fast::SampleCell));
-    h->fast_refl_off = off; off += align256(size_t(std::max(nCoat, 1)) * reflPlane * sizeof(float));
+    // the exact pipeline narrows its two CDF searches with the same guide tables (device_params.h: Tables)
+    const bool solarGuides = P.nRadii > 0 && t->fluxRadiusCDF;
     // alias tables of the same distributions (sart_set_sampler), when the packed 11-bit alias index can hold them
-    const bool aliasFits = P.nRadii > 0 && t->fluxRadiusCDF && P.nRadii <= 2048 && P.nEnergies <= 2048;
-    const size_t raOff = off; off += aliasFits ? align256(size_t(P.nRadii) * 4) : 0;
-    const size_t eaOff = off; off += aliasFits ? align256(size_t(P.nRadii) * P.nEnergies * 4) : 0;
+    const bool aliasFits = solarGuides && P.nRadii <= 2048 && P.nEnergies <= 2048;
+    const size_t nR = size_t(std::max(P.nRadii, 1));
+    auto layout = [&](Carve c) {
+      c.take(F.shells, shf.size()); c.take(F.shells32, sh32.size());
+      c.take(F.shellGuide, 4096); c.take(F.shellTab, 4096);
+      c.take(F.elut, lut.size()); c.take(F.glut, glut.size()); c.take(F.telTrans, telTrans.size());
+      c.take(F.radiusGuide, kRadGuide); c.take(F.energyGuide, nR * kEnGuide);
+      c.take(F.radiusThr, thr_pitch(int(nR))); c.take(F.energyThr, nR * thr_pitch(std::max(P.nEnergies, 1)));
+      c.take(F.radiusCells, kRadCells); c.take(F.energyCells, nR * kEnCells);
+      c.take(F.reflE, size_t(std::max(nCoat, 1)) * reflPlane);
+      c.take(F.radiusAlias, aliasFits ? nR : 0); c.take(F.energyAlias, aliasFits ? nR * P.nEnergies : 0);
+      return c.off;
+    };
+    const size_t bytes = layout(Carve());
     h->alias_ok = 0;
     if (h->fast_blob) { cudaFree(h->fast_blob); h->fast_blob = nullptr; }
-    SART_CUDA(cudaMalloc(&h->fast_blob, off + 256));
-    base = static_cast<unsigned char*>(h->fast_blob);
-    if (P.nRadii > 0 && t->fluxRadiusCDF) {
+    SART_CUDA(cudaMalloc(&h->fast_blob, bytes));
+    layout(Carve(h->fast_blob));
+    if (solarGuides) {
       const int ep = thr_pitch(P.nEnergies);
       std::vector<uint16_t> rg(kRadGuide), eg(size_t(P.nRadii) * kEnGuide);
       std::vector<uint32_t> rth(size_t(thr_pitch(P.nRadii))), eth(size_t(P.nRadii) * ep);
@@ -331,17 +317,17 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
         build_guide(t->diffFluxCDFs + size_t(r) * P.nEnergies, P.nEnergies, kEnGuide, eg.data() + size_t(r) * kEnGuide);
         build_thresholds(t->diffFluxCDFs + size_t(r) * P.nEnergies, P.nEnergies, eth.data() + size_t(r) * ep);
       }
-      SART_CUDA(cudaMemcpy(base + rgOff, rg.data(), rg.size() * 2, cudaMemcpyHostToDevice));
-      SART_CUDA(cudaMemcpy(base + egOff, eg.data(), eg.size() * 2, cudaMemcpyHostToDevice));
-      SART_CUDA(cudaMemcpy(base + rtOff, rth.data(), rth.size() * 4, cudaMemcpyHostToDevice));
-      SART_CUDA(cudaMemcpy(base + etOff, eth.data(), eth.size() * 4, cudaMemcpyHostToDevice));
+      SART_CUDA(put(F.radiusGuide, rg.data(), rg.size()));
+      SART_CUDA(put(F.energyGuide, eg.data(), eg.size()));
+      SART_CUDA(put(F.radiusThr, rth.data(), rth.size()));
+      SART_CUDA(put(F.energyThr, eth.data(), eth.size()));
       {
         std::vector<fast::SampleCell> rc(kRadCells), ec(size_t(P.nRadii) * kEnCells);
         fast::build_sample_cells(rth.data(), P.nRadii, kRadCellBits, rc.data());
         for (int r = 0; r < P.nRadii; ++r)
           fast::build_sample_cells(eth.data() + size_t(r) * ep, P.nEnergies, kEnCellBits, ec.data() + size_t(r) * kEnCells);
-        SART_CUDA(cudaMemcpy(base + rcOff, rc.data(), rc.size() * sizeof(fast::SampleCell), cudaMemcpyHostToDevice));
-        SART_CUDA(cudaMemcpy(base + ecOff, ec.data(), ec.size() * sizeof(fast::SampleCell), cudaMemcpyHostToDevice));
+        SART_CUDA(put(F.radiusCells, rc.data(), rc.size()));
+        SART_CUDA(put(F.energyCells, ec.data(), ec.size()));
       }
       if (aliasFits) {
         std::vector<uint32_t> ra(size_t(P.nRadii)), ea(size_t(P.nRadii) * P.nEnergies);
@@ -349,8 +335,8 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
         for (int r = 0; ok && r < P.nRadii; ++r)
           ok = fast::build_alias_table(eth.data() + size_t(r) * ep, P.nEnergies, ea.data() + size_t(r) * P.nEnergies);
         if (ok) {
-          SART_CUDA(cudaMemcpy(base + raOff, ra.data(), ra.size() * 4, cudaMemcpyHostToDevice));
-          SART_CUDA(cudaMemcpy(base + eaOff, ea.data(), ea.size() * 4, cudaMemcpyHostToDevice));
+          SART_CUDA(put(F.radiusAlias, ra.data(), ra.size()));
+          SART_CUDA(put(F.energyAlias, ea.data(), ea.size()));
           h->alias_ok = 1;
         }
       }
@@ -365,31 +351,13 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
           std::copy(line.begin(), line.end(), re.begin() + size_t(c) * reflPlane + size_t(i) * reflRow);
         }
       }
-      SART_CUDA(cudaMemcpy(base + h->fast_refl_off, re.data(), re.size() * sizeof(float), cudaMemcpyHostToDevice));
+      SART_CUDA(put(F.reflE, re.data(), re.size()));
     }
-    fast::FastTables& F = h->ftables;
     F.energies = h->tables.energies;
     F.radiusCDF = h->tables.fluxRadiusCDF;
     F.energyCDF = h->tables.diffFluxCDFs;
-    F.radiusGuide = reinterpret_cast<const uint16_t*>(base + rgOff);
-    F.energyGuide = reinterpret_cast<const uint16_t*>(base + egOff);
-    F.radiusThr = reinterpret_cast<const uint32_t*>(base + rtOff);
-    F.energyThr = reinterpret_cast<const uint32_t*>(base + etOff);
-    F.radiusCells = reinterpret_cast<const fast::SampleCell*>(base + rcOff);
-    F.energyCells = reinterpret_cast<const fast::SampleCell*>(base + ecOff);
-    F.elut = reinterpret_cast<const fast::EnergyLUT*>(base + h->fast_lut_off);
-    F.glut = reinterpret_cast<const fast::GasLUT*>(base + h->fast_glut_off);
-    F.reflE = reinterpret_cast<const float*>(base + h->fast_refl_off);
-    F.telTrans = reinterpret_cast<const float*>(base + h->fast_tt_off);
-    F.shells = reinterpret_cast<const fast::ShellFast*>(base + h->fast_shell_off);
-    F.shells32 = reinterpret_cast<const fast::ShellF32*>(base + h->fast_shell32_off);
-    F.shellGuide = reinterpret_cast<const uint8_t*>(base + h->fast_sguide_off);
-    F.shellTab = reinterpret_cast<const fast::ShellCell*>(base + h->fast_stab_off);
-    F.radiusAlias = h->alias_ok ? reinterpret_cast<const uint32_t*>(base + raOff) : nullptr;
-    F.energyAlias = h->alias_ok ? reinterpret_cast<const uint32_t*>(base + eaOff) : nullptr;
+    if (!h->alias_ok) { F.radiusAlias = nullptr; F.energyAlias = nullptr; }
     F.sampler = h->alias_ok ? h->sampler : SART_SAMPLER_INVERSE_CDF;
-    // the exact pipeline narrows its two CDF searches with the same guide tables (device_params.h: Tables)
-    const bool solarGuides = P.nRadii > 0 && t->fluxRadiusCDF;
     h->tables.radiusGuide = solarGuides ? F.radiusGuide : nullptr;
     h->tables.energyGuide = solarGuides ? F.energyGuide : nullptr;
   } else if (nCoat > 0) {
@@ -398,17 +366,16 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
     for (int c = 0; c < nCoat; ++c) {
       fast::refl_at_energy(P, h->h_refl32.data() + size_t(c) * P.nAngles * P.nReflEnergies, h->setup.testSource.energy, line.data());
       std::copy(line.begin(), line.end(), row.begin());
-      SART_CUDA(cudaMemcpy(base + h->fast_refl_off + (size_t(c) * reflPlane + size_t(nE) * reflRow) * sizeof(float),
-                           row.data(), reflRow * sizeof(float), cudaMemcpyHostToDevice));
+      SART_CUDA(put(F.reflE + size_t(c) * reflPlane + size_t(nE) * reflRow, row.data(), reflRow));
     }
   }
-  SART_CUDA(cudaMemcpy(base + h->fast_shell_off, shf.data(), shf.size() * sizeof(fast::ShellFast), cudaMemcpyHostToDevice));
-  SART_CUDA(cudaMemcpy(base + h->fast_shell32_off, sh32.data(), sh32.size() * sizeof(fast::ShellF32), cudaMemcpyHostToDevice));
-  SART_CUDA(cudaMemcpy(base + h->fast_lut_off, lut.data(), lut.size() * sizeof(fast::EnergyLUT), cudaMemcpyHostToDevice));
-  SART_CUDA(cudaMemcpy(base + h->fast_glut_off, glut.data(), glut.size() * sizeof(fast::GasLUT), cudaMemcpyHostToDevice));
-  SART_CUDA(cudaMemcpy(base + h->fast_tt_off, telTrans.data(), telTrans.size() * sizeof(float), cudaMemcpyHostToDevice));
-  SART_CUDA(cudaMemcpy(base + h->fast_sguide_off, sguide.data(), sguide.size(), cudaMemcpyHostToDevice));
-  SART_CUDA(cudaMemcpy(base + h->fast_stab_off, stab.data(), stab.size() * sizeof(fast::ShellCell), cudaMemcpyHostToDevice));
+  SART_CUDA(put(F.shells, shf.data(), shf.size()));
+  SART_CUDA(put(F.shells32, sh32.data(), sh32.size()));
+  SART_CUDA(put(F.elut, lut.data(), lut.size()));
+  SART_CUDA(put(F.glut, glut.data(), glut.size()));
+  SART_CUDA(put(F.telTrans, telTrans.data(), telTrans.size()));
+  SART_CUDA(put(F.shellGuide, sguide.data(), sguide.size()));
+  SART_CUDA(put(F.shellTab, stab.data(), stab.size()));
   return SART_OK;
 }
 
@@ -487,17 +454,18 @@ static int autotune(sart_handle* h) {
   h->compact = 0;
   if (!h->fast_ok || h->setup.testSource.active) return SART_OK;
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
-  const size_t bytes = 2 * plane * sizeof(double) + sizeof(sart_counters_t);
+  double *img, *img2;
+  sart_counters_t* dc;
+  auto layout = [&](Carve c) { c.take(img, plane); c.take(img2, plane); c.take(dc, 1); return c.off; };
+  const size_t bytes = layout(Carve());
   int rc = ensure_stage(h, bytes);
   if (rc) return rc;
-  unsigned char* base = static_cast<unsigned char*>(h->d_stage);
-  SART_CUDA(cudaMemsetAsync(base, 0, bytes, h->stream));
+  layout(Carve(h->d_stage));
+  SART_CUDA(cudaMemsetAsync(h->d_stage, 0, bytes, h->stream));
   const uint64_t n = 1u << 17;
-  sart_counters_t* dc = reinterpret_cast<sart_counters_t*>(base + 2 * plane * sizeof(double));
   fast::FastTables pilotTables = h->ftables;
   pilotTables.rad = RadialHist{};   // the pilot rays must not reach the user's radial histogram
-  SART_CUDA(launch_mc_image_fast(h->fparams, pilotTables, h->setup.consts.mAxion, 0, n, 0x5eedull,
-                                 reinterpret_cast<double*>(base), reinterpret_cast<double*>(base) + plane, dc,
+  SART_CUDA(launch_mc_image_fast(h->fparams, pilotTables, h->setup.consts.mAxion, 0, n, 0x5eedull, img, img2, dc,
                                  h->sm_count, false, h->stream));
   sart_counters_t c;
   SART_CUDA(cudaMemcpyAsync(&c, dc, sizeof c, cudaMemcpyDeviceToHost, h->stream));
@@ -518,22 +486,38 @@ static int ensure_stage(sart_handle* h, size_t bytes) {
   return SART_OK;
 }
 
-// One allocation of spectra (device_params.h: Spectra), 8-byte words: eW | eW2 | eN, each eRep x eStride | sW | sN, each
-// sRep x SART_MAX_SHELLS.
-static size_t spectra_bytes(int eStride, int eRep, int sRep) {
-  return 3 * align256(size_t(eRep) * eStride * 8) + 2 * align256(size_t(sRep) * SART_MAX_SHELLS * 8);
+// The copy streams and events of the two chunked host-buffer paths (sart_trace_presampled, sart_trace_mc_passed), created
+// on first use.
+static int ensure_copy_streams(sart_handle* h) {
+  if (h->stream_in) return SART_OK;
+  SART_CUDA(cudaStreamCreateWithFlags(&h->stream_in, cudaStreamNonBlocking));
+  SART_CUDA(cudaStreamCreateWithFlags(&h->stream_out, cudaStreamNonBlocking));
+  for (int i = 0; i < 6; ++i) SART_CUDA(cudaEventCreateWithFlags(reinterpret_cast<cudaEvent_t*>(&h->ev[i]), cudaEventDisableTiming));
+  return SART_OK;
 }
-static Spectra carve_spectra(void* base, int eStride, int eRep, int sRep) {
-  unsigned char* p = static_cast<unsigned char*>(base);
-  const size_t e = align256(size_t(eRep) * eStride * 8), s = align256(size_t(sRep) * SART_MAX_SHELLS * 8);
-  Spectra r{};
-  r.eW = reinterpret_cast<double*>(p);
-  r.eW2 = reinterpret_cast<double*>(p + e);
-  r.eN = reinterpret_cast<unsigned long long*>(p + 2 * e);
-  r.sW = reinterpret_cast<double*>(p + 3 * e);
-  r.sN = reinterpret_cast<unsigned long long*>(p + 3 * e + s);
-  r.eStride = uint32_t(eStride); r.eRepMask = uint32_t(eRep - 1); r.sRepMask = uint32_t(sRep - 1);
-  return r;
+
+// Copies records [0, n) of the device arrays `dev` into records [first, first + n) of the caller's arrays `host` on stream
+// s, for every array the caller asked for. Out: sart_ray_out_t or sart_passed_out_t.
+template <class Out>
+static int copy_records(const Out& host, size_t first, const Out& dev, size_t n, cudaStream_t s) {
+  cudaError_t e = cudaSuccess;
+  auto copy = [&](auto* hp, auto* dp) {
+    if (hp && e == cudaSuccess) e = cudaMemcpyAsync(hp + first, dp, n * sizeof *hp, cudaMemcpyDeviceToHost, s);
+  };
+  if constexpr (std::is_same_v<Out, sart_ray_out_t>) ray_out_fields(host, dev, copy);
+  else passed_out_fields(host, dev, copy);
+  return e == cudaSuccess ? SART_OK : cuda_fail(e, "cudaMemcpyAsync (records, device to host)");
+}
+
+// One allocation of spectra (device_params.h: Spectra): eW | eW2 | eN, each eRep x eStride | sW | sN, each
+// sRep x SART_MAX_SHELLS. Lays them over `base` (nullptr: only measures) and returns the bytes they take.
+static size_t carve_spectra(void* base, int eStride, int eRep, int sRep, Spectra* r) {
+  Carve c(base);
+  const size_t e = size_t(eRep) * eStride, s = size_t(sRep) * SART_MAX_SHELLS;
+  *r = Spectra{};
+  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
+  r->eStride = uint32_t(eStride); r->eRepMask = uint32_t(eRep - 1); r->sRepMask = uint32_t(sRep - 1);
+  return c.off;
 }
 
 // Parameter block of `s` for a live handle: setup-derived fields recomputed, table-derived fields kept.
@@ -674,6 +658,7 @@ void sart_destroy(sart_handle_t* h) {
   cudaFree(h->table_blob); cudaFree(h->fast_blob); cudaFree(h->d_masses); cudaFree(h->d_image); cudaFree(h->d_merged);
   cudaFree(h->d_counters); cudaFree(h->d_stage); cudaFree(h->d_rad_w); cudaFree(h->d_rad_n); cudaFree(h->d_rep); cudaFree(h->d_mass_acc);
   cudaFree(h->d_queue); cudaFree(h->d_spec); cudaFree(h->d_spec_rep);
+  cudaFreeHost(h->h_stage);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->stream_in) cudaStreamDestroy(h->stream_in);
   if (h->stream_out) cudaStreamDestroy(h->stream_out);
@@ -689,8 +674,8 @@ static int apply_setup(sart_handle* h, const sart_setup_t& s, bool retune) {
   std::vector<ShellF64> shells(SART_MAX_SHELLS);
   derive_shells(h->setup, shells.data());
   SART_CUDA(cudaStreamSynchronize(h->stream));
-  SART_CUDA(cudaMemcpyAsync(static_cast<unsigned char*>(h->table_blob) + h->shell_offset, shells.data(),
-                            shells.size() * sizeof(ShellF64), cudaMemcpyHostToDevice, h->stream));
+  SART_CUDA(cudaMemcpyAsync(const_cast<ShellF64*>(h->tables.shells), shells.data(), shells.size() * sizeof(ShellF64),
+                            cudaMemcpyHostToDevice, h->stream));
   SART_CUDA(cudaStreamSynchronize(h->stream));
   int rc = upload_fast(h, nullptr);
   if (rc) return rc;
@@ -904,49 +889,10 @@ int sart_trace_presampled_dev(sart_handle_t* h, size_t n, const double* d_origin
   return launch_presampled(h, n, d_origin, d_exit, d_energy, *d_out);
 }
 
-// Lays a device-side sart_ray_out_t over the staging buffer; returns bytes used.
-static size_t carve_out(unsigned char* base, size_t n, const sart_ray_out_t& host, sart_ray_out_t* dev) {
-  size_t off = 0;
-  auto takeD = [&](double* hostp) -> double* {
-    if (!hostp) return nullptr;
-    double* p = reinterpret_cast<double*>(base + off);
-    off = align256(off + n * sizeof(double));
-    return p;
-  };
-  auto takeI = [&](int32_t* hostp) -> int32_t* {
-    if (!hostp) return nullptr;
-    int32_t* p = reinterpret_cast<int32_t*>(base + off);
-    off = align256(off + n * sizeof(int32_t));
-    return p;
-  };
-  dev->x = takeD(host.x); dev->y = takeD(host.y); dev->w = takeD(host.w);
-  dev->code = takeI(host.code); dev->shell = takeI(host.shell);
-  dev->energy = takeD(host.energy); dev->reflect = takeD(host.reflect); dev->transMagnet = takeD(host.transMagnet);
-  dev->yaw = takeD(host.yaw); dev->alpha1 = takeD(host.alpha1); dev->alpha2 = takeD(host.alpha2);
-  dev->pathCB = takeD(host.pathCB); dev->r = takeD(host.r); dev->deviationDet = takeD(host.deviationDet);
-  dev->transProbArgon = takeD(host.transProbArgon);
-  return off;
+// Lays a device-side sart_ray_out_t of n rays over `c`: an array for every array the caller asked for.
+static void carve_out(Carve& c, size_t n, const sart_ray_out_t& host, sart_ray_out_t* dev) {
+  ray_out_fields(host, *dev, [&](auto* hp, auto*& dp) { if (hp) c.take(dp, n); else dp = nullptr; });
 }
-
-static int copy_out(sart_handle* h, size_t n, const sart_ray_out_t& host, const sart_ray_out_t& dev) {
-#define CPD(f) if (host.f) SART_CUDA(cudaMemcpyAsync(host.f, dev.f, n * sizeof(*host.f), cudaMemcpyDeviceToHost, h->stream))
-  CPD(x); CPD(y); CPD(w); CPD(code); CPD(shell); CPD(energy); CPD(reflect); CPD(transMagnet); CPD(yaw); CPD(alpha1);
-  CPD(alpha2); CPD(pathCB); CPD(r); CPD(deviationDet); CPD(transProbArgon);
-#undef CPD
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  return SART_OK;
-}
-
-// Offsets a host-side sart_ray_out_t by `a` rays.
-static sart_ray_out_t offset_out(const sart_ray_out_t& o, size_t a) {
-  sart_ray_out_t r = o;
-#define OFF(f) if (r.f) r.f += a
-  OFF(x); OFF(y); OFF(w); OFF(code); OFF(shell); OFF(energy); OFF(reflect); OFF(transMagnet); OFF(yaw); OFF(alpha1);
-  OFF(alpha2); OFF(pathCB); OFF(r); OFF(deviationDet); OFF(transProbArgon);
-#undef OFF
-  return r;
-}
-
 
 int sart_trace_presampled(sart_handle_t* h, size_t n, const double* origin, const double* exitxy, const double* energy,
                           const sart_ray_out_t* out) {
@@ -960,51 +906,85 @@ int sart_trace_presampled(sart_handle_t* h, size_t n, const double* origin, cons
   // chunk k and the device->host copies of chunk k-1 run on three streams at once (PCIe is full duplex; with pinned
   // host arrays the call is bound by the larger of the two directions, 48 B/ray in, instead of by their sum).
   const size_t chunk = size_t(1) << 20, m0 = n < chunk ? n : chunk;
-  const size_t inBytes = align256(3 * m0 * sizeof(double)) + align256(2 * m0 * sizeof(double)) + align256(m0 * sizeof(double));
-  sart_ray_out_t probe;
-  const size_t outBytes = carve_out(nullptr, m0, *out, &probe);
-  const size_t bufBytes = inBytes + outBytes;
   const int nbuf = n > chunk ? 2 : 1;
-  if ((rc = ensure_stage(h, nbuf * bufBytes))) return rc;
-  if (nbuf == 2 && !h->stream_in) {
-    SART_CUDA(cudaStreamCreateWithFlags(&h->stream_in, cudaStreamNonBlocking));
-    SART_CUDA(cudaStreamCreateWithFlags(&h->stream_out, cudaStreamNonBlocking));
-    for (int i = 0; i < 6; ++i) SART_CUDA(cudaEventCreateWithFlags(reinterpret_cast<cudaEvent_t*>(&h->ev[i]), cudaEventDisableTiming));
-  }
+  double *dO[2], *dX[2], *dE[2];
+  sart_ray_out_t dev[2];
+  auto layout = [&](Carve c) {   // a buffer: origin [3][m0] | exit [2][m0] | energy [m0] | records of m0 rays
+    for (int b = 0; b < nbuf; ++b) {
+      c.take(dO[b], 3 * m0); c.take(dX[b], 2 * m0); c.take(dE[b], m0);
+      carve_out(c, m0, *out, &dev[b]);
+    }
+    return c.off;
+  };
+  if ((rc = ensure_stage(h, layout(Carve())))) return rc;
+  layout(Carve(h->d_stage));
+  if (nbuf == 2 && (rc = ensure_copy_streams(h))) return rc;
   cudaStream_t sIn = nbuf == 2 ? h->stream_in : h->stream, sOut = nbuf == 2 ? h->stream_out : h->stream;
   auto ev = [&](int kind, int b) { return static_cast<cudaEvent_t>(h->ev[kind * 2 + b]); };   // 0 in, 1 kernel, 2 out
   size_t k = 0;
   for (size_t a = 0; a < n; a += chunk, ++k) {
     const size_t m = n - a < chunk ? n - a : chunk;
     const int b = int(k & 1);
-    unsigned char* base = static_cast<unsigned char*>(h->d_stage) + size_t(b) * bufBytes;
-    double* dO = reinterpret_cast<double*>(base);
-    double* dX = reinterpret_cast<double*>(base + align256(3 * m0 * sizeof(double)));
-    double* dE = reinterpret_cast<double*>(base + align256(3 * m0 * sizeof(double)) + align256(2 * m0 * sizeof(double)));
-    sart_ray_out_t dev;
-    carve_out(base + inBytes, m, *out, &dev);
     if (nbuf == 2 && k >= 2) SART_CUDA(cudaStreamWaitEvent(sIn, ev(1, b), 0));      // kernel of chunk k-2 has read this buffer
-    for (int c = 0; c < 3; ++c) SART_CUDA(cudaMemcpyAsync(dO + c * m, origin + c * n + a, m * sizeof(double), cudaMemcpyHostToDevice, sIn));
-    for (int c = 0; c < 2; ++c) SART_CUDA(cudaMemcpyAsync(dX + c * m, exitxy + c * n + a, m * sizeof(double), cudaMemcpyHostToDevice, sIn));
-    SART_CUDA(cudaMemcpyAsync(dE, energy + a, m * sizeof(double), cudaMemcpyHostToDevice, sIn));
+    for (int c = 0; c < 3; ++c) SART_CUDA(cudaMemcpyAsync(dO[b] + c * m, origin + c * n + a, m * sizeof(double), cudaMemcpyHostToDevice, sIn));
+    for (int c = 0; c < 2; ++c) SART_CUDA(cudaMemcpyAsync(dX[b] + c * m, exitxy + c * n + a, m * sizeof(double), cudaMemcpyHostToDevice, sIn));
+    SART_CUDA(cudaMemcpyAsync(dE[b], energy + a, m * sizeof(double), cudaMemcpyHostToDevice, sIn));
     if (nbuf == 2) {
       SART_CUDA(cudaEventRecord(ev(0, b), sIn));
       SART_CUDA(cudaStreamWaitEvent(h->stream, ev(0, b), 0));
       if (k >= 2) SART_CUDA(cudaStreamWaitEvent(h->stream, ev(2, b), 0));           // outputs of chunk k-2 have left this buffer
     }
-    if ((rc = launch_presampled(h, m, dO, dX, dE, dev))) return rc;
+    if ((rc = launch_presampled(h, m, dO[b], dX[b], dE[b], dev[b]))) return rc;
     if (nbuf == 2) {
       SART_CUDA(cudaEventRecord(ev(1, b), h->stream));
       SART_CUDA(cudaStreamWaitEvent(sOut, ev(1, b), 0));
     }
-    const sart_ray_out_t host = offset_out(*out, a);
-#define CPD(f) if (host.f) SART_CUDA(cudaMemcpyAsync(host.f, dev.f, m * sizeof(*host.f), cudaMemcpyDeviceToHost, sOut))
-    CPD(x); CPD(y); CPD(w); CPD(code); CPD(shell); CPD(energy); CPD(reflect); CPD(transMagnet); CPD(yaw); CPD(alpha1);
-    CPD(alpha2); CPD(pathCB); CPD(r); CPD(deviationDet); CPD(transProbArgon);
-#undef CPD
+    if ((rc = copy_records(*out, a, dev[b], m, sOut))) return rc;
     if (nbuf == 2) SART_CUDA(cudaEventRecord(ev(2, b), sOut));
   }
   if (nbuf == 2) { SART_CUDA(cudaStreamSynchronize(sIn)); SART_CUDA(cudaStreamSynchronize(sOut)); }
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  return SART_OK;
+}
+
+// Per-ray records of n Monte Carlo rays into the caller's arrays `out`: global rays first .. first + n - 1 of `seed`, or, with
+// `words`, the caller's random words (host, SoA [6][n]). `late` and `emit` (host, may be NULL) are sart_trace_words'
+// late_energy and emission shells.
+static int trace_records(sart_handle* h, uint64_t first, size_t n, uint64_t seed, const uint32_t* words, bool late,
+                         int32_t* emit, const sart_ray_out_t& out) {
+  sart_ray_out_t dev;
+  uint32_t* dW = nullptr;
+  int32_t* dEmit = nullptr;
+  auto layout = [&](Carve c) {
+    carve_out(c, n, out, &dev);
+    if (words) c.take(dW, 6 * n);
+    if (emit) c.take(dEmit, n);
+    return c.off;
+  };
+  int rc = ensure_stage(h, layout(Carve()));
+  if (rc) return rc;
+  layout(Carve(h->d_stage));
+  if (words) SART_CUDA(cudaMemcpyAsync(dW, words, 6 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+  if (h->precision == 2) {
+    fast::FastTables ft = h->ftables;
+    // the alias sampler has another ray <-> index mapping than the exact pipeline's: no re-trace
+    rc = f32_then_retrace(h, n, h->sampler != SART_SAMPLER_ALIAS,   // one launch
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          ft.rq = q;
+          return launch_mc_rays_f32(h->fparams, h->geo32, ft, h->masses[0], first, n, seed, dev, h->sm_count, h->stream, dW,
+                                    late, dEmit);
+        },
+        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
+          return launch_retrace_mc_rays(h->params, h->tables, h->masses[0], first, n, seed, dW, q, dev, h->sm_count, h->stream);
+        });
+    if (rc) return rc;
+  } else if (h->precision == 1) {
+    SART_CUDA(launch_mc_rays_fast(h->fparams, h->ftables, h->masses[0], first, n, seed, dev, h->sm_count, h->stream));
+  } else {
+    SART_CUDA(launch_mc_rays_exact(h->params, h->tables, h->masses[0], first, n, seed, dev, h->stream, dW, dEmit));
+  }
+  if (dEmit) SART_CUDA(cudaMemcpyAsync(emit, dEmit, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_records(out, 0, dev, n, h->stream))) return rc;
   SART_CUDA(cudaStreamSynchronize(h->stream));
   return SART_OK;
 }
@@ -1017,30 +997,8 @@ int sart_trace_mc_rays(sart_handle_t* h, uint64_t first_ray, size_t n, uint64_t 
   DeviceGuard dg(h->device);
   if (h->sampler == SART_SAMPLER_ALIAS && h->precision != 2)
     return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2");
-  sart_ray_out_t probe;
-  const size_t outBytes = carve_out(nullptr, n, *out, &probe);
-  if ((rc = ensure_stage(h, outBytes))) return rc;
-  sart_ray_out_t dev;
-  carve_out(static_cast<unsigned char*>(h->d_stage), n, *out, &dev);
-  if (h->precision == 2) {
-    if (n > fast::kMaxRaysPerLaunch) return fail(SART_ERR_ARG, "sart_trace_mc_rays: at most 2^31 rays per call");
-    fast::FastTables ft = h->ftables;
-    // the alias sampler has another ray <-> index mapping than the exact pipeline's: no re-trace
-    rc = f32_then_retrace(h, n, h->sampler != SART_SAMPLER_ALIAS,   // one launch
-        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
-          ft.rq = q;
-          return launch_mc_rays_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray, n, seed, dev, h->sm_count, h->stream);
-        },
-        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
-          return launch_retrace_mc_rays(h->params, h->tables, h->masses[0], first_ray, n, seed, nullptr, q, dev, h->sm_count, h->stream);
-        });
-    if (rc) return rc;
-  } else if (h->precision == 1) {
-    SART_CUDA(launch_mc_rays_fast(h->fparams, h->ftables, h->masses[0], first_ray, n, seed, dev, h->sm_count, h->stream));
-  } else {
-    SART_CUDA(launch_mc_rays_exact(h->params, h->tables, h->masses[0], first_ray, n, seed, dev, h->stream));
-  }
-  return copy_out(h, n, *out, dev);
+  if (h->precision == 2 && n > fast::kMaxRaysPerLaunch) return fail(SART_ERR_ARG, "sart_trace_mc_rays: at most 2^31 rays per call");
+  return trace_records(h, first_ray, n, seed, nullptr, false, nullptr, *out);
 }
 
 int sart_trace_mc_passed(sart_handle_t* h, uint64_t first_ray, uint64_t n, uint64_t seed, size_t capacity,
@@ -1053,39 +1011,29 @@ int sart_trace_mc_passed(sart_handle_t* h, uint64_t first_ray, uint64_t n, uint6
     return fail(SART_ERR_CONFIG, "sart_trace_mc_passed: inverse-CDF sampler and a single axion mass");
   if (n > (uint64_t(1) << 32)) return fail(SART_ERR_ARG, "sart_trace_mc_passed: at most 2^32 rays per call (32-bit ray offsets)");
   DeviceGuard dg(h->device);
-  // the fields of sart_passed_out_t in declaration order: host pointer and element size
-  void* const hostp[15] = {out->ray, out->x, out->y, out->w, out->shell, out->energy, out->r, out->reflect, out->transMagnet,
-                           out->yaw, out->alpha1, out->alpha2, out->pathCB, out->deviationDet, out->transProbArgon};
-  const size_t esize[15] = {4, 4, 4, 4, 1, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4};
   // chunks of 2^24 rays through two device buffers: the kernels of chunk k + 1 run while the records of chunk k (whose
   // number the host learns from a 4-byte read) cross PCIe on a second stream
   const uint64_t chunk = std::min<uint64_t>(std::max<uint64_t>(n, 1), uint64_t(1) << 24);
-  size_t off[15], bufBytes = 256;   // [0, 256): the record count of the chunk
-  for (int f = 0; f < 15; ++f) { off[f] = bufBytes; if (hostp[f]) bufBytes += align256(size_t(chunk) * esize[f]); }
-  const size_t cntOff = 2 * bufBytes;
-  int rc = ensure_stage(h, cntOff + align256(sizeof(sart_counters_t)));
+  unsigned int* dCount[2];
+  sart_passed_out_t dev[2];
+  sart_counters_t* dCnt;
+  auto layout = [&](Carve c) {   // two buffers (the record count of the chunk | its records), then the run's counters
+    for (int b = 0; b < 2; ++b) {
+      c.take(dCount[b], 1);
+      passed_out_fields(*out, dev[b], [&](auto* hp, auto*& dp) { if (hp) c.take(dp, chunk); else dp = nullptr; });
+    }
+    c.take(dCnt, 1);
+    return c.off;
+  };
+  int rc = ensure_stage(h, layout(Carve()));
   if (rc) return rc;
-  if (!h->stream_in) {
-    SART_CUDA(cudaStreamCreateWithFlags(&h->stream_in, cudaStreamNonBlocking));
-    SART_CUDA(cudaStreamCreateWithFlags(&h->stream_out, cudaStreamNonBlocking));
-    for (int i = 0; i < 6; ++i) SART_CUDA(cudaEventCreateWithFlags(reinterpret_cast<cudaEvent_t*>(&h->ev[i]), cudaEventDisableTiming));
-  }
-  if (!h->h_stage) { SART_CUDA(cudaHostAlloc(&h->h_stage, 256, cudaHostAllocDefault)); h->h_stage_bytes = 256; }
+  layout(Carve(h->d_stage));
+  if ((rc = ensure_copy_streams(h))) return rc;
+  if (!h->h_stage) SART_CUDA(cudaHostAlloc(&h->h_stage, 2 * sizeof(unsigned int), cudaHostAllocDefault));
   unsigned int* hcount = static_cast<unsigned int*>(h->h_stage);
-  unsigned char* base = static_cast<unsigned char*>(h->d_stage);
-  sart_counters_t* dCnt = reinterpret_cast<sart_counters_t*>(base + cntOff);
   SART_CUDA(cudaMemsetAsync(dCnt, 0, sizeof(sart_counters_t), h->stream));
   auto evDone = [&](int b) { return static_cast<cudaEvent_t>(h->ev[b]); };
   auto evCopied = [&](int b) { return static_cast<cudaEvent_t>(h->ev[2 + b]); };
-  auto devOut = [&](int b) {
-    sart_passed_out_t d;
-    unsigned char* p = base + size_t(b) * bufBytes;
-    void** dp[15] = {(void**)&d.ray, (void**)&d.x, (void**)&d.y, (void**)&d.w, (void**)&d.shell, (void**)&d.energy, (void**)&d.r,
-                     (void**)&d.reflect, (void**)&d.transMagnet, (void**)&d.yaw, (void**)&d.alpha1, (void**)&d.alpha2,
-                     (void**)&d.pathCB, (void**)&d.deviationDet, (void**)&d.transProbArgon};
-    for (int f = 0; f < 15; ++f) *dp[f] = hostp[f] ? static_cast<void*>(p + off[f]) : nullptr;
-    return d;
-  };
   uint64_t total = 0;
   bool overflow = false;
   auto finish = [&](uint64_t k) -> int {   // chunk k: wait for its kernels, learn its record count, send the records home
@@ -1095,11 +1043,10 @@ int sart_trace_mc_passed(sart_handle_t* h, uint64_t first_ray, uint64_t n, uint6
     const uint64_t room = total < capacity ? capacity - total : 0;
     const uint64_t take = std::min(c, room);
     if (take < c) overflow = true;
-    unsigned char* p = base + size_t(b) * bufBytes;
-    for (int f = 0; f < 15 && take; ++f)
-      if (hostp[f])
-        SART_CUDA(cudaMemcpyAsync(static_cast<unsigned char*>(hostp[f]) + total * esize[f], p + off[f], take * esize[f],
-                                  cudaMemcpyDeviceToHost, h->stream_out));
+    if (take) {
+      const int rc = copy_records(*out, total, dev[b], take, h->stream_out);
+      if (rc) return rc;
+    }
     SART_CUDA(cudaEventRecord(evCopied(b), h->stream_out));
     total += c;
     return SART_OK;
@@ -1108,23 +1055,21 @@ int sart_trace_mc_passed(sart_handle_t* h, uint64_t first_ray, uint64_t n, uint6
   for (uint64_t done = 0; done < n; done += chunk, ++k) {
     const uint64_t m = std::min<uint64_t>(n - done, chunk);
     const int b = int(k & 1);
-    unsigned int* dCount = reinterpret_cast<unsigned int*>(base + size_t(b) * bufBytes);
     if (k >= 2) SART_CUDA(cudaStreamWaitEvent(h->stream, evCopied(b), 0));   // the records of chunk k - 2 have left this buffer
-    SART_CUDA(cudaMemsetAsync(dCount, 0, 256, h->stream));
+    SART_CUDA(cudaMemsetAsync(dCount[b], 0, sizeof(unsigned int), h->stream));
     fast::FastTables ft = h->ftables;
-    const sart_passed_out_t d = devOut(b);
     rc = f32_then_retrace(h, m, true,   // one launch
         [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
           ft.rq = q;
-          return launch_mc_passed_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray + done, m, seed, d, dCount, unsigned(chunk),
-                                      uint32_t(done), dCnt, h->sm_count, h->stream);
+          return launch_mc_passed_f32(h->fparams, h->geo32, ft, h->masses[0], first_ray + done, m, seed, dev[b], dCount[b],
+                                      unsigned(chunk), uint32_t(done), dCnt, h->sm_count, h->stream);
         },
         [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
-          return launch_retrace_mc_passed(h->params, h->tables, h->masses[0], first_ray + done, seed, q, d, dCount, unsigned(chunk),
-                                          uint32_t(done), dCnt, h->sm_count, h->stream);
+          return launch_retrace_mc_passed(h->params, h->tables, h->masses[0], first_ray + done, seed, q, dev[b], dCount[b],
+                                          unsigned(chunk), uint32_t(done), dCnt, h->sm_count, h->stream);
         });
     if (rc) return rc;
-    SART_CUDA(cudaMemcpyAsync(hcount + b, dCount, sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
+    SART_CUDA(cudaMemcpyAsync(hcount + b, dCount[b], sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
     SART_CUDA(cudaEventRecord(evDone(b), h->stream));
     if (k >= 1 && (rc = finish(k - 1))) return rc;
   }
@@ -1147,35 +1092,9 @@ int sart_trace_words(sart_handle_t* h, size_t n, const uint32_t* words, int late
   if (h->precision == 1) return fail(SART_ERR_CONFIG, "sart_trace_words: precision mode 0 or 2 (mode 1 runs the same integer search code as mode 2)");
   if (h->setup.testSource.active) return fail(SART_ERR_CONFIG, "sart_trace_words: solar source only");
   if (late_energy && h->precision != 2) return fail(SART_ERR_CONFIG, "sart_trace_words: late_energy is a variant of precision mode 2");
+  if (h->precision == 2 && n > fast::kMaxRaysPerLaunch) return fail(SART_ERR_ARG, "sart_trace_words: at most 2^31 rays per call");
   DeviceGuard dg(h->device);
-  sart_ray_out_t probe;
-  const size_t outBytes = carve_out(nullptr, n, *out, &probe);
-  const size_t wBytes = align256(6 * n * sizeof(uint32_t)), eBytes = align256(n * sizeof(int32_t));
-  if ((rc = ensure_stage(h, outBytes + wBytes + eBytes))) return rc;
-  unsigned char* base = static_cast<unsigned char*>(h->d_stage);
-  sart_ray_out_t dev;
-  carve_out(base, n, *out, &dev);
-  uint32_t* dW = reinterpret_cast<uint32_t*>(base + outBytes);
-  int32_t* dEmit = emission_shell ? reinterpret_cast<int32_t*>(base + outBytes + wBytes) : nullptr;
-  SART_CUDA(cudaMemcpyAsync(dW, words, 6 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
-  if (h->precision == 2) {
-    if (n > fast::kMaxRaysPerLaunch) return fail(SART_ERR_ARG, "sart_trace_words: at most 2^31 rays per call");
-    fast::FastTables ft = h->ftables;
-    rc = f32_then_retrace(h, n, h->sampler != SART_SAMPLER_ALIAS,   // one launch
-        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
-          ft.rq = q;
-          return launch_mc_rays_f32(h->fparams, h->geo32, ft, h->masses[0], 0, n, 0, dev, h->sm_count, h->stream, dW,
-                                    late_energy != 0, dEmit);
-        },
-        [&](uint64_t, uint64_t, const fast::RetraceQueue& q) {
-          return launch_retrace_mc_rays(h->params, h->tables, h->masses[0], 0, n, 0, dW, q, dev, h->sm_count, h->stream);
-        });
-    if (rc) return rc;
-  } else {
-    SART_CUDA(launch_mc_rays_exact(h->params, h->tables, h->masses[0], 0, n, 0, dev, h->stream, dW, dEmit));
-  }
-  if (dEmit) SART_CUDA(cudaMemcpyAsync(emission_shell, dEmit, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-  return copy_out(h, n, *out, dev);
+  return trace_records(h, 0, n, 0, words, late_energy != 0, emission_shell, *out);
 }
 
 // A fused image run of one axion mass in the handle's precision mode, with the parameter blocks and table views the caller
@@ -1278,7 +1197,10 @@ int sart_reset_image(sart_handle_t* h) {
     SART_CUDA(cudaMemsetAsync(h->d_rad_w, 0, size_t(h->rad_bins) * sizeof(double), h->stream));
     SART_CUDA(cudaMemsetAsync(h->d_rad_n, 0, size_t(h->rad_bins) * sizeof(unsigned long long), h->stream));
   }
-  if (h->spec.eW) SART_CUDA(cudaMemsetAsync(h->d_spec, 0, spectra_bytes(h->spec_e1, 1, 1), h->stream));
+  if (h->spec.eW) {
+    Spectra s;
+    SART_CUDA(cudaMemsetAsync(h->d_spec, 0, carve_spectra(nullptr, h->spec_e1, 1, 1, &s), h->stream));
+  }
   return SART_OK;
 }
 
@@ -1302,13 +1224,15 @@ int sart_enable_spectra(sart_handle_t* h, int on) {
   };
   const int eRep = pow2("SART_SPEC_E_REPLICAS", 32), sRep = pow2("SART_SPEC_S_REPLICAS", 1024);
   const uint32_t eStride = uint32_t((nE1 + 31) & ~31);
-  SART_CUDA(cudaMalloc(&h->d_spec, spectra_bytes(nE1, 1, 1)));
-  SART_CUDA(cudaMalloc(&h->d_spec_rep, spectra_bytes(int(eStride), eRep, sRep)));
-  SART_CUDA(cudaMemsetAsync(h->d_spec, 0, spectra_bytes(nE1, 1, 1), h->stream));
-  SART_CUDA(cudaMemsetAsync(h->d_spec_rep, 0, spectra_bytes(int(eStride), eRep, sRep), h->stream));
+  Spectra spec, rep;
+  const size_t bytes = carve_spectra(nullptr, nE1, 1, 1, &spec), repBytes = carve_spectra(nullptr, int(eStride), eRep, sRep, &rep);
+  SART_CUDA(cudaMalloc(&h->d_spec, bytes));
+  SART_CUDA(cudaMalloc(&h->d_spec_rep, repBytes));
+  SART_CUDA(cudaMemsetAsync(h->d_spec, 0, bytes, h->stream));
+  SART_CUDA(cudaMemsetAsync(h->d_spec_rep, 0, repBytes, h->stream));
   SART_CUDA(cudaStreamSynchronize(h->stream));
-  h->spec = carve_spectra(h->d_spec, nE1, 1, 1);
-  h->spec_rep = carve_spectra(h->d_spec_rep, int(eStride), eRep, sRep);
+  carve_spectra(h->d_spec, nE1, 1, 1, &h->spec);
+  carve_spectra(h->d_spec_rep, int(eStride), eRep, sRep, &h->spec_rep);
   h->spec_e1 = nE1;
   return SART_OK;
 }
@@ -1382,16 +1306,14 @@ int sart_prepare_heatmap(sart_handle_t* h, int rows, int cols, double start_x, d
   if (rows < 1 || cols < 1 || !result || (n && (!X || !Y || !W))) return fail(SART_ERR_ARG, "sart_prepare_heatmap: bad argument");
   DeviceGuard dg(h->device);
   const size_t cells = size_t(rows) * cols;
-  const size_t bytes = align256(cells * sizeof(double)) + 256 + 3 * align256(n * sizeof(double));
-  int rc = ensure_stage(h, bytes);
+  double *dRes, *dX, *dY, *dW;
+  unsigned long long* dBad;
+  auto layout = [&](Carve c) { c.take(dRes, cells); c.take(dBad, 1); c.take(dX, n); c.take(dY, n); c.take(dW, n); return c.off; };
+  int rc = ensure_stage(h, layout(Carve()));
   if (rc) return rc;
-  unsigned char* base = static_cast<unsigned char*>(h->d_stage);
-  double* dRes = reinterpret_cast<double*>(base);
-  unsigned long long* dBad = reinterpret_cast<unsigned long long*>(base + align256(cells * sizeof(double)));
-  double* dX = reinterpret_cast<double*>(base + align256(cells * sizeof(double)) + 256);
-  double* dY = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(dX) + align256(n * sizeof(double)));
-  double* dW = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(dY) + align256(n * sizeof(double)));
-  SART_CUDA(cudaMemsetAsync(dRes, 0, align256(cells * sizeof(double)) + 256, h->stream));
+  layout(Carve(h->d_stage));
+  SART_CUDA(cudaMemsetAsync(dRes, 0, cells * sizeof(double), h->stream));
+  SART_CUDA(cudaMemsetAsync(dBad, 0, sizeof *dBad, h->stream));
   if (n) {
     SART_CUDA(cudaMemcpyAsync(dX, X, n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     SART_CUDA(cudaMemcpyAsync(dY, Y, n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
@@ -1417,15 +1339,17 @@ int sart_angular_scan(sart_handle_t* h, int n_angles, const double* angles_deg, 
     return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2");
   DeviceGuard dg(h->device);
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
-  const size_t imgBytes = align256(size_t(n_angles) * plane * sizeof(double));
-  const size_t bytes = 2 * imgBytes + align256(size_t(n_angles) * sizeof(sart_counters_t));
+  double *dImg, *dImg2;
+  sart_counters_t* dCnt;
+  auto layout = [&](Carve c) {
+    c.take(dImg, size_t(n_angles) * plane); c.take(dImg2, size_t(n_angles) * plane); c.take(dCnt, size_t(n_angles));
+    return c.off;
+  };
+  const size_t bytes = layout(Carve());
   int rc = ensure_stage(h, bytes);
   if (rc) return rc;
-  unsigned char* base = static_cast<unsigned char*>(h->d_stage);
-  double* dImg = reinterpret_cast<double*>(base);
-  double* dImg2 = reinterpret_cast<double*>(base + imgBytes);
-  sart_counters_t* dCnt = reinterpret_cast<sart_counters_t*>(base + 2 * imgBytes);
-  SART_CUDA(cudaMemsetAsync(base, 0, bytes, h->stream));
+  layout(Carve(h->d_stage));
+  SART_CUDA(cudaMemsetAsync(h->d_stage, 0, bytes, h->stream));
   // One launch per scan point, queued back to back on the handle's stream: only the by-value parameter block differs
   // (the rotation of the telescope frame), the tables and shell records in HBM are shared, nothing synchronises.
   fast::FastTables ft = h->ftables;

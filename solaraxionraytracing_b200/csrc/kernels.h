@@ -25,6 +25,22 @@ inline LaunchVariant launch_variant(const fast::FastParams& P, const fast::FastT
   return v;
 }
 
+// The arrays of a per-ray record struct: f(a.field, b.field) for every pointer field of a pair of sart_ray_out_t (const or
+// not) in declaration order. The only place that lists the fields; an element is sizeof(*field) bytes.
+template <class A, class B, class F>
+inline void ray_out_fields(A& a, B& b, F&& f) {
+  f(a.x, b.x); f(a.y, b.y); f(a.w, b.w); f(a.code, b.code); f(a.shell, b.shell); f(a.energy, b.energy);
+  f(a.reflect, b.reflect); f(a.transMagnet, b.transMagnet); f(a.yaw, b.yaw); f(a.alpha1, b.alpha1); f(a.alpha2, b.alpha2);
+  f(a.pathCB, b.pathCB); f(a.r, b.r); f(a.deviationDet, b.deviationDet); f(a.transProbArgon, b.transProbArgon);
+}
+// The same for a pair of sart_passed_out_t.
+template <class A, class B, class F>
+inline void passed_out_fields(A& a, B& b, F&& f) {
+  f(a.ray, b.ray); f(a.x, b.x); f(a.y, b.y); f(a.w, b.w); f(a.shell, b.shell); f(a.energy, b.energy); f(a.r, b.r);
+  f(a.reflect, b.reflect); f(a.transMagnet, b.transMagnet); f(a.yaw, b.yaw); f(a.alpha1, b.alpha1); f(a.alpha2, b.alpha2);
+  f(a.pathCB, b.pathCB); f(a.deviationDet, b.deviationDet); f(a.transProbArgon, b.transProbArgon);
+}
+
 // Grid of a grid-stride launch over n rays: one thread per ray, at most perSM blocks on each of smCount SMs. perSM = 0: one
 // resident wave, i.e. the occupancy of `kern` with `smem` bytes of dynamic shared memory (at least one block per SM).
 template <class K>

@@ -14,13 +14,7 @@
 
 namespace sart {
 
-struct RayOutDev {  // sart_ray_out_t with device pointers
-  double *x, *y, *w;
-  int32_t *code, *shell;
-  double *energy, *reflect, *transMagnet, *yaw, *alpha1, *alpha2, *pathCB, *r, *deviationDet, *transProbArgon;
-};
-
-__device__ __forceinline__ void store_ray(const RayOutDev& o, size_t i, const Geo& g, const Weights& w, const Final& f,
+__device__ __forceinline__ void store_ray(const sart_ray_out_t& o, size_t i, const Geo& g, const Weights& w, const Final& f,
                                           bool weighted) {
   o.x[i] = f.x; o.y[i] = f.y; o.w[i] = f.w;
   o.code[i] = f.code;
@@ -40,7 +34,7 @@ __device__ __forceinline__ void store_ray(const RayOutDev& o, size_t i, const Ge
 }
 
 __device__ __forceinline__ void trace_and_store(const Params& P, const Tables& T, double mAxion, V3 O, V3 E,
-                                                double energy, int preClamped, const RayOutDev& out, size_t i, int eIdx = -1) {
+                                                double energy, int preClamped, const sart_ray_out_t& out, size_t i, int eIdx = -1) {
   Geo g;
   trace_geometry<true>(P, T, O, E, energy, g);
   g.clamped |= preClamped;
@@ -60,7 +54,7 @@ __device__ __forceinline__ void trace_and_store(const Params& P, const Tables& T
 __global__ void __launch_bounds__(128)
 k_trace_presampled(const __grid_constant__ Params P, const __grid_constant__ Tables T, double mAxion, size_t n,
                    const double* __restrict__ origin, const double* __restrict__ exitxy,
-                   const double* __restrict__ energy, const __grid_constant__ RayOutDev out) {
+                   const double* __restrict__ energy, const __grid_constant__ sart_ray_out_t out) {
   const size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const V3 O = {origin[i], origin[n + i], origin[2 * n + i]};
@@ -75,7 +69,7 @@ __global__ void __launch_bounds__(128)
 k_retrace_presampled(const __grid_constant__ Params P, const __grid_constant__ Tables T, double mAxion, size_t n,
                      const double* __restrict__ origin, const double* __restrict__ exitxy,
                      const double* __restrict__ energy, const uint32_t* __restrict__ list,
-                     const uint32_t* __restrict__ count, uint32_t cap, const __grid_constant__ RayOutDev out) {
+                     const uint32_t* __restrict__ count, uint32_t cap, const __grid_constant__ sart_ray_out_t out) {
   const uint32_t m = min(*count, cap);
   for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < m; j += gridDim.x * blockDim.x) {
     const size_t i = list[j];
@@ -88,7 +82,7 @@ k_retrace_presampled(const __grid_constant__ Params P, const __grid_constant__ T
 
 __device__ __forceinline__ void mc_ray_record(const Params& P, const Tables& T, double mAxion, uint64_t first, size_t n,
                                               uint64_t seed, const uint32_t* __restrict__ words, int32_t* __restrict__ emit,
-                                              const RayOutDev& out, size_t i) {
+                                              const sart_ray_out_t& out, size_t i) {
   V3 O, E;
   double energy;
   int clamped = 0;
@@ -120,7 +114,7 @@ __device__ __forceinline__ void mc_ray_record(const Params& P, const Tables& T, 
 __global__ void __launch_bounds__(128)
 k_trace_mc_rays(const __grid_constant__ Params P, const __grid_constant__ Tables T, double mAxion, uint64_t first,
                 size_t n, uint64_t seed, const uint32_t* __restrict__ words, int32_t* __restrict__ emit,
-                const __grid_constant__ RayOutDev out) {
+                const __grid_constant__ sart_ray_out_t out) {
   const size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   mc_ray_record(P, T, mAxion, first, n, seed, words, emit, out, i);
@@ -129,7 +123,7 @@ k_trace_mc_rays(const __grid_constant__ Params P, const __grid_constant__ Tables
 __global__ void __launch_bounds__(128)
 k_retrace_mc_rays(const __grid_constant__ Params P, const __grid_constant__ Tables T, double mAxion, uint64_t first,
                   size_t n, uint64_t seed, const uint32_t* __restrict__ words, const uint32_t* __restrict__ list,
-                  const uint32_t* __restrict__ count, uint32_t cap, const __grid_constant__ RayOutDev out) {
+                  const uint32_t* __restrict__ count, uint32_t cap, const __grid_constant__ sart_ray_out_t out) {
   const uint32_t m = min(*count, cap);
   for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < m; j += gridDim.x * blockDim.x) {
     const size_t i = list[j];
@@ -410,18 +404,13 @@ cudaError_t launch_heatmap(int rows, int cols, double start_x, double step_x, do
 }
 
 // ---- launchers --------------------------------------------------------------------------------------------
-static RayOutDev to_dev(const sart_ray_out_t& o) {
-  return RayOutDev{o.x, o.y, o.w, o.code, o.shell, o.energy, o.reflect, o.transMagnet, o.yaw,
-                   o.alpha1, o.alpha2, o.pathCB, o.r, o.deviationDet, o.transProbArgon};
-}
-
 cudaError_t launch_presampled_exact(const Params& P, const Tables& T, double mAxion, size_t n, const double* origin,
                                     const double* exitxy, const double* energy, const sart_ray_out_t& out,
                                     cudaStream_t s) {
   if (n == 0) return cudaSuccess;
   const int block = 128;
   const unsigned grid = unsigned((n + block - 1) / block);
-  k_trace_presampled<<<grid, block, 0, s>>>(P, T, mAxion, n, origin, exitxy, energy, to_dev(out));
+  k_trace_presampled<<<grid, block, 0, s>>>(P, T, mAxion, n, origin, exitxy, energy, out);
   return cudaGetLastError();
 }
 
@@ -430,7 +419,7 @@ cudaError_t launch_mc_rays_exact(const Params& P, const Tables& T, double mAxion
   if (n == 0) return cudaSuccess;
   const int block = 128;
   const unsigned grid = unsigned((n + block - 1) / block);
-  k_trace_mc_rays<<<grid, block, 0, s>>>(P, T, mAxion, first, n, seed, words, emit, to_dev(out));
+  k_trace_mc_rays<<<grid, block, 0, s>>>(P, T, mAxion, first, n, seed, words, emit, out);
   return cudaGetLastError();
 }
 
@@ -466,7 +455,7 @@ cudaError_t launch_retrace_mc_image(const Params& P, const Tables& T, int nMasse
 cudaError_t launch_retrace_mc_rays(const Params& P, const Tables& T, double mAxion, uint64_t first, size_t n, uint64_t seed,
                                    const uint32_t* words, const fast::RetraceQueue& q, const sart_ray_out_t& out, int smCount,
                                    cudaStream_t s) {
-  k_retrace_mc_rays<<<unsigned(smCount) * 4u, 128, 0, s>>>(P, T, mAxion, first, n, seed, words, q.list, q.count, q.cap, to_dev(out));
+  k_retrace_mc_rays<<<unsigned(smCount) * 4u, 128, 0, s>>>(P, T, mAxion, first, n, seed, words, q.list, q.count, q.cap, out);
   return cudaGetLastError();
 }
 cudaError_t launch_retrace_mc_passed(const Params& P, const Tables& T, double mAxion, uint64_t first, uint64_t seed,
@@ -480,7 +469,7 @@ cudaError_t launch_retrace_presampled(const Params& P, const Tables& T, double m
                                       const double* exitxy, const double* energy, const fast::RetraceQueue& q,
                                       const sart_ray_out_t& out, int smCount, cudaStream_t s) {
   k_retrace_presampled<<<unsigned(smCount) * 4u, 128, 0, s>>>(P, T, mAxion, n, origin, exitxy, energy, q.list, q.count, q.cap,
-                                                            to_dev(out));
+                                                            out);
   return cudaGetLastError();
 }
 

@@ -74,11 +74,9 @@ struct sart_handle {
   sart::fast::FastTables ftables;
   sart::fast::Geo32 geo32;      // single-precision geometry block of precision mode 2
   void* fast_blob = nullptr;
-  size_t fast_shell_off = 0, fast_shell32_off = 0, fast_lut_off = 0, fast_glut_off = 0, fast_tt_off = 0, fast_sguide_off = 0, fast_stab_off = 0, fast_refl_off = 0;
   std::vector<float> h_refl32;  // host copy of the reflectivity (f32) for rebuilding the X-ray-source row
   std::vector<double> h_energies, h_tab[4][2];  // host copies (energies; strongback/window/gas/telescope transmission x,y) for LUT rebuilds
   int sm_count = 148;
-  size_t shell_offset = 0;      // byte offset of the ShellF64 array inside table_blob
   int n_masses = 1;
   int masses_default = 1;       // masses[0] still mirrors setup.consts.mAxion
   int image_masses = 0;         // mass planes the image buffers were allocated for
@@ -121,6 +119,5 @@ struct sart_handle {
   size_t stage_bytes = 0;
   cudaStream_t stream_in = nullptr, stream_out = nullptr;   // copy streams of the chunked host-buffer paths
   void* ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // cudaEvent_t: inputs landed / kernel done / outputs landed, x2 buffers
-  void* h_stage = nullptr;      // pinned
-  size_t h_stage_bytes = 0;
+  void* h_stage = nullptr;      // pinned: the record counts of the two buffers of sart_trace_mc_passed
 };
