@@ -367,12 +367,29 @@ int sart_read_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
  * alike, so precision 2 has the counts of precision 0. With spectra on, precision modes 1 and 2 run the generic kernel
  * variant (as with the radial histogram) and sart_trace_mc with more than one axion mass fails with SART_ERR_CONFIG.
  * sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev) and sart_trace_words leave
- * them untouched. on != 0 synchronises, then (re)allocates and zeroes them; on = 0 switches them off (default). */
+ * them untouched. on != 0 synchronises, then (re)allocates and zeroes them; on = 0 switches them off (default).
+ * Switching them on while the per-mass spectra (sart_enable_mass_spectra) are on fails with SART_ERR_CONFIG. */
 int sart_enable_spectra(sart_handle_t* h, int on);
 /* Synchronises and copies out; host arrays, any may be NULL: energy_* [nEnergies + 1], shell_* [SART_MAX_SHELLS].
  * SART_ERR_ARG when the spectra are off. */
 int sart_read_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                       double* shell_sum_w, uint64_t* shell_counts);
+/* Per-mass spectra of the passed rays of sart_trace_mc: for each of the M axion masses (sart_set_axion_masses) the same
+ * reductions as sart_enable_spectra — Σw, Σw², count per energy bin [nEnergies + 1] (bin nEnergies = X-ray source) and Σw,
+ * count per shell [SART_MAX_SHELLS] — from one traced ray per mass scan, as the per-mass images are. Filled in every
+ * precision mode, by the FP32 kernel and by the FP64 re-trace of its uncertain rays alike, so precision 2 has the counts
+ * of precision 0 for every mass. Accumulated (+=) like the image; cleared by sart_reset_image and by
+ * sart_set_axion_masses when it changes the number of masses. With them on, sart_trace_mc runs the mass-scan kernels for
+ * every M, M = 1 included (the image then differs from a single-mass run's only in the order of its sums), and fails with
+ * SART_ERR_CONFIG with the alias sampler. sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed,
+ * sart_trace_presampled(_dev) and sart_trace_words leave them untouched. on != 0 synchronises, then (re)allocates and
+ * zeroes them for SART_MAX_MASSES masses (about 2.4 MB at nEnergies = 1500); on = 0 switches them off (default).
+ * Switching them on while the single-mass spectra (sart_enable_spectra) are on fails with SART_ERR_CONFIG. */
+int sart_enable_mass_spectra(sart_handle_t* h, int on);
+/* Synchronises and copies out the rows of the M masses; host arrays, any may be NULL: energy_* [M][nEnergies + 1],
+ * shell_* [M][SART_MAX_SHELLS]. SART_ERR_ARG when the per-mass spectra are off. */
+int sart_read_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
+                           double* shell_sum_w, uint64_t* shell_counts);
 /* Device pointers for collectives (ncclAllReduce / torch.distributed on the caller's side). */
 double* sart_image_dev(sart_handle_t* h);       /* [M][256][256] Σw  */
 double* sart_image_w2_dev(sart_handle_t* h);    /* [M][256][256] Σw² */

@@ -36,7 +36,8 @@ def build_parser() -> argparse.ArgumentParser:
                     help="alias: emission shell / energy from alias tables of the same distributions (f32, single mass)")
     ap.add_argument("--writeSpectra", action="store_true",
                     help="also write the energy spectrum and the per-shell flux of the detected rays as CSV files next to "
-                         "the image (single-mass runs; the run then takes the generic kernel variant)")
+                         "the image (a single-mass run then takes the generic kernel variant; a mass scan writes one pair "
+                         "of files per mass, suffixed _ma{m}eV)")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--outputPath", default="", help="overrides [Resources].outputPath")
     ap.add_argument("--allowSynthetic", action="store_true",
@@ -135,12 +136,13 @@ def main(argv=None) -> int:
         if a.angularScanMin == a.angularScanMax:
             print("start")
             spectra = a.writeSpectra and len(run.mAxion) <= 1
-            if a.writeSpectra and not spectra:
-                print("--writeSpectra: spectra are written for single-mass runs only", file=sys.stderr)
+            mass_spectra = a.writeSpectra and not spectra   # a mass scan: one pair of spectra files per mass
             if len(run.mAxion) <= 1:
                 tr.enable_radial_hist()
             if spectra:
                 tr.enable_spectra()
+            if mass_spectra:
+                tr.enable_mass_spectra()
             tr.reset_image()
             tr.trace_mc(n, a.seed)
             result = tr.read_image()
@@ -157,6 +159,10 @@ def main(argv=None) -> int:
                 for m, c in zip(run.mAxion, result.counters):
                     print(f"m_a = {m:.6g} eV: passed {c['n_passed']}, total flux {c['sum_w']:.6e}")
                 np.save(Path(outpath) / "axion_images_mass_scan.npy", result.image)
+                if mass_spectra:
+                    for p in output.write_mass_spectra_csvs(tr.read_mass_spectra(), run.mAxion,
+                                                            setup.detector.windowYear, outpath):
+                        print("wrote", p)
         else:
             angles, rel, _ = rt.performAngularScan(fs, a.angularScanMin, a.angularScanMax, a.numAngularScanPoints, n,
                                                    a.seed, tracer=tr)

@@ -379,9 +379,35 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
   return SART_OK;
 }
 
+// Per-mass spectra (sart_enable_mass_spectra), each laid over `base` (nullptr: only measures); both return their bytes.
+// The handle's arrays: eW | eW2 | eN, each [SART_MAX_MASSES][nE1] | sW | sN, each [SART_MAX_MASSES][SART_MAX_SHELLS].
+static size_t carve_mass_spectra(void* base, int nE1, Spectra* r) {
+  Carve c(base);
+  const size_t e = size_t(SART_MAX_MASSES) * nE1, s = size_t(SART_MAX_MASSES) * SART_MAX_SHELLS;
+  *r = Spectra{};
+  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
+  r->eRow = uint32_t(nE1); r->sRow = uint32_t(SART_MAX_SHELLS);
+  return c.off;
+}
+// The accumulators of the throughput mass-scan kernels (fast_common.cuh: mass_spec_add): eW | eW2 | 32-bit eN, each
+// [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each [SART_MAX_SHELLS][SART_MAX_MASSES].
+static size_t carve_mass_spectra_acc(void* base, int nE1, Spectra* r) {
+  Carve c(base);
+  const size_t e = size_t(nE1) * SART_MAX_MASSES, s = size_t(SART_MAX_SHELLS) * SART_MAX_MASSES;
+  unsigned int *eN, *sN;
+  *r = Spectra{};
+  c.take(r->eW, e); c.take(r->eW2, e); c.take(eN, e); c.take(r->sW, s); c.take(sN, s);
+  r->eN = reinterpret_cast<unsigned long long*>(eN); r->sN = reinterpret_cast<unsigned long long*>(sN);
+  return c.off;
+}
+
 static int ensure_image(sart_handle* h, int nMasses) {
   const size_t len = size_t(nMasses) * SART_IMAGE_BINS * SART_IMAGE_BINS;
   if (h->d_image && h->image_masses == nMasses) return SART_OK;
+  if (h->mspec.eW) {   // a new mass list: the rows of the old one are meaningless
+    Spectra s;
+    SART_CUDA(cudaMemsetAsync(h->d_mspec, 0, carve_mass_spectra(nullptr, h->mspec_e1, &s), h->stream));
+  }
   cudaFree(h->d_image); cudaFree(h->d_counters);   // d_image_w2 points into d_image's block
   h->d_image = nullptr; h->d_image_w2 = nullptr; h->d_counters = nullptr; h->image_masses = 0; h->merged_valid = 0;
   SART_CUDA(cudaMalloc(&h->d_image, merged_words(nMasses) * sizeof(double)));
@@ -657,7 +683,7 @@ void sart_destroy(sart_handle_t* h) {
   sart_comm_destroy(h);
   cudaFree(h->table_blob); cudaFree(h->fast_blob); cudaFree(h->d_masses); cudaFree(h->d_image); cudaFree(h->d_merged);
   cudaFree(h->d_counters); cudaFree(h->d_stage); cudaFree(h->d_rad_w); cudaFree(h->d_rad_n); cudaFree(h->d_rep); cudaFree(h->d_mass_acc);
-  cudaFree(h->d_queue); cudaFree(h->d_spec); cudaFree(h->d_spec_rep);
+  cudaFree(h->d_queue); cudaFree(h->d_spec); cudaFree(h->d_spec_rep); cudaFree(h->d_mspec); cudaFree(h->d_mspec_acc);
   cudaFreeHost(h->h_stage);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->stream_in) cudaStreamDestroy(h->stream_in);
@@ -1132,11 +1158,18 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   if (h->sampler == SART_SAMPLER_ALIAS && (h->precision != 2 || h->n_masses > 1))
     return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2 and a single axion mass");
   if (h->spec.eW && h->n_masses > 1) return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass");
+  if (h->mspec.eW && h->sampler == SART_SAMPLER_ALIAS)
+    return fail(SART_ERR_CONFIG, "sart_trace_mc: the per-mass spectra run the mass-scan kernels, which need the inverse-CDF sampler");
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
   int rc = SART_OK;
-  if (h->n_masses > 1) {
+  // A mass scan, or any run with the per-mass spectra on (one contract for every mass list, M = 1 included): the exact
+  // kernels add the spectra into the handle's rows directly, the throughput kernels into mass-minor accumulators that
+  // k_fold_mass_spectra adds up after every launch.
+  if (h->n_masses > 1 || h->mspec.eW) {
+    Tables et = h->tables;
+    et.spec = h->mspec;   // or off
     if (h->precision == 0) {
-      SART_CUDA(launch_mc_image_exact(h->params, h->tables, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
+      SART_CUDA(launch_mc_image_exact(h->params, et, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
                                       h->d_image_w2, h->d_counters, h->sm_count, h->stream));
       return SART_OK;
     }
@@ -1145,22 +1178,35 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
       SART_CUDA(cudaMalloc(&h->d_mass_acc, 2 * accLen * sizeof(double)));
       SART_CUDA(cudaMemsetAsync(h->d_mass_acc, 0, 2 * accLen * sizeof(double), h->stream));
     }
+    fast::FastTables ft = h->ftables;
+    ft.spec = h->mspec_acc;   // or off
+    // the spectra's 32-bit counts are folded after every launch of at most kMaxRaysPerLaunch rays
+    auto fold_spectra = [&]() { return h->mspec.eW ? launch_fold_mass_spectra(h->mspec_acc, h->n_masses, h->mspec_e1, h->mspec, h->stream)
+                                                   : cudaSuccess; };
     if (h->precision == 2) {
-      fast::FastTables ft = h->ftables;
       rc = f32_then_retrace(h, n_rays, true,   // the alias sampler was refused above
           [&](uint64_t done, uint64_t m, const fast::RetraceQueue& q) {
             ft.rq = q;
-            return launch_mc_image_f32_masses(h->fparams, h->geo32, ft, h->n_masses, h->d_masses, first_ray + done, m, seed,
-                                              h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream);
+            const cudaError_t e = launch_mc_image_f32_masses(h->fparams, h->geo32, ft, h->n_masses, h->d_masses, first_ray + done,
+                                                             m, seed, h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters,
+                                                             h->sm_count, h->stream);
+            return e != cudaSuccess ? e : fold_spectra();
           },
           [&](uint64_t done, uint64_t, const fast::RetraceQueue& q) {
-            return launch_retrace_mc_image(h->params, h->tables, h->n_masses, h->d_masses, first_ray + done, seed, q, h->d_image,
+            return launch_retrace_mc_image(h->params, et, h->n_masses, h->d_masses, first_ray + done, seed, q, h->d_image,
                                            h->d_image_w2, h->d_counters, h->sm_count, h->stream);
           });
       if (rc) return rc;
-    } else {
-      SART_CUDA(launch_mc_image_fast_masses(h->fparams, h->ftables, h->n_masses, h->d_masses, first_ray, n_rays, seed,
+    } else if (!h->mspec.eW) {
+      SART_CUDA(launch_mc_image_fast_masses(h->fparams, ft, h->n_masses, h->d_masses, first_ray, n_rays, seed,
                                             h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream));
+    } else {
+      for (uint64_t done = 0; done < n_rays; done += fast::kMaxRaysPerLaunch) {
+        const uint64_t m = std::min<uint64_t>(n_rays - done, fast::kMaxRaysPerLaunch);
+        SART_CUDA(launch_mc_image_fast_masses(h->fparams, ft, h->n_masses, h->d_masses, first_ray + done, m, seed,
+                                              h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream));
+        SART_CUDA(fold_spectra());
+      }
     }
     SART_CUDA(launch_fold_mass_acc(h->d_mass_acc, h->d_mass_acc + accLen, h->n_masses, plane, h->d_image, h->d_image_w2,
                                    h->stream));
@@ -1201,11 +1247,55 @@ int sart_reset_image(sart_handle_t* h) {
     Spectra s;
     SART_CUDA(cudaMemsetAsync(h->d_spec, 0, carve_spectra(nullptr, h->spec_e1, 1, 1, &s), h->stream));
   }
+  if (h->mspec.eW) {
+    Spectra s;
+    SART_CUDA(cudaMemsetAsync(h->d_mspec, 0, carve_mass_spectra(nullptr, h->mspec_e1, &s), h->stream));
+  }
+  return SART_OK;
+}
+
+int sart_enable_mass_spectra(sart_handle_t* h, int on) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (on && h->spec.eW)
+    return fail(SART_ERR_CONFIG, "sart_enable_mass_spectra: the single-mass spectra are on (sart_enable_spectra); switch them off first");
+  DeviceGuard dg(h->device);
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  cudaFree(h->d_mspec); cudaFree(h->d_mspec_acc);
+  h->d_mspec = nullptr; h->d_mspec_acc = nullptr; h->mspec = Spectra{}; h->mspec_acc = Spectra{}; h->mspec_e1 = 0;
+  if (!on) return SART_OK;
+  const int nE1 = h->params.nEnergies + 1;
+  Spectra spec, acc;
+  const size_t bytes = carve_mass_spectra(nullptr, nE1, &spec), accBytes = carve_mass_spectra_acc(nullptr, nE1, &acc);
+  SART_CUDA(cudaMalloc(&h->d_mspec, bytes));
+  SART_CUDA(cudaMalloc(&h->d_mspec_acc, accBytes));
+  SART_CUDA(cudaMemsetAsync(h->d_mspec, 0, bytes, h->stream));
+  SART_CUDA(cudaMemsetAsync(h->d_mspec_acc, 0, accBytes, h->stream));
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  carve_mass_spectra(h->d_mspec, nE1, &h->mspec);
+  carve_mass_spectra_acc(h->d_mspec_acc, nE1, &h->mspec_acc);
+  h->mspec_e1 = nE1;
+  return SART_OK;
+}
+
+int sart_read_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
+                           double* shell_sum_w, uint64_t* shell_counts) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (!h->mspec.eW) return fail(SART_ERR_ARG, "sart_read_mass_spectra: no per-mass spectra enabled (sart_enable_mass_spectra)");
+  DeviceGuard dg(h->device);
+  const size_t e = size_t(h->n_masses) * h->mspec_e1 * 8, s = size_t(h->n_masses) * SART_MAX_SHELLS * 8;
+  if (energy_sum_w) SART_CUDA(cudaMemcpyAsync(energy_sum_w, h->mspec.eW, e, cudaMemcpyDeviceToHost, h->stream));
+  if (energy_sum_w2) SART_CUDA(cudaMemcpyAsync(energy_sum_w2, h->mspec.eW2, e, cudaMemcpyDeviceToHost, h->stream));
+  if (energy_counts) SART_CUDA(cudaMemcpyAsync(energy_counts, h->mspec.eN, e, cudaMemcpyDeviceToHost, h->stream));
+  if (shell_sum_w) SART_CUDA(cudaMemcpyAsync(shell_sum_w, h->mspec.sW, s, cudaMemcpyDeviceToHost, h->stream));
+  if (shell_counts) SART_CUDA(cudaMemcpyAsync(shell_counts, h->mspec.sN, s, cudaMemcpyDeviceToHost, h->stream));
+  SART_CUDA(cudaStreamSynchronize(h->stream));
   return SART_OK;
 }
 
 int sart_enable_spectra(sart_handle_t* h, int on) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (on && h->mspec.eW)
+    return fail(SART_ERR_CONFIG, "sart_enable_spectra: the per-mass spectra are on (sart_enable_mass_spectra); switch them off first");
   DeviceGuard dg(h->device);
   SART_CUDA(cudaStreamSynchronize(h->stream));
   cudaFree(h->d_spec); cudaFree(h->d_spec_rep);

@@ -78,23 +78,28 @@ struct RadialHist {
 // arrays r * SART_MAX_SHELLS; a block adds into energy replica (block & eRepMask) and a warp into shell replica
 // (global warp & sRepMask). Masks 0 = the arrays themselves (the exact kernels; the throughput kernels get replicas that a
 // fold kernel adds up after the launch). 64 bytes: the kernel parameters behind a table block keep their 16-byte alignment.
+// Per-mass spectra (sart_enable_mass_spectra) are rows of these arrays, one per axion mass: mass m's energy bins start
+// m * eRow elements in, its shell bins m * sRow. eRow = sRow = 0: the single-mass spectra, which only the first mass fills.
+// The mass-scan kernels of the throughput pipelines take another layout in the same struct (fast_common.cuh:
+// MassSpectraAcc).
 struct Spectra {
   double* eW;
   double* eW2;
   unsigned long long* eN;
   double* sW;
   unsigned long long* sN;
-  uint32_t eStride, eRepMask, sRepMask, pad[3];
+  uint32_t eStride, eRepMask, sRepMask, eRow, sRow, pad;
 };
 static_assert(sizeof(Spectra) == 64, "Spectra: 64 bytes");
 
 #if defined(__CUDACC__)
-__device__ __forceinline__ void spec_add(const Spectra& s, int eBin, int shell, double w) {
-  const uint32_t e = (blockIdx.x & s.eRepMask) * s.eStride + uint32_t(eBin);
+__device__ __forceinline__ void spec_add(const Spectra& s, int m, int eBin, int shell, double w) {
+  const uint32_t e = uint32_t(m) * s.eRow + (blockIdx.x & s.eRepMask) * s.eStride + uint32_t(eBin);
   atomicAdd(s.eW + e, w);
   atomicAdd(s.eW2 + e, w * w);
   atomicAdd(s.eN + e, 1ull);
-  const uint32_t k = ((blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) & s.sRepMask) * uint32_t(SART_MAX_SHELLS) + uint32_t(shell);
+  const uint32_t k = uint32_t(m) * s.sRow +
+                     ((blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) & s.sRepMask) * uint32_t(SART_MAX_SHELLS) + uint32_t(shell);
   atomicAdd(s.sW + k, w);
   atomicAdd(s.sN + k, 1ull);
 }

@@ -379,17 +379,32 @@ struct ImageSinkT {
 using ImageSink = ImageSinkT<true>;
 
 // ---- axion-mass scan: the part shared by the FP64-algebra and the FP32 tracing --------------------------------
+// Per-mass spectra of the mass-scan kernels (sart_enable_mass_spectra), in FastTables::spec: accumulators laid out like
+// the image's, [bin][SART_MAX_MASSES] (eW, eW2: bin = energy index, nEnergies for the X-ray source) and
+// [shell][SART_MAX_MASSES] (sW), so that the 32 mass lanes of a warp add to consecutive addresses. The counts eN / sN are
+// 32-bit arrays of the same shapes: a launch has at most kMaxRaysPerLaunch = 2^31 rays, so no bin overflows before
+// k_fold_mass_spectra widens it into the handle's 64-bit counts, and a warp's 32 lanes touch 128 bytes instead of 256.
+__device__ __forceinline__ void mass_spec_add(const Spectra& a, int m, int eBin, int shell, double w) {
+  const uint32_t e = uint32_t(eBin) * SART_MAX_MASSES + uint32_t(m), k = uint32_t(shell) * SART_MAX_MASSES + uint32_t(m);
+  atomicAdd(a.eW + e, w);
+  atomicAdd(a.eW2 + e, w * w);
+  atomicAdd(reinterpret_cast<unsigned int*>(a.eN) + e, 1u);
+  atomicAdd(a.sW + k, w);
+  atomicAdd(reinterpret_cast<unsigned int*>(a.sN) + k, 1u);
+}
+
 // Rays are traced once (lanes = rays) by `trace(global ray index, RayResult&)`; each ray that reaches the weight stage
 // is then broadcast through the warp and weighted for all M masses at once with lanes = masses (mass lane + 32 k), so
 // the per-mass sums live in registers of the lane that owns the mass and need no reduction. `image` / `imageW2` are the
 // mass-major accumulators [bin][SART_MAX_MASSES] (see k_fold_mass_acc).
 // kPer = masses per lane (1, 2 or SART_MAX_MASSES / 32): the launcher picks the smallest that holds nMasses, because the
 // per-mass sums are 15 registers per mass and lane (with 4 masses per lane the FP32 kernel spilled: 80 registers, 112 bytes).
-template <int kPer, class Trace>
-__device__ __forceinline__ void mass_scan_loop(const FastParams& P, const RadialHist& rad, const double* __restrict__ masses,
-                                               int nMasses, uint64_t first, uint64_t nRays, double* __restrict__ image,
-                                               double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
-                                               WarpCounters* wc, Trace trace) {
+// kSpectra: the passed ray-masses also go to the per-mass spectra `spec` (mass_spec_add); false compiles them out.
+template <int kPer, bool kSpectra, class Trace>
+__device__ __forceinline__ void mass_scan_loop(const FastParams& P, const RadialHist& rad, const Spectra& spec,
+                                               const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays,
+                                               double* __restrict__ image, double* __restrict__ imageW2,
+                                               sart_counters_t* __restrict__ counters, WarpCounters* wc, Trace trace) {
   static_assert(kPer >= 1 && kPer <= SART_MAX_MASSES / 32, "masses per lane");
   constexpr unsigned kFull = 0xffffffffu;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -430,6 +445,7 @@ __device__ __forceinline__ void mass_scan_loop(const FastParams& P, const Radial
       const double x = __shfl_sync(kFull, r.x, src), y = __shfl_sync(kFull, r.y, src), rr = __shfl_sync(kFull, r.r, src);
       const int bin = __shfl_sync(kFull, r.bin, src);
       const bool miss = __shfl_sync(kFull, int(r.windowMiss), src) != 0;
+      const int eBin = kSpectra ? __shfl_sync(kFull, r.eIdx, src) : 0, shell = kSpectra ? __shfl_sync(kFull, r.shell, src) : 0;
 #pragma unroll
       for (int k = 0; k < kPer; ++k) {
         const int m = lane + 32 * k;
@@ -448,6 +464,7 @@ __device__ __forceinline__ void mass_scan_loop(const FastParams& P, const Radial
             atomicAdd(imageW2 + size_t(bin) * SART_MAX_MASSES + m, w * w);
           }
           if (m == 0 && rad.w) rad_add(rad, rr, w);   // the radial histogram follows the first mass, as in the exact kernel
+          if (kSpectra) mass_spec_add(spec, m, eBin, shell, w);
         } else {
           ++nZero[k];
         }

@@ -117,6 +117,7 @@ cudaError_t launch_fold_replicas(double* rep, double* rep2, int nRep, size_t str
 cudaError_t launch_fold_spectra(const Spectra& rep, int nE1, const Spectra& dst, cudaStream_t s);
 cudaError_t launch_fold_mass_acc(double* acc, double* acc2, int nMasses, size_t plane, double* image, double* imageW2,
                                  cudaStream_t s);
+cudaError_t launch_fold_mass_spectra(const Spectra& acc, int nMasses, int nE1, const Spectra& dst, cudaStream_t s);
 cudaError_t launch_heatmap(int rows, int cols, double start_x, double step_x, double start_y, double step_y, size_t n,
                            const double* X, const double* Y, const double* W, double norm, double* result,
                            unsigned long long* nBad, cudaStream_t s);

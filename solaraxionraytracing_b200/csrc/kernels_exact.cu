@@ -269,8 +269,9 @@ __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, i
       atomicAdd(T.rad.w + b, f.w);
       atomicAdd(T.rad.n + b, 1ull);
     }
-    // spectra (sart_enable_spectra, single mass): the X-ray source's rays carry no table index and go to bin nEnergies
-    if (T.spec.eW && m == 0) spec_add(T.spec, g.eIdx >= 0 ? g.eIdx : P.nEnergies, g.shell, f.w);
+    // spectra: the first mass (sart_enable_spectra) or every mass into its own row (sart_enable_mass_spectra: eRow != 0);
+    // the X-ray source's rays carry no table index and go to bin nEnergies
+    if (T.spec.eW && (m == 0 || T.spec.eRow)) spec_add(T.spec, m, g.eIdx >= 0 ? g.eIdx : P.nEnergies, g.shell, f.w);
   }
 }
 

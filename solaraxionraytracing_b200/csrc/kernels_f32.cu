@@ -165,12 +165,11 @@ k_trace_mc_f32_compact(const __grid_constant__ FastParams P, const __grid_consta
 }
 
 // ---- axion-mass scan with FP32 tracing (the per-mass weighting is fast_common.cuh's mass_scan_loop) --------------
-template <bool kWolter, bool kMargins, int kPer>
-__global__ void __launch_bounds__(kBlockM, SART_F32_MINBLOCKS_M)
-k_trace_mc_f32_masses(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G,
-                      const __grid_constant__ FastTables T, const double* __restrict__ masses, int nMasses, uint64_t first,
-                      uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image, double* __restrict__ imageW2,
-                      sart_counters_t* __restrict__ counters) {
+template <bool kWolter, bool kMargins, int kPer, bool kSpectra>
+__device__ __forceinline__ void f32_masses(const FastParams& P, const Geo32& G, const FastTables& T,
+                                           const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays,
+                                           const PhiloxKeys& K, double* __restrict__ image, double* __restrict__ imageW2,
+                                           sart_counters_t* __restrict__ counters) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem32 S;
   unsigned char* tail;
@@ -179,7 +178,7 @@ k_trace_mc_f32_masses(const __grid_constant__ FastParams P, const __grid_constan
   smem_fill32(P, T, S);
   for (int i = threadIdx.x; i < kWarpsM * int(sizeof(WarpCounters) / 4); i += kBlockM) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
   __syncthreads();
-  mass_scan_loop<kPer>(P, T.rad, masses, nMasses, first, nRays, image, imageW2, counters, wc,
+  mass_scan_loop<kPer, kSpectra>(P, T.rad, T.spec, masses, nMasses, first, nRays, image, imageW2, counters, wc,
                  [&](uint64_t ray, uint32_t id, RayResult& r) {
     RecordSink<false> sink{r, 0.0, T.rq, true};
     Head32 hd;
@@ -190,6 +189,23 @@ k_trace_mc_f32_masses(const __grid_constant__ FastParams P, const __grid_constan
     finish32<kWolter, false, false, kMargins>(P, G, T, S, c0, rec, sink);
     return sink.unresolved;
   });
+}
+template <bool kWolter, bool kMargins, int kPer>
+__global__ void __launch_bounds__(kBlockM, SART_F32_MINBLOCKS_M)
+k_trace_mc_f32_masses(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G,
+                      const __grid_constant__ FastTables T, const double* __restrict__ masses, int nMasses, uint64_t first,
+                      uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image, double* __restrict__ imageW2,
+                      sart_counters_t* __restrict__ counters) {
+  f32_masses<kWolter, kMargins, kPer, false>(P, G, T, masses, nMasses, first, nRays, K, image, imageW2, counters);
+}
+// The same with the per-mass spectra (sart_enable_mass_spectra; T.spec holds their accumulators, see mass_spec_add).
+template <bool kWolter, bool kMargins, int kPer>
+__global__ void __launch_bounds__(kBlockM, SART_F32_MINBLOCKS_M)
+k_trace_mc_f32_masses_spectra(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G,
+                              const __grid_constant__ FastTables T, const double* __restrict__ masses, int nMasses,
+                              uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image,
+                              double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+  f32_masses<kWolter, kMargins, kPer, true>(P, G, T, masses, nMasses, first, nRays, K, image, imageW2, counters);
 }
 
 }  // namespace fast
@@ -237,10 +253,13 @@ cudaError_t launch_mc_image_f32_masses(const fast::FastParams& P, const fast::Ge
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, const double*, int, uint64_t, uint64_t, PhiloxKeys, double*,
                         double*, sart_counters_t*);
   constexpr int kAll = SART_MAX_MASSES / 32;
-#define SART_ROW(W, M) {fast::k_trace_mc_f32_masses<W, M, 1>, fast::k_trace_mc_f32_masses<W, M, 2>, fast::k_trace_mc_f32_masses<W, M, kAll>}
-  static const Kern table[2][2][3] = {{SART_ROW(false, false), SART_ROW(false, true)}, {SART_ROW(true, false), SART_ROW(true, true)}};
+  // [spectra][wolter][margins][masses per lane]; spectra: T.spec holds the per-mass spectra accumulators
+#define SART_ROW(K, W, M) {fast::K<W, M, 1>, fast::K<W, M, 2>, fast::K<W, M, kAll>}
+#define SART_KERN(K) {{SART_ROW(K, false, false), SART_ROW(K, false, true)}, {SART_ROW(K, true, false), SART_ROW(K, true, true)}}
+  static const Kern table[2][2][2][3] = {SART_KERN(k_trace_mc_f32_masses), SART_KERN(k_trace_mc_f32_masses_spectra)};
+#undef SART_KERN
 #undef SART_ROW
-  const Kern kern = table[v.wolter ? 1 : 0][v.margins ? 1 : 0][nMasses <= 32 ? 0 : (nMasses <= 64 ? 1 : 2)];   // masses per lane
+  const Kern kern = table[T.spec.eW ? 1 : 0][v.wolter ? 1 : 0][v.margins ? 1 : 0][nMasses <= 32 ? 0 : (nMasses <= 64 ? 1 : 2)];
   cudaError_t e = fast::set_smem(kern, smem);
   if (e != cudaSuccess) return e;
   unsigned grid = 0;

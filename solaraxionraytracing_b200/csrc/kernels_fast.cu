@@ -689,11 +689,10 @@ k_trace_mc_fast_compact(const __grid_constant__ FastParams P, const __grid_const
 // Rays are traced once (lanes = rays); each ray that reaches the weight stage is then broadcast through the warp and
 // weighted for all M masses at once with lanes = masses (mass lane + 32 k), so the per-mass sums live in registers of
 // the lane that owns the mass and need no reduction, and the per-mass image planes are hit by distinct lanes.
-template <bool kWolter>
-__global__ void __launch_bounds__(kBlock, 2)
-k_trace_mc_fast_masses(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T,
-                       const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays, uint64_t seed,
-                       double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+template <bool kWolter, bool kSpectra>
+__device__ __forceinline__ void fast_masses(const FastParams& P, const FastTables& T, const double* __restrict__ masses,
+                                            int nMasses, uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                                            double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem S;
   unsigned char* tail;
@@ -703,8 +702,23 @@ k_trace_mc_fast_masses(const __grid_constant__ FastParams P, const __grid_consta
   for (int i = threadIdx.x; i < kWarps * int(sizeof(WarpCounters) / 4); i += kBlock) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
   __syncthreads();
 
-  mass_scan_loop<SART_MAX_MASSES / 32>(P, T.rad, masses, nMasses, first, nRays, image, imageW2, counters, wc,
+  mass_scan_loop<SART_MAX_MASSES / 32, kSpectra>(P, T.rad, T.spec, masses, nMasses, first, nRays, image, imageW2, counters, wc,
                  [&](uint64_t ray, uint32_t, RayResult& r) { trace_one<kWolter, false>(P, T, S, seed, ray, 0.0, r); return false; });
+}
+template <bool kWolter>
+__global__ void __launch_bounds__(kBlock, 2)
+k_trace_mc_fast_masses(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T,
+                       const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays, uint64_t seed,
+                       double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+  fast_masses<kWolter, false>(P, T, masses, nMasses, first, nRays, seed, image, imageW2, counters);
+}
+// The same with the per-mass spectra (sart_enable_mass_spectra; T.spec holds their accumulators, see mass_spec_add).
+template <bool kWolter>
+__global__ void __launch_bounds__(kBlock, 2)
+k_trace_mc_fast_masses_spectra(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T,
+                               const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays, uint64_t seed,
+                               double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+  fast_masses<kWolter, true>(P, T, masses, nMasses, first, nRays, seed, image, imageW2, counters);
 }
 
 // ---- per-ray records (traceAxionWrapper in fast mode) ----------------------------------------------------------
@@ -757,7 +771,9 @@ cudaError_t launch_mc_image_fast_masses(const fast::FastParams& P, const fast::F
                                         cudaStream_t s) {
   if (nRays == 0) return cudaSuccess;
   const size_t smem = fast::smem_bytes(P);
-  auto kern = launch_variant(P, T).wolter ? fast::k_trace_mc_fast_masses<true> : fast::k_trace_mc_fast_masses<false>;
+  const bool wolter = launch_variant(P, T).wolter;
+  auto kern = T.spec.eW ? (wolter ? fast::k_trace_mc_fast_masses_spectra<true> : fast::k_trace_mc_fast_masses_spectra<false>)
+                        : (wolter ? fast::k_trace_mc_fast_masses<true> : fast::k_trace_mc_fast_masses<false>);
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
   if (e != cudaSuccess) return e;
   unsigned grid = 0;

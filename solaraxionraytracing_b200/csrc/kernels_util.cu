@@ -87,6 +87,43 @@ cudaError_t launch_fold_mass_acc(double* acc, double* acc2, int nMasses, size_t 
   return cudaGetLastError();
 }
 
+// Mass scan with per-mass spectra: adds the mass-minor accumulators of a launch (fast_common.cuh: mass_spec_add; eW, eW2,
+// 32-bit eN [nE1][SART_MAX_MASSES], sW, 32-bit sN [SART_MAX_SHELLS][SART_MAX_MASSES]) to the rows of the handle's per-mass
+// spectra (device_params.h: Spectra, row m at m * eRow / m * sRow) and clears them. One thread per accumulator element.
+__global__ void __launch_bounds__(256) k_fold_mass_spectra(const __grid_constant__ Spectra acc, int nMasses, int nE1,
+                                                           const __grid_constant__ Spectra dst) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;   // = bin * SART_MAX_MASSES + mass
+  const uint32_t nEnergy = uint32_t(nE1) * SART_MAX_MASSES;
+  if (i >= nEnergy + uint32_t(SART_MAX_SHELLS) * SART_MAX_MASSES) return;
+  const bool energy = i < nEnergy;
+  const uint32_t j = energy ? i : i - nEnergy;
+  const uint32_t m = j % SART_MAX_MASSES, bin = j / SART_MAX_MASSES;
+  unsigned int* const cnt = reinterpret_cast<unsigned int*>(energy ? acc.eN : acc.sN) + j;
+  const unsigned int n = *cnt;
+  if (n == 0u) return;   // no passed ray in this bin: its sums are zero as well
+  *cnt = 0u;
+  if (energy) {
+    const double a = acc.eW[j], b = acc.eW2[j];
+    acc.eW[j] = 0.0; acc.eW2[j] = 0.0;
+    if (int(m) < nMasses) {
+      const uint32_t o = m * dst.eRow + bin;
+      dst.eW[o] += a; dst.eW2[o] += b; dst.eN[o] += n;
+    }
+  } else {
+    const double a = acc.sW[j];
+    acc.sW[j] = 0.0;
+    if (int(m) < nMasses) {
+      const uint32_t o = m * dst.sRow + bin;
+      dst.sW[o] += a; dst.sN[o] += n;
+    }
+  }
+}
+cudaError_t launch_fold_mass_spectra(const Spectra& acc, int nMasses, int nE1, const Spectra& dst, cudaStream_t s) {
+  const unsigned n = unsigned(nE1 + SART_MAX_SHELLS) * SART_MAX_MASSES;
+  k_fold_mass_spectra<<<(n + 255) / 256, 256, 0, s>>>(acc, nMasses, nE1, dst);
+  return cudaGetLastError();
+}
+
 template <typename T, int kChains>
 __global__ void __launch_bounds__(256) k_fma_peak(T* out, T a, T b, int iters) {
   T acc[kChains];

@@ -114,6 +114,14 @@ struct sart_handle {
   void* d_spec_rep = nullptr;
   sart::Spectra spec{}, spec_rep{};   // spec.eW == nullptr: off
   int spec_e1 = 0;                    // energy bins: nEnergies + 1 (the last one is the X-ray source's)
+  // optional per-mass spectra of the passed rays (sart_enable_mass_spectra), one allocation each, sized for
+  // SART_MAX_MASSES: the handle's arrays, one row per mass (the exact kernels and the re-trace add into them directly), and
+  // the mass-minor accumulators of the throughput mass-scan kernels (fast_common.cuh: mass_spec_add), which the fold after
+  // every launch adds into those rows and clears. Only sart_trace_mc hands them to a kernel.
+  void* d_mspec = nullptr;
+  void* d_mspec_acc = nullptr;
+  sart::Spectra mspec{}, mspec_acc{};   // mspec.eW == nullptr: off
+  int mspec_e1 = 0;                     // energy bins per mass: nEnergies + 1
   // staging for the host-pointer entry points
   void* d_stage = nullptr;
   size_t stage_bytes = 0;

@@ -243,6 +243,26 @@ def write_spectra_csvs(spectra: Spectra, windowYear: int, outpath: str | Path, s
             write_shell_flux_csv(Path(outpath) / f"axion_shell_flux_{year}{suffix}.csv", spectra, precision))
 
 
+def mass_suffix(mAxion: float) -> str:
+    """File-name suffix of one axion mass of a mass scan: `_ma{m:.6g}eV`."""
+    return f"_ma{mAxion:.6g}eV"
+
+
+def write_mass_spectra_csvs(spectra: list[Spectra], masses, windowYear: int, outpath: str | Path,
+                            precision: int = 17) -> list[Path]:
+    """The spectra of a mass scan (RayTracer.read_mass_spectra), one pair of write_spectra_csvs files per mass:
+    `axion_energy_spectrum_{year}_ma{m:.6g}eV.csv` and `axion_shell_flux_{year}_ma{m:.6g}eV.csv`."""
+    masses = [float(m) for m in masses]
+    if len(spectra) != len(masses):
+        raise ValueError(f"{len(spectra)} spectra for {len(masses)} masses")
+    if len({mass_suffix(m) for m in masses}) != len(masses):
+        raise ValueError("two masses of the scan share a file name (they agree to 6 significant digits)")
+    paths: list[Path] = []
+    for s, m in zip(spectra, masses):
+        paths.extend(write_spectra_csvs(s, windowYear, outpath, suffix=mass_suffix(m), precision=precision))
+    return paths
+
+
 def generateResultPlots(result, windowYear: int, outpath: str | Path, suffix: str = "",
                         radii: ContainmentRadii | None = None, chipXMax: float = 14.0, chipYMax: float = 14.0,
                         precision: int = 17, echo=print) -> Path:

@@ -303,20 +303,37 @@ class RayTracer:
         Switching them on clears them; precision modes 1 and 2 then run their generic kernel variant."""
         check(lib.sart_enable_spectra(self._h, int(bool(on))))
 
-    def read_spectra(self) -> Spectra:
-        """The spectra accumulated since enable_spectra / reset_image (raises SartError while they are off)."""
+    def _read_spectra_rows(self, read, rows: int) -> list[Spectra]:
+        """`rows` spectra copied out by `read` (sart_read_spectra / sart_read_mass_spectra), each with the energies of the
+        bins: the tabulated energies, then the X-ray source's (NaN without a source); shells cut to the telescope's."""
         en = np.asarray(self.fullSetup.tables.energies if self.fullSetup.tables.energies is not None else [], dtype=np.float64)
         nE1 = en.size + 1
-        w, w2 = np.empty(nE1), np.empty(nE1)
-        n = np.empty(nE1, dtype=np.uint64)
-        sw = np.empty(abi.MAX_SHELLS)
-        sn = np.empty(abi.MAX_SHELLS, dtype=np.uint64)
+        w, w2 = np.empty((rows, nE1)), np.empty((rows, nE1))
+        n = np.empty((rows, nE1), dtype=np.uint64)
+        sw = np.empty((rows, abi.MAX_SHELLS))
+        sn = np.empty((rows, abi.MAX_SHELLS), dtype=np.uint64)
         u64 = C.POINTER(C.c_uint64)
-        check(lib.sart_read_spectra(self._h, _dp(w), _dp(w2), n.ctypes.data_as(u64), _dp(sw), sn.ctypes.data_as(u64)))
+        check(read(self._h, _dp(w), _dp(w2), n.ctypes.data_as(u64), _dp(sw), sn.ctypes.data_as(u64)))
         s = self.fullSetup.expSetup
         src = s.testSource.energy if s.testSource.active else np.nan
         ns = s.telescope.nShells
-        return Spectra(np.append(en, src), w, w2, n, sw[:ns].copy(), sn[:ns].copy())
+        energies = np.append(en, src)
+        return [Spectra(energies.copy(), w[k], w2[k], n[k], sw[k, :ns].copy(), sn[k, :ns].copy()) for k in range(rows)]
+
+    def read_spectra(self) -> Spectra:
+        """The spectra accumulated since enable_spectra / reset_image (raises SartError while they are off)."""
+        return self._read_spectra_rows(lib.sart_read_spectra, 1)[0]
+
+    def enable_mass_spectra(self, on: bool = True):
+        """Energy spectrum and per-shell flux of the rays that pass in trace_mc, for every axion mass of set_axion_masses
+        (sart_enable_mass_spectra), from the one traced ray per mass scan. Switching them on clears them; trace_mc then runs
+        the mass-scan kernels for any number of masses. Not together with enable_spectra or the alias sampler."""
+        check(lib.sart_enable_mass_spectra(self._h, int(bool(on))))
+
+    def read_mass_spectra(self) -> list[Spectra]:
+        """One Spectra per axion mass, in the order of set_axion_masses, accumulated since enable_mass_spectra /
+        reset_image (raises SartError while they are off)."""
+        return self._read_spectra_rows(lib.sart_read_mass_spectra, self.n_masses)
 
     def synchronize(self):
         check(lib.sart_synchronize(self._h))
