@@ -412,6 +412,28 @@ int sart_comm_init_all(sart_handle_t* const* handles, int n);
 void sart_comm_destroy(sart_handle_t* h);   /* also done by sart_destroy */
 int sart_allreduce(sart_handle_t* const* handles, int n);
 int sart_read_merged(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);
+/* Sums the optional accumulators of the fused run over all ranks: the radial histogram, the spectra, the per-mass
+ * spectra, whichever are on. Each goes into a merged copy per handle; the handles' own accumulators are untouched.
+ * Every rank must have the same ones on with the same shapes. This is checked collectively, so a mismatch fails
+ * with SART_ERR_CONFIG on every rank instead of hanging. Synchronises the handles' streams.
+ *   The ranks first exchange a few words describing what each has on (one small all-reduce); every refusal that depends
+ * on one rank's state is decided from those words on every rank alike: a mismatch (SART_ERR_CONFIG), a rank that could not
+ * allocate its merged copies (SART_ERR_NOMEM), nothing on anywhere (SART_ERR_ARG). Handles of one call (one process) are
+ * compared on the host first (SART_ERR_CONFIG, before any collective). Then one group of all-reduces sums counts as u64
+ * and sums as f64, so the counts stay exact; of the per-mass spectra only the rows of the M masses set are summed. These
+ * are queued on the handles' streams; the readers synchronise. Same forms as sart_allreduce (&h, 1 per rank, or n handles
+ * of sart_comm_init_all); it does not need sart_allreduce and leaves its merged image alone.
+ *   The merged copies are allocated at the first call (resized when a shape changes, freed by sart_destroy) and stay
+ * readable until the next sart_allreduce_outputs; sart_reset_image leaves them. Switching an accumulator on, off or to
+ * another size (and a new number of axion masses, for the per-mass spectra) invalidates its merged copy. */
+int sart_allreduce_outputs(sart_handle_t* const* handles, int n);
+/* The merged copies; same arguments and array shapes as sart_read_radial_hist, sart_read_spectra and
+ * sart_read_mass_spectra. Synchronise and copy out; SART_ERR_ARG without a valid merged copy. */
+int sart_read_merged_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
+int sart_read_merged_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
+                             double* shell_sum_w, uint64_t* shell_counts);
+int sart_read_merged_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
+                                  double* shell_sum_w, uint64_t* shell_counts);
 
 /* Synchronise and copy out. image/image_w2 may be NULL. counters is [M]. */
 int sart_read_image(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);

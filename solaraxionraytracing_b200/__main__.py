@@ -4,7 +4,7 @@
   python -m solaraxionraytracing_b200 [--ignoreDetWindow] [--ignoreGasAbs] [--ignoreConvProb] [--ignoreReflection]
       [--xrayTest] [--detectorInstall] [--magnet] [--angularScanMin A --angularScanMax B --numAngularScanPoints N]
       [--noPlots] [--config FILE | --configPath DIR] [--nRays N] [--precision f32|fast|exact] [--writeSpectra]
-      [--device D]
+      [--device D | --devices 0,1,... | --devices all]
 
 Inputs the reference reads from `resources/` and that are not shipped with it (solar_model_dataframe.csv, the two
 reflectivity HDF5 files) are taken from [Resources] when present, else generated: Primakoff emission rates from AGSS09
@@ -39,11 +39,51 @@ def build_parser() -> argparse.ArgumentParser:
                          "the image (a single-mass run then takes the generic kernel variant; a mass scan writes one pair "
                          "of files per mass, suffixed _ma{m}eV)")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--devices", default=None,
+                    help="trace on several GPUs: a comma-separated list of CUDA ordinals or `all`. A fused run shards the "
+                         "rays over them and merges image, counters, radial histogram and spectra with NCCL; an angular "
+                         "scan deals each a contiguous block of scan points. The output files are those of one GPU")
     ap.add_argument("--outputPath", default="", help="overrides [Resources].outputPath")
     ap.add_argument("--allowSynthetic", action="store_true",
                     help="continue with stand-in tables (and a warning) when a [Resources] input file is missing; the "
                          "reference stops in that case")
     return ap
+
+
+def parse_devices(text: str, n_visible: int) -> list[int]:
+    """The value of --devices: `all` (every visible device) or distinct, comma-separated ordinals below `n_visible`."""
+    if text.strip() == "all":
+        if n_visible < 1:
+            raise ValueError("no CUDA device is visible")
+        return list(range(n_visible))
+    try:
+        devices = [int(x) for x in text.split(",")]
+    except ValueError:
+        raise ValueError(f"expected `all` or comma-separated device ordinals, got {text!r}") from None
+    for k, d in enumerate(devices):
+        if d in devices[:k]:
+            raise ValueError(f"device {d} is listed twice")
+        if not 0 <= d < n_visible:
+            raise ValueError(f"device {d} does not exist ({n_visible} visible)")
+    return devices
+
+
+def visible_devices() -> int:
+    from ._lib import lib
+    return lib.sart_device_count()
+
+
+def parse_args(argv=None) -> argparse.Namespace:
+    ap = build_parser()
+    a = ap.parse_args(argv)
+    if a.devices is not None:
+        if a.device != 0:
+            ap.error("--devices and --device exclude each other")
+        try:
+            a.devices = parse_devices(a.devices, visible_devices())
+        except ValueError as e:
+            ap.error(f"--devices: {e}")
+    return a
 
 
 def _substitute(what: str, missing, used: str, allow: bool):
@@ -104,9 +144,40 @@ def load_tables(rt, tables, res, setup, device: int, allow_synthetic: bool = Fal
     return tables.TableSet(energies=em.energies, fluxRadiusCDF=rc, diffFluxCDFs=dc, reflectivity=refl, **extra, **det)
 
 
+def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath):
+    """The files of a fused run: the image CSV and containment radii (at most one mass), or the per-mass images of a mass
+    scan; with `spectra` also the spectra CSVs (one Spectra, or one per mass)."""
+    from . import output
+    if len(masses) <= 1:
+        radii = output.containment_radii_from_hist(*radial_hist)
+        path = output.generateResultPlots(result, setup.detector.windowYear, outpath, radii=radii,
+                                          chipXMax=setup.consts.chipXMax, chipYMax=setup.consts.chipYMax)
+        print("wrote", path)
+        if spectra is not None:
+            for p in output.write_spectra_csvs(spectra, setup.detector.windowYear, outpath):
+                print("wrote", p)
+    else:   # mass scan: one image per mass, total flux per mass on stdout
+        Path(outpath).mkdir(parents=True, exist_ok=True)
+        for m, c in zip(masses, result.counters):
+            print(f"m_a = {m:.6g} eV: passed {c['n_passed']}, total flux {c['sum_w']:.6e}")
+        np.save(Path(outpath) / "axion_images_mass_scan.npy", result.image)
+        if spectra is not None:
+            for p in output.write_mass_spectra_csvs(spectra, masses, setup.detector.windowYear, outpath):
+                print("wrote", p)
+
+
+def write_angular_scan(angles, rel, outpath):
+    print("Angle [deg], relative flux")
+    for ang, r in zip(angles, rel):
+        print(f"{ang:.4f}, {r:.6f}")
+    Path(outpath).mkdir(parents=True, exist_ok=True)
+    np.savetxt(Path(outpath) / "angular_scan_telescope_y.csv", np.column_stack([angles, rel]), delimiter=",",
+               header="Angle [deg],relative flux", comments="")
+
+
 def main(argv=None) -> int:
-    a = build_parser().parse_args(argv)
-    from . import abi, config as cfgmod, output, raytracer as rt, tables
+    a = parse_args(argv)
+    from . import abi, config as cfgmod, multi_gpu, raytracer as rt, tables
     cfg_file = a.config or (str(Path(a.configPath) / "config.toml") if a.configPath else None)
     flags = rt.flags_from_cli(a.ignoreDetWindow, a.ignoreGasAbs, a.ignoreConvProb, a.ignoreReflection, a.xrayTest,
                               a.magnet, a.detectorInstall)
@@ -117,61 +188,56 @@ def main(argv=None) -> int:
     a.seed = run.seed if a.seed is None else a.seed
     a.precision = a.precision or run.precision
     outpath = a.outputPath or res.outputPath
-    tb = load_tables(rt, tables, res, setup, a.device, a.allowSynthetic)
+    devices = a.devices or [a.device]
+    tb = load_tables(rt, tables, res, setup, devices[0], a.allowSynthetic)
     fs = rt.FullRaytraceSetup(setup, tb, outpath)
     n = int(a.nRays)
-    with rt.RayTracer(fs, a.device) as tr:
-        want = {"exact": 0, "fast": 1, "f32": 2}[a.precision]
-        for mode in range(want, -1, -1):     # f32 -> fast -> exact: the fastest pipeline that supports this setup
+    want = {"exact": 0, "fast": 1, "f32": 2}[a.precision]
+    sampler = abi.SAMPLER_ALIAS if (a.sampler or run.sampler) == "alias" else None
+    warn = lambda msg: print(msg, file=sys.stderr)   # noqa: E731
+    single = len(run.mAxion) <= 1
+    fused = a.angularScanMin == a.angularScanMax
+    if a.devices is not None:
+        if fused:
+            print("start")
             try:
-                tr.set_precision(mode)
-                break
+                r = multi_gpu.trace_on_devices(fs, devices, n, a.seed, precision=want, sampler=sampler,
+                                               masses=run.mAxion or None, radial_hist=single, spectra=a.writeSpectra,
+                                               warn=warn)
             except rt.SartError as e:
-                print(f"precision {['exact', 'fast', 'f32'][mode]} is not available for this setup ({e}); falling back",
-                      file=sys.stderr)
-        if (a.sampler or run.sampler) == "alias":
-            tr.set_sampler(abi.SAMPLER_ALIAS)
+                if "NCCL" in str(e):
+                    raise SystemExit(f"raytracer: {e}") from None
+                raise
+            write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath)
+        else:
+            angles, rel, _ = multi_gpu.angular_scan_on_devices(fs, devices, a.angularScanMin, a.angularScanMax,
+                                                               a.numAngularScanPoints, n, a.seed, precision=want,
+                                                               sampler=sampler, masses=run.mAxion or None, warn=warn)
+            write_angular_scan(angles, rel, outpath)
+        return 0
+    with rt.RayTracer(fs, a.device) as tr:
+        rt.set_fastest_precision(tr, want, warn)
+        if sampler is not None:
+            tr.set_sampler(sampler)
         if run.mAxion:
             tr.set_axion_masses(run.mAxion)
-        if a.angularScanMin == a.angularScanMax:
+        if fused:
             print("start")
-            spectra = a.writeSpectra and len(run.mAxion) <= 1
-            mass_spectra = a.writeSpectra and not spectra   # a mass scan: one pair of spectra files per mass
-            if len(run.mAxion) <= 1:
+            if single:
                 tr.enable_radial_hist()
-            if spectra:
-                tr.enable_spectra()
-            if mass_spectra:
-                tr.enable_mass_spectra()
+            if a.writeSpectra:   # a mass scan: one pair of spectra files per mass
+                tr.enable_spectra() if single else tr.enable_mass_spectra()
             tr.reset_image()
             tr.trace_mc(n, a.seed)
             result = tr.read_image()
-            if len(run.mAxion) <= 1:
-                radii = output.containment_radii_from_hist(*tr.read_radial_hist())
-                path = output.generateResultPlots(result, setup.detector.windowYear, outpath, radii=radii,
-                                                  chipXMax=setup.consts.chipXMax, chipYMax=setup.consts.chipYMax)
-                print("wrote", path)
-                if spectra:
-                    for p in output.write_spectra_csvs(tr.read_spectra(), setup.detector.windowYear, outpath):
-                        print("wrote", p)
-            else:   # mass scan: one image per mass, total flux per mass on stdout
-                Path(outpath).mkdir(parents=True, exist_ok=True)
-                for m, c in zip(run.mAxion, result.counters):
-                    print(f"m_a = {m:.6g} eV: passed {c['n_passed']}, total flux {c['sum_w']:.6e}")
-                np.save(Path(outpath) / "axion_images_mass_scan.npy", result.image)
-                if mass_spectra:
-                    for p in output.write_mass_spectra_csvs(tr.read_mass_spectra(), run.mAxion,
-                                                            setup.detector.windowYear, outpath):
-                        print("wrote", p)
+            spectra = None
+            if a.writeSpectra:
+                spectra = tr.read_spectra() if single else tr.read_mass_spectra()
+            write_fused_outputs(result, tr.read_radial_hist() if single else None, spectra, run.mAxion, setup, outpath)
         else:
             angles, rel, _ = rt.performAngularScan(fs, a.angularScanMin, a.angularScanMax, a.numAngularScanPoints, n,
                                                    a.seed, tracer=tr)
-            print("Angle [deg], relative flux")
-            for ang, r in zip(angles, rel):
-                print(f"{ang:.4f}, {r:.6f}")
-            Path(outpath).mkdir(parents=True, exist_ok=True)
-            np.savetxt(Path(outpath) / "angular_scan_telescope_y.csv", np.column_stack([angles, rel]), delimiter=",",
-                       header="Angle [deg],relative flux", comments="")
+            write_angular_scan(angles, rel, outpath)
     return 0
 
 

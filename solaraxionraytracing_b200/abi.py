@@ -219,6 +219,12 @@ SIGNATURES = {
     "sart_comm_destroy": (None, [H]),
     "sart_allreduce": (C.c_int, [C.POINTER(H), C.c_int]),
     "sart_read_merged": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(Counters)]),
+    "sart_allreduce_outputs": (C.c_int, [C.POINTER(H), C.c_int]),
+    "sart_read_merged_radial_hist": (C.c_int, [H, c_double_p, C.POINTER(C.c_uint64)]),
+    "sart_read_merged_spectra": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64), c_double_p,
+                                           C.POINTER(C.c_uint64)]),
+    "sart_read_merged_mass_spectra": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64), c_double_p,
+                                                C.POINTER(C.c_uint64)]),
     "sart_angular_scan": (C.c_int, [H, C.c_int, c_double_p, C.c_uint64, C.c_uint64, C.c_uint64, c_double_p, C.POINTER(Counters),
                                     c_double_p]),
     "sart_measure_fma_peak": (C.c_int, [C.c_int, C.c_int, c_double_p]),

@@ -37,18 +37,6 @@ static int cuda_fail(cudaError_t e, const char* what) {
     if (e__ != cudaSuccess) return cuda_fail(e__, #call); \
   } while (0)
 
-// Bump allocator over one device buffer: every piece starts on a 256-byte boundary. Over a null base it only measures, so a
-// layout is written once and run twice: over nullptr to size the buffer, then over the allocation to hand out its pointers.
-struct Carve {
-  unsigned char* base;
-  size_t off = 0;
-  explicit Carve(void* b = nullptr) : base(static_cast<unsigned char*>(b)) {}
-  template <class T> void take(T*& p, size_t count) {
-    p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-    off = (off + count * sizeof(T) + 255) & ~size_t(255);
-  }
-};
-
 // Synchronous host -> device copy of n elements into a table the kernels only read.
 template <class T> static cudaError_t put(const T* dst, const T* src, size_t n) {
   return cudaMemcpy(const_cast<T*>(dst), src, n * sizeof(T), cudaMemcpyHostToDevice);
@@ -379,18 +367,9 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
   return SART_OK;
 }
 
-// Per-mass spectra (sart_enable_mass_spectra), each laid over `base` (nullptr: only measures); both return their bytes.
-// The handle's arrays: eW | eW2 | eN, each [SART_MAX_MASSES][nE1] | sW | sN, each [SART_MAX_MASSES][SART_MAX_SHELLS].
-static size_t carve_mass_spectra(void* base, int nE1, Spectra* r) {
-  Carve c(base);
-  const size_t e = size_t(SART_MAX_MASSES) * nE1, s = size_t(SART_MAX_MASSES) * SART_MAX_SHELLS;
-  *r = Spectra{};
-  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
-  r->eRow = uint32_t(nE1); r->sRow = uint32_t(SART_MAX_SHELLS);
-  return c.off;
-}
-// The accumulators of the throughput mass-scan kernels (fast_common.cuh: mass_spec_add): eW | eW2 | 32-bit eN, each
-// [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each [SART_MAX_SHELLS][SART_MAX_MASSES].
+// The accumulators of the throughput mass-scan kernels (fast_common.cuh: mass_spec_add), laid over `base` (nullptr: only
+// measures); returns their bytes: eW | eW2 | 32-bit eN, each [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each
+// [SART_MAX_SHELLS][SART_MAX_MASSES]. The per-mass rows themselves are carve_mass_spectra (sart_internal.h).
 static size_t carve_mass_spectra_acc(void* base, int nE1, Spectra* r) {
   Carve c(base);
   const size_t e = size_t(nE1) * SART_MAX_MASSES, s = size_t(SART_MAX_SHELLS) * SART_MAX_MASSES;
@@ -408,6 +387,7 @@ static int ensure_image(sart_handle* h, int nMasses) {
     Spectra s;
     SART_CUDA(cudaMemsetAsync(h->d_mspec, 0, carve_mass_spectra(nullptr, h->mspec_e1, &s), h->stream));
   }
+  h->merged_out.mspec_valid = 0;
   cudaFree(h->d_image); cudaFree(h->d_counters);   // d_image_w2 points into d_image's block
   h->d_image = nullptr; h->d_image_w2 = nullptr; h->d_counters = nullptr; h->image_masses = 0; h->merged_valid = 0;
   SART_CUDA(cudaMalloc(&h->d_image, merged_words(nMasses) * sizeof(double)));
@@ -533,17 +513,6 @@ static int copy_records(const Out& host, size_t first, const Out& dev, size_t n,
   if constexpr (std::is_same_v<Out, sart_ray_out_t>) ray_out_fields(host, dev, copy);
   else passed_out_fields(host, dev, copy);
   return e == cudaSuccess ? SART_OK : cuda_fail(e, "cudaMemcpyAsync (records, device to host)");
-}
-
-// One allocation of spectra (device_params.h: Spectra): eW | eW2 | eN, each eRep x eStride | sW | sN, each
-// sRep x SART_MAX_SHELLS. Lays them over `base` (nullptr: only measures) and returns the bytes they take.
-static size_t carve_spectra(void* base, int eStride, int eRep, int sRep, Spectra* r) {
-  Carve c(base);
-  const size_t e = size_t(eRep) * eStride, s = size_t(sRep) * SART_MAX_SHELLS;
-  *r = Spectra{};
-  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
-  r->eStride = uint32_t(eStride); r->eRepMask = uint32_t(eRep - 1); r->sRepMask = uint32_t(sRep - 1);
-  return c.off;
 }
 
 // Parameter block of `s` for a live handle: setup-derived fields recomputed, table-derived fields kept.
@@ -684,7 +653,7 @@ void sart_destroy(sart_handle_t* h) {
   cudaFree(h->table_blob); cudaFree(h->fast_blob); cudaFree(h->d_masses); cudaFree(h->d_image); cudaFree(h->d_merged);
   cudaFree(h->d_counters); cudaFree(h->d_stage); cudaFree(h->d_rad_w); cudaFree(h->d_rad_n); cudaFree(h->d_rep); cudaFree(h->d_mass_acc);
   cudaFree(h->d_queue); cudaFree(h->d_spec); cudaFree(h->d_spec_rep); cudaFree(h->d_mspec); cudaFree(h->d_mspec_acc);
-  cudaFreeHost(h->h_stage);
+  cudaFree(h->merged_out.blob); cudaFreeHost(h->h_stage);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->stream_in) cudaStreamDestroy(h->stream_in);
   if (h->stream_out) cudaStreamDestroy(h->stream_out);
@@ -1262,6 +1231,7 @@ int sart_enable_mass_spectra(sart_handle_t* h, int on) {
   SART_CUDA(cudaStreamSynchronize(h->stream));
   cudaFree(h->d_mspec); cudaFree(h->d_mspec_acc);
   h->d_mspec = nullptr; h->d_mspec_acc = nullptr; h->mspec = Spectra{}; h->mspec_acc = Spectra{}; h->mspec_e1 = 0;
+  h->merged_out.mspec_valid = 0;
   if (!on) return SART_OK;
   const int nE1 = h->params.nEnergies + 1;
   Spectra spec, acc;
@@ -1300,6 +1270,7 @@ int sart_enable_spectra(sart_handle_t* h, int on) {
   SART_CUDA(cudaStreamSynchronize(h->stream));
   cudaFree(h->d_spec); cudaFree(h->d_spec_rep);
   h->d_spec = nullptr; h->d_spec_rep = nullptr; h->spec = Spectra{}; h->spec_rep = Spectra{}; h->spec_e1 = 0;
+  h->merged_out.spec_valid = 0;
   if (!on) return SART_OK;
   const int nE1 = h->params.nEnergies + 1;
   // Replicas of the throughput kernels (powers of two; SART_SPEC_E_REPLICAS / SART_SPEC_S_REPLICAS override them for
@@ -1349,6 +1320,7 @@ int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max) {
   SART_CUDA(cudaStreamSynchronize(h->stream));
   cudaFree(h->d_rad_w); cudaFree(h->d_rad_n);
   h->d_rad_w = nullptr; h->d_rad_n = nullptr; h->rad_bins = 0; h->rad_rmax = 0.0;
+  h->merged_out.rad_valid = 0;
   RadialHist r{};
   if (nbins > 0) {
     SART_CUDA(cudaMalloc(&h->d_rad_w, size_t(nbins) * sizeof(double)));

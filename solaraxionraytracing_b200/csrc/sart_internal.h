@@ -49,6 +49,52 @@ constexpr int kCounterWords = int(sizeof(sart_counters_t) / 8);
 inline size_t merged_words(int nMasses) {
   return size_t(nMasses) * (2 * size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS + size_t(kCounterWords));
 }
+
+// Bump allocator over one device buffer: every piece starts on a 256-byte boundary. Over a null base it only measures, so a
+// layout is written once and run twice: over nullptr to size the buffer, then over the allocation to hand out its pointers.
+struct Carve {
+  unsigned char* base;
+  size_t off = 0;
+  explicit Carve(void* b = nullptr) : base(static_cast<unsigned char*>(b)) {}
+  template <class T> void take(T*& p, size_t count) {
+    p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+    off = (off + count * sizeof(T) + 255) & ~size_t(255);
+  }
+};
+
+// One allocation of spectra (device_params.h: Spectra): eW | eW2 | eN, each eRep x eStride | sW | sN, each
+// sRep x SART_MAX_SHELLS. Lays them over `base` (nullptr: only measures) and returns the bytes they take.
+inline size_t carve_spectra(void* base, int eStride, int eRep, int sRep, Spectra* r) {
+  Carve c(base);
+  const size_t e = size_t(eRep) * eStride, s = size_t(sRep) * SART_MAX_SHELLS;
+  *r = Spectra{};
+  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
+  r->eStride = uint32_t(eStride); r->eRepMask = uint32_t(eRep - 1); r->sRepMask = uint32_t(sRep - 1);
+  return c.off;
+}
+
+// Per-mass spectra (sart_enable_mass_spectra), laid over `base` (nullptr: only measures); returns their bytes.
+// The handle's arrays: eW | eW2 | eN, each [SART_MAX_MASSES][nE1] | sW | sN, each [SART_MAX_MASSES][SART_MAX_SHELLS].
+inline size_t carve_mass_spectra(void* base, int nE1, Spectra* r) {
+  Carve c(base);
+  const size_t e = size_t(SART_MAX_MASSES) * nE1, s = size_t(SART_MAX_MASSES) * SART_MAX_SHELLS;
+  *r = Spectra{};
+  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
+  r->eRow = uint32_t(nE1); r->sRow = uint32_t(SART_MAX_SHELLS);
+  return c.off;
+}
+
+// sart_allreduce_outputs (comm.cu): the sums over all ranks of the optional accumulators, in one allocation laid out like
+// the handle's own (radial histogram w | n, then carve_spectra / carve_mass_spectra). Each has its own valid flag: the
+// enable call of an accumulator clears it, and so does a new number of axion masses for the per-mass spectra.
+struct MergedOutputs {
+  void* blob = nullptr;
+  int rad_bins = 0, spec_e1 = 0, mspec_e1 = 0;   // what blob is laid out for (0: not in it)
+  double* rad_w = nullptr;
+  unsigned long long* rad_n = nullptr;
+  Spectra spec{}, mspec{};
+  int rad_valid = 0, spec_valid = 0, mspec_valid = 0;
+};
 }  // namespace sart
 
 struct sart_handle {
@@ -122,6 +168,7 @@ struct sart_handle {
   void* d_mspec_acc = nullptr;
   sart::Spectra mspec{}, mspec_acc{};   // mspec.eW == nullptr: off
   int mspec_e1 = 0;                     // energy bins per mass: nEnergies + 1
+  sart::MergedOutputs merged_out;       // the result of the last sart_allreduce_outputs
   // staging for the host-pointer entry points
   void* d_stage = nullptr;
   size_t stage_bytes = 0;

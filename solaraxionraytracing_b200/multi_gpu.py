@@ -5,14 +5,22 @@ contiguous index ranges, one per rank, with no data-path exchange; the only coll
 detector image, the sum-of-squares image and the counters (512 KiB + 512 KiB + 224 B per axion mass) — one
 all-reduce over NVLink (NCCL) on the device buffers libsart exposes. The reference's only parallel construct is the
 Weave parallelFor over rays inside one process (src/raytracer.nim:2234-2244).
+
+One process can also drive several GPUs itself (trace_on_devices, angular_scan_on_devices): one RayTracer per device,
+one NCCL communicator over all of them (sart_comm_init_all), and the same collectives behind the C-ABI, which then take
+every handle of the process in one call.
 """
 from __future__ import annotations
 
 import ctypes as C
+import threading
+from dataclasses import dataclass
 
 import numpy as np
 
 from . import abi
+from ._lib import check, lib
+from .output import Spectra
 
 
 def shard(n_rays: int, rank: int, world: int, first_ray: int = 0) -> tuple[int, int]:
@@ -133,3 +141,125 @@ def calculateFluxFractionsSharded(raytraceSetup, nRays: int, seed: int = 2997924
         tr.trace_mc(count, seed, first_ray=first)
         tr.allreduce()
         return tr.read_merged()
+
+
+# -- one process, n GPUs: NCCL needs every handle of the process in one call (RayTracer.allreduce is the per-rank form)
+def _handles(tracers):
+    return (abi.H * len(tracers))(*[t._h for t in tracers])
+
+
+def comm_init_all(tracers):
+    """One NCCL communicator over `tracers`, each on its own device (sart_comm_init_all); rank i = tracers[i]."""
+    check(lib.sart_comm_init_all(_handles(tracers), len(tracers)))
+
+
+def allreduce(tracers):
+    """sart_allreduce over every tracer of comm_init_all: image, w^2 image and counters into each one's read_merged()."""
+    check(lib.sart_allreduce(_handles(tracers), len(tracers)))
+
+
+def allreduce_outputs(tracers):
+    """sart_allreduce_outputs over every tracer of comm_init_all: the radial histogram and the (per-mass) spectra that are
+    on, into each one's read_merged_radial_hist / read_merged_spectra / read_merged_mass_spectra. Synchronises."""
+    check(lib.sart_allreduce_outputs(_handles(tracers), len(tracers)))
+
+
+@dataclass
+class DevicesResult:
+    """A fused run traced on several GPUs and merged over them."""
+    result: object                          # raytracer.RunResult: image, w^2 image and counters of the whole run
+    radial_hist: tuple | None               # (bin edges, sum of weights, counts) as RayTracer.read_radial_hist
+    spectra: Spectra | list[Spectra] | None  # one Spectra (at most one mass) or one per mass (a mass scan)
+    precision: int                           # the precision mode the run took
+
+
+def _open_tracers(fullSetup, devices, precision: int, sampler, masses, warn):
+    """One RayTracer per device, configured as the command line configures one: the fastest precision mode up to
+    `precision` the setup supports (decided on the first device), the sampler and the axion masses."""
+    from . import raytracer as rt
+    if not devices or len(set(devices)) != len(devices):
+        raise ValueError(f"need distinct devices, got {list(devices)}")
+    tracers = []
+    try:
+        for d in devices:
+            tracers.append(rt.RayTracer(fullSetup, d))
+        mode = rt.set_fastest_precision(tracers[0], precision, warn)
+        for t in tracers:
+            t.set_precision(mode)
+            if sampler is not None:
+                t.set_sampler(sampler)
+            if masses is not None and len(masses):
+                t.set_axion_masses(masses)
+    except BaseException:
+        for t in tracers:
+            t.close()
+        raise
+    return tracers, mode
+
+
+def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, precision: int = 2, sampler=None,
+                     masses=None, radial_hist: bool = False, spectra: bool = False, warn=None) -> DevicesResult:
+    """The fused run of `nRays` rays over `devices`, one process: device k traces shard(nRays, k, n) of the global rays,
+    so the result is that of one GPU tracing all of them, up to the order of the floating-point sums. The shards run
+    concurrently (trace_mc only queues work); then sart_allreduce and, with `radial_hist` or `spectra`,
+    sart_allreduce_outputs merge them. `spectra` means the single-mass spectra for at most one axion mass and the per-mass
+    spectra for a mass scan. `warn` receives the precision fall-back messages (see raytracer.set_fastest_precision)."""
+    tracers, mode = _open_tracers(fullSetup, devices, precision, sampler, masses, warn)
+    try:
+        scan = masses is not None and len(masses) > 1
+        for t in tracers:
+            if radial_hist:
+                t.enable_radial_hist()
+            if spectra:
+                t.enable_mass_spectra() if scan else t.enable_spectra()
+            t.reset_image()
+        comm_init_all(tracers)
+        for rank, t in enumerate(tracers):
+            first, count = shard(nRays, rank, len(tracers))
+            if count:
+                t.trace_mc(count, seed, first_ray=first)
+        allreduce(tracers)
+        if radial_hist or spectra:
+            allreduce_outputs(tracers)
+        t0 = tracers[0]
+        merged_spectra = None
+        if spectra:
+            merged_spectra = t0.read_merged_mass_spectra() if scan else t0.read_merged_spectra()
+        return DevicesResult(t0.read_merged(), t0.read_merged_radial_hist() if radial_hist else None, merged_spectra, mode)
+    finally:
+        for t in tracers:
+            t.close()
+
+
+def angular_scan_on_devices(fullSetup, devices, angularScanMin: float, angularScanMax: float,
+                            numAngularScanPoints: int = 50, nRays: int = 1_000_000, seed: int = 299792458, *,
+                            precision: int = 2, sampler=None, masses=None, warn=None):
+    """performAngularScan over `devices` in one process: device k takes the contiguous block shard(points, k, n) of the
+    scan points, and scan point i traces the global rays [i*nRays, (i+1)*nRays) as on one GPU. sart_angular_scan blocks,
+    so each device runs in its own thread; the fluxes are put together on the host. Returns (angles [deg],
+    flux / max flux, fluxes)."""
+    angles = np.linspace(angularScanMin, angularScanMax, numAngularScanPoints)
+    fluxes = np.zeros(numAngularScanPoints)
+    tracers, _ = _open_tracers(fullSetup, devices, precision, sampler, masses, warn)
+    errors = []
+
+    def scan(rank, t):
+        lo, cnt = shard(numAngularScanPoints, rank, len(tracers))
+        try:
+            if cnt:
+                fluxes[lo:lo + cnt] = t.angular_scan(angles[lo:lo + cnt], nRays, seed, first_ray=lo * nRays)[0]
+        except BaseException as e:   # re-raised in the calling thread
+            errors.append(e)
+
+    try:
+        threads = [threading.Thread(target=scan, args=(k, t)) for k, t in enumerate(tracers)]
+        for th in threads:
+            th.start()
+        for th in threads:
+            th.join()
+    finally:
+        for t in tracers:
+            t.close()
+    if errors:
+        raise errors[0]
+    return angles, fluxes / fluxes.max(), fluxes

@@ -290,13 +290,16 @@ class RayTracer:
         check(lib.sart_enable_radial_hist(self._h, nbins, r_max))
         self._rad = (nbins, r_max)
 
-    def read_radial_hist(self):
-        """(bin edges [nbins + 1], sum of weights [nbins], ray counts [nbins])."""
+    def _read_radial(self, read):
         nbins, r_max = self._rad
         w = np.empty(nbins)
         n = np.empty(nbins, dtype=np.uint64)
-        check(lib.sart_read_radial_hist(self._h, _dp(w), n.ctypes.data_as(C.POINTER(C.c_uint64))))
+        check(read(self._h, _dp(w), n.ctypes.data_as(C.POINTER(C.c_uint64))))
         return np.linspace(0.0, r_max, nbins + 1), w, n
+
+    def read_radial_hist(self):
+        """(bin edges [nbins + 1], sum of weights [nbins], ray counts [nbins])."""
+        return self._read_radial(lib.sart_read_radial_hist)
 
     def enable_spectra(self, on: bool = True):
         """Energy spectrum and per-shell flux of the rays that pass in trace_mc (single axion mass; sart_enable_spectra).
@@ -373,6 +376,24 @@ class RayTracer:
         hs = (abi.H * 1)(self._h)
         check(lib.sart_allreduce(hs, 1))
 
+    def allreduce_outputs(self):
+        """sart_allreduce_outputs for this rank (every rank calls it): sums the radial histogram and the (per-mass)
+        spectra that are on over all ranks into merged copies, read with the read_merged_* methods. Synchronises."""
+        hs = (abi.H * 1)(self._h)
+        check(lib.sart_allreduce_outputs(hs, 1))
+
+    def read_merged_radial_hist(self):
+        """read_radial_hist of the last allreduce_outputs (raises SartError without one)."""
+        return self._read_radial(lib.sart_read_merged_radial_hist)
+
+    def read_merged_spectra(self) -> Spectra:
+        """read_spectra of the last allreduce_outputs (raises SartError without one)."""
+        return self._read_spectra_rows(lib.sart_read_merged_spectra, 1)[0]
+
+    def read_merged_mass_spectra(self) -> list[Spectra]:
+        """read_mass_spectra of the last allreduce_outputs (raises SartError without one)."""
+        return self._read_spectra_rows(lib.sart_read_merged_mass_spectra, self.n_masses)
+
     def read_merged(self, want_w2: bool = True) -> RunResult:
         m = self.n_masses
         img = np.empty((m, abi.IMAGE_BINS, abi.IMAGE_BINS))
@@ -388,6 +409,23 @@ class RayTracer:
         cnt = (abi.Counters * m)()
         check(lib.sart_read_image(self._h, _dp(img), _dp(img2) if want_w2 else None, cnt))
         return RunResult(img, img2, [c.as_dict() for c in cnt])
+
+
+PRECISION_NAMES = ("exact", "fast", "f32")
+
+
+def set_fastest_precision(tracer: RayTracer, want: int, warn=None) -> int:
+    """Sets precision mode `want`, else the fastest slower one this setup supports (f32 -> fast -> exact); returns the
+    mode set. `warn` receives a message for every mode the setup refuses."""
+    for mode in range(want, 0, -1):
+        try:
+            tracer.set_precision(mode)
+            return mode
+        except SartError as e:
+            if warn:
+                warn(f"precision {PRECISION_NAMES[mode]} is not available for this setup ({e}); falling back")
+    tracer.set_precision(0)
+    return 0
 
 
 def initFullSetup(setup, detectorSetup, stage, telescope, flags: int = 0, tables: _tables.TableSet | None = None,
