@@ -11,6 +11,7 @@
 #include <type_traits>
 #include <vector>
 
+#include "host_cuda.h"
 #include "kernels.h"
 #include "philox.cuh"
 #include "sart_internal.h"
@@ -27,26 +28,10 @@ int fail(int code, const char* fmt, ...) {
   return code;
 }
 
-static int cuda_fail(cudaError_t e, const char* what) {
-  return fail(SART_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e));
-}
-
-#define SART_CUDA(call)                                  \
-  do {                                                   \
-    cudaError_t e__ = (call);                            \
-    if (e__ != cudaSuccess) return cuda_fail(e__, #call); \
-  } while (0)
-
 // Synchronous host -> device copy of n elements into a table the kernels only read.
 template <class T> static cudaError_t put(const T* dst, const T* src, size_t n) {
   return cudaMemcpy(const_cast<T*>(dst), src, n * sizeof(T), cudaMemcpyHostToDevice);
 }
-
-struct DeviceGuard {
-  int prev = -1;
-  explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 static int validate(const sart_setup_t* s, const sart_tables_t* t) {
   if (!s) return fail(SART_ERR_ARG, "setup is NULL");
@@ -367,27 +352,121 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
   return SART_OK;
 }
 
-// The accumulators of the throughput mass-scan kernels (fast_common.cuh: mass_spec_add), laid over `base` (nullptr: only
-// measures); returns their bytes: eW | eW2 | 32-bit eN, each [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each
-// [SART_MAX_SHELLS][SART_MAX_MASSES]. The per-mass rows themselves are carve_mass_spectra (sart_internal.h).
-static size_t carve_mass_spectra_acc(void* base, int nE1, Spectra* r) {
+// Lays block `a` of accumulator k (bins and rmax set) over `base` (nullptr: only measures): the arrays of accum_arrays for
+// SART_MAX_MASSES masses, each on a 256-byte boundary. Returns their bytes.
+static size_t carve_accum(AccumKind k, void* base, Accum* a) {
   Carve c(base);
-  const size_t e = size_t(nE1) * SART_MAX_MASSES, s = size_t(SART_MAX_SHELLS) * SART_MAX_MASSES;
-  unsigned int *eN, *sN;
-  *r = Spectra{};
-  c.take(r->eW, e); c.take(r->eW2, e); c.take(eN, e); c.take(r->sW, s); c.take(sN, s);
-  r->eN = reinterpret_cast<unsigned long long*>(eN); r->sN = reinterpret_cast<unsigned long long*>(sN);
+  accum_arrays(k, *a, *a, accum_rows(k, SART_MAX_MASSES), [&](auto*& p, auto*&, size_t n) { c.take(p, n); });
+  if (k == kRadialHist) { a->rad.invStep = double(a->bins) / a->rmax; a->rad.nbins = a->bins; }
+  if (k == kMassSpectra) { a->spec.eRow = uint32_t(a->bins); a->spec.sRow = uint32_t(SART_MAX_SHELLS); }
   return c.off;
+}
+
+int alloc_accum(AccumKind k, int bins, double rmax, Accum* a) {
+  *a = Accum{};
+  a->bins = bins; a->rmax = rmax;
+  const size_t bytes = carve_accum(k, nullptr, a);
+  const cudaError_t e = cudaMalloc(&a->blob, bytes);
+  if (e != cudaSuccess) { *a = Accum{}; return cuda_fail(e, "cudaMalloc (accumulator)"); }
+  a->bytes = bytes;
+  carve_accum(k, a->blob, a);
+  return SART_OK;
+}
+
+// The buffers the throughput kernels of accumulator k add into (Accum::tput), laid over `base` (nullptr: only measures);
+// returns their bytes. The spectra's replicas (device_params.h: Spectra): eW | eW2 | eN, each eRep x eStride | sW | sN,
+// each sRep x SART_MAX_SHELLS. The per-mass spectra's mass-minor accumulators (fast_common.cuh: mass_spec_add):
+// eW | eW2 | 32-bit eN, each [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each [SART_MAX_SHELLS][SART_MAX_MASSES].
+static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, void* base, Spectra* r) {
+  Carve c(base);
+  *r = Spectra{};
+  if (k == kSpectra) {
+    const uint32_t eStride = uint32_t((nE1 + 31) & ~31);
+    const size_t e = size_t(eRep) * eStride, s = size_t(sRep) * SART_MAX_SHELLS;
+    c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
+    r->eStride = eStride; r->eRepMask = uint32_t(eRep - 1); r->sRepMask = uint32_t(sRep - 1);
+  } else if (k == kMassSpectra) {
+    const size_t e = size_t(nE1) * SART_MAX_MASSES, s = size_t(SART_MAX_SHELLS) * SART_MAX_MASSES;
+    unsigned int *eN, *sN;
+    c.take(r->eW, e); c.take(r->eW2, e); c.take(eN, e); c.take(r->sW, s); c.take(sN, s);
+    r->eN = reinterpret_cast<unsigned long long*>(eN); r->sN = reinterpret_cast<unsigned long long*>(sN);
+  }
+  return c.off;
+}
+
+// Switches accumulator k off: frees the handle's block, its throughput buffers and its merged copy. The other accumulators
+// and their merged copies stay as they are.
+static void free_accum(sart_handle* h, AccumKind k) {
+  cudaFree(h->accum[k].blob); cudaFree(h->accum[k].tput_blob); cudaFree(h->merged_accum[k].blob);
+  h->accum[k] = Accum{};
+  h->merged_accum[k] = Accum{};
+  if (k == kRadialHist) h->tables.rad = h->ftables.rad = RadialHist{};
+}
+
+// Accumulator k on with `bins` bins: the handle's block and its throughput buffers, allocated, cleared and carved.
+static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax) {
+  Accum& a = h->accum[k];
+  int rc = alloc_accum(k, bins, rmax, &a);
+  if (rc) return rc;
+  // Replicas of the spectra (powers of two; SART_SPEC_E_REPLICAS / SART_SPEC_S_REPLICAS override them for measurements).
+  // The energy bins spread the passed rays over hundreds of addresses, like the focal spot the image replicas serve: one
+  // replica per block residue. The shell bins are a handful of addresses (4 for LLNL): one per warp.
+  auto pow2 = [](const char* env, int dflt) {
+    int n = dflt;
+    if (const char* e = std::getenv(env)) n = std::max(1, std::min(1 << 16, std::atoi(e)));
+    int p = 1;
+    while (p * 2 <= n) p *= 2;
+    return p;
+  };
+  const int eRep = pow2("SART_SPEC_E_REPLICAS", 32), sRep = pow2("SART_SPEC_S_REPLICAS", 1024);
+  const size_t tputBytes = carve_throughput(k, bins, eRep, sRep, nullptr, &a.tput);
+  if (tputBytes) SART_CUDA(cudaMalloc(&a.tput_blob, tputBytes));
+  SART_CUDA(cudaMemsetAsync(a.blob, 0, a.bytes, h->stream));
+  if (tputBytes) SART_CUDA(cudaMemsetAsync(a.tput_blob, 0, tputBytes, h->stream));
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  carve_throughput(k, bins, eRep, sRep, a.tput_blob, &a.tput);
+  if (k == kRadialHist) h->tables.rad = h->ftables.rad = a.rad;
+  return SART_OK;
+}
+
+// What every sart_enable_* does after its own checks: synchronises, switches accumulator k off, and with bins > 0 on again,
+// cleared. A failure leaves it off.
+static int set_accum(sart_handle* h, AccumKind k, int bins, double rmax = 0.0) {
+  DeviceGuard dg(h->device);
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  free_accum(h, k);
+  const int rc = bins > 0 ? new_accum(h, k, bins, rmax) : SART_OK;
+  if (rc) free_accum(h, k);
+  return rc;
+}
+
+// Clears the handle's block of accumulator k on its stream (nothing while it is off).
+static int clear_accum(sart_handle* h, AccumKind k) {
+  if (h->accum[k].blob) SART_CUDA(cudaMemsetAsync(h->accum[k].blob, 0, h->accum[k].bytes, h->stream));
+  return SART_OK;
+}
+
+int read_accum(sart_handle* h, AccumKind k, bool merged, std::initializer_list<void*> host, const char* off) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  const Accum& a = merged ? h->merged_accum[k] : h->accum[k];
+  if (merged ? !a.valid : !a.blob) return fail(SART_ERR_ARG, "%s", off);
+  DeviceGuard dg(h->device);
+  void* const* hp = host.begin();
+  cudaError_t e = cudaSuccess;
+  accum_arrays(k, a, a, accum_rows(k, h->n_masses), [&](auto* d, auto*, size_t n) {
+    void* p = *hp++;
+    if (p && e == cudaSuccess) e = cudaMemcpyAsync(p, d, n * sizeof *d, cudaMemcpyDeviceToHost, h->stream);
+  });
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  return e == cudaSuccess ? SART_OK : cuda_fail(e, "cudaMemcpyAsync (accumulator, device to host)");
 }
 
 static int ensure_image(sart_handle* h, int nMasses) {
   const size_t len = size_t(nMasses) * SART_IMAGE_BINS * SART_IMAGE_BINS;
   if (h->d_image && h->image_masses == nMasses) return SART_OK;
-  if (h->mspec.eW) {   // a new mass list: the rows of the old one are meaningless
-    Spectra s;
-    SART_CUDA(cudaMemsetAsync(h->d_mspec, 0, carve_mass_spectra(nullptr, h->mspec_e1, &s), h->stream));
-  }
-  h->merged_out.mspec_valid = 0;
+  const int rc = clear_accum(h, kMassSpectra);   // a new mass list: the per-mass rows of the old one are meaningless
+  if (rc) return rc;
+  h->merged_accum[kMassSpectra].valid = 0;
   cudaFree(h->d_image); cudaFree(h->d_counters);   // d_image_w2 points into d_image's block
   h->d_image = nullptr; h->d_image_w2 = nullptr; h->d_counters = nullptr; h->image_masses = 0; h->merged_valid = 0;
   SART_CUDA(cudaMalloc(&h->d_image, merged_words(nMasses) * sizeof(double)));
@@ -651,9 +730,9 @@ void sart_destroy(sart_handle_t* h) {
   if (h->stream) cudaStreamSynchronize(h->stream);
   sart_comm_destroy(h);
   cudaFree(h->table_blob); cudaFree(h->fast_blob); cudaFree(h->d_masses); cudaFree(h->d_image); cudaFree(h->d_merged);
-  cudaFree(h->d_counters); cudaFree(h->d_stage); cudaFree(h->d_rad_w); cudaFree(h->d_rad_n); cudaFree(h->d_rep); cudaFree(h->d_mass_acc);
-  cudaFree(h->d_queue); cudaFree(h->d_spec); cudaFree(h->d_spec_rep); cudaFree(h->d_mspec); cudaFree(h->d_mspec_acc);
-  cudaFree(h->merged_out.blob); cudaFreeHost(h->h_stage);
+  cudaFree(h->d_counters); cudaFree(h->d_stage); cudaFree(h->d_rep); cudaFree(h->d_mass_acc); cudaFree(h->d_queue);
+  for (AccumKind k : kAllAccums) free_accum(h, k);
+  cudaFreeHost(h->h_stage);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->stream_in) cudaStreamDestroy(h->stream_in);
   if (h->stream_out) cudaStreamDestroy(h->stream_out);
@@ -1126,17 +1205,18 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   DeviceGuard dg(h->device);
   if (h->sampler == SART_SAMPLER_ALIAS && (h->precision != 2 || h->n_masses > 1))
     return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2 and a single axion mass");
-  if (h->spec.eW && h->n_masses > 1) return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass");
-  if (h->mspec.eW && h->sampler == SART_SAMPLER_ALIAS)
+  const Accum &spec = h->accum[kSpectra], &mspec = h->accum[kMassSpectra];
+  if (spec.blob && h->n_masses > 1) return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass");
+  if (mspec.blob && h->sampler == SART_SAMPLER_ALIAS)
     return fail(SART_ERR_CONFIG, "sart_trace_mc: the per-mass spectra run the mass-scan kernels, which need the inverse-CDF sampler");
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
   int rc = SART_OK;
   // A mass scan, or any run with the per-mass spectra on (one contract for every mass list, M = 1 included): the exact
   // kernels add the spectra into the handle's rows directly, the throughput kernels into mass-minor accumulators that
   // k_fold_mass_spectra adds up after every launch.
-  if (h->n_masses > 1 || h->mspec.eW) {
+  if (h->n_masses > 1 || mspec.blob) {
     Tables et = h->tables;
-    et.spec = h->mspec;   // or off
+    et.spec = mspec.spec;   // or off
     if (h->precision == 0) {
       SART_CUDA(launch_mc_image_exact(h->params, et, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
                                       h->d_image_w2, h->d_counters, h->sm_count, h->stream));
@@ -1148,10 +1228,10 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
       SART_CUDA(cudaMemsetAsync(h->d_mass_acc, 0, 2 * accLen * sizeof(double), h->stream));
     }
     fast::FastTables ft = h->ftables;
-    ft.spec = h->mspec_acc;   // or off
+    ft.spec = mspec.tput;   // or off
     // the spectra's 32-bit counts are folded after every launch of at most kMaxRaysPerLaunch rays
-    auto fold_spectra = [&]() { return h->mspec.eW ? launch_fold_mass_spectra(h->mspec_acc, h->n_masses, h->mspec_e1, h->mspec, h->stream)
-                                                   : cudaSuccess; };
+    auto fold_spectra = [&]() { return mspec.blob ? launch_fold_mass_spectra(mspec.tput, h->n_masses, mspec.bins, mspec.spec, h->stream)
+                                                  : cudaSuccess; };
     if (h->precision == 2) {
       rc = f32_then_retrace(h, n_rays, true,   // the alias sampler was refused above
           [&](uint64_t done, uint64_t m, const fast::RetraceQueue& q) {
@@ -1166,7 +1246,7 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
                                            h->d_image_w2, h->d_counters, h->sm_count, h->stream);
           });
       if (rc) return rc;
-    } else if (!h->mspec.eW) {
+    } else if (!mspec.blob) {
       SART_CUDA(launch_mc_image_fast_masses(h->fparams, ft, h->n_masses, h->d_masses, first_ray, n_rays, seed,
                                             h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream));
     } else {
@@ -1182,12 +1262,12 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
     return SART_OK;
   }
   Tables et = h->tables;
-  et.spec = h->spec;   // mode 0 and the re-trace of mode 2 add into the spectra directly
+  et.spec = spec.spec;   // mode 0 and the re-trace of mode 2 add into the spectra directly
   fast::FastTables ft = h->ftables;
   double *img = h->d_image, *img2 = h->d_image_w2;
   if (h->precision >= 1) {
     if ((rc = ensure_replicas(h))) return rc;
-    ft.spec = h->spec_rep;   // the spectra replicas, or off
+    ft.spec = spec.tput;   // the spectra replicas, or off
     if (h->n_rep > 1) {
       ft.nImgRep = h->n_rep; ft.imgRepStride = h->rep_stride;
       img = h->d_rep; img2 = h->d_rep + size_t(h->n_rep) * h->rep_stride;
@@ -1198,7 +1278,7 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   if (rc || h->precision == 0) return rc;
   if (h->n_rep > 1)
     SART_CUDA(launch_fold_replicas(img, img2, h->n_rep, h->rep_stride, plane, h->d_image, h->d_image_w2, h->stream));
-  if (h->spec.eW) SART_CUDA(launch_fold_spectra(h->spec_rep, h->spec_e1, h->spec, h->stream));
+  if (spec.blob) SART_CUDA(launch_fold_spectra(spec.tput, spec.bins, spec.spec, h->stream));
   return SART_OK;
 }
 
@@ -1208,141 +1288,45 @@ int sart_reset_image(sart_handle_t* h) {
   const size_t len = size_t(h->n_masses) * SART_IMAGE_BINS * SART_IMAGE_BINS;
   SART_CUDA(cudaMemsetAsync(h->d_image, 0, 2 * len * sizeof(double), h->stream));   // image | w^2 image: one block
   SART_CUDA(cudaMemsetAsync(h->d_counters, 0, size_t(h->n_masses) * sizeof(sart_counters_t), h->stream));
-  if (h->rad_bins > 0) {
-    SART_CUDA(cudaMemsetAsync(h->d_rad_w, 0, size_t(h->rad_bins) * sizeof(double), h->stream));
-    SART_CUDA(cudaMemsetAsync(h->d_rad_n, 0, size_t(h->rad_bins) * sizeof(unsigned long long), h->stream));
-  }
-  if (h->spec.eW) {
-    Spectra s;
-    SART_CUDA(cudaMemsetAsync(h->d_spec, 0, carve_spectra(nullptr, h->spec_e1, 1, 1, &s), h->stream));
-  }
-  if (h->mspec.eW) {
-    Spectra s;
-    SART_CUDA(cudaMemsetAsync(h->d_mspec, 0, carve_mass_spectra(nullptr, h->mspec_e1, &s), h->stream));
-  }
+  for (AccumKind k : kAllAccums)
+    if (int rc = clear_accum(h, k)) return rc;
   return SART_OK;
 }
 
 int sart_enable_mass_spectra(sart_handle_t* h, int on) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
-  if (on && h->spec.eW)
+  if (on && h->accum[kSpectra].blob)
     return fail(SART_ERR_CONFIG, "sart_enable_mass_spectra: the single-mass spectra are on (sart_enable_spectra); switch them off first");
-  DeviceGuard dg(h->device);
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  cudaFree(h->d_mspec); cudaFree(h->d_mspec_acc);
-  h->d_mspec = nullptr; h->d_mspec_acc = nullptr; h->mspec = Spectra{}; h->mspec_acc = Spectra{}; h->mspec_e1 = 0;
-  h->merged_out.mspec_valid = 0;
-  if (!on) return SART_OK;
-  const int nE1 = h->params.nEnergies + 1;
-  Spectra spec, acc;
-  const size_t bytes = carve_mass_spectra(nullptr, nE1, &spec), accBytes = carve_mass_spectra_acc(nullptr, nE1, &acc);
-  SART_CUDA(cudaMalloc(&h->d_mspec, bytes));
-  SART_CUDA(cudaMalloc(&h->d_mspec_acc, accBytes));
-  SART_CUDA(cudaMemsetAsync(h->d_mspec, 0, bytes, h->stream));
-  SART_CUDA(cudaMemsetAsync(h->d_mspec_acc, 0, accBytes, h->stream));
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  carve_mass_spectra(h->d_mspec, nE1, &h->mspec);
-  carve_mass_spectra_acc(h->d_mspec_acc, nE1, &h->mspec_acc);
-  h->mspec_e1 = nE1;
-  return SART_OK;
+  return set_accum(h, kMassSpectra, on ? h->params.nEnergies + 1 : 0);
 }
 
 int sart_read_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                            double* shell_sum_w, uint64_t* shell_counts) {
-  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
-  if (!h->mspec.eW) return fail(SART_ERR_ARG, "sart_read_mass_spectra: no per-mass spectra enabled (sart_enable_mass_spectra)");
-  DeviceGuard dg(h->device);
-  const size_t e = size_t(h->n_masses) * h->mspec_e1 * 8, s = size_t(h->n_masses) * SART_MAX_SHELLS * 8;
-  if (energy_sum_w) SART_CUDA(cudaMemcpyAsync(energy_sum_w, h->mspec.eW, e, cudaMemcpyDeviceToHost, h->stream));
-  if (energy_sum_w2) SART_CUDA(cudaMemcpyAsync(energy_sum_w2, h->mspec.eW2, e, cudaMemcpyDeviceToHost, h->stream));
-  if (energy_counts) SART_CUDA(cudaMemcpyAsync(energy_counts, h->mspec.eN, e, cudaMemcpyDeviceToHost, h->stream));
-  if (shell_sum_w) SART_CUDA(cudaMemcpyAsync(shell_sum_w, h->mspec.sW, s, cudaMemcpyDeviceToHost, h->stream));
-  if (shell_counts) SART_CUDA(cudaMemcpyAsync(shell_counts, h->mspec.sN, s, cudaMemcpyDeviceToHost, h->stream));
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  return SART_OK;
+  return read_accum(h, kMassSpectra, false, {energy_sum_w, energy_sum_w2, energy_counts, shell_sum_w, shell_counts},
+                    "sart_read_mass_spectra: no per-mass spectra enabled (sart_enable_mass_spectra)");
 }
 
 int sart_enable_spectra(sart_handle_t* h, int on) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
-  if (on && h->mspec.eW)
+  if (on && h->accum[kMassSpectra].blob)
     return fail(SART_ERR_CONFIG, "sart_enable_spectra: the per-mass spectra are on (sart_enable_mass_spectra); switch them off first");
-  DeviceGuard dg(h->device);
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  cudaFree(h->d_spec); cudaFree(h->d_spec_rep);
-  h->d_spec = nullptr; h->d_spec_rep = nullptr; h->spec = Spectra{}; h->spec_rep = Spectra{}; h->spec_e1 = 0;
-  h->merged_out.spec_valid = 0;
-  if (!on) return SART_OK;
-  const int nE1 = h->params.nEnergies + 1;
-  // Replicas of the throughput kernels (powers of two; SART_SPEC_E_REPLICAS / SART_SPEC_S_REPLICAS override them for
-  // measurements). The energy bins spread the passed rays over hundreds of addresses, like the focal spot the image
-  // replicas serve: one replica per block residue. The shell bins are a handful of addresses (4 for LLNL): one per warp.
-  auto pow2 = [](const char* env, int dflt) {
-    int n = dflt;
-    if (const char* e = std::getenv(env)) n = std::max(1, std::min(1 << 16, std::atoi(e)));
-    int p = 1;
-    while (p * 2 <= n) p *= 2;
-    return p;
-  };
-  const int eRep = pow2("SART_SPEC_E_REPLICAS", 32), sRep = pow2("SART_SPEC_S_REPLICAS", 1024);
-  const uint32_t eStride = uint32_t((nE1 + 31) & ~31);
-  Spectra spec, rep;
-  const size_t bytes = carve_spectra(nullptr, nE1, 1, 1, &spec), repBytes = carve_spectra(nullptr, int(eStride), eRep, sRep, &rep);
-  SART_CUDA(cudaMalloc(&h->d_spec, bytes));
-  SART_CUDA(cudaMalloc(&h->d_spec_rep, repBytes));
-  SART_CUDA(cudaMemsetAsync(h->d_spec, 0, bytes, h->stream));
-  SART_CUDA(cudaMemsetAsync(h->d_spec_rep, 0, repBytes, h->stream));
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  carve_spectra(h->d_spec, nE1, 1, 1, &h->spec);
-  carve_spectra(h->d_spec_rep, int(eStride), eRep, sRep, &h->spec_rep);
-  h->spec_e1 = nE1;
-  return SART_OK;
+  return set_accum(h, kSpectra, on ? h->params.nEnergies + 1 : 0);   // the last energy bin is the X-ray source's
 }
 
 int sart_read_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                       double* shell_sum_w, uint64_t* shell_counts) {
-  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
-  if (!h->spec.eW) return fail(SART_ERR_ARG, "sart_read_spectra: no spectra enabled (sart_enable_spectra)");
-  DeviceGuard dg(h->device);
-  const size_t e = size_t(h->spec_e1) * 8, s = size_t(SART_MAX_SHELLS) * 8;
-  if (energy_sum_w) SART_CUDA(cudaMemcpyAsync(energy_sum_w, h->spec.eW, e, cudaMemcpyDeviceToHost, h->stream));
-  if (energy_sum_w2) SART_CUDA(cudaMemcpyAsync(energy_sum_w2, h->spec.eW2, e, cudaMemcpyDeviceToHost, h->stream));
-  if (energy_counts) SART_CUDA(cudaMemcpyAsync(energy_counts, h->spec.eN, e, cudaMemcpyDeviceToHost, h->stream));
-  if (shell_sum_w) SART_CUDA(cudaMemcpyAsync(shell_sum_w, h->spec.sW, s, cudaMemcpyDeviceToHost, h->stream));
-  if (shell_counts) SART_CUDA(cudaMemcpyAsync(shell_counts, h->spec.sN, s, cudaMemcpyDeviceToHost, h->stream));
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  return SART_OK;
+  return read_accum(h, kSpectra, false, {energy_sum_w, energy_sum_w2, energy_counts, shell_sum_w, shell_counts},
+                    "sart_read_spectra: no spectra enabled (sart_enable_spectra)");
 }
 
 int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
   if (nbins < 0 || nbins > (1 << 24) || (nbins > 0 && !(r_max > 0.0))) return fail(SART_ERR_ARG, "sart_enable_radial_hist: bad argument");
-  DeviceGuard dg(h->device);
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  cudaFree(h->d_rad_w); cudaFree(h->d_rad_n);
-  h->d_rad_w = nullptr; h->d_rad_n = nullptr; h->rad_bins = 0; h->rad_rmax = 0.0;
-  h->merged_out.rad_valid = 0;
-  RadialHist r{};
-  if (nbins > 0) {
-    SART_CUDA(cudaMalloc(&h->d_rad_w, size_t(nbins) * sizeof(double)));
-    SART_CUDA(cudaMalloc(&h->d_rad_n, size_t(nbins) * sizeof(unsigned long long)));
-    SART_CUDA(cudaMemsetAsync(h->d_rad_w, 0, size_t(nbins) * sizeof(double), h->stream));
-    SART_CUDA(cudaMemsetAsync(h->d_rad_n, 0, size_t(nbins) * sizeof(unsigned long long), h->stream));
-    h->rad_bins = nbins; h->rad_rmax = r_max;
-    r.w = h->d_rad_w; r.n = h->d_rad_n; r.invStep = double(nbins) / r_max; r.nbins = nbins;
-  }
-  h->tables.rad = r;
-  h->ftables.rad = r;
-  return SART_OK;
+  return set_accum(h, kRadialHist, nbins, r_max);
 }
 
 int sart_read_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts) {
-  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
-  if (h->rad_bins < 1) return fail(SART_ERR_ARG, "sart_read_radial_hist: no radial histogram enabled");
-  DeviceGuard dg(h->device);
-  if (sum_w) SART_CUDA(cudaMemcpyAsync(sum_w, h->d_rad_w, size_t(h->rad_bins) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  if (counts) SART_CUDA(cudaMemcpyAsync(counts, h->d_rad_n, size_t(h->rad_bins) * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
-  SART_CUDA(cudaStreamSynchronize(h->stream));
-  return SART_OK;
+  return read_accum(h, kRadialHist, false, {sum_w, counts}, "sart_read_radial_hist: no radial histogram enabled");
 }
 
 double* sart_image_dev(sart_handle_t* h) { return h ? h->d_image : nullptr; }

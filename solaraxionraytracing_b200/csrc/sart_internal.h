@@ -1,9 +1,10 @@
-// sart_internal.h — private to libsart.so: the handle, error reporting, launcher prototypes.
+// sart_internal.h — private to libsart.so: the handle and its optional accumulators, error reporting, launcher prototypes.
 #pragma once
 #include <cstdarg>
 #include <cstddef>
 #include <cstdint>
 
+#include <initializer_list>
 #include <vector>
 
 #include "../../include/sart.h"
@@ -62,39 +63,53 @@ struct Carve {
   }
 };
 
-// One allocation of spectra (device_params.h: Spectra): eW | eW2 | eN, each eRep x eStride | sW | sN, each
-// sRep x SART_MAX_SHELLS. Lays them over `base` (nullptr: only measures) and returns the bytes they take.
-inline size_t carve_spectra(void* base, int eStride, int eRep, int sRep, Spectra* r) {
-  Carve c(base);
-  const size_t e = size_t(eRep) * eStride, s = size_t(sRep) * SART_MAX_SHELLS;
-  *r = Spectra{};
-  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
-  r->eStride = uint32_t(eStride); r->eRepMask = uint32_t(eRep - 1); r->sRepMask = uint32_t(sRep - 1);
-  return c.off;
-}
+// The optional accumulators of the passed rays, each switched on and off by its own entry point: the radial histogram
+// (sart_enable_radial_hist), the spectra (sart_enable_spectra) and the per-mass spectra (sart_enable_mass_spectra).
+enum AccumKind { kRadialHist, kSpectra, kMassSpectra, kAccums };
+constexpr AccumKind kAllAccums[kAccums] = {kRadialHist, kSpectra, kMassSpectra};
 
-// Per-mass spectra (sart_enable_mass_spectra), laid over `base` (nullptr: only measures); returns their bytes.
-// The handle's arrays: eW | eW2 | eN, each [SART_MAX_MASSES][nE1] | sW | sN, each [SART_MAX_MASSES][SART_MAX_SHELLS].
-inline size_t carve_mass_spectra(void* base, int nE1, Spectra* r) {
-  Carve c(base);
-  const size_t e = size_t(SART_MAX_MASSES) * nE1, s = size_t(SART_MAX_MASSES) * SART_MAX_SHELLS;
-  *r = Spectra{};
-  c.take(r->eW, e); c.take(r->eW2, e); c.take(r->eN, e); c.take(r->sW, s); c.take(r->sN, s);
-  r->eRow = uint32_t(nE1); r->sRow = uint32_t(SART_MAX_SHELLS);
-  return c.off;
-}
-
-// sart_allreduce_outputs (comm.cu): the sums over all ranks of the optional accumulators, in one allocation laid out like
-// the handle's own (radial histogram w | n, then carve_spectra / carve_mass_spectra). Each has its own valid flag: the
-// enable call of an accumulator clears it, and so does a new number of axion masses for the per-mass spectra.
-struct MergedOutputs {
+// One block of an accumulator: the handle's own (sart_handle::accum) or its merged copy (sart_handle::merged_accum), both
+// one allocation laid out by the same code (api.cu: alloc_accum). blob == nullptr: off (and bins == 0).
+struct Accum {
   void* blob = nullptr;
-  int rad_bins = 0, spec_e1 = 0, mspec_e1 = 0;   // what blob is laid out for (0: not in it)
-  double* rad_w = nullptr;
-  unsigned long long* rad_n = nullptr;
-  Spectra spec{}, mspec{};
-  int rad_valid = 0, spec_valid = 0, mspec_valid = 0;
+  size_t bytes = 0;
+  int bins = 0;         // radial histogram: its bins; (per-mass) spectra: energy bins per row, nEnergies + 1
+  double rmax = 0.0;    // radial histogram: its range
+  RadialHist rad{};     // radial histogram: w, n
+  Spectra spec{};       // (per-mass) spectra: eW, eW2, eN, sW, sN; the per-mass spectra have one row per mass (eRow, sRow)
+  int valid = 0;        // merged copy: it holds the sums of the last sart_allreduce_outputs for the masses set
+  // The handle's own block only: the buffers the throughput kernels add into instead (api.cu: carve_throughput), which the
+  // fold after every launch adds into the arrays above and clears. The spectra's replicas, the per-mass spectra's
+  // mass-minor accumulators; the radial histogram has none.
+  void* tput_blob = nullptr;
+  Spectra tput{};
 };
+
+// Rows of accumulator k for nMasses axion masses: one per mass for the per-mass spectra (allocated for SART_MAX_MASSES,
+// read and merged for the masses set), one for the others.
+inline size_t accum_rows(AccumKind k, int nMasses) { return k == kMassSpectra ? size_t(nMasses) : 1; }
+
+// The arrays of an accumulator: f(a.array, b.array, count) for every device array of a pair of blocks of kind k (a block
+// and itself, or a handle's block and its merged copy) in layout order, `count` elements for `rows` rows of a.bins bins.
+// The only place that lists them; an element is an f64 sum (double) or a u64 count (unsigned long long).
+template <class A, class B, class F>
+inline void accum_arrays(AccumKind k, A& a, B& b, size_t rows, F&& f) {
+  const size_t e = rows * size_t(a.bins), s = rows * SART_MAX_SHELLS;
+  if (k == kRadialHist) {
+    f(a.rad.w, b.rad.w, e); f(a.rad.n, b.rad.n, e);
+    return;
+  }
+  f(a.spec.eW, b.spec.eW, e); f(a.spec.eW2, b.spec.eW2, e); f(a.spec.eN, b.spec.eN, e);
+  f(a.spec.sW, b.spec.sW, s); f(a.spec.sN, b.spec.sN, s);
+}
+
+// api.cu: a block of accumulator k with `bins` bins (rmax: the radial histogram's range), allocated and carved but not
+// cleared. On failure `a` stays empty and the error is recorded.
+int alloc_accum(AccumKind k, int bins, double rmax, Accum* a);
+// api.cu: the reader behind sart_read_radial_hist / _spectra / _mass_spectra and their sart_read_merged_* twins. Copies the
+// rows in use of accumulator k, the handle's own block or its merged copy, into the caller's arrays `host`, one per array
+// in the order of accum_arrays (NULL: skipped), and synchronises. `off`: the error while there is nothing to read.
+int read_accum(sart_handle* h, AccumKind k, bool merged, std::initializer_list<void*> host, const char* off);
 }  // namespace sart
 
 struct sart_handle {
@@ -148,27 +163,10 @@ struct sart_handle {
   size_t queue_cap = 0;
   int retrace = 1;              // sart_set_retrace: uncertain FP32 rays are re-traced in FP64
   float retrace_scale = 1.0f;   // multiplies every error budget (Tol32)
-  // optional radial histogram of the passed rays (sart_enable_radial_hist)
-  double* d_rad_w = nullptr;
-  unsigned long long* d_rad_n = nullptr;
-  int rad_bins = 0;
-  double rad_rmax = 0.0;
-  // optional spectra of the passed rays (sart_enable_spectra), one allocation each: the handle's arrays (the exact kernels
-  // and the re-trace add into them directly) and the replicas of the throughput kernels (device_params.h: Spectra), which
-  // the fold after every launch adds up and clears. Only sart_trace_mc hands them to a kernel.
-  void* d_spec = nullptr;
-  void* d_spec_rep = nullptr;
-  sart::Spectra spec{}, spec_rep{};   // spec.eW == nullptr: off
-  int spec_e1 = 0;                    // energy bins: nEnergies + 1 (the last one is the X-ray source's)
-  // optional per-mass spectra of the passed rays (sart_enable_mass_spectra), one allocation each, sized for
-  // SART_MAX_MASSES: the handle's arrays, one row per mass (the exact kernels and the re-trace add into them directly), and
-  // the mass-minor accumulators of the throughput mass-scan kernels (fast_common.cuh: mass_spec_add), which the fold after
-  // every launch adds into those rows and clears. Only sart_trace_mc hands them to a kernel.
-  void* d_mspec = nullptr;
-  void* d_mspec_acc = nullptr;
-  sart::Spectra mspec{}, mspec_acc{};   // mspec.eW == nullptr: off
-  int mspec_e1 = 0;                     // energy bins per mass: nEnergies + 1
-  sart::MergedOutputs merged_out;       // the result of the last sart_allreduce_outputs
+  // the optional accumulators (indexed by sart::AccumKind): the handle's arrays, which the exact kernels and the re-trace
+  // add into directly (the radial histogram also reaches the kernels through tables.rad / ftables.rad, the others only
+  // through sart_trace_mc), and their merged copies, the sums over all ranks of the last sart_allreduce_outputs
+  sart::Accum accum[sart::kAccums], merged_accum[sart::kAccums];
   // staging for the host-pointer entry points
   void* d_stage = nullptr;
   size_t stage_bytes = 0;
