@@ -34,6 +34,7 @@ extern "C" {
 #define SART_MAX_COATINGS 8  /* LLNL has 4 coating recipes (raytracer.nim:1167) */
 #define SART_IMAGE_BINS 256  /* prepareHeatmap(256, 256, ...) raytracer.nim:2629 */
 #define SART_MAX_MASSES 64   /* axion masses traced per launch in a mass scan */
+#define SART_MAX_BANDS 16    /* energy bands of sart_enable_band_images */
 
 typedef enum {
   SART_OK = 0,
@@ -390,6 +391,27 @@ int sart_enable_mass_spectra(sart_handle_t* h, int on);
  * shell_* [M][SART_MAX_SHELLS]. SART_ERR_ARG when the per-mass spectra are off. */
 int sart_read_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                            double* shell_sum_w, uint64_t* shell_counts);
+/* Optional detector images of the passed rays of sart_trace_mc per energy band, single axion mass: band b collects the
+ * passed rays whose energy (energiesAx, rt:2197, as a per-ray record reports it: max(0.03 keV, the tabulated energy),
+ * rt:470-471; the X-ray source's energy for its rays) lies in [edges_keV[b], edges_keV[b+1]). Each band has Σw and Σw² per
+ * image bin, binned like the image (rt:818-842), and the number of its passed rays (those outside the image included).
+ * Rays outside every band still go to the ordinary image, which the band images leave as it is. The band of each tabulated
+ * energy is decided once on the host; sart_update_setup redecides the X-ray source's when its energy changes.
+ *   Accumulated (+=) like the image and cleared by sart_reset_image; filled in every precision mode, by the FP32 kernel and by
+ * the FP64 re-trace of its uncertain rays alike, so precision 2 has the counts of precision 0. With them on, precision modes
+ * 1 and 2 run kernel variants of their own that also fill the radial histogram and the spectra when those are on; the alias
+ * sampler is supported like in a run without them. sart_trace_mc with more than one axion mass, or with the per-mass spectra
+ * on, fails with SART_ERR_CONFIG. sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev)
+ * and sart_trace_words leave them untouched.
+ *   n_bands in 1..SART_MAX_BANDS with n_bands + 1 finite, non-negative, strictly ascending edges synchronises, then
+ * (re)allocates and zeroes them; n_bands = 0 switches them off (default; edges_keV may then be NULL); anything else is
+ * SART_ERR_ARG. Device memory at n_bands bands: 1 MB per band for Σw and Σw², the same again for each of the 8 replicas the
+ * throughput kernels add into (a fold after every launch adds them up), and 1 MB per band for the merged copy of
+ * sart_allreduce_outputs: 16 + 128 + 16 MB at 16 bands. */
+int sart_enable_band_images(sart_handle_t* h, int n_bands, const double* edges_keV);
+/* Synchronises and copies out; host arrays, any may be NULL: image, image_w2 [n_bands][256][256] (the layout of the image),
+ * counts [n_bands]. SART_ERR_ARG when the band images are off. */
+int sart_read_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts);
 /* Device pointers for collectives (ncclAllReduce / torch.distributed on the caller's side). */
 double* sart_image_dev(sart_handle_t* h);       /* [M][256][256] Σw  */
 double* sart_image_w2_dev(sart_handle_t* h);    /* [M][256][256] Σw² */
@@ -413,7 +435,7 @@ void sart_comm_destroy(sart_handle_t* h);   /* also done by sart_destroy */
 int sart_allreduce(sart_handle_t* const* handles, int n);
 int sart_read_merged(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);
 /* Sums the optional accumulators of the fused run over all ranks: the radial histogram, the spectra, the per-mass
- * spectra, whichever are on. Each goes into a merged copy per handle; the handles' own accumulators are untouched.
+ * spectra, the band images, whichever are on (the band images with the same edges on every rank). Each goes into a merged copy per handle; the handles' own accumulators are untouched.
  * Every rank must have the same ones on with the same shapes. This is checked collectively, so a mismatch fails
  * with SART_ERR_CONFIG on every rank instead of hanging. Synchronises the handles' streams.
  *   The ranks first exchange a few words describing what each has on (one small all-reduce); every refusal that depends
@@ -427,13 +449,14 @@ int sart_read_merged(sart_handle_t* h, double* image, double* image_w2, sart_cou
  * readable until the next sart_allreduce_outputs; sart_reset_image leaves them. Switching an accumulator on, off or to
  * another size (and a new number of axion masses, for the per-mass spectra) invalidates its merged copy. */
 int sart_allreduce_outputs(sart_handle_t* const* handles, int n);
-/* The merged copies; same arguments and array shapes as sart_read_radial_hist, sart_read_spectra and
- * sart_read_mass_spectra. Synchronise and copy out; SART_ERR_ARG without a valid merged copy. */
+/* The merged copies; same arguments and array shapes as sart_read_radial_hist, sart_read_spectra,
+ * sart_read_mass_spectra and sart_read_band_images. Synchronise and copy out; SART_ERR_ARG without a valid merged copy. */
 int sart_read_merged_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
 int sart_read_merged_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                              double* shell_sum_w, uint64_t* shell_counts);
 int sart_read_merged_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                                   double* shell_sum_w, uint64_t* shell_counts);
+int sart_read_merged_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts);
 
 /* Synchronise and copy out. image/image_w2 may be NULL. counters is [M]. */
 int sart_read_image(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);

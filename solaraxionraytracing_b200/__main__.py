@@ -4,7 +4,7 @@
   python -m solaraxionraytracing_b200 [--ignoreDetWindow] [--ignoreGasAbs] [--ignoreConvProb] [--ignoreReflection]
       [--xrayTest] [--detectorInstall] [--magnet] [--angularScanMin A --angularScanMax B --numAngularScanPoints N]
       [--noPlots] [--config FILE | --configPath DIR] [--nRays N] [--precision f32|fast|exact] [--writeSpectra]
-      [--device D | --devices 0,1,... | --devices all]
+      [--energyBands E0,E1,...] [--device D | --devices 0,1,... | --devices all]
 
 Inputs the reference reads from `resources/` and that are not shipped with it (solar_model_dataframe.csv, the two
 reflectivity HDF5 files) are taken from [Resources] when present, else generated: Primakoff emission rates from AGSS09
@@ -38,6 +38,10 @@ def build_parser() -> argparse.ArgumentParser:
                     help="also write the energy spectrum and the per-shell flux of the detected rays as CSV files next to "
                          "the image (a single-mass run then takes the generic kernel variant; a mass scan writes one pair "
                          "of files per mass, suffixed _ma{m}eV)")
+    ap.add_argument("--energyBands", default=None,
+                    help="also write one detector image per energy band: comma-separated band edges in keV, e.g. 0.5,2,4,8 "
+                         "(2 to 17 values, ascending) writes axion_image_{year}_E0.5-2keV.csv and so on next to the image; "
+                         "a single axion mass only")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--devices", default=None,
                     help="trace on several GPUs: a comma-separated list of CUDA ordinals or `all`. A fused run shards the "
@@ -83,6 +87,12 @@ def parse_args(argv=None) -> argparse.Namespace:
             a.devices = parse_devices(a.devices, visible_devices())
         except ValueError as e:
             ap.error(f"--devices: {e}")
+    if a.energyBands is not None:
+        from .output import parse_energy_bands
+        try:
+            a.energyBands = parse_energy_bands(a.energyBands)
+        except ValueError as e:
+            ap.error(f"--energyBands: {e}")
     return a
 
 
@@ -144,15 +154,20 @@ def load_tables(rt, tables, res, setup, device: int, allow_synthetic: bool = Fal
     return tables.TableSet(energies=em.energies, fluxRadiusCDF=rc, diffFluxCDFs=dc, reflectivity=refl, **extra, **det)
 
 
-def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath):
+def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath, bands=None):
     """The files of a fused run: the image CSV and containment radii (at most one mass), or the per-mass images of a mass
-    scan; with `spectra` also the spectra CSVs (one Spectra, or one per mass)."""
+    scan; with `spectra` also the spectra CSVs (one Spectra, or one per mass); with `bands` (output.BandImages, at most one
+    mass) one image CSV per energy band."""
     from . import output
     if len(masses) <= 1:
         radii = output.containment_radii_from_hist(*radial_hist)
         path = output.generateResultPlots(result, setup.detector.windowYear, outpath, radii=radii,
                                           chipXMax=setup.consts.chipXMax, chipYMax=setup.consts.chipYMax)
         print("wrote", path)
+        if bands is not None:
+            for p in output.write_band_image_csvs(bands, setup.detector.windowYear, outpath, radii,
+                                                  setup.consts.chipXMax, setup.consts.chipYMax):
+                print("wrote", p)
         if spectra is not None:
             for p in output.write_spectra_csvs(spectra, setup.detector.windowYear, outpath):
                 print("wrote", p)
@@ -184,6 +199,8 @@ def main(argv=None) -> int:
     print("Flags:", {n for n, on in vars(a).items() if on is True and n != "noPlots"})
     setup, res = cfgmod.setup_from_config(cfg_file, flags)
     run = cfgmod.parseRun(cfgmod.load_config(cfg_file))
+    if a.energyBands is not None and len(run.mAxion) > 1:
+        build_parser().error("--energyBands: the band images need a single axion mass, and the configuration sets a mass scan")
     a.nRays = run.nRays if a.nRays is None else a.nRays
     a.seed = run.seed if a.seed is None else a.seed
     a.precision = a.precision or run.precision
@@ -203,12 +220,12 @@ def main(argv=None) -> int:
             try:
                 r = multi_gpu.trace_on_devices(fs, devices, n, a.seed, precision=want, sampler=sampler,
                                                masses=run.mAxion or None, radial_hist=single, spectra=a.writeSpectra,
-                                               warn=warn)
+                                               bands=a.energyBands, warn=warn)
             except rt.SartError as e:
                 if "NCCL" in str(e):
                     raise SystemExit(f"raytracer: {e}") from None
                 raise
-            write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath)
+            write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath, r.band_images)
         else:
             angles, rel, _ = multi_gpu.angular_scan_on_devices(fs, devices, a.angularScanMin, a.angularScanMax,
                                                                a.numAngularScanPoints, n, a.seed, precision=want,
@@ -227,13 +244,16 @@ def main(argv=None) -> int:
                 tr.enable_radial_hist()
             if a.writeSpectra:   # a mass scan: one pair of spectra files per mass
                 tr.enable_spectra() if single else tr.enable_mass_spectra()
+            if a.energyBands is not None:
+                tr.enable_band_images(a.energyBands)
             tr.reset_image()
             tr.trace_mc(n, a.seed)
             result = tr.read_image()
             spectra = None
             if a.writeSpectra:
                 spectra = tr.read_spectra() if single else tr.read_mass_spectra()
-            write_fused_outputs(result, tr.read_radial_hist() if single else None, spectra, run.mAxion, setup, outpath)
+            bands = tr.read_band_images() if a.energyBands is not None else None
+            write_fused_outputs(result, tr.read_radial_hist() if single else None, spectra, run.mAxion, setup, outpath, bands)
         else:
             angles, rel, _ = rt.performAngularScan(fs, a.angularScanMin, a.angularScanMax, a.numAngularScanPoints, n,
                                                    a.seed, tracer=tr)

@@ -10,6 +10,7 @@ MAX_SHELLS = 64
 MAX_COATINGS = 8
 IMAGE_BINS = 256
 MAX_MASSES = 64
+MAX_BANDS = 16
 COMM_ID_BYTES = 128
 
 # enums (raytracer.nim:16-46, 59-64, 164-167)
@@ -207,6 +208,8 @@ SIGNATURES = {
     "sart_enable_mass_spectra": (C.c_int, [H, C.c_int]),
     "sart_read_mass_spectra": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64), c_double_p,
                                          C.POINTER(C.c_uint64)]),
+    "sart_enable_band_images": (C.c_int, [H, C.c_int, c_double_p]),
+    "sart_read_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_image_dev": (C.c_void_p, [H]),
     "sart_image_w2_dev": (C.c_void_p, [H]),
     "sart_counters_dev": (C.c_void_p, [H]),
@@ -225,6 +228,7 @@ SIGNATURES = {
                                            C.POINTER(C.c_uint64)]),
     "sart_read_merged_mass_spectra": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64), c_double_p,
                                                 C.POINTER(C.c_uint64)]),
+    "sart_read_merged_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_angular_scan": (C.c_int, [H, C.c_int, c_double_p, C.c_uint64, C.c_uint64, C.c_uint64, c_double_p, C.POINTER(Counters),
                                     c_double_p]),
     "sart_measure_fma_peak": (C.c_int, [C.c_int, C.c_int, c_double_p]),

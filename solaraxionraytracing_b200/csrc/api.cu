@@ -359,6 +359,7 @@ static size_t carve_accum(AccumKind k, void* base, Accum* a) {
   accum_arrays(k, *a, *a, accum_rows(k, SART_MAX_MASSES), [&](auto*& p, auto*&, size_t n) { c.take(p, n); });
   if (k == kRadialHist) { a->rad.invStep = double(a->bins) / a->rmax; a->rad.nbins = a->bins; }
   if (k == kMassSpectra) { a->spec.eRow = uint32_t(a->bins); a->spec.sRow = uint32_t(SART_MAX_SHELLS); }
+  if (k == kBandImages) a->band.nBands = a->bins;
   return c.off;
 }
 
@@ -373,12 +374,15 @@ int alloc_accum(AccumKind k, int bins, double rmax, Accum* a) {
   return SART_OK;
 }
 
-// The buffers the throughput kernels of accumulator k add into (Accum::tput), laid over `base` (nullptr: only measures);
-// returns their bytes. The spectra's replicas (device_params.h: Spectra): eW | eW2 | eN, each eRep x eStride | sW | sN,
-// each sRep x SART_MAX_SHELLS. The per-mass spectra's mass-minor accumulators (fast_common.cuh: mass_spec_add):
-// eW | eW2 | 32-bit eN, each [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each [SART_MAX_SHELLS][SART_MAX_MASSES].
-static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, void* base, Spectra* r) {
+// The buffers the throughput kernels of accumulator k add into (Accum::tput, tput_band), laid over `base` (nullptr: only
+// measures); returns their bytes. The spectra's replicas (device_params.h: Spectra): eW | eW2 | eN, each eRep x eStride |
+// sW | sN, each sRep x SART_MAX_SHELLS. The per-mass spectra's mass-minor accumulators (fast_common.cuh: mass_spec_add):
+// eW | eW2 | 32-bit eN, each [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each [SART_MAX_SHELLS][SART_MAX_MASSES]. The band
+// images' replicas (device_params.h: BandImages): w | w2, each bRep x [bins][256][256], and the band of each of the nE1
+// energy bins, which the exact kernels read through the handle's block (a->band) as well; their counts are the handle's.
+static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, int bRep, void* base, Accum* a) {
   Carve c(base);
+  Spectra* r = &a->tput;
   *r = Spectra{};
   if (k == kSpectra) {
     const uint32_t eStride = uint32_t((nE1 + 31) & ~31);
@@ -390,8 +394,36 @@ static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, void* b
     unsigned int *eN, *sN;
     c.take(r->eW, e); c.take(r->eW2, e); c.take(eN, e); c.take(r->sW, s); c.take(sN, s);
     r->eN = reinterpret_cast<unsigned long long*>(eN); r->sN = reinterpret_cast<unsigned long long*>(sN);
+  } else if (k == kBandImages) {
+    BandImages& b = a->tput_band;
+    b = a->band;
+    const size_t len = size_t(a->bins) * SART_IMAGE_BINS * SART_IMAGE_BINS;
+    c.take(b.w, size_t(bRep) * len); c.take(b.w2, size_t(bRep) * len); c.take(b.band, size_t(nE1));
+    b.repStride = uint32_t(len); b.repMask = uint32_t(bRep - 1);
+    a->band.band = b.band;
   }
   return c.off;
+}
+
+// The band images' table of the energy bins from bin `from` on (sart_enable_band_images; device_params.h: BandImages): the band
+// of the energy a per-ray record reports, max(0.03 keV, energies[i]) for tabulated energy i (rt:470-471) and the X-ray
+// source's energy for bin nEnergies.
+static int put_band_table(sart_handle* h, int from) {
+  const Accum& a = h->accum[kBandImages];
+  const int nE = h->params.nEnergies;
+  auto band_of = [&](double E) {
+    for (int b = 0; b < a.bins; ++b)
+      if (a.edges[b] <= E && E < a.edges[b + 1]) return uint8_t(b);
+    return kNoBand;
+  };
+  std::vector<uint8_t> t(size_t(nE) + 1);
+  for (int i = from; i <= nE; ++i)
+    t[size_t(i)] = band_of(i == nE ? h->setup.testSource.energy
+                                   : (size_t(i) < h->h_energies.size() ? std::max(0.03, h->h_energies[size_t(i)]) : NAN));
+  SART_CUDA(cudaMemcpyAsync(const_cast<uint8_t*>(a.band.band) + from, t.data() + from, size_t(nE + 1 - from),
+                            cudaMemcpyHostToDevice, h->stream));
+  SART_CUDA(cudaStreamSynchronize(h->stream));
+  return SART_OK;
 }
 
 // Switches accumulator k off: frees the handle's block, its throughput buffers and its merged copy. The other accumulators
@@ -403,14 +435,18 @@ static void free_accum(sart_handle* h, AccumKind k) {
   if (k == kRadialHist) h->tables.rad = h->ftables.rad = RadialHist{};
 }
 
-// Accumulator k on with `bins` bins: the handle's block and its throughput buffers, allocated, cleared and carved.
-static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax) {
+// Accumulator k on with `bins` bins: the handle's block and its throughput buffers, allocated, cleared and carved; the band
+// images also get their `edges` and energy -> band table.
+static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax, const double* edges) {
   Accum& a = h->accum[k];
   int rc = alloc_accum(k, bins, rmax, &a);
   if (rc) return rc;
+  if (edges) std::copy(edges, edges + bins + 1, a.edges);
   // Replicas of the spectra (powers of two; SART_SPEC_E_REPLICAS / SART_SPEC_S_REPLICAS override them for measurements).
   // The energy bins spread the passed rays over hundreds of addresses, like the focal spot the image replicas serve: one
-  // replica per block residue. The shell bins are a handful of addresses (4 for LLNL): one per warp.
+  // replica per block residue. The shell bins are a handful of addresses (4 for LLNL): one per warp. The band images have a
+  // focal spot per band plane, like the image: 8 replicas (SART_BAND_REPLICAS overrides it; measured on B200, CAST+LLNL, 4
+  // bands, 1e9 rays: 1 replica 39.5 ms, 8 replicas 31.4 ms, 16 replicas at 16 bands no faster than 8).
   auto pow2 = [](const char* env, int dflt) {
     int n = dflt;
     if (const char* e = std::getenv(env)) n = std::max(1, std::min(1 << 16, std::atoi(e)));
@@ -419,23 +455,25 @@ static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax) {
     return p;
   };
   const int eRep = pow2("SART_SPEC_E_REPLICAS", 32), sRep = pow2("SART_SPEC_S_REPLICAS", 1024);
-  const size_t tputBytes = carve_throughput(k, bins, eRep, sRep, nullptr, &a.tput);
+  const int bRep = std::min(pow2("SART_BAND_REPLICAS", 8), 64);
+  const int nE1 = h->params.nEnergies + 1;
+  const size_t tputBytes = carve_throughput(k, nE1, eRep, sRep, bRep, nullptr, &a);
   if (tputBytes) SART_CUDA(cudaMalloc(&a.tput_blob, tputBytes));
   SART_CUDA(cudaMemsetAsync(a.blob, 0, a.bytes, h->stream));
   if (tputBytes) SART_CUDA(cudaMemsetAsync(a.tput_blob, 0, tputBytes, h->stream));
   SART_CUDA(cudaStreamSynchronize(h->stream));
-  carve_throughput(k, bins, eRep, sRep, a.tput_blob, &a.tput);
+  carve_throughput(k, nE1, eRep, sRep, bRep, a.tput_blob, &a);
   if (k == kRadialHist) h->tables.rad = h->ftables.rad = a.rad;
-  return SART_OK;
+  return k == kBandImages ? put_band_table(h, 0) : SART_OK;
 }
 
 // What every sart_enable_* does after its own checks: synchronises, switches accumulator k off, and with bins > 0 on again,
 // cleared. A failure leaves it off.
-static int set_accum(sart_handle* h, AccumKind k, int bins, double rmax = 0.0) {
+static int set_accum(sart_handle* h, AccumKind k, int bins, double rmax = 0.0, const double* edges = nullptr) {
   DeviceGuard dg(h->device);
   SART_CUDA(cudaStreamSynchronize(h->stream));
   free_accum(h, k);
-  const int rc = bins > 0 ? new_accum(h, k, bins, rmax) : SART_OK;
+  const int rc = bins > 0 ? new_accum(h, k, bins, rmax, edges) : SART_OK;
   if (rc) free_accum(h, k);
   return rc;
 }
@@ -714,6 +752,7 @@ int sart_create(const sart_setup_t* setup, const sart_tables_t* tables, int devi
   if ((rc = upload_tables(h, tables))) { sart_destroy(h); return rc; }
   if ((rc = upload_fast(h, tables))) { sart_destroy(h); return rc; }
   if ((e = cudaMalloc(&h->d_masses, SART_MAX_MASSES * sizeof(double))) != cudaSuccess) { sart_destroy(h); return cuda_fail(e, "cudaMalloc"); }
+  if ((e = cudaMalloc(&h->d_desc, kDescCapacity * sizeof(long long))) != cudaSuccess) { sart_destroy(h); return cuda_fail(e, "cudaMalloc"); }
   h->n_masses = 1;
   h->masses[0] = setup->consts.mAxion;
   if ((e = cudaMemcpyAsync(h->d_masses, h->masses, sizeof(double), cudaMemcpyHostToDevice, h->stream)) != cudaSuccess) { sart_destroy(h); return cuda_fail(e, "cudaMemcpyAsync"); }
@@ -731,6 +770,7 @@ void sart_destroy(sart_handle_t* h) {
   sart_comm_destroy(h);
   cudaFree(h->table_blob); cudaFree(h->fast_blob); cudaFree(h->d_masses); cudaFree(h->d_image); cudaFree(h->d_merged);
   cudaFree(h->d_counters); cudaFree(h->d_stage); cudaFree(h->d_rep); cudaFree(h->d_mass_acc); cudaFree(h->d_queue);
+  cudaFree(h->d_desc);
   for (AccumKind k : kAllAccums) free_accum(h, k);
   cudaFreeHost(h->h_stage);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -782,6 +822,9 @@ int sart_update_setup(sart_handle_t* h, const sart_setup_t* setup) {
     h->precision = oldPrecision; h->compact = oldCompact; h->pilot_survival = oldSurvival;
     return fail(rc, "sart_update_setup failed, previous setup kept: %s", msg);
   }
+  // the band of the X-ray source's energy bin, like its reflectivity row (upload_fast)
+  if (h->accum[kBandImages].blob && old.testSource.energy != setup->testSource.energy && (rc = put_band_table(h, h->params.nEnergies)))
+    return rc;
   if (h->n_masses == 1 && h->masses_default) {
     h->masses[0] = setup->consts.mAxion;
     SART_CUDA(cudaMemcpyAsync(h->d_masses, h->masses, sizeof(double), cudaMemcpyHostToDevice, h->stream));
@@ -1173,17 +1216,19 @@ int sart_trace_words(sart_handle_t* h, size_t n, const uint32_t* words, int late
 
 // A fused image run of one axion mass in the handle's precision mode, with the parameter blocks and table views the caller
 // prepared (the handle's, or those of a scan point). The throughput kernels add into img / img2, which ft may spread over
-// replicas; the exact kernels (mode 0, and the re-trace of mode 2) add into exImg / exImg2. All add into `counters`.
+// replicas, and into the band images `band`; the exact kernels (mode 0, and the re-trace of mode 2) add into exImg / exImg2
+// and `exBand`. All add into `counters`. Band images off: band.w == exBand.w == nullptr.
 static int trace_image(sart_handle* h, const Params& P, const fast::FastParams& F, const fast::Geo32& G, fast::FastTables ft,
                        const Tables& et, uint64_t first, uint64_t n, uint64_t seed, double* img, double* img2, double* exImg,
-                       double* exImg2, sart_counters_t* counters) {
+                       double* exImg2, sart_counters_t* counters, const BandImages& band = {}, const BandImages& exBand = {}) {
   if (h->precision == 0) {
-    SART_CUDA(launch_mc_image_exact(P, et, 1, h->d_masses, first, n, seed, exImg, exImg2, counters, h->sm_count, h->stream));
+    SART_CUDA(launch_mc_image_exact(P, et, 1, h->d_masses, first, n, seed, exImg, exImg2, counters, h->sm_count, h->stream,
+                                    exBand));
     return SART_OK;
   }
   if (h->precision == 1) {
     SART_CUDA(launch_mc_image_fast(F, ft, h->masses[0], first, n, seed, img, img2, counters, h->sm_count, h->compact != 0,
-                                   h->stream));
+                                   h->stream, band));
     return SART_OK;
   }
   // the alias sampler has another ray <-> index mapping than the exact pipeline's: no re-trace
@@ -1191,11 +1236,11 @@ static int trace_image(sart_handle* h, const Params& P, const fast::FastParams& 
       [&](uint64_t done, uint64_t m, const fast::RetraceQueue& q) {
         ft.rq = q;
         return launch_mc_image_f32(F, G, ft, h->masses[0], first + done, m, seed, img, img2, counters, h->sm_count,
-                                   h->compact != 0, h->stream);
+                                   h->compact != 0, h->stream, band);
       },
       [&](uint64_t done, uint64_t, const fast::RetraceQueue& q) {
         return launch_retrace_mc_image(P, et, 1, h->d_masses, first + done, seed, q, exImg, exImg2, counters, h->sm_count,
-                                       h->stream);
+                                       h->stream, exBand);
       });
 }
 
@@ -1209,6 +1254,9 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   if (spec.blob && h->n_masses > 1) return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass");
   if (mspec.blob && h->sampler == SART_SAMPLER_ALIAS)
     return fail(SART_ERR_CONFIG, "sart_trace_mc: the per-mass spectra run the mass-scan kernels, which need the inverse-CDF sampler");
+  const Accum& bands = h->accum[kBandImages];
+  if (bands.blob && (h->n_masses > 1 || mspec.blob))
+    return fail(SART_ERR_CONFIG, "sart_trace_mc: the band images need a single axion mass and the per-mass spectra off");
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
   int rc = SART_OK;
   // A mass scan, or any run with the per-mass spectra on (one contract for every mass list, M = 1 included): the exact
@@ -1273,12 +1321,17 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
       img = h->d_rep; img2 = h->d_rep + size_t(h->n_rep) * h->rep_stride;
     }
   }
+  // band images: the throughput kernels add into their replicas, the exact kernels into the handle's arrays
   rc = trace_image(h, h->params, h->fparams, h->geo32, ft, et, first_ray, n_rays, seed, img, img2, h->d_image, h->d_image_w2,
-                   h->d_counters);
+                   h->d_counters, bands.tput_band, bands.band);
   if (rc || h->precision == 0) return rc;
   if (h->n_rep > 1)
     SART_CUDA(launch_fold_replicas(img, img2, h->n_rep, h->rep_stride, plane, h->d_image, h->d_image_w2, h->stream));
   if (spec.blob) SART_CUDA(launch_fold_spectra(spec.tput, spec.bins, spec.spec, h->stream));
+  if (bands.blob) {
+    const BandImages& r = bands.tput_band;
+    SART_CUDA(launch_fold_replicas(r.w, r.w2, int(r.repMask) + 1, r.repStride, r.repStride, bands.band.w, bands.band.w2, h->stream));
+  }
   return SART_OK;
 }
 
@@ -1317,6 +1370,21 @@ int sart_read_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum
                       double* shell_sum_w, uint64_t* shell_counts) {
   return read_accum(h, kSpectra, false, {energy_sum_w, energy_sum_w2, energy_counts, shell_sum_w, shell_counts},
                     "sart_read_spectra: no spectra enabled (sart_enable_spectra)");
+}
+
+int sart_enable_band_images(sart_handle_t* h, int n_bands, const double* edges_keV) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (n_bands < 0 || n_bands > SART_MAX_BANDS || (n_bands > 0 && !edges_keV))
+    return fail(SART_ERR_ARG, "sart_enable_band_images: need 1..%d bands and their edges, or 0 (off)", SART_MAX_BANDS);
+  for (int b = 0; n_bands > 0 && b <= n_bands; ++b)
+    if (!std::isfinite(edges_keV[b]) || edges_keV[b] < 0.0 || (b > 0 && !(edges_keV[b] > edges_keV[b - 1])))
+      return fail(SART_ERR_ARG, "sart_enable_band_images: the band edges must be finite, >= 0 and strictly ascending");
+  return set_accum(h, kBandImages, n_bands, 0.0, edges_keV);
+}
+
+int sart_read_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts) {
+  return read_accum(h, kBandImages, false, {image, image_w2, counts},
+                    "sart_read_band_images: no band images enabled (sart_enable_band_images)");
 }
 
 int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max) {

@@ -5,8 +5,9 @@
 // image and sum-of-squares image in ONE allocation followed by a small f64 area; sart_allreduce writes the counters into
 // that area as f64 (exact below 2^53) and issues ONE ncclAllReduce(sum, f64) over the whole block into a separate
 // "merged" block, so a rank's own accumulators stay untouched (no reset between steps) and the call can be repeated.
-// sart_allreduce_outputs does the same for the optional accumulators (radial histogram, spectra, per-mass spectra): the
-// ranks first agree on which are on and their shapes, then sum them into merged copies, counts as u64 and sums as f64.
+// sart_allreduce_outputs does the same for the optional accumulators (radial histogram, spectra, per-mass spectra, band
+// images): the ranks first agree on which are on and their shapes, then sum them into merged copies, counts as u64 and sums
+// as f64.
 //
 // NCCL is resolved with dlopen at first use: libsart.so has no link-time dependency on it, a process that already
 // loaded NCCL (PyTorch) shares that copy, and a host without NCCL can use everything else.
@@ -87,14 +88,16 @@ __global__ void k_pack_counters(const sart_counters_t* __restrict__ c, int nMass
 
 // sart_allreduce_outputs: what a handle has on, in the words every rank must agree on, then an error word. All ranks send
 // [d, -d] through one ncclMax, so each learns the largest and (negated) smallest value of every word. Words 0 .. kAccums - 1
-// are the bins of each accumulator (0: off).
-enum { kDescRadMax = kAccums, kDescMasses, kDescErr, kDescWords };
-static_assert(2 * kDescWords <= kCounterWords, "the descriptor travels in the counter words behind the images");
+// are the bins of each accumulator (0: off), then the bits of r_max, the number of masses and the bits of the
+// SART_MAX_BANDS + 1 band edges (0 beyond the last edge; edges are >= 0, so their bits are non-negative int64 words).
+enum { kDescRadMax = kAccums, kDescMasses, kDescEdges, kDescErr = kDescEdges + SART_MAX_BANDS + 1, kDescWords };
+static_assert(2 * kDescWords <= kDescCapacity, "the descriptor travels in sart_handle::d_desc");
 
 static void describe_outputs(const sart_handle* h, long long d[kDescWords]) {
   for (AccumKind k : kAllAccums) d[k] = h->accum[k].bins;
   std::memcpy(&d[kDescRadMax], &h->accum[kRadialHist].rmax, sizeof(long long));
   d[kDescMasses] = h->n_masses;
+  std::memcpy(&d[kDescEdges], h->accum[kBandImages].edges, (SART_MAX_BANDS + 1) * sizeof(long long));
   d[kDescErr] = 0;
 }
 
@@ -250,11 +253,8 @@ int sart_allreduce_outputs(sart_handle_t* const* handles, int n) {
     for (int k = 0; k < kDescErr; ++k)
       if (desc[size_t(i) * 2 * kDescWords + k] != desc[k])
         return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: handles 0 and %d differ in their radial histogram, spectra, "
-                                     "per-mass spectra or number of axion masses", i);
-  // the descriptor travels in the counter words behind the images: sart_allreduce rewrites them before every use
-  auto desc_dev = [](sart_handle* h) {
-    return reinterpret_cast<long long*>(h->d_image + 2 * size_t(h->n_masses) * SART_IMAGE_BINS * SART_IMAGE_BINS);
-  };
+                                     "per-mass spectra, band images or number of axion masses", i);
+  auto desc_dev = [](sart_handle* h) { return h->d_desc; };
   for (int i = 0; i < n; ++i) {
     sart_handle* h = handles[i];
     long long* d = &desc[size_t(i) * 2 * kDescWords];
@@ -295,12 +295,13 @@ int sart_allreduce_outputs(sart_handle_t* const* handles, int n) {
   const long long* hi = &red[0];
   const long long* neg_lo = &red[kDescWords];
   if (hi[kDescErr]) return fail(SART_ERR_NOMEM, "sart_allreduce_outputs: a rank could not allocate its merged copies");
-  static const char* const what[kDescErr] = {"radial histogram bins", "spectra bins", "per-mass spectra bins",
-                                             "radial histogram r_max", "number of axion masses"};
+  static const char* const what[kDescEdges] = {"radial histogram bins", "spectra bins", "per-mass spectra bins",
+                                               "number of energy bands", "radial histogram r_max", "number of axion masses"};
   for (int k = 0; k < kDescErr; ++k)
-    if (hi[k] != -neg_lo[k]) return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: the ranks differ in their %s", what[k]);
-  if (!hi[kRadialHist] && !hi[kSpectra] && !hi[kMassSpectra])
-    return fail(SART_ERR_ARG, "sart_allreduce_outputs: no radial histogram, spectra or per-mass spectra enabled");
+    if (hi[k] != -neg_lo[k])
+      return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: the ranks differ in their %s", k < kDescEdges ? what[k] : "energy band edges");
+  if (!hi[kRadialHist] && !hi[kSpectra] && !hi[kMassSpectra] && !hi[kBandImages])
+    return fail(SART_ERR_ARG, "sart_allreduce_outputs: no radial histogram, spectra or per-mass spectra enabled, and no band images");
   // the payload: counts as u64, sums as f64, of the per-mass rows only those of the M masses set, every all-reduce of every
   // handle in one group
   r = api->GroupStart();
@@ -331,6 +332,11 @@ int sart_read_merged_spectra(sart_handle_t* h, double* energy_sum_w, double* ene
                              double* shell_sum_w, uint64_t* shell_counts) {
   return read_accum(h, kSpectra, true, {energy_sum_w, energy_sum_w2, energy_counts, shell_sum_w, shell_counts},
                     "sart_read_merged_spectra: no merged spectra (call sart_allreduce_outputs first)");
+}
+
+int sart_read_merged_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts) {
+  return read_accum(h, kBandImages, true, {image, image_w2, counts},
+                    "sart_read_merged_band_images: no merged band images (call sart_allreduce_outputs first)");
 }
 
 int sart_read_merged_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,

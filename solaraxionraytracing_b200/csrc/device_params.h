@@ -105,6 +105,35 @@ __device__ __forceinline__ void spec_add(const Spectra& s, int m, int eBin, int 
 }
 #endif
 
+// Optional band images of the passed rays (sart_enable_band_images): plane b of w / w2 holds Σw / Σw² per image bin of the
+// passed rays whose energy lies in band b, n[b] their number (every passed ray of the band, in the image or not).
+// band[i] is the band of tabulated energy i (i = nEnergies: the X-ray source), 0xff for none; built on the host, so the
+// kernels do no search. A block adds its sums into replica (block & repMask), repStride elements after replica 0; repMask 0
+// = the arrays themselves (the exact kernels). The counts are never replicated. w == nullptr: off. Passed to the kernels
+// that fill them as a parameter of its own, so that the parameter blocks of every other kernel keep their layout.
+struct BandImages {
+  double* w;                   // [nBands][256 * 256]
+  double* w2;
+  unsigned long long* n;       // [nBands]
+  const uint8_t* band;         // [nEnergies + 1]
+  uint32_t repStride, repMask;
+  int32_t nBands, pad;
+};
+constexpr uint8_t kNoBand = 0xff;
+
+#if defined(__CUDACC__)
+// A passed ray of energy index eIdx into the handle's band images (the exact kernels: one atomic per quantity).
+__device__ __forceinline__ void band_add(const BandImages& b, int eIdx, int bin, double w) {
+  const unsigned k = __ldg(b.band + eIdx);
+  if (k == kNoBand) return;
+  atomicAdd(b.n + k, 1ull);
+  if (bin < 0) return;
+  const uint32_t at = k * uint32_t(SART_IMAGE_BINS * SART_IMAGE_BINS) + uint32_t(bin);
+  atomicAdd(b.w + at, w);
+  atomicAdd(b.w2 + at, w * w);
+}
+#endif
+
 // Table pointers (device memory).
 struct Tables {
   const double* energies;

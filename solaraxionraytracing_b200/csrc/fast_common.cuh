@@ -378,6 +378,53 @@ struct ImageSinkT {
 };
 using ImageSink = ImageSinkT<true>;
 
+// Sink of the band-image kernel variants (sart_enable_band_images): the generic sink, with the radial histogram and the
+// spectra checked at run time, plus the band images B (device_params.h: BandImages; here their replicas, bandRep this block's
+// replica) and the block's per-band counts bandN in shared memory, which the kernel flushes once at its end. A derived sink,
+// so that ImageSinkT, and every kernel variant built on it, stays what it was before the band images existed.
+struct BandImageSink : ImageSinkT<true, true> {
+  const BandImages& B;
+  unsigned int* bandN;
+  uint32_t bandRep;
+  __device__ __forceinline__ void hit(const RayResult& h) {
+    ImageSinkT<true, true>::hit(h);
+    const double wd = h.wPre * h.wPost;   // the weight ImageSinkT::hit tested
+    if (h.windowMiss || wd == 0.0) return;
+    const unsigned k = __ldg(B.band + h.eIdx);
+    if (k == kNoBand) return;
+    atomicAdd(bandN + k, 1u);
+    if (h.bin < 0) return;
+    const uint32_t at = bandRep + k * uint32_t(SART_IMAGE_BINS * SART_IMAGE_BINS) + uint32_t(h.bin);
+    atomicAdd(B.w + at, wd);
+    atomicAdd(B.w2 + at, wd * wd);
+  }
+};
+
+// The block's per-band counts of the band-image kernel variants (BandImageSink::bandN): shared memory, zeroed by the threads
+// 0 .. SART_MAX_BANDS - 1 before the kernel's first __syncthreads, added to the handle's counts once at the end of the
+// kernel (one global atomic per band and block instead of one per ray). nullptr without band images.
+template <bool kBands>
+__device__ __forceinline__ unsigned int* band_counts() {
+  if constexpr (kBands) {
+    __shared__ unsigned int n[SART_MAX_BANDS];
+    if (threadIdx.x < SART_MAX_BANDS) n[threadIdx.x] = 0u;
+    return n;
+  } else {
+    return nullptr;
+  }
+}
+__device__ __forceinline__ uint32_t band_replica(const BandImages& B) { return (blockIdx.x & B.repMask) * B.repStride; }
+// The sink of a fused kernel body shared by a variant without band images (kBands = false: `sink` itself) and one with them.
+template <bool kBands, class Sink>
+__device__ __forceinline__ auto with_bands(const Sink& sink, const BandImages& B, unsigned int* bandN) {
+  if constexpr (kBands) return BandImageSink{sink, B, bandN, band_replica(B)};
+  else return sink;
+}
+__device__ __forceinline__ void band_counts_flush(const BandImages& B, const unsigned int* n) {
+  __syncthreads();
+  if (threadIdx.x < unsigned(B.nBands) && n[threadIdx.x]) atomicAdd(B.n + threadIdx.x, (unsigned long long)n[threadIdx.x]);
+}
+
 // ---- axion-mass scan: the part shared by the FP64-algebra and the FP32 tracing --------------------------------
 // Per-mass spectra of the mass-scan kernels (sart_enable_mass_spectra), in FastTables::spec: accumulators laid out like
 // the image's, [bin][SART_MAX_MASSES] (eW, eW2: bin = energy index, nEnergies for the X-ray source) and

@@ -208,10 +208,13 @@ struct MassCounters {
   double sum_w, sum_w2, sum_x, sum_y, sum_r;
 };
 
-// One ray of the fused run: sample, trace, weight for every axion mass, histogram (rt:1736-2221 + 818-842).
+// One ray of the fused run: sample, trace, weight for every axion mass, histogram (rt:1736-2221 + 818-842). kBands: the
+// passed rays of the first mass also go to the band images B (sart_enable_band_images); false compiles them out.
+template <bool kBands>
 __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, int nMasses, const double* __restrict__ masses,
                                              uint64_t seed, uint64_t ray, double* __restrict__ image,
-                                             double* __restrict__ imageW2, BlockCounters* bc, MassCounters* mc, ThreadSums& ts) {
+                                             double* __restrict__ imageW2, const BandImages& B, BlockCounters* bc,
+                                             MassCounters* mc, ThreadSums& ts) {
   const double step = (P.chipCX * 2.0 - 0.0) / double(SART_IMAGE_BINS);  // (stop - start)/rows rt:828-830
   const double stepY = (P.chipCY * 2.0 - 0.0) / double(SART_IMAGE_BINS);
   V3 O, E;
@@ -272,6 +275,11 @@ __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, i
     // spectra: the first mass (sart_enable_spectra) or every mass into its own row (sart_enable_mass_spectra: eRow != 0);
     // the X-ray source's rays carry no table index and go to bin nEnergies
     if (T.spec.eW && (m == 0 || T.spec.eRow)) spec_add(T.spec, m, g.eIdx >= 0 ? g.eIdx : P.nEnergies, g.shell, f.w);
+    // band images (single mass only): the same energy index, the image bin of plane 0
+    if (kBands && m == 0) {
+      const bool inImage = cx >= 0.0 && cx < double(SART_IMAGE_BINS) && cy >= 0.0 && cy < double(SART_IMAGE_BINS);
+      band_add(B, g.eIdx >= 0 ? g.eIdx : P.nEnergies, inImage ? int(cy) * SART_IMAGE_BINS + int(cx) : -1, f.w);
+    }
   }
 }
 
@@ -279,11 +287,12 @@ __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, i
 #define SART_EXACT_MINBLOCKS 6   // 85 registers instead of 108: 24 instead of 16 warps per SM for this latency-bound kernel (+5 %; 8 is slower)
 #endif
 // `list` != nullptr: trace the rays first + list[j], j < min(*listCount, listCap), instead of first + [0, nRays).
-__global__ void __launch_bounds__(128, SART_EXACT_MINBLOCKS)
-k_trace_mc_image(const __grid_constant__ Params P, const __grid_constant__ Tables T, int nMasses,
-                 const double* __restrict__ masses, uint64_t first, uint64_t nRays, uint64_t seed,
-                 const uint32_t* __restrict__ list, const uint32_t* __restrict__ listCount, uint32_t listCap,
-                 double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+template <bool kBands>
+__device__ __forceinline__ void mc_image(const Params& P, const Tables& T, int nMasses, const double* __restrict__ masses,
+                                         uint64_t first, uint64_t nRays, uint64_t seed, const uint32_t* __restrict__ list,
+                                         const uint32_t* __restrict__ listCount, uint32_t listCap, double* __restrict__ image,
+                                         double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                                         const BandImages& B) {
   extern __shared__ unsigned char smem_raw[];
   BlockCounters* bc = reinterpret_cast<BlockCounters*>(smem_raw);
   MassCounters* mc = reinterpret_cast<MassCounters*>(smem_raw + sizeof(BlockCounters));
@@ -304,7 +313,7 @@ k_trace_mc_image(const __grid_constant__ Params P, const __grid_constant__ Table
   for (uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < total; i += stride) {
     const uint64_t ray = first + (listMode ? uint64_t(list[i]) : i);
     if (!listMode) ++ts.n_rays;
-    mc_image_ray(P, T, nMasses, masses, seed, ray, image, imageW2, bc, mc, ts);
+    mc_image_ray<kBands>(P, T, nMasses, masses, seed, ray, image, imageW2, B, bc, mc, ts);
   }
   if (listMode && blockIdx.x == 0 && threadIdx.x == 0)
     for (int m = 0; m < nMasses; ++m) atomicAdd(reinterpret_cast<unsigned long long*>(&counters[m].n_retraced), (unsigned long long)total);
@@ -348,6 +357,23 @@ k_trace_mc_image(const __grid_constant__ Params P, const __grid_constant__ Table
     atomicAdd(&c->sum_y, mc[m].sum_y);
     atomicAdd(&c->sum_r, mc[m].sum_r);
   }
+}
+
+__global__ void __launch_bounds__(128, SART_EXACT_MINBLOCKS)
+k_trace_mc_image(const __grid_constant__ Params P, const __grid_constant__ Tables T, int nMasses,
+                 const double* __restrict__ masses, uint64_t first, uint64_t nRays, uint64_t seed,
+                 const uint32_t* __restrict__ list, const uint32_t* __restrict__ listCount, uint32_t listCap,
+                 double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+  mc_image<false>(P, T, nMasses, masses, first, nRays, seed, list, listCount, listCap, image, imageW2, counters, BandImages{});
+}
+// The same with the band images B (a kernel of its own: the check inside the per-ray code made mode 0 2 % slower).
+__global__ void __launch_bounds__(128, SART_EXACT_MINBLOCKS)
+k_trace_mc_image_bands(const __grid_constant__ Params P, const __grid_constant__ Tables T, int nMasses,
+                       const double* __restrict__ masses, uint64_t first, uint64_t nRays, uint64_t seed,
+                       const uint32_t* __restrict__ list, const uint32_t* __restrict__ listCount, uint32_t listCap,
+                       double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                       const __grid_constant__ BandImages B) {
+  mc_image<true>(P, T, nMasses, masses, first, nRays, seed, list, listCount, listCap, image, imageW2, counters, B);
 }
 
 // ---- CDF build rt:2679-2705 -------------------------------------------------------------------------------
@@ -426,31 +452,41 @@ cudaError_t launch_mc_rays_exact(const Params& P, const Tables& T, double mAxion
 
 cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                   uint64_t nRays, uint64_t seed, double* image, double* imageW2,
-                                  sart_counters_t* counters, int smCount, cudaStream_t s) {
+                                  sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands) {
   if (nRays == 0) return cudaSuccess;
   const int block = 128;
   const size_t smem = sizeof(BlockCounters) + size_t(nMasses) * sizeof(MassCounters);
   unsigned grid = 0;   // one resident wave; the grid-stride loop covers the rest
-  const cudaError_t e = grid_size(k_trace_mc_image, block, smem, nRays, smCount, 0, &grid);
+  const cudaError_t e = bands.w ? grid_size(k_trace_mc_image_bands, block, smem, nRays, smCount, 0, &grid)
+                                 : grid_size(k_trace_mc_image, block, smem, nRays, smCount, 0, &grid);
   if (e != cudaSuccess) return e;
-  k_trace_mc_image<<<grid, block, smem, s>>>(P, T, nMasses, masses, first, nRays, seed, nullptr, nullptr, 0u, image, imageW2,
-                                             counters);
+  if (bands.w)
+    k_trace_mc_image_bands<<<grid, block, smem, s>>>(P, T, nMasses, masses, first, nRays, seed, nullptr, nullptr, 0u, image,
+                                                     imageW2, counters, bands);
+  else
+    k_trace_mc_image<<<grid, block, smem, s>>>(P, T, nMasses, masses, first, nRays, seed, nullptr, nullptr, 0u, image, imageW2,
+                                               counters);
   return cudaGetLastError();
 }
 
 // ---- re-trace launchers (fixed grids: the list length lives on the device) -------------------------------------
 cudaError_t launch_retrace_mc_image(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                     uint64_t seed, const fast::RetraceQueue& q, double* image, double* imageW2,
-                                    sart_counters_t* counters, int smCount, cudaStream_t s) {
+                                    sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands) {
   const int block = 128;
   const size_t smem = sizeof(BlockCounters) + size_t(nMasses) * sizeof(MassCounters);
   int perSM = 0;
-  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image, block, smem);
+  cudaError_t e = bands.w ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image_bands, block, smem)
+                           : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image, block, smem);
   if (e != cudaSuccess) return e;
   if (perSM < 1) perSM = 1;
   // one resident wave (the list length lives on the device): latency-bound FP64 code wants every warp slot it can get
-  k_trace_mc_image<<<unsigned(smCount * perSM), block, smem, s>>>(P, T, nMasses, masses, first, 0, seed, q.list, q.count, q.cap, image,
-                                                                 imageW2, counters);
+  if (bands.w)
+    k_trace_mc_image_bands<<<unsigned(smCount * perSM), block, smem, s>>>(P, T, nMasses, masses, first, 0, seed, q.list, q.count,
+                                                                         q.cap, image, imageW2, counters, bands);
+  else
+    k_trace_mc_image<<<unsigned(smCount * perSM), block, smem, s>>>(P, T, nMasses, masses, first, 0, seed, q.list, q.count, q.cap,
+                                                                   image, imageW2, counters);
   return cudaGetLastError();
 }
 cudaError_t launch_retrace_mc_rays(const Params& P, const Tables& T, double mAxion, uint64_t first, size_t n, uint64_t seed,

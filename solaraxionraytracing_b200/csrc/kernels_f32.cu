@@ -22,12 +22,14 @@ namespace fast {
 // ---- fused kernel ---------------------------------------------------------------------------------------------
 // A ray of stage A that is uncertain (rec.unc) goes to the re-trace queue whatever its code; stage B does the same at its
 // own exits. A launch has at most kMaxRaysPerLaunch rays (fast_params.h), so the queue entry (ray index - first) fits 32 bits.
-// kSpectra: the generic variant that also fills the spectra (sart_enable_spectra; fast_common.cuh: ImageSinkT).
-template <bool kWolter, bool kPlain, bool kAlias, bool kMargins, bool kSpectra = false>
-__global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
-k_trace_mc_f32(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G, const __grid_constant__ FastTables T,
-               double mAxion2, uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image,
-               double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+// kSpectra: the generic variant that also fills the spectra (sart_enable_spectra; fast_common.cuh: ImageSinkT). kBands: the
+// generic variant that also fills the band images B (sart_enable_band_images), the spectra and the radial histogram checked at
+// run time (k_trace_mc_f32_bands).
+template <bool kWolter, bool kPlain, bool kAlias, bool kMargins, bool kSpectra, bool kBands>
+__device__ __forceinline__ void f32_fused(const FastParams& P, const Geo32& G, const FastTables& T, double mAxion2, uint64_t first,
+                                          uint64_t nRays, const PhiloxKeys& K, double* __restrict__ image,
+                                          double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                                          const BandImages& B) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem32 S;
   unsigned char* tail;
@@ -35,13 +37,15 @@ k_trace_mc_f32(const __grid_constant__ FastParams P, const __grid_constant__ Geo
   WarpCounters* wc = reinterpret_cast<WarpCounters*>(tail);
   smem_fill32<kAlias>(P, T, S);
   for (int i = threadIdx.x; i < kWarps32 * int(sizeof(WarpCounters) / 4); i += kBlock32) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
+  unsigned int* bandN = band_counts<kBands>();
   __syncthreads();
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   unsigned int nPassed = 0, nTill = 0, nIter = 0;
   double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
   const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
-  ImageSinkT<!kPlain, kSpectra> sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
+  auto sink = with_bands<kBands>(ImageSinkT<!kPlain, kSpectra>{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2,
+                                                                 sumX, sumY, sumR}, B, bandN);
   const uint64_t stride = uint64_t(gridDim.x) * kBlock32;
   // 32-bit trip count + running 64-bit ray index: 5 loop instructions per ray instead of 12 (nRays <= kMaxRaysPerLaunch,
   // so the count fits)
@@ -70,6 +74,23 @@ k_trace_mc_f32(const __grid_constant__ FastParams P, const __grid_constant__ Geo
   }
   __syncwarp();
   if (lane == 0) flush_counters(counters, wc[warp], nIter, nPassed, nTill, sumW, sumW2, sumX, sumY, sumR);
+  if (kBands) band_counts_flush(B, bandN);
+}
+template <bool kWolter, bool kPlain, bool kAlias, bool kMargins, bool kSpectra = false>
+__global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
+k_trace_mc_f32(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G, const __grid_constant__ FastTables T,
+               double mAxion2, uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image,
+               double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+  f32_fused<kWolter, kPlain, kAlias, kMargins, kSpectra, false>(P, G, T, mAxion2, first, nRays, K, image, imageW2, counters,
+                                                                BandImages{});
+}
+template <bool kWolter, bool kAlias, bool kMargins>
+__global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
+k_trace_mc_f32_bands(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G, const __grid_constant__ FastTables T,
+                     double mAxion2, uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K,
+                     double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                     const __grid_constant__ BandImages B) {
+  f32_fused<kWolter, false, kAlias, kMargins, true, true>(P, G, T, mAxion2, first, nRays, K, image, imageW2, counters, B);
 }
 
 // ---- fused kernel with warp-level compaction between stage A and stage B (see kernels_fast.cu) ----------------
@@ -164,6 +185,96 @@ k_trace_mc_f32_compact(const __grid_constant__ FastParams P, const __grid_consta
   if (lane == 0) flush_counters(counters, wc[warp], nIter, nPassed, nTill, sumW, sumW2, sumX, sumY, sumR);
 }
 
+// The same with the band images B, the generic kind (k_trace_mc_f32_bands). Its own copy of the kernel above: the plain variants
+// of that kernel, compiled from a body shared with this one, came out with another register allocation than before the band
+// images existed, and a run without them is to run the code it ran before.
+template <bool kWolter, bool kAlias, bool kMargins>
+__global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
+k_trace_mc_f32_compact_bands(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G,
+                             const __grid_constant__ FastTables T, double mAxion2, uint64_t first, uint64_t nRays,
+                             const __grid_constant__ PhiloxKeys K, double* __restrict__ image, double* __restrict__ imageW2,
+                             sart_counters_t* __restrict__ counters, const __grid_constant__ BandImages B) {
+  constexpr bool kPlain = false;
+  extern __shared__ __align__(16) unsigned char smem[];
+  Smem32 S;
+  unsigned char* tail;
+  smem_layout32<kAlias>(P, smem, S, tail);
+  WarpCounters* wc = reinterpret_cast<WarpCounters*>(tail);
+  WarpQueue32* queues = reinterpret_cast<WarpQueue32*>(tail + kWarps32 * sizeof(WarpCounters));
+  smem_fill32<kAlias>(P, T, S);
+  for (int i = threadIdx.x; i < kWarps32 * int(sizeof(WarpCounters) / 4); i += kBlock32) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
+  unsigned int* bandN = band_counts<true>();
+  __syncthreads();
+
+  constexpr unsigned kFull = 0xffffffffu;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  WarpQueue32& Q = queues[warp];
+  unsigned int nPassed = 0, nTill = 0, nIter = 0;
+  double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
+  const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
+  BandImageSink sink{{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR}, B, bandN,
+                     band_replica(B)};
+  const uint64_t stride = uint64_t(gridDim.x) * kBlock32;
+  uint64_t base = uint64_t(blockIdx.x) * kBlock32 + (threadIdx.x & ~31);
+  const bool solar = kPlain || !P.testXray;
+  int qn = 0;
+  for (;;) {
+    while (qn <= kQueue32 - 32 && base < nRays) {
+      const uint64_t i = base + lane;
+      base += stride;
+      Rec32 rec;
+      int code = SART_N_EXIT_CODES;
+      if (i < nRays) {
+        Head32 hd;
+        stage_a32_head<kPlain, true, kAlias>(P, T, S, K, first + i, hd);
+        rec.id = uint32_t(i);
+        code = stage_a32<kWolter, false, kPlain, true, kAlias, kMargins>(P, G, T, S, hd, rec);
+        ++nIter;
+        if (code >= 0 && !(kMargins && rec.unc && sink.defer(rec.id))) sink.fail(code);
+      }
+      const unsigned m = __ballot_sync(kFull, code < 0);
+      if (code < 0) {
+        const int pos = qn + __popc(m & ((1u << lane) - 1u));
+        Q.x0[pos] = rec.x0; Q.y0[pos] = rec.y0; Q.tx[pos] = rec.tx; Q.ty[pos] = rec.ty; Q.rho0[pos] = rec.rho0;
+        Q.path2[pos] = rec.path2;
+        Q.meta[pos] = rec.hitLayer | ((solar ? rec.rIdx : rec.eIdx) << 8) | (rec.clamped ? (1 << 30) : 0) | (rec.unc ? (1 << 31) : 0);
+        Q.we[pos] = rec.we;
+        Q.id[pos] = rec.id;
+      }
+      qn += __popc(m);
+    }
+    if (qn == 0) break;
+    __syncwarp();
+    const int take = qn < 32 ? qn : 32;
+    if (lane < take) {
+      const int pos = qn - take + lane;
+      Rec32 rec;
+      rec.x0 = Q.x0[pos]; rec.y0 = Q.y0[pos]; rec.tx = Q.tx[pos]; rec.ty = Q.ty[pos]; rec.rho0 = Q.rho0[pos];
+      rec.path2 = Q.path2[pos];
+      const int meta = Q.meta[pos];
+      rec.hitLayer = meta & 0xff; rec.eIdx = (meta >> 8) & 0x3fffff; rec.clamped = (meta >> 30) & 1; rec.unc = meta < 0;
+      rec.id = Q.id[pos];
+      rec.bud = solar ? (0.0015f + float(rec.eIdx) * 0.0005f) : 1.0f;   // rs of the emission shell (rec.eIdx still holds it)
+      if (solar) rec.eIdx = energy_index<kAlias>(P, T, rec.eIdx, Q.we[pos], rec.clamped);
+      finish32<kWolter, kPlain, false, kMargins>(P, G, T, S, -1, rec, sink);
+    }
+    qn -= take;
+    __syncwarp();
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    nPassed += __shfl_down_sync(kFull, nPassed, o);
+    nTill += __shfl_down_sync(kFull, nTill, o);
+    nIter += __shfl_down_sync(kFull, nIter, o);
+    sumW += __shfl_down_sync(kFull, sumW, o);
+    sumW2 += __shfl_down_sync(kFull, sumW2, o);
+    sumX += __shfl_down_sync(kFull, sumX, o);
+    sumY += __shfl_down_sync(kFull, sumY, o);
+    sumR += __shfl_down_sync(kFull, sumR, o);
+  }
+  __syncwarp();
+  if (lane == 0) flush_counters(counters, wc[warp], nIter, nPassed, nTill, sumW, sumW2, sumX, sumY, sumR);
+  band_counts_flush(B, bandN);
+}
 // ---- axion-mass scan with FP32 tracing (the per-mass weighting is fast_common.cuh's mass_scan_loop) --------------
 template <bool kWolter, bool kMargins, int kPer, bool kSpectra>
 __device__ __forceinline__ void f32_masses(const FastParams& P, const Geo32& G, const FastTables& T,
@@ -214,17 +325,41 @@ k_trace_mc_f32_masses_spectra(const __grid_constant__ FastParams P, const __grid
 // One launch of at most fast::kMaxRaysPerLaunch rays (api.cu cuts longer runs).
 cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T, double mAxion,
                                 uint64_t first, uint64_t nRays, uint64_t seed, double* image, double* imageW2,
-                                sart_counters_t* counters, int smCount, bool compact, cudaStream_t s) {
+                                sart_counters_t* counters, int smCount, bool compact, cudaStream_t s, const BandImages& bands) {
   if (nRays == 0) return cudaSuccess;
   const LaunchVariant v = launch_variant(P, T);
-  // the plain-run kernels compile the radial histogram and the spectra out
-  const bool plain = v.plain && !T.rad.w && !T.spec.eW;
+  // the plain-run kernels compile the radial histogram, the spectra and the band images out
+  const bool plain = v.plain && !T.rad.w && !T.spec.eW && !bands.w;
   const size_t smem = fast::smem_bytes32(P, fast::kWarps32, v.alias) + (compact ? fast::kWarps32 * sizeof(fast::WarpQueue32) : 0);
+  // variant 0: inverse-CDF sampler, pure FP32; 1: inverse-CDF sampler with the margin tests (re-trace queue attached); 2: alias
+  // sampler (no re-trace: its ray <-> index mapping is not the exact pipeline's)
+  const int variant = v.alias ? 2 : (v.margins ? 1 : 0);
+  auto run = [&](auto kern, auto... bandArg) {
+    cudaError_t e = fast::set_smem(kern, smem);
+    if (e != cudaSuccess) return e;
+    unsigned grid = 0;
+    if ((e = grid_size(kern, fast::kBlock32, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
+    kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, first, nRays, philox_round_keys(seed), image, imageW2, counters,
+                                            bandArg...);
+    return cudaGetLastError();
+  };
+  if (getenv("SART_DEBUG"))
+    fprintf(stderr, "[sart] k_trace_mc_f32 compact=%d wolter=%d plain=%d alias=%d bands=%d (sampler=%d ra=%p ea=%p) smem=%zu\n",
+            int(compact), int(v.wolter), int(plain), int(v.alias), bands.nBands, T.sampler, (const void*)T.radiusAlias,
+            (const void*)T.energyAlias, smem);
+  if (bands.w) {   // the generic kind with the band images: the radial histogram and the spectra are checked at run time
+    using KernB = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, uint64_t, uint64_t, PhiloxKeys, double*,
+                           double*, sart_counters_t*, BandImages);
+    // [compact][wolter][variant]
+#define SART_ROW(K, W) {fast::K<W, false, false>, fast::K<W, false, true>, fast::K<W, true, false>}
+    static const KernB table[2][2][3] = {{SART_ROW(k_trace_mc_f32_bands, false), SART_ROW(k_trace_mc_f32_bands, true)},
+                                         {SART_ROW(k_trace_mc_f32_compact_bands, false), SART_ROW(k_trace_mc_f32_compact_bands, true)}};
+#undef SART_ROW
+    return run(table[compact ? 1 : 0][v.wolter ? 1 : 0][variant], bands);
+  }
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, uint64_t, uint64_t, PhiloxKeys, double*, double*,
                         sart_counters_t*);
-  // [compact][wolter][kind][variant]; kind 0: generic, 1: plain, 2: generic with the spectra; variant 0: inverse-CDF sampler,
-  // pure FP32; 1: inverse-CDF sampler with the margin tests (re-trace queue attached); 2: alias sampler (no re-trace: its
-  // ray <-> index mapping is not the exact pipeline's)
+  // [compact][wolter][kind][variant]; kind 0: generic, 1: plain, 2: generic with the spectra
 #define SART_ROW(K, W, PL, SP) {fast::K<W, PL, false, false, SP>, fast::K<W, PL, false, true, SP>, fast::K<W, PL, true, false, SP>}
 #define SART_KINDS(K, W) {SART_ROW(K, W, false, false), SART_ROW(K, W, true, false), SART_ROW(K, W, false, true)}
   static const Kern table[2][2][3][3] = {{SART_KINDS(k_trace_mc_f32, false), SART_KINDS(k_trace_mc_f32, true)},
@@ -232,16 +367,7 @@ cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G,
 #undef SART_KINDS
 #undef SART_ROW
   const int kind = plain ? 1 : (T.spec.eW ? 2 : 0);
-  const Kern kern = table[compact ? 1 : 0][v.wolter ? 1 : 0][kind][v.alias ? 2 : (v.margins ? 1 : 0)];
-  if (getenv("SART_DEBUG"))
-    fprintf(stderr, "[sart] k_trace_mc_f32 compact=%d wolter=%d plain=%d alias=%d (sampler=%d ra=%p ea=%p) smem=%zu\n", int(compact),
-            int(v.wolter), int(plain), int(v.alias), T.sampler, (const void*)T.radiusAlias, (const void*)T.energyAlias, smem);
-  cudaError_t e = fast::set_smem(kern, smem);
-  if (e != cudaSuccess) return e;
-  unsigned grid = 0;
-  if ((e = grid_size(kern, fast::kBlock32, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
-  kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, first, nRays, philox_round_keys(seed), image, imageW2, counters);
-  return cudaGetLastError();
+  return run(table[compact ? 1 : 0][v.wolter ? 1 : 0][kind][variant]);
 }
 
 cudaError_t launch_mc_image_f32_masses(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T,

@@ -534,11 +534,12 @@ __device__ __forceinline__ void trace_one(const FastParams& P, const FastTables&
 }
 
 // ---- fused kernel ---------------------------------------------------------------------------------------------
-template <bool kWolter>
-__global__ void __launch_bounds__(kBlockF, 1)
-k_trace_mc_fast(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
-                uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
-                double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+// kBands: the variant that also fills the band images B (sart_enable_band_images; fast_common.cuh: ImageSinkT).
+template <bool kWolter, bool kBands>
+__device__ __forceinline__ void fast_fused(const FastParams& P, const FastTables& T, double mAxion2, uint64_t first,
+                                           uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                                           double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                                           const BandImages& B) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem S;
   unsigned char* tail;
@@ -546,6 +547,7 @@ k_trace_mc_fast(const __grid_constant__ FastParams P, const __grid_constant__ Fa
   WarpCounters* wc = reinterpret_cast<WarpCounters*>(tail);
   smem_fill(P, T, S);
   for (int i = threadIdx.x; i < kWarpsF * int(sizeof(WarpCounters) / 4); i += kBlockF) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
+  unsigned int* bandN = band_counts<kBands>();
   __syncthreads();
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -553,7 +555,8 @@ k_trace_mc_fast(const __grid_constant__ FastParams P, const __grid_constant__ Fa
   double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
 
   const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
-  ImageSink sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
+  auto sink = with_bands<kBands>(ImageSink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR},
+                                  B, bandN);
   const uint64_t stride = uint64_t(gridDim.x) * kBlockF;
   for (uint64_t i = uint64_t(blockIdx.x) * kBlockF + threadIdx.x; i < nRays; i += stride) {
     ++nIter;
@@ -588,6 +591,21 @@ k_trace_mc_fast(const __grid_constant__ FastParams P, const __grid_constant__ Fa
     atomicAdd(&c->sum_w, sumW); atomicAdd(&c->sum_w2, sumW2);
     atomicAdd(&c->sum_x, sumX); atomicAdd(&c->sum_y, sumY); atomicAdd(&c->sum_r, sumR);
   }
+  if (kBands) band_counts_flush(B, bandN);
+}
+template <bool kWolter>
+__global__ void __launch_bounds__(kBlockF, 1)
+k_trace_mc_fast(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
+                uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+  fast_fused<kWolter, false>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, BandImages{});
+}
+template <bool kWolter>
+__global__ void __launch_bounds__(kBlockF, 1)
+k_trace_mc_fast_bands(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
+                      uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                      double* __restrict__ imageW2, sart_counters_t* __restrict__ counters, const __grid_constant__ BandImages B) {
+  fast_fused<kWolter, true>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, B);
 }
 
 // ---- fused kernel with warp-level compaction ------------------------------------------------------------------
@@ -601,11 +619,11 @@ struct WarpQueue {
   int meta[kQueue];   // hitLayer | eIdx << 8 | clamped << 30
 };
 
-template <bool kWolter>
-__global__ void __launch_bounds__(kBlockF, 1)
-k_trace_mc_fast_compact(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
-                        uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
-                        double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+template <bool kWolter, bool kBands>
+__device__ __forceinline__ void fast_fused_compact(const FastParams& P, const FastTables& T, double mAxion2, uint64_t first,
+                                                   uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                                                   double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                                                   const BandImages& B) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem S;
   unsigned char* tail;
@@ -614,6 +632,7 @@ k_trace_mc_fast_compact(const __grid_constant__ FastParams P, const __grid_const
   WarpQueue* queues = reinterpret_cast<WarpQueue*>(tail + kWarpsF * sizeof(WarpCounters));
   smem_fill(P, T, S);
   for (int i = threadIdx.x; i < kWarpsF * int(sizeof(WarpCounters) / 4); i += kBlockF) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
+  unsigned int* bandN = band_counts<kBands>();
   __syncthreads();
 
   constexpr unsigned kFull = 0xffffffffu;
@@ -623,7 +642,8 @@ k_trace_mc_fast_compact(const __grid_constant__ FastParams P, const __grid_const
   double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
   const uint64_t stride = uint64_t(gridDim.x) * kBlockF;
   const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
-  ImageSink sink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR};
+  auto sink = with_bands<kBands>(ImageSink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR},
+                                  B, bandN);
   uint64_t base = uint64_t(blockIdx.x) * kBlockF + (threadIdx.x & ~31);   // warp-uniform
   int qn = 0;                                                              // warp-uniform queue fill
   for (;;) {
@@ -683,6 +703,22 @@ k_trace_mc_fast_compact(const __grid_constant__ FastParams P, const __grid_const
     atomicAdd(&c->sum_w, sumW); atomicAdd(&c->sum_w2, sumW2);
     atomicAdd(&c->sum_x, sumX); atomicAdd(&c->sum_y, sumY); atomicAdd(&c->sum_r, sumR);
   }
+  if (kBands) band_counts_flush(B, bandN);
+}
+template <bool kWolter>
+__global__ void __launch_bounds__(kBlockF, 1)
+k_trace_mc_fast_compact(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
+                        uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                        double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+  fast_fused_compact<kWolter, false>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, BandImages{});
+}
+template <bool kWolter>
+__global__ void __launch_bounds__(kBlockF, 1)
+k_trace_mc_fast_compact_bands(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
+                              uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                              double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                              const __grid_constant__ BandImages B) {
+  fast_fused_compact<kWolter, true>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, B);
 }
 
 // ---- fused kernel, axion-mass scan ---------------------------------------------------------------------------
@@ -751,18 +787,23 @@ size_t smem_bytes(const FastParams& P, int nWarps = kWarps) {
 
 cudaError_t launch_mc_image_fast(const fast::FastParams& P, const fast::FastTables& T, double mAxion, uint64_t first,
                                  uint64_t nRays, uint64_t seed, double* image, double* imageW2,
-                                 sart_counters_t* counters, int smCount, bool compact, cudaStream_t s) {
+                                 sart_counters_t* counters, int smCount, bool compact, cudaStream_t s, const BandImages& bands) {
   if (nRays == 0) return cudaSuccess;
   const bool wolter = launch_variant(P, T).wolter;
   const size_t smem = fast::smem_bytes(P, fast::kWarpsF) + (compact ? fast::kWarpsF * sizeof(fast::WarpQueue) : 0);
-  auto kern = compact ? (wolter ? fast::k_trace_mc_fast_compact<true> : fast::k_trace_mc_fast_compact<false>)
-                      : (wolter ? fast::k_trace_mc_fast<true> : fast::k_trace_mc_fast<false>);
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-  if (e != cudaSuccess) return e;
-  unsigned grid = 0;
-  if ((e = grid_size(kern, fast::kBlockF, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
-  kern<<<grid, fast::kBlockF, smem, s>>>(P, T, mAxion * mAxion, first, nRays, seed, image, imageW2, counters);
-  return cudaGetLastError();
+  auto run = [&](auto kern, auto... bandArg) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return e;
+    unsigned grid = 0;
+    if ((e = grid_size(kern, fast::kBlockF, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
+    kern<<<grid, fast::kBlockF, smem, s>>>(P, T, mAxion * mAxion, first, nRays, seed, image, imageW2, counters, bandArg...);
+    return cudaGetLastError();
+  };
+  if (bands.w)
+    return run(compact ? (wolter ? fast::k_trace_mc_fast_compact_bands<true> : fast::k_trace_mc_fast_compact_bands<false>)
+                       : (wolter ? fast::k_trace_mc_fast_bands<true> : fast::k_trace_mc_fast_bands<false>), bands);
+  return run(compact ? (wolter ? fast::k_trace_mc_fast_compact<true> : fast::k_trace_mc_fast_compact<false>)
+                     : (wolter ? fast::k_trace_mc_fast<true> : fast::k_trace_mc_fast<false>));
 }
 
 cudaError_t launch_mc_image_fast_masses(const fast::FastParams& P, const fast::FastTables& T, int nMasses,

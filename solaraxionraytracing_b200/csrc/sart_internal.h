@@ -51,6 +51,9 @@ inline size_t merged_words(int nMasses) {
   return size_t(nMasses) * (2 * size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS + size_t(kCounterWords));
 }
 
+// sart_allreduce_outputs (comm.cu): int64 words of the descriptor the ranks exchange, in sart_handle::d_desc
+constexpr int kDescCapacity = 64;
+
 // Bump allocator over one device buffer: every piece starts on a 256-byte boundary. Over a null base it only measures, so a
 // layout is written once and run twice: over nullptr to size the buffer, then over the allocation to hand out its pointers.
 struct Carve {
@@ -64,25 +67,30 @@ struct Carve {
 };
 
 // The optional accumulators of the passed rays, each switched on and off by its own entry point: the radial histogram
-// (sart_enable_radial_hist), the spectra (sart_enable_spectra) and the per-mass spectra (sart_enable_mass_spectra).
-enum AccumKind { kRadialHist, kSpectra, kMassSpectra, kAccums };
-constexpr AccumKind kAllAccums[kAccums] = {kRadialHist, kSpectra, kMassSpectra};
+// (sart_enable_radial_hist), the spectra (sart_enable_spectra), the per-mass spectra (sart_enable_mass_spectra) and the
+// band images (sart_enable_band_images).
+enum AccumKind { kRadialHist, kSpectra, kMassSpectra, kBandImages, kAccums };
+constexpr AccumKind kAllAccums[kAccums] = {kRadialHist, kSpectra, kMassSpectra, kBandImages};
 
 // One block of an accumulator: the handle's own (sart_handle::accum) or its merged copy (sart_handle::merged_accum), both
 // one allocation laid out by the same code (api.cu: alloc_accum). blob == nullptr: off (and bins == 0).
 struct Accum {
   void* blob = nullptr;
   size_t bytes = 0;
-  int bins = 0;         // radial histogram: its bins; (per-mass) spectra: energy bins per row, nEnergies + 1
+  int bins = 0;         // radial histogram: its bins; (per-mass) spectra: energy bins per row, nEnergies + 1; band images: bands
   double rmax = 0.0;    // radial histogram: its range
+  double edges[SART_MAX_BANDS + 1] = {};   // band images: the bins + 1 band edges [keV]
   RadialHist rad{};     // radial histogram: w, n
   Spectra spec{};       // (per-mass) spectra: eW, eW2, eN, sW, sN; the per-mass spectra have one row per mass (eRow, sRow)
+  BandImages band{};    // band images: w, w2 [bins][256][256], n [bins]; the handle's block also its energy -> band table
   int valid = 0;        // merged copy: it holds the sums of the last sart_allreduce_outputs for the masses set
   // The handle's own block only: the buffers the throughput kernels add into instead (api.cu: carve_throughput), which the
   // fold after every launch adds into the arrays above and clears. The spectra's replicas, the per-mass spectra's
-  // mass-minor accumulators; the radial histogram has none.
+  // mass-minor accumulators, the band images' replicas (tput_band, which also holds the energy -> band table); the radial
+  // histogram has none.
   void* tput_blob = nullptr;
   Spectra tput{};
+  BandImages tput_band{};
 };
 
 // Rows of accumulator k for nMasses axion masses: one per mass for the per-mass spectra (allocated for SART_MAX_MASSES,
@@ -97,6 +105,11 @@ inline void accum_arrays(AccumKind k, A& a, B& b, size_t rows, F&& f) {
   const size_t e = rows * size_t(a.bins), s = rows * SART_MAX_SHELLS;
   if (k == kRadialHist) {
     f(a.rad.w, b.rad.w, e); f(a.rad.n, b.rad.n, e);
+    return;
+  }
+  if (k == kBandImages) {
+    const size_t p = e * SART_IMAGE_BINS * SART_IMAGE_BINS;
+    f(a.band.w, b.band.w, p); f(a.band.w2, b.band.w2, p); f(a.band.n, b.band.n, e);
     return;
   }
   f(a.spec.eW, b.spec.eW, e); f(a.spec.eW2, b.spec.eW2, e); f(a.spec.eN, b.spec.eN, e);
@@ -143,6 +156,7 @@ struct sart_handle {
   int image_masses = 0;         // mass planes the image buffers were allocated for
   double masses[SART_MAX_MASSES] = {0};
   double* d_masses = nullptr;   // [SART_MAX_MASSES]
+  long long* d_desc = nullptr;  // [kDescCapacity] the descriptor of sart_allreduce_outputs (comm.cu: describe_outputs)
   // one allocation of merged_words(n_masses) doubles: image [n_masses][256][256] | w^2 image | counter words (the send
   // buffer of sart_allreduce); d_image_w2 points into it
   double* d_image = nullptr;

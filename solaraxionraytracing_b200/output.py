@@ -263,6 +263,51 @@ def write_mass_spectra_csvs(spectra: list[Spectra], masses, windowYear: int, out
     return paths
 
 
+@dataclass
+class BandImages:
+    """Detector images of the passed rays of a run per energy band (RayTracer.enable_band_images): band b holds the rays
+    whose energy lies in [edges[b], edges[b + 1]) keV."""
+    edges: np.ndarray       # [B + 1] keV, strictly ascending
+    image: np.ndarray       # [B, 256, 256] Σw, image[b, y, x] like the run's image
+    image_w2: np.ndarray    # [B, 256, 256] Σw²
+    counts: np.ndarray      # [B] uint64: the passed rays of each band, in the image or not
+
+
+def parse_energy_bands(text: str) -> list[float]:
+    """The value of --energyBands: 2 .. abi.MAX_BANDS + 1 comma-separated edges in keV, finite, >= 0 and strictly
+    ascending ("0.5,2,4,8": three bands)."""
+    try:
+        edges = [float(x) for x in text.split(",")]
+    except ValueError:
+        raise ValueError(f"expected comma-separated energies in keV, got {text!r}") from None
+    if not 2 <= len(edges) <= abi.MAX_BANDS + 1:
+        raise ValueError(f"need 2 to {abi.MAX_BANDS + 1} edges (1 to {abi.MAX_BANDS} bands), got {len(edges)}")
+    if not all(np.isfinite(e) and e >= 0.0 for e in edges) or any(b <= a for a, b in zip(edges, edges[1:])):
+        raise ValueError(f"the edges must be finite, >= 0 and strictly ascending, got {text!r}")
+    return edges
+
+
+def band_suffix(lo: float, hi: float) -> str:
+    """File-name suffix of the energy band [lo, hi) keV: `_E{lo:g}-{hi:g}keV`."""
+    return f"_E{lo:g}-{hi:g}keV"
+
+
+def write_band_image_csvs(bands: BandImages, windowYear: int, outpath: str | Path, radii: ContainmentRadii | None = None,
+                          chipXMax: float = 14.0, chipYMax: float = 14.0, precision: int = 17) -> list[Path]:
+    """One write_axion_image_csv file per energy band, `axion_image_{year}_E{lo:g}-{hi:g}keV.csv`, next to the run's
+    image. The radius columns carry `radii`, the containment radii of the whole run: per-band radii are not computed."""
+    edges = [float(e) for e in bands.edges]
+    if len(edges) != bands.image.shape[0] + 1:
+        raise ValueError(f"{len(edges)} edges for {bands.image.shape[0]} band images")
+    names = [band_suffix(lo, hi) for lo, hi in zip(edges, edges[1:])]
+    if len(set(names)) != len(names):
+        raise ValueError("two bands share a file name (their edges agree to 6 significant digits)")
+    radii = radii or ContainmentRadii(0.0, 0.0, 0.0, 0.0)
+    year = WINDOW_YEAR_NAMES.get(windowYear, str(windowYear))
+    return [write_axion_image_csv(Path(outpath) / f"axion_image_{year}{sfx}.csv", img, radii.rSigma1W, radii.rSigma2W,
+                                  chipXMax, chipYMax, precision) for sfx, img in zip(names, bands.image)]
+
+
 def generateResultPlots(result, windowYear: int, outpath: str | Path, suffix: str = "",
                         radii: ContainmentRadii | None = None, chipXMax: float = 14.0, chipYMax: float = 14.0,
                         precision: int = 17, echo=print) -> Path:

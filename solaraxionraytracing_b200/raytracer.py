@@ -15,7 +15,7 @@ import numpy as np
 
 from . import abi, tables as _tables
 from ._lib import SartError, check, lib  # noqa: F401  (re-exported)
-from .output import Spectra
+from .output import BandImages, Spectra
 
 
 def _dp(a: np.ndarray):
@@ -338,6 +338,34 @@ class RayTracer:
         reset_image (raises SartError while they are off)."""
         return self._read_spectra_rows(lib.sart_read_mass_spectra, self.n_masses)
 
+    def enable_band_images(self, edges_keV=None):
+        """Detector images of the rays that pass in trace_mc per energy band [edges[b], edges[b + 1]) keV (single axion mass;
+        sart_enable_band_images); None switches them off. Switching them on clears them."""
+        if edges_keV is None:
+            check(lib.sart_enable_band_images(self._h, 0, None))
+            self._band_edges = None
+            return
+        e = np.ascontiguousarray(edges_keV, dtype=np.float64)
+        check(lib.sart_enable_band_images(self._h, e.size - 1 if e.size > 1 else -1, _dp(e)))   # one edge: no band, refused
+        self._band_edges = e.copy()
+
+    def _read_bands(self, read) -> BandImages:
+        edges = getattr(self, "_band_edges", None)
+        nb = 0 if edges is None else edges.size - 1
+        img = np.empty((nb, abi.IMAGE_BINS, abi.IMAGE_BINS))
+        img2 = np.empty_like(img)
+        n = np.empty(nb, dtype=np.uint64)
+        check(read(self._h, _dp(img), _dp(img2), n.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return BandImages(edges.copy(), img, img2, n)
+
+    def read_band_images(self) -> BandImages:
+        """The band images accumulated since enable_band_images / reset_image (raises SartError while they are off)."""
+        return self._read_bands(lib.sart_read_band_images)
+
+    def read_merged_band_images(self) -> BandImages:
+        """read_band_images of the last allreduce_outputs (raises SartError without one)."""
+        return self._read_bands(lib.sart_read_merged_band_images)
+
     def synchronize(self):
         check(lib.sart_synchronize(self._h))
 
@@ -377,8 +405,8 @@ class RayTracer:
         check(lib.sart_allreduce(hs, 1))
 
     def allreduce_outputs(self):
-        """sart_allreduce_outputs for this rank (every rank calls it): sums the radial histogram and the (per-mass)
-        spectra that are on over all ranks into merged copies, read with the read_merged_* methods. Synchronises."""
+        """sart_allreduce_outputs for this rank (every rank calls it): sums the radial histogram, the (per-mass) spectra and
+        the band images that are on over all ranks into merged copies, read with the read_merged_* methods. Synchronises."""
         hs = (abi.H * 1)(self._h)
         check(lib.sart_allreduce_outputs(hs, 1))
 
