@@ -35,6 +35,7 @@ extern "C" {
 #define SART_IMAGE_BINS 256  /* prepareHeatmap(256, 256, ...) raytracer.nim:2629 */
 #define SART_MAX_MASSES 64   /* axion masses traced per launch in a mass scan */
 #define SART_MAX_BANDS 16    /* energy bands of sart_enable_band_images */
+#define SART_MAX_QHIST_BINS 512   /* regular bins of one histogram of sart_enable_quantity_hists */
 
 typedef enum {
   SART_OK = 0,
@@ -412,6 +413,38 @@ int sart_enable_band_images(sart_handle_t* h, int n_bands, const double* edges_k
 /* Synchronises and copies out; host arrays, any may be NULL: image, image_w2 [n_bands][256][256] (the layout of the image),
  * counts [n_bands]. SART_ERR_ARG when the band images are off. */
 int sart_read_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts);
+/* Optional weighted histograms of per-ray record quantities of the passed rays (w != 0, rt:2220) of sart_trace_mc, single
+ * axion mass: the distributions generateResultPlots (rt:2246-2635) draws from reflect, transmissionMagnet, yawAngles,
+ * deviationDet and transProbArgon, and those of the grazing angles and pathCB, without per-ray records. The value of a ray
+ * is the one sart_trace_mc_rays reports for it in the field of sart_ray_out_t the quantity names, in the same precision
+ * mode with the same sampler, the FP64 re-trace included (modes 1 and 2: the FP32 value widened to double).
+ *   Histogram k has nbins_k + 2 entries: entry 0 underflow (v < lo), entries 1 .. nbins_k the regular bins, entry
+ * nbins_k + 1 overflow (!(v < hi), NaN included). Regular bin: 1 + fmin(floor((v - lo) * inv), nbins - 1) with
+ * inv = nbins / (hi - lo) computed once on the host in double, each operation rounded on its own (no contraction), so that
+ * a host reference reproduces it bit for bit. Each entry holds Σw, Σw² and a count; the rows are concatenated in the order
+ * of `hists`, Σ(nbins_k + 2) entries in all.
+ *   Accumulated (+=) like the image and cleared by sart_reset_image; filled in every precision mode, by the FP32 kernel and
+ * by the FP64 re-trace of its uncertain rays alike. With them on, precision modes 1 and 2 run kernel variants of their own
+ * that also fill the radial histogram, the spectra and the band images when those are on; the alias sampler is supported.
+ * sart_trace_mc with more than one axion mass, or with the per-mass spectra on, fails with SART_ERR_CONFIG.
+ * sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev) and sart_trace_words leave them
+ * untouched.
+ *   n in 1..SART_N_QUANTITIES histograms, each quantity at most once, nbins in 1..SART_MAX_QHIST_BINS, lo and hi finite
+ * with lo < hi: synchronises, then (re)allocates and zeroes them. n = 0 switches them off (default; hists may then be
+ * NULL). Anything else is SART_ERR_ARG. Device memory: 24 bytes per entry for the handle's arrays and for the merged copy
+ * of sart_allreduce_outputs, 16 per entry for each of the 8 block replicas (under 1 MB in all at 8 x 512 bins). */
+enum {
+  SART_Q_REFLECT = 0, SART_Q_TRANS_MAGNET = 1, SART_Q_YAW = 2, SART_Q_ALPHA1 = 3, SART_Q_ALPHA2 = 4,
+  SART_Q_PATH_CB = 5, SART_Q_DEVIATION_DET = 6, SART_Q_TRANS_PROB_ARGON = 7, SART_N_QUANTITIES = 8
+};
+typedef struct {
+  int32_t quantity;   /* SART_Q_* */
+  int32_t nbins;      /* regular bins, 1..SART_MAX_QHIST_BINS */
+  double lo, hi;      /* range of the regular bins */
+} sart_quantity_hist_t;
+int sart_enable_quantity_hists(sart_handle_t* h, int n, const sart_quantity_hist_t* hists);
+/* Synchronises and copies out; host arrays of Σ(nbins_k + 2) entries, any may be NULL. SART_ERR_ARG when they are off. */
+int sart_read_quantity_hists(sart_handle_t* h, double* sum_w, double* sum_w2, uint64_t* counts);
 /* Device pointers for collectives (ncclAllReduce / torch.distributed on the caller's side). */
 double* sart_image_dev(sart_handle_t* h);       /* [M][256][256] Σw  */
 double* sart_image_w2_dev(sart_handle_t* h);    /* [M][256][256] Σw² */
@@ -435,7 +468,9 @@ void sart_comm_destroy(sart_handle_t* h);   /* also done by sart_destroy */
 int sart_allreduce(sart_handle_t* const* handles, int n);
 int sart_read_merged(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);
 /* Sums the optional accumulators of the fused run over all ranks: the radial histogram, the spectra, the per-mass
- * spectra, the band images, whichever are on (the band images with the same edges on every rank). Each goes into a merged copy per handle; the handles' own accumulators are untouched.
+ * spectra, the band images, the quantity histograms, whichever are on (the band images with the same edges, the quantity
+ * histograms with the same specs on every rank). Each goes into a merged copy per handle; the handles' own accumulators
+ * are untouched.
  * Every rank must have the same ones on with the same shapes. This is checked collectively, so a mismatch fails
  * with SART_ERR_CONFIG on every rank instead of hanging. Synchronises the handles' streams.
  *   The ranks first exchange a few words describing what each has on (one small all-reduce); every refusal that depends
@@ -450,13 +485,15 @@ int sart_read_merged(sart_handle_t* h, double* image, double* image_w2, sart_cou
  * another size (and a new number of axion masses, for the per-mass spectra) invalidates its merged copy. */
 int sart_allreduce_outputs(sart_handle_t* const* handles, int n);
 /* The merged copies; same arguments and array shapes as sart_read_radial_hist, sart_read_spectra,
- * sart_read_mass_spectra and sart_read_band_images. Synchronise and copy out; SART_ERR_ARG without a valid merged copy. */
+ * sart_read_mass_spectra, sart_read_band_images and sart_read_quantity_hists. Synchronise and copy out; SART_ERR_ARG
+ * without a valid merged copy. */
 int sart_read_merged_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
 int sart_read_merged_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                              double* shell_sum_w, uint64_t* shell_counts);
 int sart_read_merged_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                                   double* shell_sum_w, uint64_t* shell_counts);
 int sart_read_merged_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts);
+int sart_read_merged_quantity_hists(sart_handle_t* h, double* sum_w, double* sum_w2, uint64_t* counts);
 
 /* Synchronise and copy out. image/image_w2 may be NULL. counters is [M]. */
 int sart_read_image(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);

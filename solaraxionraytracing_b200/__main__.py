@@ -4,7 +4,7 @@
   python -m solaraxionraytracing_b200 [--ignoreDetWindow] [--ignoreGasAbs] [--ignoreConvProb] [--ignoreReflection]
       [--xrayTest] [--detectorInstall] [--magnet] [--angularScanMin A --angularScanMax B --numAngularScanPoints N]
       [--noPlots] [--config FILE | --configPath DIR] [--nRays N] [--precision f32|fast|exact] [--writeSpectra]
-      [--energyBands E0,E1,...] [--device D | --devices 0,1,... | --devices all]
+      [--energyBands E0,E1,...] [--histogram NAME:NBINS:LO:HI ...] [--device D | --devices 0,1,... | --devices all]
 
 Inputs the reference reads from `resources/` and that are not shipped with it (solar_model_dataframe.csv, the two
 reflectivity HDF5 files) are taken from [Resources] when present, else generated: Primakoff emission rates from AGSS09
@@ -42,6 +42,12 @@ def build_parser() -> argparse.ArgumentParser:
                     help="also write one detector image per energy band: comma-separated band edges in keV, e.g. 0.5,2,4,8 "
                          "(2 to 17 values, ascending) writes axion_image_{year}_E0.5-2keV.csv and so on next to the image; "
                          "a single axion mass only")
+    ap.add_argument("--histogram", action="append", default=None, metavar="NAME:NBINS:LO:HI",
+                    help="also write a weighted histogram of a per-ray record quantity of the passed rays, e.g. "
+                         "transMagnet:256:0:1e-20, to axion_hist_{NAME}_{year}.csv next to the image (NBINS regular bins over "
+                         "[LO, HI) plus an underflow and an overflow row); repeatable, each quantity once; NAME is one of "
+                         "reflect, transMagnet, yaw, alpha1, alpha2, pathCB, deviationDet, transProbArgon; a single axion mass "
+                         "only")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--devices", default=None,
                     help="trace on several GPUs: a comma-separated list of CUDA ordinals or `all`. A fused run shards the "
@@ -93,6 +99,12 @@ def parse_args(argv=None) -> argparse.Namespace:
             a.energyBands = parse_energy_bands(a.energyBands)
         except ValueError as e:
             ap.error(f"--energyBands: {e}")
+    if a.histogram is not None:
+        from .output import check_quantity_hist_specs, parse_quantity_hist
+        try:
+            a.histogram = check_quantity_hist_specs([parse_quantity_hist(t) for t in a.histogram])
+        except ValueError as e:
+            ap.error(f"--histogram: {e}")
     return a
 
 
@@ -154,10 +166,10 @@ def load_tables(rt, tables, res, setup, device: int, allow_synthetic: bool = Fal
     return tables.TableSet(energies=em.energies, fluxRadiusCDF=rc, diffFluxCDFs=dc, reflectivity=refl, **extra, **det)
 
 
-def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath, bands=None):
+def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath, bands=None, qhists=None):
     """The files of a fused run: the image CSV and containment radii (at most one mass), or the per-mass images of a mass
     scan; with `spectra` also the spectra CSVs (one Spectra, or one per mass); with `bands` (output.BandImages, at most one
-    mass) one image CSV per energy band."""
+    mass) one image CSV per energy band; with `qhists` (output.QuantityHist list, at most one mass) one CSV per histogram."""
     from . import output
     if len(masses) <= 1:
         radii = output.containment_radii_from_hist(*radial_hist)
@@ -167,6 +179,9 @@ def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath, ba
         if bands is not None:
             for p in output.write_band_image_csvs(bands, setup.detector.windowYear, outpath, radii,
                                                   setup.consts.chipXMax, setup.consts.chipYMax):
+                print("wrote", p)
+        if qhists is not None:
+            for p in output.write_quantity_hist_csvs(qhists, setup.detector.windowYear, outpath):
                 print("wrote", p)
         if spectra is not None:
             for p in output.write_spectra_csvs(spectra, setup.detector.windowYear, outpath):
@@ -201,6 +216,8 @@ def main(argv=None) -> int:
     run = cfgmod.parseRun(cfgmod.load_config(cfg_file))
     if a.energyBands is not None and len(run.mAxion) > 1:
         build_parser().error("--energyBands: the band images need a single axion mass, and the configuration sets a mass scan")
+    if a.histogram is not None and len(run.mAxion) > 1:
+        build_parser().error("--histogram: the quantity histograms need a single axion mass, and the configuration sets a mass scan")
     a.nRays = run.nRays if a.nRays is None else a.nRays
     a.seed = run.seed if a.seed is None else a.seed
     a.precision = a.precision or run.precision
@@ -220,12 +237,12 @@ def main(argv=None) -> int:
             try:
                 r = multi_gpu.trace_on_devices(fs, devices, n, a.seed, precision=want, sampler=sampler,
                                                masses=run.mAxion or None, radial_hist=single, spectra=a.writeSpectra,
-                                               bands=a.energyBands, warn=warn)
+                                               bands=a.energyBands, quantity_hists=a.histogram, warn=warn)
             except rt.SartError as e:
                 if "NCCL" in str(e):
                     raise SystemExit(f"raytracer: {e}") from None
                 raise
-            write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath, r.band_images)
+            write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath, r.band_images, r.quantity_hists)
         else:
             angles, rel, _ = multi_gpu.angular_scan_on_devices(fs, devices, a.angularScanMin, a.angularScanMax,
                                                                a.numAngularScanPoints, n, a.seed, precision=want,
@@ -246,6 +263,8 @@ def main(argv=None) -> int:
                 tr.enable_spectra() if single else tr.enable_mass_spectra()
             if a.energyBands is not None:
                 tr.enable_band_images(a.energyBands)
+            if a.histogram is not None:
+                tr.enable_quantity_hists(a.histogram)
             tr.reset_image()
             tr.trace_mc(n, a.seed)
             result = tr.read_image()
@@ -253,7 +272,9 @@ def main(argv=None) -> int:
             if a.writeSpectra:
                 spectra = tr.read_spectra() if single else tr.read_mass_spectra()
             bands = tr.read_band_images() if a.energyBands is not None else None
-            write_fused_outputs(result, tr.read_radial_hist() if single else None, spectra, run.mAxion, setup, outpath, bands)
+            qhists = tr.read_quantity_hists() if a.histogram is not None else None
+            write_fused_outputs(result, tr.read_radial_hist() if single else None, spectra, run.mAxion, setup, outpath, bands,
+                                qhists)
         else:
             angles, rel, _ = rt.performAngularScan(fs, a.angularScanMin, a.angularScanMax, a.numAngularScanPoints, n,
                                                    a.seed, tracer=tr)

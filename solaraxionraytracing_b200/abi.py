@@ -11,6 +11,10 @@ MAX_COATINGS = 8
 IMAGE_BINS = 256
 MAX_MASSES = 64
 MAX_BANDS = 16
+MAX_QHIST_BINS = 512
+# the record quantities of sart_enable_quantity_hists (SART_Q_*), named like the fields of sart_ray_out_t
+QUANTITIES = ("reflect", "transMagnet", "yaw", "alpha1", "alpha2", "pathCB", "deviationDet", "transProbArgon")
+N_QUANTITIES = len(QUANTITIES)
 COMM_ID_BYTES = 128
 
 # enums (raytracer.nim:16-46, 59-64, 164-167)
@@ -134,6 +138,10 @@ class PassedOut(C.Structure):
     _fields_ = [(n, C.POINTER(t)) for n, t in PASSED_OUT_FIELDS]
 
 
+class QuantityHistSpec(C.Structure):   # sart_quantity_hist_t
+    _fields_ = [("quantity", C.c_int32), ("nbins", C.c_int32), ("lo", C.c_double), ("hi", C.c_double)]
+
+
 class Counters(C.Structure):
     _fields_ = [("n_rays", C.c_uint64), ("n_exit", C.c_uint64 * 16), ("n_passed", C.c_uint64),
                 ("n_passed_till_window", C.c_uint64), ("n_hit_nickel", C.c_uint64), ("n_interp_clamped", C.c_uint64),
@@ -210,6 +218,8 @@ SIGNATURES = {
                                          C.POINTER(C.c_uint64)]),
     "sart_enable_band_images": (C.c_int, [H, C.c_int, c_double_p]),
     "sart_read_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
+    "sart_enable_quantity_hists": (C.c_int, [H, C.c_int, C.POINTER(QuantityHistSpec)]),
+    "sart_read_quantity_hists": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_image_dev": (C.c_void_p, [H]),
     "sart_image_w2_dev": (C.c_void_p, [H]),
     "sart_counters_dev": (C.c_void_p, [H]),
@@ -229,6 +239,7 @@ SIGNATURES = {
     "sart_read_merged_mass_spectra": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64), c_double_p,
                                                 C.POINTER(C.c_uint64)]),
     "sart_read_merged_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
+    "sart_read_merged_quantity_hists": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_angular_scan": (C.c_int, [H, C.c_int, c_double_p, C.c_uint64, C.c_uint64, C.c_uint64, c_double_p, C.POINTER(Counters),
                                     c_double_p]),
     "sart_measure_fma_peak": (C.c_int, [C.c_int, C.c_int, c_double_p]),

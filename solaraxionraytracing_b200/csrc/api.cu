@@ -379,8 +379,9 @@ int alloc_accum(AccumKind k, int bins, double rmax, Accum* a) {
 // sW | sN, each sRep x SART_MAX_SHELLS. The per-mass spectra's mass-minor accumulators (fast_common.cuh: mass_spec_add):
 // eW | eW2 | 32-bit eN, each [nE1][SART_MAX_MASSES] | sW | 32-bit sN, each [SART_MAX_SHELLS][SART_MAX_MASSES]. The band
 // images' replicas (device_params.h: BandImages): w | w2, each bRep x [bins][256][256], and the band of each of the nE1
-// energy bins, which the exact kernels read through the handle's block (a->band) as well; their counts are the handle's.
-static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, int bRep, void* base, Accum* a) {
+// energy bins, which the exact kernels read through the handle's block (a->band) as well; their counts are the handle's. The
+// quantity histograms' replicas of Σw and Σw² (device_params.h: QuantityHists::rw, rw2), each qRep x bins, in a->qh itself.
+static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, int bRep, int qRep, void* base, Accum* a) {
   Carve c(base);
   Spectra* r = &a->tput;
   *r = Spectra{};
@@ -401,6 +402,10 @@ static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, int bRe
     c.take(b.w, size_t(bRep) * len); c.take(b.w2, size_t(bRep) * len); c.take(b.band, size_t(nE1));
     b.repStride = uint32_t(len); b.repMask = uint32_t(bRep - 1);
     a->band.band = b.band;
+  } else if (k == kQuantityHists) {
+    QuantityHists& q = a->qh;
+    c.take(q.rw, size_t(qRep) * size_t(a->bins)); c.take(q.rw2, size_t(qRep) * size_t(a->bins));
+    q.repStride = uint32_t(a->bins); q.repMask = uint32_t(qRep - 1);
   }
   return c.off;
 }
@@ -435,18 +440,35 @@ static void free_accum(sart_handle* h, AccumKind k) {
   if (k == kRadialHist) h->tables.rad = h->ftables.rad = RadialHist{};
 }
 
+// The specs of the quantity histograms into their device view (device_params.h: QuantityHists), bins = their entries.
+static void put_qhist_specs(Accum& a, int n, const sart_quantity_hist_t* specs) {
+  QuantityHists& q = a.qh;
+  a.n_qhists = n;
+  q.nHists = n; q.entries = a.bins;
+  int off = 0;
+  for (int j = 0; j < n; ++j) {
+    a.qspecs[j] = specs[j];
+    q.quantity[j] = specs[j].quantity; q.nbins[j] = specs[j].nbins; q.off[j] = off;
+    q.lo[j] = specs[j].lo; q.hi[j] = specs[j].hi; q.inv[j] = double(specs[j].nbins) / (specs[j].hi - specs[j].lo);
+    off += specs[j].nbins + 2;
+  }
+}
+
 // Accumulator k on with `bins` bins: the handle's block and its throughput buffers, allocated, cleared and carved; the band
-// images also get their `edges` and energy -> band table.
-static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax, const double* edges) {
+// images also get their `edges` and energy -> band table, the quantity histograms their `n_q` specs `qspecs`.
+static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax, const double* edges, int n_q,
+                     const sart_quantity_hist_t* qspecs) {
   Accum& a = h->accum[k];
   int rc = alloc_accum(k, bins, rmax, &a);
   if (rc) return rc;
   if (edges) std::copy(edges, edges + bins + 1, a.edges);
+  if (qspecs) put_qhist_specs(a, n_q, qspecs);
   // Replicas of the spectra (powers of two; SART_SPEC_E_REPLICAS / SART_SPEC_S_REPLICAS override them for measurements).
   // The energy bins spread the passed rays over hundreds of addresses, like the focal spot the image replicas serve: one
   // replica per block residue. The shell bins are a handful of addresses (4 for LLNL): one per warp. The band images have a
   // focal spot per band plane, like the image: 8 replicas (SART_BAND_REPLICAS overrides it; measured on B200, CAST+LLNL, 4
-  // bands, 1e9 rays: 1 replica 39.5 ms, 8 replicas 31.4 ms, 16 replicas at 16 bands no faster than 8).
+  // bands, 1e9 rays: 1 replica 39.5 ms, 8 replicas 31.4 ms, 16 replicas at 16 bands no faster than 8). The quantity
+  // histograms' sums go to 8 replicas only in the kernels whose block leaves no room for them in shared memory.
   auto pow2 = [](const char* env, int dflt) {
     int n = dflt;
     if (const char* e = std::getenv(env)) n = std::max(1, std::min(1 << 16, std::atoi(e)));
@@ -456,24 +478,26 @@ static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax, const d
   };
   const int eRep = pow2("SART_SPEC_E_REPLICAS", 32), sRep = pow2("SART_SPEC_S_REPLICAS", 1024);
   const int bRep = std::min(pow2("SART_BAND_REPLICAS", 8), 64);
+  const int qRep = std::min(pow2("SART_QHIST_REPLICAS", 8), 64);
   const int nE1 = h->params.nEnergies + 1;
-  const size_t tputBytes = carve_throughput(k, nE1, eRep, sRep, bRep, nullptr, &a);
+  const size_t tputBytes = carve_throughput(k, nE1, eRep, sRep, bRep, qRep, nullptr, &a);
   if (tputBytes) SART_CUDA(cudaMalloc(&a.tput_blob, tputBytes));
   SART_CUDA(cudaMemsetAsync(a.blob, 0, a.bytes, h->stream));
   if (tputBytes) SART_CUDA(cudaMemsetAsync(a.tput_blob, 0, tputBytes, h->stream));
   SART_CUDA(cudaStreamSynchronize(h->stream));
-  carve_throughput(k, nE1, eRep, sRep, bRep, a.tput_blob, &a);
+  carve_throughput(k, nE1, eRep, sRep, bRep, qRep, a.tput_blob, &a);
   if (k == kRadialHist) h->tables.rad = h->ftables.rad = a.rad;
   return k == kBandImages ? put_band_table(h, 0) : SART_OK;
 }
 
 // What every sart_enable_* does after its own checks: synchronises, switches accumulator k off, and with bins > 0 on again,
 // cleared. A failure leaves it off.
-static int set_accum(sart_handle* h, AccumKind k, int bins, double rmax = 0.0, const double* edges = nullptr) {
+static int set_accum(sart_handle* h, AccumKind k, int bins, double rmax = 0.0, const double* edges = nullptr, int n_q = 0,
+                     const sart_quantity_hist_t* qspecs = nullptr) {
   DeviceGuard dg(h->device);
   SART_CUDA(cudaStreamSynchronize(h->stream));
   free_accum(h, k);
-  const int rc = bins > 0 ? new_accum(h, k, bins, rmax, edges) : SART_OK;
+  const int rc = bins > 0 ? new_accum(h, k, bins, rmax, edges, n_q, qspecs) : SART_OK;
   if (rc) free_accum(h, k);
   return rc;
 }
@@ -1217,18 +1241,21 @@ int sart_trace_words(sart_handle_t* h, size_t n, const uint32_t* words, int late
 // A fused image run of one axion mass in the handle's precision mode, with the parameter blocks and table views the caller
 // prepared (the handle's, or those of a scan point). The throughput kernels add into img / img2, which ft may spread over
 // replicas, and into the band images `band`; the exact kernels (mode 0, and the re-trace of mode 2) add into exImg / exImg2
-// and `exBand`. All add into `counters`. Band images off: band.w == exBand.w == nullptr.
+// and `exBand`. All add into `counters` and into the quantity histograms `qh` (the exact kernels into its arrays, the
+// throughput kernels from shared memory or through its replicas). Band images off: band.w == exBand.w == nullptr; quantity
+// histograms off: qh.w == nullptr.
 static int trace_image(sart_handle* h, const Params& P, const fast::FastParams& F, const fast::Geo32& G, fast::FastTables ft,
                        const Tables& et, uint64_t first, uint64_t n, uint64_t seed, double* img, double* img2, double* exImg,
-                       double* exImg2, sart_counters_t* counters, const BandImages& band = {}, const BandImages& exBand = {}) {
+                       double* exImg2, sart_counters_t* counters, const BandImages& band = {}, const BandImages& exBand = {},
+                       const QuantityHists& qh = {}) {
   if (h->precision == 0) {
     SART_CUDA(launch_mc_image_exact(P, et, 1, h->d_masses, first, n, seed, exImg, exImg2, counters, h->sm_count, h->stream,
-                                    exBand));
+                                    exBand, qh));
     return SART_OK;
   }
   if (h->precision == 1) {
     SART_CUDA(launch_mc_image_fast(F, ft, h->masses[0], first, n, seed, img, img2, counters, h->sm_count, h->compact != 0,
-                                   h->stream, band));
+                                   h->stream, band, qh));
     return SART_OK;
   }
   // the alias sampler has another ray <-> index mapping than the exact pipeline's: no re-trace
@@ -1236,11 +1263,11 @@ static int trace_image(sart_handle* h, const Params& P, const fast::FastParams& 
       [&](uint64_t done, uint64_t m, const fast::RetraceQueue& q) {
         ft.rq = q;
         return launch_mc_image_f32(F, G, ft, h->masses[0], first + done, m, seed, img, img2, counters, h->sm_count,
-                                   h->compact != 0, h->stream, band);
+                                   h->compact != 0, h->stream, band, qh);
       },
       [&](uint64_t done, uint64_t, const fast::RetraceQueue& q) {
         return launch_retrace_mc_image(P, et, 1, h->d_masses, first + done, seed, q, exImg, exImg2, counters, h->sm_count,
-                                       h->stream, exBand);
+                                       h->stream, exBand, qh);
       });
 }
 
@@ -1257,6 +1284,9 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   const Accum& bands = h->accum[kBandImages];
   if (bands.blob && (h->n_masses > 1 || mspec.blob))
     return fail(SART_ERR_CONFIG, "sart_trace_mc: the band images need a single axion mass and the per-mass spectra off");
+  const Accum& qhists = h->accum[kQuantityHists];
+  if (qhists.blob && (h->n_masses > 1 || mspec.blob))
+    return fail(SART_ERR_CONFIG, "sart_trace_mc: the quantity histograms need a single axion mass and the per-mass spectra off");
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
   int rc = SART_OK;
   // A mass scan, or any run with the per-mass spectra on (one contract for every mass list, M = 1 included): the exact
@@ -1323,7 +1353,7 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   }
   // band images: the throughput kernels add into their replicas, the exact kernels into the handle's arrays
   rc = trace_image(h, h->params, h->fparams, h->geo32, ft, et, first_ray, n_rays, seed, img, img2, h->d_image, h->d_image_w2,
-                   h->d_counters, bands.tput_band, bands.band);
+                   h->d_counters, bands.tput_band, bands.band, qhists.qh);
   if (rc || h->precision == 0) return rc;
   if (h->n_rep > 1)
     SART_CUDA(launch_fold_replicas(img, img2, h->n_rep, h->rep_stride, plane, h->d_image, h->d_image_w2, h->stream));
@@ -1331,6 +1361,10 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   if (bands.blob) {
     const BandImages& r = bands.tput_band;
     SART_CUDA(launch_fold_replicas(r.w, r.w2, int(r.repMask) + 1, r.repStride, r.repStride, bands.band.w, bands.band.w2, h->stream));
+  }
+  if (qhists.blob) {   // the replicas hold sums only where the kernel kept them out of shared memory; zeros cost no adds
+    const QuantityHists& q = qhists.qh;
+    SART_CUDA(launch_fold_replicas(q.rw, q.rw2, int(q.repMask) + 1, q.repStride, size_t(q.entries), q.w, q.w2, h->stream));
   }
   return SART_OK;
 }
@@ -1385,6 +1419,31 @@ int sart_enable_band_images(sart_handle_t* h, int n_bands, const double* edges_k
 int sart_read_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts) {
   return read_accum(h, kBandImages, false, {image, image_w2, counts},
                     "sart_read_band_images: no band images enabled (sart_enable_band_images)");
+}
+
+int sart_enable_quantity_hists(sart_handle_t* h, int n, const sart_quantity_hist_t* hists) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (n < 0 || n > SART_N_QUANTITIES || (n > 0 && !hists))
+    return fail(SART_ERR_ARG, "sart_enable_quantity_hists: need 1..%d histograms and their specs, or 0 (off)", SART_N_QUANTITIES);
+  int entries = 0;
+  unsigned seen = 0;
+  for (int j = 0; j < n; ++j) {
+    const sart_quantity_hist_t& q = hists[j];
+    if (q.quantity < 0 || q.quantity >= SART_N_QUANTITIES || (seen & (1u << q.quantity)))
+      return fail(SART_ERR_ARG, "sart_enable_quantity_hists: histogram %d: unknown or repeated quantity %d", j, int(q.quantity));
+    if (q.nbins < 1 || q.nbins > SART_MAX_QHIST_BINS)
+      return fail(SART_ERR_ARG, "sart_enable_quantity_hists: histogram %d: need 1..%d bins", j, SART_MAX_QHIST_BINS);
+    if (!std::isfinite(q.lo) || !std::isfinite(q.hi) || !(q.lo < q.hi))
+      return fail(SART_ERR_ARG, "sart_enable_quantity_hists: histogram %d: lo and hi must be finite with lo < hi", j);
+    seen |= 1u << q.quantity;
+    entries += q.nbins + 2;
+  }
+  return set_accum(h, kQuantityHists, entries, 0.0, nullptr, n, hists);
+}
+
+int sart_read_quantity_hists(sart_handle_t* h, double* sum_w, double* sum_w2, uint64_t* counts) {
+  return read_accum(h, kQuantityHists, false, {sum_w, sum_w2, counts},
+                    "sart_read_quantity_hists: no quantity histograms enabled (sart_enable_quantity_hists)");
 }
 
 int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max) {

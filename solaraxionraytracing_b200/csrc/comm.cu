@@ -89,8 +89,14 @@ __global__ void k_pack_counters(const sart_counters_t* __restrict__ c, int nMass
 // sart_allreduce_outputs: what a handle has on, in the words every rank must agree on, then an error word. All ranks send
 // [d, -d] through one ncclMax, so each learns the largest and (negated) smallest value of every word. Words 0 .. kAccums - 1
 // are the bins of each accumulator (0: off), then the bits of r_max, the number of masses and the bits of the
-// SART_MAX_BANDS + 1 band edges (0 beyond the last edge; edges are >= 0, so their bits are non-negative int64 words).
-enum { kDescRadMax = kAccums, kDescMasses, kDescEdges, kDescErr = kDescEdges + SART_MAX_BANDS + 1, kDescWords };
+// SART_MAX_BANDS + 1 band edges (0 beyond the last edge; edges are >= 0, so their bits are non-negative int64 words), then
+// per quantity histogram (0 beyond the last) a word of quantity | nbins << 8 | the sign bits of lo and hi << 20, 21, and
+// the other 63 bits of lo and of hi (non-negative words, so that -d never overflows).
+enum {
+  kDescRadMax = kAccums, kDescMasses, kDescEdges, kDescQSpec = kDescEdges + SART_MAX_BANDS + 1,
+  kDescQLo = kDescQSpec + SART_N_QUANTITIES, kDescQHi = kDescQLo + SART_N_QUANTITIES, kDescErr = kDescQHi + SART_N_QUANTITIES,
+  kDescWords
+};
 static_assert(2 * kDescWords <= kDescCapacity, "the descriptor travels in sart_handle::d_desc");
 
 static void describe_outputs(const sart_handle* h, long long d[kDescWords]) {
@@ -98,6 +104,20 @@ static void describe_outputs(const sart_handle* h, long long d[kDescWords]) {
   std::memcpy(&d[kDescRadMax], &h->accum[kRadialHist].rmax, sizeof(long long));
   d[kDescMasses] = h->n_masses;
   std::memcpy(&d[kDescEdges], h->accum[kBandImages].edges, (SART_MAX_BANDS + 1) * sizeof(long long));
+  const Accum& q = h->accum[kQuantityHists];
+  for (int j = 0; j < SART_N_QUANTITIES; ++j) {
+    uint64_t lo = 0, hi = 0;
+    long long spec = 0;
+    if (j < q.n_qhists) {
+      std::memcpy(&lo, &q.qspecs[j].lo, sizeof lo);
+      std::memcpy(&hi, &q.qspecs[j].hi, sizeof hi);
+      spec = (long long)q.qspecs[j].quantity | (long long)q.qspecs[j].nbins << 8 | (long long)(lo >> 63) << 20 |
+             (long long)(hi >> 63) << 21;
+    }
+    d[kDescQSpec + j] = spec;
+    d[kDescQLo + j] = (long long)(lo & ~(uint64_t(1) << 63));
+    d[kDescQHi + j] = (long long)(hi & ~(uint64_t(1) << 63));
+  }
   d[kDescErr] = 0;
 }
 
@@ -253,7 +273,7 @@ int sart_allreduce_outputs(sart_handle_t* const* handles, int n) {
     for (int k = 0; k < kDescErr; ++k)
       if (desc[size_t(i) * 2 * kDescWords + k] != desc[k])
         return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: handles 0 and %d differ in their radial histogram, spectra, "
-                                     "per-mass spectra, band images or number of axion masses", i);
+                                     "per-mass spectra, band images, quantity histograms or number of axion masses", i);
   auto desc_dev = [](sart_handle* h) { return h->d_desc; };
   for (int i = 0; i < n; ++i) {
     sart_handle* h = handles[i];
@@ -296,12 +316,15 @@ int sart_allreduce_outputs(sart_handle_t* const* handles, int n) {
   const long long* neg_lo = &red[kDescWords];
   if (hi[kDescErr]) return fail(SART_ERR_NOMEM, "sart_allreduce_outputs: a rank could not allocate its merged copies");
   static const char* const what[kDescEdges] = {"radial histogram bins", "spectra bins", "per-mass spectra bins",
-                                               "number of energy bands", "radial histogram r_max", "number of axion masses"};
+                                               "number of energy bands", "quantity histogram entries", "radial histogram r_max",
+                                               "number of axion masses"};
   for (int k = 0; k < kDescErr; ++k)
     if (hi[k] != -neg_lo[k])
-      return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: the ranks differ in their %s", k < kDescEdges ? what[k] : "energy band edges");
-  if (!hi[kRadialHist] && !hi[kSpectra] && !hi[kMassSpectra] && !hi[kBandImages])
-    return fail(SART_ERR_ARG, "sart_allreduce_outputs: no radial histogram, spectra or per-mass spectra enabled, and no band images");
+      return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: the ranks differ in their %s",
+                  k < kDescEdges ? what[k] : (k < kDescQSpec ? "energy band edges" : "quantity histogram specs"));
+  if (!hi[kRadialHist] && !hi[kSpectra] && !hi[kMassSpectra] && !hi[kBandImages] && !hi[kQuantityHists])
+    return fail(SART_ERR_ARG, "sart_allreduce_outputs: no radial histogram, spectra or per-mass spectra enabled, and no band "
+                              "images or quantity histograms");
   // the payload: counts as u64, sums as f64, of the per-mass rows only those of the M masses set, every all-reduce of every
   // handle in one group
   r = api->GroupStart();
@@ -337,6 +360,11 @@ int sart_read_merged_spectra(sart_handle_t* h, double* energy_sum_w, double* ene
 int sart_read_merged_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts) {
   return read_accum(h, kBandImages, true, {image, image_w2, counts},
                     "sart_read_merged_band_images: no merged band images (call sart_allreduce_outputs first)");
+}
+
+int sart_read_merged_quantity_hists(sart_handle_t* h, double* sum_w, double* sum_w2, uint64_t* counts) {
+  return read_accum(h, kQuantityHists, true, {sum_w, sum_w2, counts},
+                    "sart_read_merged_quantity_hists: no merged quantity histograms (call sart_allreduce_outputs first)");
 }
 
 int sart_read_merged_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,

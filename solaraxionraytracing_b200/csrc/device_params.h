@@ -134,6 +134,34 @@ __device__ __forceinline__ void band_add(const BandImages& b, int eIdx, int bin,
 }
 #endif
 
+// Optional weighted histograms of per-ray record quantities of the passed rays (sart_enable_quantity_hists): histogram j
+// (quantity[j], a SART_Q_*) has nbins[j] + 2 entries from entry off[j] on — underflow, the regular bins, overflow — of
+// `entries` in all. w / w2 / n: Σw, Σw² and the count per entry, the handle's arrays (the exact kernels add into them per
+// ray; the throughput kernels their counts once per block from shared memory, and their sums too when they keep those
+// there, SART_QHIST_SMEM). rw / rw2: block replicas of Σw and Σw² (replica block & repMask, repStride elements apart),
+// where the throughput kernels add their sums by default; folded into w / w2 after every launch. w == nullptr: off. Passed to the kernels that fill them as a parameter of its own.
+struct QuantityHists {
+  double* w;
+  double* w2;
+  unsigned long long* n;
+  double* rw;
+  double* rw2;
+  uint32_t repStride, repMask;
+  int32_t nHists, entries;
+  int32_t quantity[SART_N_QUANTITIES], nbins[SART_N_QUANTITIES], off[SART_N_QUANTITIES];
+  double lo[SART_N_QUANTITIES], hi[SART_N_QUANTITIES], inv[SART_N_QUANTITIES];   // inv = nbins / (hi - lo)
+};
+
+#if defined(__CUDACC__)
+// The entry of value v in histogram j, relative to its first: 0 underflow (v < lo), nbins + 1 overflow (!(v < hi), NaN
+// included), else 1 + fmin(floor((v - lo) * inv), nbins - 1), each operation rounded on its own (no contraction).
+__device__ __forceinline__ int qhist_entry(const QuantityHists& Q, int j, double v) {
+  if (v < Q.lo[j]) return 0;
+  if (!(v < Q.hi[j])) return Q.nbins[j] + 1;
+  return 1 + int(fmin(floor(__dmul_rn(__dsub_rn(v, Q.lo[j]), Q.inv[j])), double(Q.nbins[j] - 1)));
+}
+#endif
+
 // Table pointers (device memory).
 struct Tables {
   const double* energies;

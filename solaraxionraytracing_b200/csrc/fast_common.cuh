@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <cfloat>
+#include <cstdlib>
 
 #include "fast_params.h"
 #include "kernels.h"
@@ -271,6 +272,12 @@ __device__ __forceinline__ int finish_ray(const FastParams& P, const RayResult& 
   return ((w != 0.0) ? SART_EXIT_PASSED : SART_EXIT_ZERO_WEIGHT) | flags;
 }
 
+// transmissionMagnet of a ray that reached the weight stage (rt:2120) for axion mass^2 m2: the record's value
+// (store_record) and the quantity histograms' (QuantityHistSink).
+__device__ __forceinline__ double trans_magnet(const FastParams& P, const RayResult& r, double m2) {
+  return double(r.pre) * conv_factor(P, r.convVac, r.gasGamma, r.gasE1, r.gasE2, r.gasInv2E, r.gasL, m2);
+}
+
 // The Axion record (rt:192-221) of one ray of the throughput pipelines, written to the structure of arrays `o` (device
 // pointers). Fields of the weight stage (reflect, transmissionMagnet, yawAngles, the grazing angles, pathCB, deviationDet)
 // are defined for the rays that reach it — exit codes PASSED, ZERO_WEIGHT, WINDOW_APERTURE, which is every ray
@@ -292,8 +299,7 @@ __device__ __forceinline__ void store_record(const FastParams& P, const sart_ray
   if (!kOptional) return;
   if (o.energy) o.energy[i] = energyKeV;
   if (o.reflect) o.reflect[i] = weighted ? r.refl : 0.0;
-  if (o.transMagnet)
-    o.transMagnet[i] = weighted ? double(r.pre) * conv_factor(P, r.convVac, r.gasGamma, r.gasE1, r.gasE2, r.gasInv2E, r.gasL, m2) : 0.0;
+  if (o.transMagnet) o.transMagnet[i] = weighted ? trans_magnet(P, r, m2) : 0.0;
   if (o.yaw) o.yaw[i] = weighted ? double(r.yaw) : 0.0;
   if (o.alpha1) o.alpha1[i] = weighted ? double(r.a1) : 0.0;
   if (o.alpha2) o.alpha2[i] = weighted ? double(r.a2) : 0.0;
@@ -382,6 +388,18 @@ using ImageSink = ImageSinkT<true>;
 // spectra checked at run time, plus the band images B (device_params.h: BandImages; here their replicas, bandRep this block's
 // replica) and the block's per-band counts bandN in shared memory, which the kernel flushes once at its end. A derived sink,
 // so that ImageSinkT, and every kernel variant built on it, stays what it was before the band images existed.
+// A passed ray of weight wd into the band images of a throughput kernel: its band's count in shared memory, Σw and Σw² into
+// replica bandRep of its band's plane.
+__device__ __forceinline__ void band_hit(const BandImages& B, unsigned int* bandN, uint32_t bandRep, const RayResult& h,
+                                         double wd) {
+  const unsigned k = __ldg(B.band + h.eIdx);
+  if (k == kNoBand) return;
+  atomicAdd(bandN + k, 1u);
+  if (h.bin < 0) return;
+  const uint32_t at = bandRep + k * uint32_t(SART_IMAGE_BINS * SART_IMAGE_BINS) + uint32_t(h.bin);
+  atomicAdd(B.w + at, wd);
+  atomicAdd(B.w2 + at, wd * wd);
+}
 struct BandImageSink : ImageSinkT<true, true> {
   const BandImages& B;
   unsigned int* bandN;
@@ -390,13 +408,7 @@ struct BandImageSink : ImageSinkT<true, true> {
     ImageSinkT<true, true>::hit(h);
     const double wd = h.wPre * h.wPost;   // the weight ImageSinkT::hit tested
     if (h.windowMiss || wd == 0.0) return;
-    const unsigned k = __ldg(B.band + h.eIdx);
-    if (k == kNoBand) return;
-    atomicAdd(bandN + k, 1u);
-    if (h.bin < 0) return;
-    const uint32_t at = bandRep + k * uint32_t(SART_IMAGE_BINS * SART_IMAGE_BINS) + uint32_t(h.bin);
-    atomicAdd(B.w + at, wd);
-    atomicAdd(B.w2 + at, wd * wd);
+    band_hit(B, bandN, bandRep, h, wd);
   }
 };
 
@@ -423,6 +435,140 @@ __device__ __forceinline__ auto with_bands(const Sink& sink, const BandImages& B
 __device__ __forceinline__ void band_counts_flush(const BandImages& B, const unsigned int* n) {
   __syncthreads();
   if (threadIdx.x < unsigned(B.nBands) && n[threadIdx.x]) atomicAdd(B.n + threadIdx.x, (unsigned long long)n[threadIdx.x]);
+}
+
+// ---- quantity histograms of the throughput kernels (sart_enable_quantity_hists; device_params.h: QuantityHists) ------
+// The record quantity q (SART_Q_*) of a ray that passed, as store_record writes it.
+__device__ __forceinline__ double record_quantity(const FastParams& P, const RayResult& h, double m2, int q) {
+  switch (q) {
+    case SART_Q_REFLECT: return h.refl;
+    case SART_Q_TRANS_MAGNET: return trans_magnet(P, h, m2);
+    case SART_Q_YAW: return double(h.yaw);
+    case SART_Q_ALPHA1: return double(h.a1);
+    case SART_Q_ALPHA2: return double(h.a2);
+    case SART_Q_PATH_CB: return double(h.path);
+    case SART_Q_DEVIATION_DET: return double(h.devDet);
+    default: return double(h.agas);
+  }
+}
+
+// The block-private part of the histograms in dynamic shared memory, behind everything else the kernel keeps there: the
+// counts as u32 (a block traces fewer than 2^32 rays), and with kSmemSums also Σw and Σw² as f64, so that a passed ray costs
+// shared-memory atomics only and the block adds its entries into the handle's arrays once, at its end (the f64 adds are
+// CAS loops in shared memory: ATOMS.CAST.SPIN.64). Without kSmemSums the sums go to the block replicas in global memory
+// (QuantityHists::rw, rw2) instead.
+struct QhistSmem {
+  double* w;
+  double* w2;
+  unsigned int* n;
+};
+// Bytes the launcher adds to the block's dynamic shared memory (16 for the alignment of the part).
+__host__ __device__ inline size_t qhist_smem_bytes(int entries, bool sums) {
+  return 16 + ((size_t(entries) * (sums ? 20 : 4) + 15) & ~size_t(15));
+}
+// The launchers' choice between the two: the replicas, unless SART_QHIST_SMEM is set and the block, `smem` bytes without the
+// histograms, still fits the per-block limit with the sums. Measured on B200 (tools/bench_quantity_hists.py, 1e9 rays,
+// 2 and 8 histograms at 256 bins, CAST+LLNL and BabyIAXO+XMM): the two within 2 % of each other, the replicas ahead in
+// three of the four cases.
+inline bool qhist_sums_in_smem(size_t smem, int entries) {
+  if (!std::getenv("SART_QHIST_SMEM")) return false;
+  int dev = 0, optin = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
+    return false;
+  return smem + qhist_smem_bytes(entries, true) <= size_t(optin);
+}
+// Lays the part over `base` (the end of the kernel's own shared memory) and zeroes it; before the kernel's first
+// __syncthreads.
+template <bool kSmemSums>
+__device__ __forceinline__ QhistSmem qhist_smem(unsigned char* base, const QuantityHists& Q) {
+  QhistSmem s;
+  const int e = Q.entries;
+  unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(base) + 15) & ~uintptr_t(15));
+  if (kSmemSums) {
+    s.w = reinterpret_cast<double*>(p); s.w2 = s.w + e; s.n = reinterpret_cast<unsigned int*>(s.w2 + e);
+  } else {
+    s.w = s.w2 = nullptr; s.n = reinterpret_cast<unsigned int*>(p);
+  }
+  for (int i = threadIdx.x; i < e; i += blockDim.x) {
+    s.n[i] = 0u;
+    if (kSmemSums) { s.w[i] = 0.0; s.w2[i] = 0.0; }
+  }
+  return s;
+}
+// The block's entries into the handle's arrays: the counts, and with kSmemSums the sums; once, at the end of the kernel.
+template <bool kSmemSums>
+__device__ __forceinline__ void qhist_flush(const QuantityHists& Q, const QhistSmem& s) {
+  __syncthreads();
+  for (int e = threadIdx.x; e < Q.entries; e += blockDim.x) {
+    const unsigned int c = s.n[e];
+    if (!c) continue;
+    atomicAdd(Q.n + e, (unsigned long long)c);
+    if (kSmemSums) { atomicAdd(Q.w + e, s.w[e]); atomicAdd(Q.w2 + e, s.w2[e]); }
+  }
+}
+
+// Sink of the quantity-histogram kernel variants: the generic sink with the radial histogram and the spectra checked at run
+// time, the band images checked at run time (B.w), and the histograms Q. kRecord: pathCB and deviationDet are computed,
+// as for a per-ray record. A derived sink like BandImageSink, so that every kernel variant without the histograms stays
+// what it was.
+template <bool kSmemSums>
+struct QuantityHistSink : ImageSinkT<true, true> {
+  static constexpr bool kRecord = true;
+  const FastParams& P;
+  const BandImages& B;
+  unsigned int* bandN;
+  uint32_t bandRep;
+  const QuantityHists& Q;
+  QhistSmem s;
+  uint32_t qRep;   // element offset of this block's replica of the sums (without kSmemSums)
+  __device__ __forceinline__ void hit(const RayResult& h) {
+    ImageSinkT<true, true>::hit(h);
+    const double wd = h.wPre * h.wPost;   // the weight ImageSinkT::hit tested
+    if (h.windowMiss || wd == 0.0) return;
+    if (B.w) band_hit(B, bandN, bandRep, h, wd);
+    // The lanes of a warp that hit the same entry first sum through the warp and one of them adds (as spec_add_warp): a
+    // distribution piles most rays into a few entries, and same-address f64 adds are serialised (in shared memory a CAS
+    // loop per add).
+    for (int j = 0; j < Q.nHists; ++j) {
+      const uint32_t e = uint32_t(Q.off[j] + qhist_entry(Q, j, record_quantity(P, h, m2, Q.quantity[j])));
+      const unsigned active = __activemask();
+      const unsigned peers = __match_any_sync(active, e);
+      double sw = 0.0, sw2 = 0.0;
+      if (peers == 0xffffffffu) {   // the whole warp in one entry (a distribution's peak): 5 butterfly steps, not 32 shuffles
+        sw = wd; sw2 = wd * wd;
+        for (int o = 16; o > 0; o >>= 1) {
+          sw += __shfl_xor_sync(peers, sw, o);
+          sw2 += __shfl_xor_sync(peers, sw2, o);
+        }
+      } else {
+        for (unsigned m = peers; m; m &= m - 1u) {
+          const double x = __shfl_sync(peers, wd, __ffs(m) - 1);
+          sw += x;
+          sw2 += x * x;
+        }
+      }
+      if ((threadIdx.x & 31u) != unsigned(__ffs(peers) - 1)) continue;
+      atomicAdd(s.n + e, unsigned(__popc(peers)));
+      if (kSmemSums) {
+        atomicAdd(s.w + e, sw);
+        atomicAdd(s.w2 + e, sw2);
+      } else {
+        atomicAdd(Q.rw + (qRep + e), sw);
+        atomicAdd(Q.rw2 + (qRep + e), sw2);
+      }
+    }
+  }
+};
+__device__ __forceinline__ uint32_t qhist_replica(const QuantityHists& Q) { return (blockIdx.x & Q.repMask) * Q.repStride; }
+// The sink of a fused kernel body shared by the variants without quantity histograms (kQH = 0: with_bands) and those with
+// them (kQH = 1: sums in shared memory, 2: sums in the block replicas).
+template <bool kBands, int kQH, class Sink>
+__device__ __forceinline__ auto with_extras(const Sink& sink, const FastParams& P, const BandImages& B, unsigned int* bandN,
+                                            const QuantityHists& Q, const QhistSmem& qs) {
+  if constexpr (kQH != 0)
+    return QuantityHistSink<kQH == 1>{sink, P, B, bandN, band_replica(B), Q, qs, qhist_replica(Q)};
+  else
+    return with_bands<kBands>(sink, B, bandN);
 }
 
 // ---- axion-mass scan: the part shared by the FP64-algebra and the FP32 tracing --------------------------------

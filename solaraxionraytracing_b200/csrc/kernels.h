@@ -64,11 +64,13 @@ cudaError_t launch_mc_rays_exact(const Params& P, const Tables& T, double mAxion
                                  int32_t* emit = nullptr);
 cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                   uint64_t nRays, uint64_t seed, double* image, double* imageW2,
-                                  sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands = {});
+                                  sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands = {},
+                                  const QuantityHists& qh = {});
 // re-trace of the uncertain rays of an FP32 launch (fast_params.h: RetraceQueue) by the exact pipeline
 cudaError_t launch_retrace_mc_image(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                     uint64_t seed, const fast::RetraceQueue& q, double* image, double* imageW2,
-                                    sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands = {});
+                                    sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands = {},
+                                    const QuantityHists& qh = {});
 cudaError_t launch_retrace_mc_rays(const Params& P, const Tables& T, double mAxion, uint64_t first, size_t n, uint64_t seed,
                                    const uint32_t* words, const fast::RetraceQueue& q, const sart_ray_out_t& out, int smCount,
                                    cudaStream_t s);
@@ -86,11 +88,13 @@ cudaError_t launch_build_cdfs(int nR, int nE, const double* radii, const double*
 
 // ---- "fast" pipeline (kernels_fast.cu)
 // bands: the band images (device_params.h: BandImages; w == nullptr: off), in modes 1 and 2 their replicas, which
-// launch_fold_replicas adds up after the launch; with them on, the launchers run the kernel variants that fill them
+// launch_fold_replicas adds up after the launch; with them on, the launchers run the kernel variants that fill them.
+// qh: the quantity histograms (device_params.h: QuantityHists; w == nullptr: off), whose replicas rw / rw2 the caller folds
+// after the launch as well; with them on, the launchers run the kernel variants that fill them and the band images.
 cudaError_t launch_mc_image_fast(const fast::FastParams& P, const fast::FastTables& T, double mAxion, uint64_t first,
                                  uint64_t nRays, uint64_t seed, double* image, double* imageW2,
                                  sart_counters_t* counters, int smCount, bool compact, cudaStream_t s,
-                                 const BandImages& bands = {});
+                                 const BandImages& bands = {}, const QuantityHists& qh = {});
 
 cudaError_t launch_mc_image_fast_masses(const fast::FastParams& P, const fast::FastTables& T, int nMasses,
                                         const double* dMasses, uint64_t first, uint64_t nRays, uint64_t seed,
@@ -105,7 +109,7 @@ cudaError_t launch_emission_rates(int nR, int nE, const double* dTemp, const dou
 cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T, double mAxion,
                                 uint64_t first, uint64_t nRays, uint64_t seed, double* image, double* imageW2,
                                 sart_counters_t* counters, int smCount, bool compact, cudaStream_t s,
-                                const BandImages& bands = {});
+                                const BandImages& bands = {}, const QuantityHists& qh = {});
 cudaError_t launch_mc_image_f32_masses(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T,
                                        int nMasses, const double* dMasses, uint64_t first, uint64_t nRays, uint64_t seed,
                                        double* acc, double* accW2, sart_counters_t* counters, int smCount, cudaStream_t s);

@@ -283,6 +283,104 @@ __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, i
   }
 }
 
+// A passed ray of the exact kernels into the quantity histograms Q (sart_enable_quantity_hists): its record values
+// (store_ray), one global atomic per array and histogram.
+__device__ __forceinline__ void qhist_add_exact(const QuantityHists& Q, const Geo& g, const Weights& w, const Final& f) {
+  for (int j = 0; j < Q.nHists; ++j) {
+    double v;
+    switch (Q.quantity[j]) {
+      case SART_Q_REFLECT: v = w.reflect; break;
+      case SART_Q_TRANS_MAGNET: v = f.transMagnet; break;
+      case SART_Q_YAW: v = g.ya; break;
+      case SART_Q_ALPHA1: v = g.alpha1; break;
+      case SART_Q_ALPHA2: v = g.alpha2; break;
+      case SART_Q_PATH_CB: v = g.pathCB; break;
+      case SART_Q_DEVIATION_DET: v = g.deviationDet; break;
+      default: v = w.absGas; break;
+    }
+    const int e = Q.off[j] + qhist_entry(Q, j, v);
+    atomicAdd(Q.n + e, 1ull);
+    atomicAdd(Q.w + e, f.w);
+    atomicAdd(Q.w2 + e, f.w * f.w);
+  }
+}
+
+// mc_image_ray with the quantity histograms Q: the passed rays of the first mass also go to Q, and to the band images B when
+// B.w != nullptr; the geometry is traced with the record fields (deviationDet) that trace_geometry<false> leaves out. A copy,
+// so that the kernels built from mc_image_ray keep the code they had before.
+__device__ __forceinline__ void mc_image_ray_qh(const Params& P, const Tables& T, int nMasses, const double* __restrict__ masses,
+                                                uint64_t seed, uint64_t ray, double* __restrict__ image,
+                                                double* __restrict__ imageW2, const BandImages& B, const QuantityHists& Q,
+                                                BlockCounters* bc, MassCounters* mc, ThreadSums& ts) {
+  const double step = (P.chipCX * 2.0 - 0.0) / double(SART_IMAGE_BINS);  // (stop - start)/rows rt:828-830
+  const double stepY = (P.chipCY * 2.0 - 0.0) / double(SART_IMAGE_BINS);
+  V3 O, E;
+  double energy;
+  int clamped = 0;
+  int eIdx = -1;
+  if (!sample_ray(P, T, seed, ray, O, E, energy, clamped, &eIdx)) {
+    atomicAdd(&bc->n_exit[SART_EXIT_COLLIMATOR], 1u);
+    return;
+  }
+  Geo g;
+  trace_geometry<true>(P, T, O, E, energy, g);
+  g.clamped |= clamped;
+  g.eIdx = eIdx;
+  if (g.code >= 0) {
+    atomicAdd(&bc->n_exit[g.code], 1u);
+    if (g.clamped) atomicAdd(&bc->n_clamped, 1u);
+    return;
+  }
+  Weights w;
+  ray_weights(P, T, g, w);
+  if (g.clamped) atomicAdd(&bc->n_clamped, 1u);
+  if (g.windowMiss) atomicAdd(&bc->n_exit[SART_EXIT_WINDOW_APERTURE], 1u);
+  for (int m = 0; m < nMasses; ++m) {
+    Final f;
+    ray_finish(P, g, w, masses[m], f);
+    const int code = f.code & SART_CODE_MASK;
+    if (m == 0) {   // the first (usually only) mass: per-thread registers
+      if (f.code & SART_FLAG_PASSED_TILL_WINDOW) ++ts.n_till;
+      if (code == SART_EXIT_ZERO_WEIGHT) ++ts.n_zero;
+      if (code != SART_EXIT_PASSED) continue;
+      ++ts.n_passed;
+      ts.sum_w += f.w; ts.sum_w2 += f.w * f.w; ts.sum_x += f.x; ts.sum_y += f.y; ts.sum_r += f.r;
+    } else {
+      if (f.code & SART_FLAG_PASSED_TILL_WINDOW) atomicAdd(&mc[m].n_till_window, 1ull);
+      if (code == SART_EXIT_ZERO_WEIGHT) atomicAdd(&mc[m].n_zero, 1ull);
+      if (code != SART_EXIT_PASSED) continue;
+      atomicAdd(&mc[m].n_passed, 1ull);
+      atomicAdd(&mc[m].sum_w, f.w);
+      atomicAdd(&mc[m].sum_w2, f.w * f.w);
+      atomicAdd(&mc[m].sum_x, f.x);
+      atomicAdd(&mc[m].sum_y, f.y);
+      atomicAdd(&mc[m].sum_r, f.r);
+    }
+    // prepareHeatmap rt:839-842
+    const double cx = floor((f.x - 0.0) / step), cy = floor((f.y - 0.0) / stepY);
+    if (cx >= 0.0 && cx < double(SART_IMAGE_BINS) && cy >= 0.0 && cy < double(SART_IMAGE_BINS)) {
+      const size_t bin = size_t(m) * SART_IMAGE_BINS * SART_IMAGE_BINS + size_t(int(cy)) * SART_IMAGE_BINS + size_t(int(cx));
+      atomicAdd(image + bin, f.w);
+      atomicAdd(imageW2 + bin, f.w * f.w);
+    }
+    if (T.rad.w && m == 0) {
+      int b = int(f.r * T.rad.invStep);
+      b = b < 0 ? 0 : (b > T.rad.nbins - 1 ? T.rad.nbins - 1 : b);
+      atomicAdd(T.rad.w + b, f.w);
+      atomicAdd(T.rad.n + b, 1ull);
+    }
+    // spectra: the first mass (sart_enable_spectra) or every mass into its own row (sart_enable_mass_spectra: eRow != 0);
+    // the X-ray source's rays carry no table index and go to bin nEnergies
+    if (T.spec.eW && (m == 0 || T.spec.eRow)) spec_add(T.spec, m, g.eIdx >= 0 ? g.eIdx : P.nEnergies, g.shell, f.w);
+    // band images (single mass only): the same energy index, the image bin of plane 0
+    if (m == 0 && B.w) {
+      const bool inImage = cx >= 0.0 && cx < double(SART_IMAGE_BINS) && cy >= 0.0 && cy < double(SART_IMAGE_BINS);
+      band_add(B, g.eIdx >= 0 ? g.eIdx : P.nEnergies, inImage ? int(cy) * SART_IMAGE_BINS + int(cx) : -1, f.w);
+    }
+    if (m == 0) qhist_add_exact(Q, g, w, f);
+  }
+}
+
 #ifndef SART_EXACT_MINBLOCKS
 #define SART_EXACT_MINBLOCKS 6   // 85 registers instead of 108: 24 instead of 16 warps per SM for this latency-bound kernel (+5 %; 8 is slower)
 #endif
@@ -375,6 +473,80 @@ k_trace_mc_image_bands(const __grid_constant__ Params P, const __grid_constant__
                        const __grid_constant__ BandImages B) {
   mc_image<true>(P, T, nMasses, masses, first, nRays, seed, list, listCount, listCap, image, imageW2, counters, B);
 }
+// The same with the quantity histograms Q, and the band images B when B.w != nullptr (single mass); a copy of mc_image for the
+// reason of mc_image_ray_qh.
+__global__ void __launch_bounds__(128, SART_EXACT_MINBLOCKS)
+k_trace_mc_image_qhists(const __grid_constant__ Params P, const __grid_constant__ Tables T, int nMasses,
+                        const double* __restrict__ masses, uint64_t first, uint64_t nRays, uint64_t seed,
+                        const uint32_t* __restrict__ list, const uint32_t* __restrict__ listCount, uint32_t listCap,
+                        double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                        const __grid_constant__ BandImages B, const __grid_constant__ QuantityHists Q) {
+  extern __shared__ unsigned char smem_raw[];
+  BlockCounters* bc = reinterpret_cast<BlockCounters*>(smem_raw);
+  MassCounters* mc = reinterpret_cast<MassCounters*>(smem_raw + sizeof(BlockCounters));
+  unsigned long long* nRaysBlock = &mc[0].pad;   // rays of this block (zeroed with the mass counters)
+  for (int k = threadIdx.x; k < int(sizeof(BlockCounters) / 4); k += blockDim.x)
+    reinterpret_cast<unsigned int*>(bc)[k] = 0u;
+  for (int k = threadIdx.x; k < int(nMasses * sizeof(MassCounters) / 8); k += blockDim.x)
+    reinterpret_cast<unsigned long long*>(mc)[k] = 0ull;
+  __syncthreads();
+
+  const uint64_t stride = uint64_t(gridDim.x) * blockDim.x;
+  ThreadSums ts;
+  // One loop for both modes, so that the per-ray code (8500 SASS instructions, most of them inlined f64 libm) exists once:
+  // this kernel waits for instruction fetches more than for anything else (profiles/README.md).
+  // List mode: the re-trace of the uncertain rays of an FP32 launch, which has counted them in n_rays already.
+  const bool listMode = list != nullptr;
+  const uint64_t total = listMode ? uint64_t(min(*listCount, listCap)) : nRays;
+  for (uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < total; i += stride) {
+    const uint64_t ray = first + (listMode ? uint64_t(list[i]) : i);
+    if (!listMode) ++ts.n_rays;
+    mc_image_ray_qh(P, T, nMasses, masses, seed, ray, image, imageW2, B, Q, bc, mc, ts);
+  }
+  if (listMode && blockIdx.x == 0 && threadIdx.x == 0)
+    for (int m = 0; m < nMasses; ++m) atomicAdd(reinterpret_cast<unsigned long long*>(&counters[m].n_retraced), (unsigned long long)total);
+  // the thread sums of the first mass: warp shuffle, then one shared-memory atomic per warp and quantity
+  for (int o = 16; o > 0; o >>= 1) {
+    ts.n_rays += __shfl_down_sync(0xffffffffu, ts.n_rays, o);
+    ts.n_passed += __shfl_down_sync(0xffffffffu, ts.n_passed, o);
+    ts.n_zero += __shfl_down_sync(0xffffffffu, ts.n_zero, o);
+    ts.n_till += __shfl_down_sync(0xffffffffu, ts.n_till, o);
+    ts.sum_w += __shfl_down_sync(0xffffffffu, ts.sum_w, o);
+    ts.sum_w2 += __shfl_down_sync(0xffffffffu, ts.sum_w2, o);
+    ts.sum_x += __shfl_down_sync(0xffffffffu, ts.sum_x, o);
+    ts.sum_y += __shfl_down_sync(0xffffffffu, ts.sum_y, o);
+    ts.sum_r += __shfl_down_sync(0xffffffffu, ts.sum_r, o);
+  }
+  if ((threadIdx.x & 31) == 0) {
+    atomicAdd(nRaysBlock, (unsigned long long)ts.n_rays);
+    atomicAdd(&mc[0].n_passed, (unsigned long long)ts.n_passed);
+    atomicAdd(&mc[0].n_zero, (unsigned long long)ts.n_zero);
+    atomicAdd(&mc[0].n_till_window, (unsigned long long)ts.n_till);
+    atomicAdd(&mc[0].sum_w, ts.sum_w); atomicAdd(&mc[0].sum_w2, ts.sum_w2);
+    atomicAdd(&mc[0].sum_x, ts.sum_x); atomicAdd(&mc[0].sum_y, ts.sum_y); atomicAdd(&mc[0].sum_r, ts.sum_r);
+  }
+  __syncthreads();
+  // flush
+  for (int m = threadIdx.x; m < nMasses; m += blockDim.x) {
+    sart_counters_t* c = counters + m;
+    atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_rays), *nRaysBlock);
+    for (int e = 1; e < SART_N_EXIT_CODES; ++e)
+      if (e != SART_EXIT_ZERO_WEIGHT && bc->n_exit[e])
+        atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_exit[e]), (unsigned long long)bc->n_exit[e]);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_exit[SART_EXIT_PASSED]), mc[m].n_passed);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_exit[SART_EXIT_ZERO_WEIGHT]), mc[m].n_zero);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_passed), mc[m].n_passed);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_passed_till_window), mc[m].n_till_window);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_hit_nickel), (unsigned long long)bc->n_exit[SART_EXIT_NICKEL]);
+    atomicAdd(reinterpret_cast<unsigned long long*>(&c->n_interp_clamped), (unsigned long long)bc->n_clamped);
+    atomicAdd(&c->sum_w, mc[m].sum_w);
+    atomicAdd(&c->sum_w2, mc[m].sum_w2);
+    atomicAdd(&c->sum_x, mc[m].sum_x);
+    atomicAdd(&c->sum_y, mc[m].sum_y);
+    atomicAdd(&c->sum_r, mc[m].sum_r);
+  }
+}
+
 
 // ---- CDF build rt:2679-2705 -------------------------------------------------------------------------------
 // One thread walks one radius row sequentially (the reference's summation order => identical bits).
@@ -452,15 +624,20 @@ cudaError_t launch_mc_rays_exact(const Params& P, const Tables& T, double mAxion
 
 cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                   uint64_t nRays, uint64_t seed, double* image, double* imageW2,
-                                  sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands) {
+                                  sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands,
+                                  const QuantityHists& qh) {
   if (nRays == 0) return cudaSuccess;
   const int block = 128;
   const size_t smem = sizeof(BlockCounters) + size_t(nMasses) * sizeof(MassCounters);
   unsigned grid = 0;   // one resident wave; the grid-stride loop covers the rest
-  const cudaError_t e = bands.w ? grid_size(k_trace_mc_image_bands, block, smem, nRays, smCount, 0, &grid)
-                                 : grid_size(k_trace_mc_image, block, smem, nRays, smCount, 0, &grid);
+  const cudaError_t e = qh.w      ? grid_size(k_trace_mc_image_qhists, block, smem, nRays, smCount, 0, &grid)
+                        : bands.w ? grid_size(k_trace_mc_image_bands, block, smem, nRays, smCount, 0, &grid)
+                                  : grid_size(k_trace_mc_image, block, smem, nRays, smCount, 0, &grid);
   if (e != cudaSuccess) return e;
-  if (bands.w)
+  if (qh.w)
+    k_trace_mc_image_qhists<<<grid, block, smem, s>>>(P, T, nMasses, masses, first, nRays, seed, nullptr, nullptr, 0u, image,
+                                                      imageW2, counters, bands, qh);
+  else if (bands.w)
     k_trace_mc_image_bands<<<grid, block, smem, s>>>(P, T, nMasses, masses, first, nRays, seed, nullptr, nullptr, 0u, image,
                                                      imageW2, counters, bands);
   else
@@ -472,16 +649,21 @@ cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses,
 // ---- re-trace launchers (fixed grids: the list length lives on the device) -------------------------------------
 cudaError_t launch_retrace_mc_image(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                     uint64_t seed, const fast::RetraceQueue& q, double* image, double* imageW2,
-                                    sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands) {
+                                    sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands,
+                                    const QuantityHists& qh) {
   const int block = 128;
   const size_t smem = sizeof(BlockCounters) + size_t(nMasses) * sizeof(MassCounters);
   int perSM = 0;
-  cudaError_t e = bands.w ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image_bands, block, smem)
-                           : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image, block, smem);
+  cudaError_t e = qh.w      ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image_qhists, block, smem)
+                  : bands.w ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image_bands, block, smem)
+                            : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image, block, smem);
   if (e != cudaSuccess) return e;
   if (perSM < 1) perSM = 1;
   // one resident wave (the list length lives on the device): latency-bound FP64 code wants every warp slot it can get
-  if (bands.w)
+  if (qh.w)
+    k_trace_mc_image_qhists<<<unsigned(smCount * perSM), block, smem, s>>>(P, T, nMasses, masses, first, 0, seed, q.list, q.count,
+                                                                          q.cap, image, imageW2, counters, bands, qh);
+  else if (bands.w)
     k_trace_mc_image_bands<<<unsigned(smCount * perSM), block, smem, s>>>(P, T, nMasses, masses, first, 0, seed, q.list, q.count,
                                                                          q.cap, image, imageW2, counters, bands);
   else

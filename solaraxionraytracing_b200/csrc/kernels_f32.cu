@@ -92,6 +92,64 @@ k_trace_mc_f32_bands(const __grid_constant__ FastParams P, const __grid_constant
                      const __grid_constant__ BandImages B) {
   f32_fused<kWolter, false, kAlias, kMargins, true, true>(P, G, T, mAxion2, first, nRays, K, image, imageW2, counters, B);
 }
+// The generic kind with the quantity histograms QH (sart_enable_quantity_hists; fast_common.cuh: QuantityHistSink), the band
+// images B checked at run time. kQH = 1: the block's sums in shared memory, 2: in the block replicas QH.rw / QH.rw2. A copy
+// of f32_fused rather than another instantiation of it: the kernels built from f32_fused keep the code they had before.
+template <bool kWolter, bool kAlias, bool kMargins, int kQH>
+__global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
+k_trace_mc_f32_qhists(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G, const __grid_constant__ FastTables T,
+                      double mAxion2, uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K,
+                      double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                      const __grid_constant__ BandImages B, const __grid_constant__ QuantityHists QH) {
+  constexpr bool kPlain = false;
+  extern __shared__ __align__(16) unsigned char smem[];
+  Smem32 S;
+  unsigned char* tail;
+  smem_layout32<kAlias>(P, smem, S, tail);
+  WarpCounters* wc = reinterpret_cast<WarpCounters*>(tail);
+  smem_fill32<kAlias>(P, T, S);
+  for (int i = threadIdx.x; i < kWarps32 * int(sizeof(WarpCounters) / 4); i += kBlock32) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
+  unsigned int* bandN = band_counts<true>();
+  const QhistSmem qs = qhist_smem<kQH == 1>(tail + kWarps32 * sizeof(WarpCounters), QH);
+  __syncthreads();
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  unsigned int nPassed = 0, nTill = 0, nIter = 0;
+  double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
+  const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
+  QuantityHistSink<kQH == 1> sink{{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR}, P, B,
+                                  bandN, band_replica(B), QH, qs, qhist_replica(QH)};
+  const uint64_t stride = uint64_t(gridDim.x) * kBlock32;
+  // 32-bit trip count + running 64-bit ray index: 5 loop instructions per ray instead of 12 (nRays <= kMaxRaysPerLaunch,
+  // so the count fits)
+  const uint64_t i0 = uint64_t(blockIdx.x) * kBlock32 + threadIdx.x;
+  nIter = i0 < nRays ? unsigned((nRays - 1 - i0) / stride) + 1u : 0u;
+  uint64_t ray = first + i0;
+  uint32_t id = uint32_t(i0);
+  const uint32_t stride32 = uint32_t(stride);
+  for (unsigned k = nIter; k != 0u; --k, ray += stride, id += stride32) {
+    Head32 hd;
+    stage_a32_head<kPlain, false, kAlias>(P, T, S, K, ray, hd);
+    Rec32 rec;
+    rec.id = id;
+    const int code = stage_a32<kWolter, false, kPlain, false, kAlias, kMargins>(P, G, T, S, hd, rec);
+    finish32<kWolter, kPlain, false, kMargins>(P, G, T, S, code, rec, sink);
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    nPassed += __shfl_down_sync(0xffffffffu, nPassed, o);
+    nTill += __shfl_down_sync(0xffffffffu, nTill, o);
+    nIter += __shfl_down_sync(0xffffffffu, nIter, o);
+    sumW += __shfl_down_sync(0xffffffffu, sumW, o);
+    sumW2 += __shfl_down_sync(0xffffffffu, sumW2, o);
+    sumX += __shfl_down_sync(0xffffffffu, sumX, o);
+    sumY += __shfl_down_sync(0xffffffffu, sumY, o);
+    sumR += __shfl_down_sync(0xffffffffu, sumR, o);
+  }
+  __syncwarp();
+  if (lane == 0) flush_counters(counters, wc[warp], nIter, nPassed, nTill, sumW, sumW2, sumX, sumY, sumR);
+  band_counts_flush(B, bandN);
+  qhist_flush<kQH == 1>(QH, qs);
+}
 
 // ---- fused kernel with warp-level compaction between stage A and stage B (see kernels_fast.cu) ----------------
 constexpr int kQueue32 = 64;
@@ -275,6 +333,98 @@ k_trace_mc_f32_compact_bands(const __grid_constant__ FastParams P, const __grid_
   if (lane == 0) flush_counters(counters, wc[warp], nIter, nPassed, nTill, sumW, sumW2, sumX, sumY, sumR);
   band_counts_flush(B, bandN);
 }
+// The same with the quantity histograms QH as well (k_trace_mc_f32_qhists), the band images checked at run time; a copy for
+// the same reason.
+template <bool kWolter, bool kAlias, bool kMargins, int kQH>
+__global__ void __launch_bounds__(kBlock32, SART_F32_MINBLOCKS)
+k_trace_mc_f32_compact_qhists(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G,
+                              const __grid_constant__ FastTables T, double mAxion2, uint64_t first, uint64_t nRays,
+                              const __grid_constant__ PhiloxKeys K, double* __restrict__ image, double* __restrict__ imageW2,
+                              sart_counters_t* __restrict__ counters, const __grid_constant__ BandImages B,
+                              const __grid_constant__ QuantityHists QH) {
+  constexpr bool kPlain = false;
+  extern __shared__ __align__(16) unsigned char smem[];
+  Smem32 S;
+  unsigned char* tail;
+  smem_layout32<kAlias>(P, smem, S, tail);
+  WarpCounters* wc = reinterpret_cast<WarpCounters*>(tail);
+  WarpQueue32* queues = reinterpret_cast<WarpQueue32*>(tail + kWarps32 * sizeof(WarpCounters));
+  smem_fill32<kAlias>(P, T, S);
+  for (int i = threadIdx.x; i < kWarps32 * int(sizeof(WarpCounters) / 4); i += kBlock32) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
+  unsigned int* bandN = band_counts<true>();
+  const QhistSmem qs = qhist_smem<kQH == 1>(reinterpret_cast<unsigned char*>(queues + kWarps32), QH);
+  __syncthreads();
+
+  constexpr unsigned kFull = 0xffffffffu;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  WarpQueue32& Q = queues[warp];
+  unsigned int nPassed = 0, nTill = 0, nIter = 0;
+  double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
+  const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
+  QuantityHistSink<kQH == 1> sink{{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR}, P, B,
+                                  bandN, band_replica(B), QH, qs, qhist_replica(QH)};
+  const uint64_t stride = uint64_t(gridDim.x) * kBlock32;
+  uint64_t base = uint64_t(blockIdx.x) * kBlock32 + (threadIdx.x & ~31);
+  const bool solar = kPlain || !P.testXray;
+  int qn = 0;
+  for (;;) {
+    while (qn <= kQueue32 - 32 && base < nRays) {
+      const uint64_t i = base + lane;
+      base += stride;
+      Rec32 rec;
+      int code = SART_N_EXIT_CODES;
+      if (i < nRays) {
+        Head32 hd;
+        stage_a32_head<kPlain, true, kAlias>(P, T, S, K, first + i, hd);
+        rec.id = uint32_t(i);
+        code = stage_a32<kWolter, false, kPlain, true, kAlias, kMargins>(P, G, T, S, hd, rec);
+        ++nIter;
+        if (code >= 0 && !(kMargins && rec.unc && sink.defer(rec.id))) sink.fail(code);
+      }
+      const unsigned m = __ballot_sync(kFull, code < 0);
+      if (code < 0) {
+        const int pos = qn + __popc(m & ((1u << lane) - 1u));
+        Q.x0[pos] = rec.x0; Q.y0[pos] = rec.y0; Q.tx[pos] = rec.tx; Q.ty[pos] = rec.ty; Q.rho0[pos] = rec.rho0;
+        Q.path2[pos] = rec.path2;
+        Q.meta[pos] = rec.hitLayer | ((solar ? rec.rIdx : rec.eIdx) << 8) | (rec.clamped ? (1 << 30) : 0) | (rec.unc ? (1 << 31) : 0);
+        Q.we[pos] = rec.we;
+        Q.id[pos] = rec.id;
+      }
+      qn += __popc(m);
+    }
+    if (qn == 0) break;
+    __syncwarp();
+    const int take = qn < 32 ? qn : 32;
+    if (lane < take) {
+      const int pos = qn - take + lane;
+      Rec32 rec;
+      rec.x0 = Q.x0[pos]; rec.y0 = Q.y0[pos]; rec.tx = Q.tx[pos]; rec.ty = Q.ty[pos]; rec.rho0 = Q.rho0[pos];
+      rec.path2 = Q.path2[pos];
+      const int meta = Q.meta[pos];
+      rec.hitLayer = meta & 0xff; rec.eIdx = (meta >> 8) & 0x3fffff; rec.clamped = (meta >> 30) & 1; rec.unc = meta < 0;
+      rec.id = Q.id[pos];
+      rec.bud = solar ? (0.0015f + float(rec.eIdx) * 0.0005f) : 1.0f;   // rs of the emission shell (rec.eIdx still holds it)
+      if (solar) rec.eIdx = energy_index<kAlias>(P, T, rec.eIdx, Q.we[pos], rec.clamped);
+      finish32<kWolter, kPlain, false, kMargins>(P, G, T, S, -1, rec, sink);
+    }
+    qn -= take;
+    __syncwarp();
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    nPassed += __shfl_down_sync(kFull, nPassed, o);
+    nTill += __shfl_down_sync(kFull, nTill, o);
+    nIter += __shfl_down_sync(kFull, nIter, o);
+    sumW += __shfl_down_sync(kFull, sumW, o);
+    sumW2 += __shfl_down_sync(kFull, sumW2, o);
+    sumX += __shfl_down_sync(kFull, sumX, o);
+    sumY += __shfl_down_sync(kFull, sumY, o);
+    sumR += __shfl_down_sync(kFull, sumR, o);
+  }
+  __syncwarp();
+  if (lane == 0) flush_counters(counters, wc[warp], nIter, nPassed, nTill, sumW, sumW2, sumX, sumY, sumR);
+  band_counts_flush(B, bandN);
+  qhist_flush<kQH == 1>(QH, qs);
+}
 // ---- axion-mass scan with FP32 tracing (the per-mass weighting is fast_common.cuh's mass_scan_loop) --------------
 template <bool kWolter, bool kMargins, int kPer, bool kSpectra>
 __device__ __forceinline__ void f32_masses(const FastParams& P, const Geo32& G, const FastTables& T,
@@ -325,28 +475,45 @@ k_trace_mc_f32_masses_spectra(const __grid_constant__ FastParams P, const __grid
 // One launch of at most fast::kMaxRaysPerLaunch rays (api.cu cuts longer runs).
 cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T, double mAxion,
                                 uint64_t first, uint64_t nRays, uint64_t seed, double* image, double* imageW2,
-                                sart_counters_t* counters, int smCount, bool compact, cudaStream_t s, const BandImages& bands) {
+                                sart_counters_t* counters, int smCount, bool compact, cudaStream_t s, const BandImages& bands,
+                                const QuantityHists& qh) {
   if (nRays == 0) return cudaSuccess;
   const LaunchVariant v = launch_variant(P, T);
-  // the plain-run kernels compile the radial histogram, the spectra and the band images out
-  const bool plain = v.plain && !T.rad.w && !T.spec.eW && !bands.w;
+  // the plain-run kernels compile the radial histogram, the spectra, the band images and the quantity histograms out
+  const bool plain = v.plain && !T.rad.w && !T.spec.eW && !bands.w && !qh.w;
   const size_t smem = fast::smem_bytes32(P, fast::kWarps32, v.alias) + (compact ? fast::kWarps32 * sizeof(fast::WarpQueue32) : 0);
   // variant 0: inverse-CDF sampler, pure FP32; 1: inverse-CDF sampler with the margin tests (re-trace queue attached); 2: alias
   // sampler (no re-trace: its ray <-> index mapping is not the exact pipeline's)
   const int variant = v.alias ? 2 : (v.margins ? 1 : 0);
-  auto run = [&](auto kern, auto... bandArg) {
-    cudaError_t e = fast::set_smem(kern, smem);
+  auto run_smem = [&](size_t sm, auto kern, auto... extra) {
+    cudaError_t e = fast::set_smem(kern, sm);
     if (e != cudaSuccess) return e;
     unsigned grid = 0;
-    if ((e = grid_size(kern, fast::kBlock32, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
-    kern<<<grid, fast::kBlock32, smem, s>>>(P, G, T, mAxion * mAxion, first, nRays, philox_round_keys(seed), image, imageW2, counters,
-                                            bandArg...);
+    if ((e = grid_size(kern, fast::kBlock32, sm, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
+    kern<<<grid, fast::kBlock32, sm, s>>>(P, G, T, mAxion * mAxion, first, nRays, philox_round_keys(seed), image, imageW2, counters,
+                                           extra...);
     return cudaGetLastError();
   };
+  auto run = [&](auto kern, auto... bandArg) { return run_smem(smem, kern, bandArg...); };
   if (getenv("SART_DEBUG"))
-    fprintf(stderr, "[sart] k_trace_mc_f32 compact=%d wolter=%d plain=%d alias=%d bands=%d (sampler=%d ra=%p ea=%p) smem=%zu\n",
-            int(compact), int(v.wolter), int(plain), int(v.alias), bands.nBands, T.sampler, (const void*)T.radiusAlias,
-            (const void*)T.energyAlias, smem);
+    fprintf(stderr, "[sart] k_trace_mc_f32 compact=%d wolter=%d plain=%d alias=%d bands=%d qhists=%d (sampler=%d ra=%p ea=%p) "
+            "smem=%zu\n", int(compact), int(v.wolter), int(plain), int(v.alias), bands.nBands, qh.nHists, T.sampler,
+            (const void*)T.radiusAlias, (const void*)T.energyAlias, smem);
+  if (qh.w) {   // the generic kind with the quantity histograms: everything else is checked at run time
+    const bool smemSums = fast::qhist_sums_in_smem(smem, qh.entries);
+    using KernQ = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, uint64_t, uint64_t, PhiloxKeys, double*,
+                           double*, sart_counters_t*, BandImages, QuantityHists);
+    // [compact][wolter][variant][sums in shared memory]
+#define SART_VAR(K, W, A, M) {fast::K<W, A, M, 2>, fast::K<W, A, M, 1>}
+#define SART_ROW(K, W) {SART_VAR(K, W, false, false), SART_VAR(K, W, false, true), SART_VAR(K, W, true, false)}
+    static const KernQ table[2][2][3][2] = {{SART_ROW(k_trace_mc_f32_qhists, false), SART_ROW(k_trace_mc_f32_qhists, true)},
+                                            {SART_ROW(k_trace_mc_f32_compact_qhists, false),
+                                             SART_ROW(k_trace_mc_f32_compact_qhists, true)}};
+#undef SART_ROW
+#undef SART_VAR
+    return run_smem(smem + fast::qhist_smem_bytes(qh.entries, smemSums),
+                    table[compact ? 1 : 0][v.wolter ? 1 : 0][variant][smemSums ? 1 : 0], bands, qh);
+  }
   if (bands.w) {   // the generic kind with the band images: the radial histogram and the spectra are checked at run time
     using KernB = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, double, uint64_t, uint64_t, PhiloxKeys, double*,
                            double*, sart_counters_t*, BandImages);

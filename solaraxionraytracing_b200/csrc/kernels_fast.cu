@@ -534,12 +534,14 @@ __device__ __forceinline__ void trace_one(const FastParams& P, const FastTables&
 }
 
 // ---- fused kernel ---------------------------------------------------------------------------------------------
-// kBands: the variant that also fills the band images B (sart_enable_band_images; fast_common.cuh: ImageSinkT).
-template <bool kWolter, bool kBands>
+// kBands: the variant that also fills the band images B (sart_enable_band_images; fast_common.cuh: ImageSinkT). kQH: the
+// variant that also fills the quantity histograms Q (sart_enable_quantity_hists; fast_common.cuh: QuantityHistSink), with
+// the band images checked at run time; 1: the block's sums in shared memory, 2: in the block replicas Q.rw / Q.rw2.
+template <bool kWolter, bool kBands, int kQH = 0>
 __device__ __forceinline__ void fast_fused(const FastParams& P, const FastTables& T, double mAxion2, uint64_t first,
                                            uint64_t nRays, uint64_t seed, double* __restrict__ image,
                                            double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
-                                           const BandImages& B) {
+                                           const BandImages& B, const QuantityHists& Q) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem S;
   unsigned char* tail;
@@ -547,7 +549,9 @@ __device__ __forceinline__ void fast_fused(const FastParams& P, const FastTables
   WarpCounters* wc = reinterpret_cast<WarpCounters*>(tail);
   smem_fill(P, T, S);
   for (int i = threadIdx.x; i < kWarpsF * int(sizeof(WarpCounters) / 4); i += kBlockF) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
-  unsigned int* bandN = band_counts<kBands>();
+  unsigned int* bandN = band_counts<kBands || kQH != 0>();
+  QhistSmem qs{};
+  if constexpr (kQH != 0) qs = qhist_smem<kQH == 1>(tail + kWarpsF * sizeof(WarpCounters), Q);
   __syncthreads();
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -555,8 +559,8 @@ __device__ __forceinline__ void fast_fused(const FastParams& P, const FastTables
   double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
 
   const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
-  auto sink = with_bands<kBands>(ImageSink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR},
-                                  B, bandN);
+  auto sink = with_extras<kBands, kQH>(ImageSink{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY,
+                                                 sumR}, P, B, bandN, Q, qs);
   const uint64_t stride = uint64_t(gridDim.x) * kBlockF;
   for (uint64_t i = uint64_t(blockIdx.x) * kBlockF + threadIdx.x; i < nRays; i += stride) {
     ++nIter;
@@ -591,21 +595,30 @@ __device__ __forceinline__ void fast_fused(const FastParams& P, const FastTables
     atomicAdd(&c->sum_w, sumW); atomicAdd(&c->sum_w2, sumW2);
     atomicAdd(&c->sum_x, sumX); atomicAdd(&c->sum_y, sumY); atomicAdd(&c->sum_r, sumR);
   }
-  if (kBands) band_counts_flush(B, bandN);
+  if (kBands || kQH != 0) band_counts_flush(B, bandN);
+  if constexpr (kQH != 0) qhist_flush<kQH == 1>(Q, qs);
 }
 template <bool kWolter>
 __global__ void __launch_bounds__(kBlockF, 1)
 k_trace_mc_fast(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
                 uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
                 double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
-  fast_fused<kWolter, false>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, BandImages{});
+  fast_fused<kWolter, false>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, BandImages{}, QuantityHists{});
 }
 template <bool kWolter>
 __global__ void __launch_bounds__(kBlockF, 1)
 k_trace_mc_fast_bands(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
                       uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
                       double* __restrict__ imageW2, sart_counters_t* __restrict__ counters, const __grid_constant__ BandImages B) {
-  fast_fused<kWolter, true>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, B);
+  fast_fused<kWolter, true>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, B, QuantityHists{});
+}
+template <bool kWolter, int kQH>
+__global__ void __launch_bounds__(kBlockF, 1)
+k_trace_mc_fast_qhists(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
+                       uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                       double* __restrict__ imageW2, sart_counters_t* __restrict__ counters, const __grid_constant__ BandImages B,
+                       const __grid_constant__ QuantityHists Q) {
+  fast_fused<kWolter, false, kQH>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, B, Q);
 }
 
 // ---- fused kernel with warp-level compaction ------------------------------------------------------------------
@@ -721,6 +734,98 @@ k_trace_mc_fast_compact_bands(const __grid_constant__ FastParams P, const __grid
   fast_fused_compact<kWolter, true>(P, T, mAxion2, first, nRays, seed, image, imageW2, counters, B);
 }
 
+// The same with the quantity histograms QH (kQH as in fast_fused), the band images checked at run time. A copy rather than
+// another instantiation of fast_fused_compact, so that the kernels built from that keep the code they had before.
+template <bool kWolter, int kQH>
+__global__ void __launch_bounds__(kBlockF, 1)
+k_trace_mc_fast_compact_qhists(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T, double mAxion2,
+                               uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
+                               double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                               const __grid_constant__ BandImages B, const __grid_constant__ QuantityHists QH) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  Smem S;
+  unsigned char* tail;
+  smem_layout(P, smem, S, tail);
+  WarpCounters* wc = reinterpret_cast<WarpCounters*>(tail);
+  WarpQueue* queues = reinterpret_cast<WarpQueue*>(tail + kWarpsF * sizeof(WarpCounters));
+  smem_fill(P, T, S);
+  for (int i = threadIdx.x; i < kWarpsF * int(sizeof(WarpCounters) / 4); i += kBlockF) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
+  unsigned int* bandN = band_counts<true>();
+  const QhistSmem qs = qhist_smem<kQH == 1>(reinterpret_cast<unsigned char*>(queues + kWarpsF), QH);
+  __syncthreads();
+
+  constexpr unsigned kFull = 0xffffffffu;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  WarpQueue& Q = queues[warp];
+  unsigned int nPassed = 0, nTill = 0, nIter = 0;
+  double sumW = 0.0, sumW2 = 0.0, sumX = 0.0, sumY = 0.0, sumR = 0.0;
+  const uint64_t stride = uint64_t(gridDim.x) * kBlockF;
+  const uint32_t rep = T.nImgRep > 1 ? (blockIdx.x % unsigned(T.nImgRep)) * uint32_t(T.imgRepStride) : 0u;
+  QuantityHistSink<kQH == 1> sink{{T, mAxion2, image, imageW2, rep, wc[warp], nPassed, nTill, sumW, sumW2, sumX, sumY, sumR}, P, B,
+                                  bandN, band_replica(B), QH, qs, qhist_replica(QH)};
+  uint64_t base = uint64_t(blockIdx.x) * kBlockF + (threadIdx.x & ~31);   // warp-uniform
+  int qn = 0;                                                              // warp-uniform queue fill
+  for (;;) {
+    while (qn <= kQueue - 32 && base < nRays) {
+      const uint64_t i = base + lane;
+      base += stride;
+      Rec rec;
+      int code = SART_N_EXIT_CODES;
+      if (i < nRays) {
+        code = stage_a<kWolter>(P, T, S, seed, first + i, rec);
+        ++nIter;
+        if (code >= 0) atomicAdd(&wc[warp].n_exit[code], 1u);
+      }
+      const unsigned m = __ballot_sync(kFull, code < 0);
+      if (code < 0) {
+        const int pos = qn + __popc(m & ((1u << lane) - 1u));
+        Q.x0[pos] = rec.x0; Q.y0[pos] = rec.y0; Q.tx[pos] = rec.tx; Q.ty[pos] = rec.ty; Q.path2[pos] = rec.path2;
+        Q.meta[pos] = rec.hitLayer | (rec.eIdx << 8) | (rec.clamped ? (1 << 30) : 0);
+      }
+      qn += __popc(m);
+    }
+    if (qn == 0) break;
+    __syncwarp();
+    const int take = qn < 32 ? qn : 32;
+    if (lane < take) {
+      const int pos = qn - take + lane;
+      Rec rec;
+      rec.x0 = Q.x0[pos]; rec.y0 = Q.y0[pos]; rec.tx = Q.tx[pos]; rec.ty = Q.ty[pos]; rec.path2 = Q.path2[pos];
+      const int meta = Q.meta[pos];
+      rec.hitLayer = meta & 0xff; rec.eIdx = (meta >> 8) & 0x3fffff; rec.clamped = (meta >> 30) & 1;
+      stage_b<kWolter>(P, T, S, rec, sink);
+    }
+    qn -= take;
+    __syncwarp();
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    nPassed += __shfl_down_sync(kFull, nPassed, o);
+    nTill += __shfl_down_sync(kFull, nTill, o);
+    nIter += __shfl_down_sync(kFull, nIter, o);
+    sumW += __shfl_down_sync(kFull, sumW, o);
+    sumW2 += __shfl_down_sync(kFull, sumW2, o);
+    sumX += __shfl_down_sync(kFull, sumX, o);
+    sumY += __shfl_down_sync(kFull, sumY, o);
+    sumR += __shfl_down_sync(kFull, sumR, o);
+  }
+  __syncwarp();
+  if (lane == 0) {
+    sart_counters_t* c = counters;
+    auto addu = [](uint64_t* p, unsigned long long v) { if (v) atomicAdd(reinterpret_cast<unsigned long long*>(p), v); };
+    addu(&c->n_rays, nIter);
+    addu(&c->n_exit[SART_EXIT_PASSED], nPassed);
+    addu(&c->n_passed, nPassed);
+    addu(&c->n_passed_till_window, nTill);
+    for (int e = 1; e < SART_N_EXIT_CODES; ++e) addu(&c->n_exit[e], wc[warp].n_exit[e]);
+    addu(&c->n_hit_nickel, wc[warp].n_exit[SART_EXIT_NICKEL]);
+    addu(&c->n_interp_clamped, wc[warp].n_clamped);
+    atomicAdd(&c->sum_w, sumW); atomicAdd(&c->sum_w2, sumW2);
+    atomicAdd(&c->sum_x, sumX); atomicAdd(&c->sum_y, sumY); atomicAdd(&c->sum_r, sumR);
+  }
+  band_counts_flush(B, bandN);
+  qhist_flush<kQH == 1>(QH, qs);
+}
+
 // ---- fused kernel, axion-mass scan ---------------------------------------------------------------------------
 // Rays are traced once (lanes = rays); each ray that reaches the weight stage is then broadcast through the warp and
 // weighted for all M masses at once with lanes = masses (mass lane + 32 k), so the per-mass sums live in registers of
@@ -787,18 +892,33 @@ size_t smem_bytes(const FastParams& P, int nWarps = kWarps) {
 
 cudaError_t launch_mc_image_fast(const fast::FastParams& P, const fast::FastTables& T, double mAxion, uint64_t first,
                                  uint64_t nRays, uint64_t seed, double* image, double* imageW2,
-                                 sart_counters_t* counters, int smCount, bool compact, cudaStream_t s, const BandImages& bands) {
+                                 sart_counters_t* counters, int smCount, bool compact, cudaStream_t s, const BandImages& bands,
+                                 const QuantityHists& qh) {
   if (nRays == 0) return cudaSuccess;
   const bool wolter = launch_variant(P, T).wolter;
   const size_t smem = fast::smem_bytes(P, fast::kWarpsF) + (compact ? fast::kWarpsF * sizeof(fast::WarpQueue) : 0);
-  auto run = [&](auto kern, auto... bandArg) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+  auto run_smem = [&](size_t sm, auto kern, auto... extra) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(sm));
     if (e != cudaSuccess) return e;
     unsigned grid = 0;
-    if ((e = grid_size(kern, fast::kBlockF, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
-    kern<<<grid, fast::kBlockF, smem, s>>>(P, T, mAxion * mAxion, first, nRays, seed, image, imageW2, counters, bandArg...);
+    if ((e = grid_size(kern, fast::kBlockF, sm, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
+    kern<<<grid, fast::kBlockF, sm, s>>>(P, T, mAxion * mAxion, first, nRays, seed, image, imageW2, counters, extra...);
     return cudaGetLastError();
   };
+  auto run = [&](auto kern, auto... bandArg) { return run_smem(smem, kern, bandArg...); };
+  if (qh.w) {   // the variants with the quantity histograms, the band images checked at run time
+    const bool smemSums = fast::qhist_sums_in_smem(smem, qh.entries);
+    using KernQ = void (*)(fast::FastParams, fast::FastTables, double, uint64_t, uint64_t, uint64_t, double*, double*,
+                           sart_counters_t*, BandImages, QuantityHists);
+    // [compact][wolter][sums in shared memory]
+    static const KernQ table[2][2][2] = {
+        {{fast::k_trace_mc_fast_qhists<false, 2>, fast::k_trace_mc_fast_qhists<false, 1>},
+         {fast::k_trace_mc_fast_qhists<true, 2>, fast::k_trace_mc_fast_qhists<true, 1>}},
+        {{fast::k_trace_mc_fast_compact_qhists<false, 2>, fast::k_trace_mc_fast_compact_qhists<false, 1>},
+         {fast::k_trace_mc_fast_compact_qhists<true, 2>, fast::k_trace_mc_fast_compact_qhists<true, 1>}}};
+    return run_smem(smem + fast::qhist_smem_bytes(qh.entries, smemSums), table[compact ? 1 : 0][wolter ? 1 : 0][smemSums ? 1 : 0],
+                    bands, qh);
+  }
   if (bands.w)
     return run(compact ? (wolter ? fast::k_trace_mc_fast_compact_bands<true> : fast::k_trace_mc_fast_compact_bands<false>)
                        : (wolter ? fast::k_trace_mc_fast_bands<true> : fast::k_trace_mc_fast_bands<false>), bands);

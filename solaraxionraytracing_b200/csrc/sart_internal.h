@@ -52,7 +52,7 @@ inline size_t merged_words(int nMasses) {
 }
 
 // sart_allreduce_outputs (comm.cu): int64 words of the descriptor the ranks exchange, in sart_handle::d_desc
-constexpr int kDescCapacity = 64;
+constexpr int kDescCapacity = 128;
 
 // Bump allocator over one device buffer: every piece starts on a 256-byte boundary. Over a null base it only measures, so a
 // layout is written once and run twice: over nullptr to size the buffer, then over the allocation to hand out its pointers.
@@ -68,26 +68,30 @@ struct Carve {
 
 // The optional accumulators of the passed rays, each switched on and off by its own entry point: the radial histogram
 // (sart_enable_radial_hist), the spectra (sart_enable_spectra), the per-mass spectra (sart_enable_mass_spectra) and the
-// band images (sart_enable_band_images).
-enum AccumKind { kRadialHist, kSpectra, kMassSpectra, kBandImages, kAccums };
-constexpr AccumKind kAllAccums[kAccums] = {kRadialHist, kSpectra, kMassSpectra, kBandImages};
+// band images (sart_enable_band_images) and the quantity histograms (sart_enable_quantity_hists).
+enum AccumKind { kRadialHist, kSpectra, kMassSpectra, kBandImages, kQuantityHists, kAccums };
+constexpr AccumKind kAllAccums[kAccums] = {kRadialHist, kSpectra, kMassSpectra, kBandImages, kQuantityHists};
 
 // One block of an accumulator: the handle's own (sart_handle::accum) or its merged copy (sart_handle::merged_accum), both
 // one allocation laid out by the same code (api.cu: alloc_accum). blob == nullptr: off (and bins == 0).
 struct Accum {
   void* blob = nullptr;
   size_t bytes = 0;
-  int bins = 0;         // radial histogram: its bins; (per-mass) spectra: energy bins per row, nEnergies + 1; band images: bands
+  int bins = 0;         // radial histogram: its bins; (per-mass) spectra: energy bins per row, nEnergies + 1; band images: bands;
+                        // quantity histograms: their entries, Σ(nbins + 2)
   double rmax = 0.0;    // radial histogram: its range
   double edges[SART_MAX_BANDS + 1] = {};   // band images: the bins + 1 band edges [keV]
+  int n_qhists = 0;                        // quantity histograms: their specs, in the caller's order
+  sart_quantity_hist_t qspecs[SART_N_QUANTITIES] = {};
   RadialHist rad{};     // radial histogram: w, n
   Spectra spec{};       // (per-mass) spectra: eW, eW2, eN, sW, sN; the per-mass spectra have one row per mass (eRow, sRow)
   BandImages band{};    // band images: w, w2 [bins][256][256], n [bins]; the handle's block also its energy -> band table
+  QuantityHists qh{};   // quantity histograms: w, w2, n [bins]; the handle's block also the specs and the replicas rw, rw2
   int valid = 0;        // merged copy: it holds the sums of the last sart_allreduce_outputs for the masses set
   // The handle's own block only: the buffers the throughput kernels add into instead (api.cu: carve_throughput), which the
   // fold after every launch adds into the arrays above and clears. The spectra's replicas, the per-mass spectra's
   // mass-minor accumulators, the band images' replicas (tput_band, which also holds the energy -> band table); the radial
-  // histogram has none.
+  // histogram has none, the quantity histograms keep theirs in qh.
   void* tput_blob = nullptr;
   Spectra tput{};
   BandImages tput_band{};
@@ -110,6 +114,10 @@ inline void accum_arrays(AccumKind k, A& a, B& b, size_t rows, F&& f) {
   if (k == kBandImages) {
     const size_t p = e * SART_IMAGE_BINS * SART_IMAGE_BINS;
     f(a.band.w, b.band.w, p); f(a.band.w2, b.band.w2, p); f(a.band.n, b.band.n, e);
+    return;
+  }
+  if (k == kQuantityHists) {
+    f(a.qh.w, b.qh.w, e); f(a.qh.w2, b.qh.w2, e); f(a.qh.n, b.qh.n, e);
     return;
   }
   f(a.spec.eW, b.spec.eW, e); f(a.spec.eW2, b.spec.eW2, e); f(a.spec.eN, b.spec.eN, e);

@@ -20,7 +20,7 @@ import numpy as np
 
 from . import abi
 from ._lib import check, lib
-from .output import BandImages, Spectra
+from .output import BandImages, QuantityHist, Spectra
 
 
 def shard(n_rays: int, rank: int, world: int, first_ray: int = 0) -> tuple[int, int]:
@@ -172,6 +172,7 @@ class DevicesResult:
     spectra: Spectra | list[Spectra] | None  # one Spectra (at most one mass) or one per mass (a mass scan)
     precision: int                           # the precision mode the run took
     band_images: BandImages | None = None    # the band images of `bands` (RayTracer.read_band_images)
+    quantity_hists: list[QuantityHist] | None = None   # the histograms of `quantity_hists` (RayTracer.read_quantity_hists)
 
 
 def _open_tracers(fullSetup, devices, precision: int, sampler, masses, warn):
@@ -199,13 +200,15 @@ def _open_tracers(fullSetup, devices, precision: int, sampler, masses, warn):
 
 
 def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, precision: int = 2, sampler=None,
-                     masses=None, radial_hist: bool = False, spectra: bool = False, bands=None, warn=None) -> DevicesResult:
+                     masses=None, radial_hist: bool = False, spectra: bool = False, bands=None, quantity_hists=None,
+                     warn=None) -> DevicesResult:
     """The fused run of `nRays` rays over `devices`, one process: device k traces shard(nRays, k, n) of the global rays,
     so the result is that of one GPU tracing all of them, up to the order of the floating-point sums. The shards run
     concurrently (trace_mc only queues work); then sart_allreduce and, with `radial_hist` or `spectra`,
     sart_allreduce_outputs merge them. `spectra` means the single-mass spectra for at most one axion mass and the per-mass
     spectra for a mass scan. `bands`: the edges of the band images (RayTracer.enable_band_images; at most one axion
-    mass). `warn` receives the precision fall-back messages (see raytracer.set_fastest_precision)."""
+    mass). `quantity_hists`: the specs of the quantity histograms (RayTracer.enable_quantity_hists; at most one axion mass).
+    `warn` receives the precision fall-back messages (see raytracer.set_fastest_precision)."""
     tracers, mode = _open_tracers(fullSetup, devices, precision, sampler, masses, warn)
     try:
         scan = masses is not None and len(masses) > 1
@@ -216,6 +219,8 @@ def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, p
                 t.enable_mass_spectra() if scan else t.enable_spectra()
             if bands is not None:
                 t.enable_band_images(bands)
+            if quantity_hists:
+                t.enable_quantity_hists(quantity_hists)
             t.reset_image()
         comm_init_all(tracers)
         for rank, t in enumerate(tracers):
@@ -223,14 +228,15 @@ def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, p
             if count:
                 t.trace_mc(count, seed, first_ray=first)
         allreduce(tracers)
-        if radial_hist or spectra or bands is not None:
+        if radial_hist or spectra or bands is not None or quantity_hists:
             allreduce_outputs(tracers)
         t0 = tracers[0]
         merged_spectra = None
         if spectra:
             merged_spectra = t0.read_merged_mass_spectra() if scan else t0.read_merged_spectra()
         return DevicesResult(t0.read_merged(), t0.read_merged_radial_hist() if radial_hist else None, merged_spectra, mode,
-                             t0.read_merged_band_images() if bands is not None else None)
+                             t0.read_merged_band_images() if bands is not None else None,
+                             t0.read_merged_quantity_hists() if quantity_hists else None)
     finally:
         for t in tracers:
             t.close()

@@ -308,6 +308,112 @@ def write_band_image_csvs(bands: BandImages, windowYear: int, outpath: str | Pat
                                   chipXMax, chipYMax, precision) for sfx, img in zip(names, bands.image)]
 
 
+@dataclass
+class QuantityHist:
+    """Weighted histogram of one per-ray record quantity of the passed rays of a run (RayTracer.enable_quantity_hists).
+    Entry 0 is the underflow (v < lo), entries 1 .. nbins the regular bins [edges[k-1], edges[k]), entry nbins + 1 the
+    overflow (v >= hi or NaN)."""
+    name: str               # a field of sart_ray_out_t: abi.QUANTITIES
+    edges: np.ndarray       # [nbins + 1] lo + (hi - lo) k / nbins
+    sum_w: np.ndarray       # [nbins + 2] Σw
+    sum_w2: np.ndarray      # [nbins + 2] Σw²
+    counts: np.ndarray      # [nbins + 2] uint64
+
+
+def check_quantity_hist_specs(specs) -> list[tuple[str, int, float, float]]:
+    """The specs of RayTracer.enable_quantity_hists, [(name, nbins, lo, hi), ...], checked like sart_enable_quantity_hists
+    checks them: at most one histogram per quantity, names from abi.QUANTITIES, 1 .. abi.MAX_QHIST_BINS bins, lo and hi
+    finite with lo < hi. Raises ValueError."""
+    out = []
+    for spec in specs:
+        try:
+            name, nbins, lo, hi = spec
+        except (TypeError, ValueError):
+            raise ValueError(f"a histogram spec is (name, nbins, lo, hi), got {spec!r}") from None
+        if name not in abi.QUANTITIES:
+            raise ValueError(f"unknown quantity {name!r}; one of {', '.join(abi.QUANTITIES)}")
+        if any(name == o[0] for o in out):
+            raise ValueError(f"quantity {name!r} is histogrammed twice")
+        if isinstance(nbins, bool) or int(nbins) != nbins or not 1 <= int(nbins) <= abi.MAX_QHIST_BINS:
+            raise ValueError(f"{name}: need 1 to {abi.MAX_QHIST_BINS} bins, got {nbins!r}")
+        lo, hi = float(lo), float(hi)
+        if not (np.isfinite(lo) and np.isfinite(hi) and lo < hi):
+            raise ValueError(f"{name}: lo and hi must be finite with lo < hi, got {lo!r}, {hi!r}")
+        out.append((name, int(nbins), lo, hi))
+    return out
+
+
+def parse_quantity_hist(text: str) -> tuple[str, int, float, float]:
+    """One value of --histogram: `NAME:NBINS:LO:HI`, e.g. `transMagnet:256:0:1e-20`."""
+    parts = text.split(":")
+    if len(parts) != 4:
+        raise ValueError(f"expected NAME:NBINS:LO:HI, got {text!r}")
+    name, nbins, lo, hi = parts
+    try:
+        n, a, b = int(nbins), float(lo), float(hi)
+    except ValueError:
+        raise ValueError(f"expected NAME:NBINS:LO:HI with an integer NBINS and numbers LO, HI, got {text!r}") from None
+    return check_quantity_hist_specs([(name, n, a, b)])[0]
+
+
+def quantity_hist_entries(values, nbins: int, lo: float, hi: float) -> np.ndarray:
+    """The entry of each value in a histogram of `nbins` bins over [lo, hi), the binning of sart_enable_quantity_hists bit
+    for bit: 0 if v < lo, nbins + 1 if not v < hi (NaN included), else 1 + fmin(floor((v - lo) * inv), nbins - 1) with
+    inv = nbins / (hi - lo), every operation rounded on its own."""
+    v = np.asarray(values, dtype=np.float64)
+    lo, hi = np.float64(lo), np.float64(hi)
+    inv = np.float64(nbins) / (hi - lo)
+    with np.errstate(invalid="ignore", over="ignore"):
+        reg = 1.0 + np.fmin(np.floor((v - lo) * inv), np.float64(nbins - 1))
+        e = np.where(v < lo, 0.0, np.where(~(v < hi), np.float64(nbins + 1), reg))
+    return e.astype(np.int64)
+
+
+def quantity_hists_from_records(records, specs) -> list[QuantityHist]:
+    """The quantity histograms of per-ray records (an AxionBatch of RayTracer.trace_mc_rays, or anything with the arrays `w`
+    and those the specs name), the host-side counterpart of RayTracer.read_quantity_hists: the rays with w != 0 (rt:2220)
+    are counted, each with the value of its record."""
+    W = np.asarray(records.w, dtype=np.float64)
+    sel = W != 0.0
+    W = W[sel]
+    out = []
+    for name, nbins, lo, hi in check_quantity_hist_specs(specs):
+        v = getattr(records, name)
+        if v is None:
+            raise ValueError(f"the records have no {name!r} array")
+        e = quantity_hist_entries(np.asarray(v, dtype=np.float64)[sel], nbins, lo, hi)
+        out.append(QuantityHist(name, quantity_hist_edges(nbins, lo, hi),
+                                np.bincount(e, weights=W, minlength=nbins + 2),
+                                np.bincount(e, weights=W * W, minlength=nbins + 2),
+                                np.bincount(e, minlength=nbins + 2).astype(np.uint64)))
+    return out
+
+
+def quantity_hist_edges(nbins: int, lo: float, hi: float) -> np.ndarray:
+    """The nbins + 1 edges of the regular bins, lo + (hi - lo) k / nbins (the last one exactly hi)."""
+    e = lo + (hi - lo) * (np.arange(nbins + 1, dtype=np.float64) / nbins)
+    e[-1] = hi
+    return e
+
+
+QUANTITY_HIST_COLUMNS = ["lower edge", "upper edge", "flux", "flux error", "rays"]
+
+
+def write_quantity_hist_csvs(hists: list[QuantityHist], windowYear: int, outpath: str | Path,
+                             precision: int = 17) -> list[Path]:
+    """One `axion_hist_{name}_{year}.csv` per histogram next to the image CSV: columns `lower edge`, `upper edge`, `flux`
+    (Σw), `flux error` (√Σw²) and `rays`, one row per entry; the underflow row has the lower edge -inf, the overflow row
+    (NaN values included) the upper edge inf."""
+    year = WINDOW_YEAR_NAMES.get(windowYear, str(windowYear))
+    paths = []
+    for h in hists:
+        lower = np.concatenate(([-np.inf], h.edges))
+        upper = np.concatenate((h.edges, [np.inf]))
+        paths.append(_write_columns(Path(outpath) / f"axion_hist_{h.name}_{year}.csv", QUANTITY_HIST_COLUMNS,
+                                    [lower, upper, h.sum_w, np.sqrt(h.sum_w2), h.counts], {4}, precision))
+    return paths
+
+
 def generateResultPlots(result, windowYear: int, outpath: str | Path, suffix: str = "",
                         radii: ContainmentRadii | None = None, chipXMax: float = 14.0, chipYMax: float = 14.0,
                         precision: int = 17, echo=print) -> Path:

@@ -15,7 +15,7 @@ import numpy as np
 
 from . import abi, tables as _tables
 from ._lib import SartError, check, lib  # noqa: F401  (re-exported)
-from .output import BandImages, Spectra
+from .output import BandImages, QuantityHist, Spectra, check_quantity_hist_specs, quantity_hist_edges
 
 
 def _dp(a: np.ndarray):
@@ -366,6 +366,39 @@ class RayTracer:
         """read_band_images of the last allreduce_outputs (raises SartError without one)."""
         return self._read_bands(lib.sart_read_merged_band_images)
 
+    def enable_quantity_hists(self, specs=None):
+        """Weighted histograms of per-ray record quantities of the rays that pass in trace_mc (single axion mass;
+        sart_enable_quantity_hists): specs [(name, nbins, lo, hi), ...], names from abi.QUANTITIES (the fields of
+        sart_ray_out_t); None or [] switches them off. Switching them on clears them."""
+        specs = check_quantity_hist_specs(specs or [])
+        arr = (abi.QuantityHistSpec * max(len(specs), 1))()
+        for k, (name, nbins, lo, hi) in enumerate(specs):
+            arr[k] = abi.QuantityHistSpec(abi.QUANTITIES.index(name), nbins, lo, hi)
+        check(lib.sart_enable_quantity_hists(self._h, len(specs), arr if specs else None))
+        self._qhist_specs = specs or None
+
+    def _read_qhists(self, read) -> list[QuantityHist]:
+        specs = getattr(self, "_qhist_specs", None) or []
+        n = sum(nb + 2 for _, nb, _, _ in specs)
+        w, w2 = np.empty(n), np.empty(n)
+        c = np.empty(n, dtype=np.uint64)
+        check(read(self._h, _dp(w), _dp(w2), c.ctypes.data_as(C.POINTER(C.c_uint64))))
+        out, off = [], 0
+        for name, nb, lo, hi in specs:
+            sl = slice(off, off + nb + 2)
+            out.append(QuantityHist(name, quantity_hist_edges(nb, lo, hi), w[sl].copy(), w2[sl].copy(), c[sl].copy()))
+            off += nb + 2
+        return out
+
+    def read_quantity_hists(self) -> list[QuantityHist]:
+        """The quantity histograms accumulated since enable_quantity_hists / reset_image, one output.QuantityHist per spec
+        (raises SartError while they are off)."""
+        return self._read_qhists(lib.sart_read_quantity_hists)
+
+    def read_merged_quantity_hists(self) -> list[QuantityHist]:
+        """read_quantity_hists of the last allreduce_outputs (raises SartError without one)."""
+        return self._read_qhists(lib.sart_read_merged_quantity_hists)
+
     def synchronize(self):
         check(lib.sart_synchronize(self._h))
 
@@ -405,8 +438,9 @@ class RayTracer:
         check(lib.sart_allreduce(hs, 1))
 
     def allreduce_outputs(self):
-        """sart_allreduce_outputs for this rank (every rank calls it): sums the radial histogram, the (per-mass) spectra and
-        the band images that are on over all ranks into merged copies, read with the read_merged_* methods. Synchronises."""
+        """sart_allreduce_outputs for this rank (every rank calls it): sums the radial histogram, the (per-mass) spectra, the
+        band images and the quantity histograms that are on over all ranks into merged copies, read with the read_merged_*
+        methods. Synchronises."""
         hs = (abi.H * 1)(self._h)
         check(lib.sart_allreduce_outputs(hs, 1))
 
