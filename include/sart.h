@@ -357,7 +357,8 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
 int sart_reset_image(sart_handle_t* h);
 /* Optional weighted radial histogram of the passed rays, for the 68 % / 95.5 % containment radii of
  * generateResultPlots (rt:2459-2527, which sorts pointdataR of every passed ray): bin = floor(pointdataR * nbins / r_max),
- * the last bin also collects r >= r_max. Filled by sart_trace_mc for a single axion mass, cleared by sart_reset_image.
+ * the last bin also collects r >= r_max. Filled by sart_trace_mc for a single axion mass, cleared by sart_reset_image;
+ * sart_angular_scan leaves it untouched and sart_angular_scan_outputs fills rows of its own.
  * nbins = 0 switches it off (default). sum_w / counts are host arrays [nbins] (either may be NULL). */
 int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max);
 int sart_read_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
@@ -368,8 +369,8 @@ int sart_read_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
  * sart_reset_image; filled in every precision mode, by the FP32 kernel and by the FP64 re-trace of its uncertain rays
  * alike, so precision 2 has the counts of precision 0. With spectra on, precision modes 1 and 2 run the generic kernel
  * variant (as with the radial histogram) and sart_trace_mc with more than one axion mass fails with SART_ERR_CONFIG.
- * sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev) and sart_trace_words leave
- * them untouched. on != 0 synchronises, then (re)allocates and zeroes them; on = 0 switches them off (default).
+ * sart_angular_scan, sart_angular_scan_outputs (which fills rows of its own), sart_trace_mc_rays, sart_trace_mc_passed,
+ * sart_trace_presampled(_dev) and sart_trace_words leave them untouched. on != 0 synchronises, then (re)allocates and zeroes them; on = 0 switches them off (default).
  * Switching them on while the per-mass spectra (sart_enable_mass_spectra) are on fails with SART_ERR_CONFIG. */
 int sart_enable_spectra(sart_handle_t* h, int on);
 /* Synchronises and copies out; host arrays, any may be NULL: energy_* [nEnergies + 1], shell_* [SART_MAX_SHELLS].
@@ -384,7 +385,7 @@ int sart_read_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum
  * sart_set_axion_masses when it changes the number of masses. With them on, sart_trace_mc runs the mass-scan kernels for
  * every M, M = 1 included (the image then differs from a single-mass run's only in the order of its sums), and fails with
  * SART_ERR_CONFIG with the alias sampler. sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed,
- * sart_trace_presampled(_dev) and sart_trace_words leave them untouched. on != 0 synchronises, then (re)allocates and
+ * sart_trace_presampled(_dev) and sart_trace_words leave them untouched; sart_angular_scan_outputs refuses them. on != 0 synchronises, then (re)allocates and
  * zeroes them for SART_MAX_MASSES masses (about 2.4 MB at nEnergies = 1500); on = 0 switches them off (default).
  * Switching them on while the single-mass spectra (sart_enable_spectra) are on fails with SART_ERR_CONFIG. */
 int sart_enable_mass_spectra(sart_handle_t* h, int on);
@@ -402,8 +403,8 @@ int sart_read_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energ
  * the FP64 re-trace of its uncertain rays alike, so precision 2 has the counts of precision 0. With them on, precision modes
  * 1 and 2 run kernel variants of their own that also fill the radial histogram and the spectra when those are on; the alias
  * sampler is supported like in a run without them. sart_trace_mc with more than one axion mass, or with the per-mass spectra
- * on, fails with SART_ERR_CONFIG. sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev)
- * and sart_trace_words leave them untouched.
+ * on, fails with SART_ERR_CONFIG. sart_angular_scan, sart_angular_scan_outputs (which fills rows of its own),
+ * sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev) and sart_trace_words leave them untouched.
  *   n_bands in 1..SART_MAX_BANDS with n_bands + 1 finite, non-negative, strictly ascending edges synchronises, then
  * (re)allocates and zeroes them; n_bands = 0 switches them off (default; edges_keV may then be NULL); anything else is
  * SART_ERR_ARG. Device memory at n_bands bands: 1 MB per band for Σw and Σw², the same again for each of the 8 replicas the
@@ -427,8 +428,8 @@ int sart_read_band_images(sart_handle_t* h, double* image, double* image_w2, uin
  * by the FP64 re-trace of its uncertain rays alike. With them on, precision modes 1 and 2 run kernel variants of their own
  * that also fill the radial histogram, the spectra and the band images when those are on; the alias sampler is supported.
  * sart_trace_mc with more than one axion mass, or with the per-mass spectra on, fails with SART_ERR_CONFIG.
- * sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev) and sart_trace_words leave them
- * untouched.
+ * sart_angular_scan, sart_angular_scan_outputs (which fills rows of its own), sart_trace_mc_rays, sart_trace_mc_passed,
+ * sart_trace_presampled(_dev) and sart_trace_words leave them untouched.
  *   n in 1..SART_N_QUANTITIES histograms, each quantity at most once, nbins in 1..SART_MAX_QHIST_BINS, lo and hi finite
  * with lo < hi: synchronises, then (re)allocates and zeroes them. n = 0 switches them off (default; hists may then be
  * NULL). Anything else is SART_ERR_ARG. Device memory: 24 bytes per entry for the handle's arrays and for the merged copy
@@ -508,6 +509,33 @@ int sart_synchronize(sart_handle_t* h);
  * [n_angles][256][256] are optional host arrays (NULL to skip). Leaves the handle's own setup and image untouched. */
 int sart_angular_scan(sart_handle_t* h, int n_angles, const double* angles_deg, uint64_t first_ray,
                       uint64_t n_rays_per_angle, uint64_t seed, double* fluxes, sart_counters_t* counters, double* images);
+/* sart_angular_scan, and every scan point also fills its own row of each single-mass accumulator the handle has on: the
+ * radial histogram, the spectra, the band images and the quantity histograms, each in the shape its sart_enable_* call
+ * gave it (bins and r_max, band edges, histogram specs). Row i holds what sart_trace_mc of scan point i's rays, with the
+ * same accumulators on and the setup turned to angles_deg[i], adds to a freshly reset handle, in every precision mode, the
+ * FP64 re-trace and the alias sampler (mode 2) included. The containment radii of a row are about the chip centre
+ * (pointdataR, rt:2202), so an off-axis row includes the displacement of the spot.
+ *   The rows are this call's result only: they are not accumulated across calls or kept on the handle. fluxes, counters,
+ * images and the ray indices are those of sart_angular_scan; the handle's own accumulators, image and counters are left
+ * bit-identical. The arrays of `out` are host arrays, any may be NULL (out itself too), with the scan point as their leading
+ * dimension; one for an accumulator that is off is SART_ERR_ARG, and so is a call with none of the four on (use
+ * sart_angular_scan). The per-mass spectra on give SART_ERR_CONFIG, more than one axion mass SART_ERR_ARG.
+ *   Device memory: the rows live in the handle's stage buffer next to the per-point images (1 MB per scan point), which
+ * keeps its size after the call: the band images take n_angles x n_bands x 1 MB (800 MB for 50 points at 16 bands), the
+ * radial histogram 16 bytes per bin and point, the spectra about 36 KB per point at nEnergies = 1500, the quantity
+ * histograms 24 bytes per entry and point. When that does not fit the call returns SART_ERR_NOMEM before it launches
+ * anything. */
+typedef struct {
+  double* radial_sum_w;   uint64_t* radial_counts;                          /* [n_angles][nbins] */
+  double* energy_sum_w;   double* energy_sum_w2;  uint64_t* energy_counts;  /* [n_angles][nEnergies + 1] */
+  double* shell_sum_w;    uint64_t* shell_counts;                           /* [n_angles][SART_MAX_SHELLS] */
+  double* band_image;     double* band_image_w2;                            /* [n_angles][n_bands][256][256] */
+  uint64_t* band_counts;                                                    /* [n_angles][n_bands] */
+  double* qhist_sum_w;    double* qhist_sum_w2;   uint64_t* qhist_counts;   /* [n_angles][Σ(nbins_k + 2)] */
+} sart_scan_out_t;
+int sart_angular_scan_outputs(sart_handle_t* h, int n_angles, const double* angles_deg, uint64_t first_ray,
+                              uint64_t n_rays_per_angle, uint64_t seed, double* fluxes, sart_counters_t* counters,
+                              double* images, const sart_scan_out_t* out);
 
 /* ---- prepareHeatmap (rt:818-842), general form, for per-ray records held by the host (e.g. the output of
  * sart_trace_mc_rays filtered by `passed`): result[floor((y-start_y)/dy)][floor((x-start_x)/dx)] += w/norm on the

@@ -37,17 +37,20 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--writeSpectra", action="store_true",
                     help="also write the energy spectrum and the per-shell flux of the detected rays as CSV files next to "
                          "the image (a single-mass run then takes the generic kernel variant; a mass scan writes one pair "
-                         "of files per mass, suffixed _ma{m}eV)")
+                         "of files per mass, suffixed _ma{m}eV, an angular scan one pair per scan point, suffixed "
+                         "_angle{a}deg)")
     ap.add_argument("--energyBands", default=None,
                     help="also write one detector image per energy band: comma-separated band edges in keV, e.g. 0.5,2,4,8 "
-                         "(2 to 17 values, ascending) writes axion_image_{year}_E0.5-2keV.csv and so on next to the image; "
-                         "a single axion mass only")
+                         "(2 to 17 values, ascending) writes axion_image_{year}_E0.5-2keV.csv and so on next to the image "
+                         "(an angular scan: one set per scan point, suffixed _angle{a}deg); a single axion mass only")
     ap.add_argument("--histogram", action="append", default=None, metavar="NAME:NBINS:LO:HI",
                     help="also write a weighted histogram of a per-ray record quantity of the passed rays, e.g. "
                          "transMagnet:256:0:1e-20, to axion_hist_{NAME}_{year}.csv next to the image (NBINS regular bins over "
                          "[LO, HI) plus an underflow and an overflow row); repeatable, each quantity once; NAME is one of "
-                         "reflect, transMagnet, yaw, alpha1, alpha2, pathCB, deviationDet, transProbArgon; a single axion mass "
-                         "only")
+                         "reflect, transMagnet, yaw, alpha1, alpha2, pathCB, deviationDet, transProbArgon; an angular scan "
+                         "writes one file per scan point, suffixed _angle{a}deg; a single axion mass only. With an angular "
+                         "scan, each of these three switches also writes the containment radii of every scan point to "
+                         "angular_scan_telescope_y_radii.csv")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--devices", default=None,
                     help="trace on several GPUs: a comma-separated list of CUDA ordinals or `all`. A fused run shards the "
@@ -205,6 +208,15 @@ def write_angular_scan(angles, rel, outpath):
                header="Angle [deg],relative flux", comments="")
 
 
+def write_angular_scan_outputs(scan, setup, outpath):
+    """The files of an angular scan with accumulators (output.ScanOutputs): those of write_angular_scan, the containment
+    radii of every scan point and its spectra, band images and quantity histograms (output.write_scan_outputs)."""
+    from . import output
+    write_angular_scan(scan.angles, scan.fluxes / scan.fluxes.max(), outpath)
+    for p in output.write_scan_outputs(scan, setup.detector.windowYear, outpath, setup.consts.chipXMax, setup.consts.chipYMax):
+        print("wrote", p)
+
+
 def main(argv=None) -> int:
     a = parse_args(argv)
     from . import abi, config as cfgmod, multi_gpu, raytracer as rt, tables
@@ -231,6 +243,8 @@ def main(argv=None) -> int:
     warn = lambda msg: print(msg, file=sys.stderr)   # noqa: E731
     single = len(run.mAxion) <= 1
     fused = a.angularScanMin == a.angularScanMax
+    # an angular scan of one axion mass writes the files of these switches once per scan point, with its containment radii
+    scan_outputs = single and (a.writeSpectra or a.energyBands is not None or a.histogram is not None)
     if a.devices is not None:
         if fused:
             print("start")
@@ -243,6 +257,13 @@ def main(argv=None) -> int:
                     raise SystemExit(f"raytracer: {e}") from None
                 raise
             write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath, r.band_images, r.quantity_hists)
+        elif scan_outputs:
+            scan = multi_gpu.angular_scan_outputs_on_devices(fs, devices, a.angularScanMin, a.angularScanMax,
+                                                             a.numAngularScanPoints, n, a.seed, precision=want,
+                                                             sampler=sampler, masses=run.mAxion or None, radial_hist=True,
+                                                             spectra=a.writeSpectra, bands=a.energyBands,
+                                                             quantity_hists=a.histogram, warn=warn)
+            write_angular_scan_outputs(scan, setup, outpath)
         else:
             angles, rel, _ = multi_gpu.angular_scan_on_devices(fs, devices, a.angularScanMin, a.angularScanMax,
                                                                a.numAngularScanPoints, n, a.seed, precision=want,
@@ -275,6 +296,16 @@ def main(argv=None) -> int:
             qhists = tr.read_quantity_hists() if a.histogram is not None else None
             write_fused_outputs(result, tr.read_radial_hist() if single else None, spectra, run.mAxion, setup, outpath, bands,
                                 qhists)
+        elif scan_outputs:
+            tr.enable_radial_hist()
+            if a.writeSpectra:
+                tr.enable_spectra()
+            if a.energyBands is not None:
+                tr.enable_band_images(a.energyBands)
+            if a.histogram is not None:
+                tr.enable_quantity_hists(a.histogram)
+            angles = np.linspace(a.angularScanMin, a.angularScanMax, a.numAngularScanPoints)
+            write_angular_scan_outputs(tr.angular_scan_outputs(angles, n, a.seed), setup, outpath)
         else:
             angles, rel, _ = rt.performAngularScan(fs, a.angularScanMin, a.angularScanMax, a.numAngularScanPoints, n,
                                                    a.seed, tracer=tr)

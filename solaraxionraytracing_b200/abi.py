@@ -142,6 +142,19 @@ class QuantityHistSpec(C.Structure):   # sart_quantity_hist_t
     _fields_ = [("quantity", C.c_int32), ("nbins", C.c_int32), ("lo", C.c_double), ("hi", C.c_double)]
 
 
+# sart_scan_out_t: the host arrays of sart_angular_scan_outputs, [n_angles] rows each, grouped by accumulator in the order
+# of the fields of sart_scan_out_t
+SCAN_OUT_FIELDS = {"radial": (("radial_sum_w", C.c_double), ("radial_counts", C.c_uint64)),
+                   "spectra": (("energy_sum_w", C.c_double), ("energy_sum_w2", C.c_double), ("energy_counts", C.c_uint64),
+                               ("shell_sum_w", C.c_double), ("shell_counts", C.c_uint64)),
+                   "bands": (("band_image", C.c_double), ("band_image_w2", C.c_double), ("band_counts", C.c_uint64)),
+                   "qhists": (("qhist_sum_w", C.c_double), ("qhist_sum_w2", C.c_double), ("qhist_counts", C.c_uint64))}
+
+
+class ScanOut(C.Structure):   # sart_scan_out_t
+    _fields_ = [(n, C.POINTER(t)) for fields in SCAN_OUT_FIELDS.values() for n, t in fields]
+
+
 class Counters(C.Structure):
     _fields_ = [("n_rays", C.c_uint64), ("n_exit", C.c_uint64 * 16), ("n_passed", C.c_uint64),
                 ("n_passed_till_window", C.c_uint64), ("n_hit_nickel", C.c_uint64), ("n_interp_clamped", C.c_uint64),
@@ -242,6 +255,8 @@ SIGNATURES = {
     "sart_read_merged_quantity_hists": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_angular_scan": (C.c_int, [H, C.c_int, c_double_p, C.c_uint64, C.c_uint64, C.c_uint64, c_double_p, C.POINTER(Counters),
                                     c_double_p]),
+    "sart_angular_scan_outputs": (C.c_int, [H, C.c_int, c_double_p, C.c_uint64, C.c_uint64, C.c_uint64, c_double_p,
+                                            C.POINTER(Counters), c_double_p, C.POINTER(ScanOut)]),
     "sart_measure_fma_peak": (C.c_int, [C.c_int, C.c_int, c_double_p]),
     "sart_prepare_heatmap": (C.c_int, [H, C.c_int, C.c_int, C.c_double, C.c_double, C.c_double, C.c_double, C.c_size_t,
                                        c_double_p, c_double_p, c_double_p, C.c_double, c_double_p,

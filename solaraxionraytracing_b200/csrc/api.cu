@@ -1271,6 +1271,23 @@ static int trace_image(sart_handle* h, const Params& P, const fast::FastParams& 
       });
 }
 
+// The folds that follow a run of the throughput kernels with the accumulators `acc` (the handle's, or the rows of a scan
+// point): the replicas of the spectra, the band images and the quantity histograms, which belong to the handle, are added
+// into acc's arrays and cleared.
+static int fold_accums(sart_handle* h, const Accum* acc) {
+  const Accum &spec = acc[kSpectra], &bands = acc[kBandImages], &qhists = acc[kQuantityHists];
+  if (spec.blob) SART_CUDA(launch_fold_spectra(spec.tput, spec.bins, spec.spec, h->stream));
+  if (bands.blob) {
+    const BandImages& r = bands.tput_band;
+    SART_CUDA(launch_fold_replicas(r.w, r.w2, int(r.repMask) + 1, r.repStride, r.repStride, bands.band.w, bands.band.w2, h->stream));
+  }
+  if (qhists.blob) {   // the replicas hold sums only where the kernel kept them out of shared memory; zeros cost no adds
+    const QuantityHists& q = qhists.qh;
+    SART_CUDA(launch_fold_replicas(q.rw, q.rw2, int(q.repMask) + 1, q.repStride, size_t(q.entries), q.w, q.w2, h->stream));
+  }
+  return SART_OK;
+}
+
 int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_t seed) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
   if (!h->d_image) return fail(SART_ERR_NOMEM, "the image buffers of this handle could not be allocated");
@@ -1357,16 +1374,7 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   if (rc || h->precision == 0) return rc;
   if (h->n_rep > 1)
     SART_CUDA(launch_fold_replicas(img, img2, h->n_rep, h->rep_stride, plane, h->d_image, h->d_image_w2, h->stream));
-  if (spec.blob) SART_CUDA(launch_fold_spectra(spec.tput, spec.bins, spec.spec, h->stream));
-  if (bands.blob) {
-    const BandImages& r = bands.tput_band;
-    SART_CUDA(launch_fold_replicas(r.w, r.w2, int(r.repMask) + 1, r.repStride, r.repStride, bands.band.w, bands.band.w2, h->stream));
-  }
-  if (qhists.blob) {   // the replicas hold sums only where the kernel kept them out of shared memory; zeros cost no adds
-    const QuantityHists& q = qhists.qh;
-    SART_CUDA(launch_fold_replicas(q.rw, q.rw2, int(q.repMask) + 1, q.repStride, size_t(q.entries), q.w, q.w2, h->stream));
-  }
-  return SART_OK;
+  return fold_accums(h, h->accum);
 }
 
 int sart_reset_image(sart_handle_t* h) {
@@ -1503,32 +1511,67 @@ int sart_prepare_heatmap(sart_handle_t* h, int rows, int cols, double start_x, d
   return SART_OK;
 }
 
-int sart_angular_scan(sart_handle_t* h, int n_angles, const double* angles_deg, uint64_t first_ray,
-                      uint64_t n_rays_per_angle, uint64_t seed, double* fluxes, sart_counters_t* counters, double* images) {
-  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
-  if (n_angles < 1 || !angles_deg || !fluxes) return fail(SART_ERR_ARG, "sart_angular_scan: bad argument");
-  if (h->n_masses != 1) return fail(SART_ERR_ARG, "sart_angular_scan: set a single axion mass");
-  if (h->sampler == SART_SAMPLER_ALIAS && h->precision != 2)
-    return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2");
+// The caller's arrays of accumulator k in a sart_scan_out_t, in the order of accum_arrays, into p; returns their number (0:
+// an accumulator without rows in a scan).
+static int scan_out_arrays(const sart_scan_out_t& o, AccumKind k, void** p) {
+  switch (k) {
+    case kRadialHist: p[0] = o.radial_sum_w; p[1] = o.radial_counts; return 2;
+    case kSpectra:
+      p[0] = o.energy_sum_w; p[1] = o.energy_sum_w2; p[2] = o.energy_counts; p[3] = o.shell_sum_w; p[4] = o.shell_counts;
+      return 5;
+    case kBandImages: p[0] = o.band_image; p[1] = o.band_image_w2; p[2] = o.band_counts; return 3;
+    case kQuantityHists: p[0] = o.qhist_sum_w; p[1] = o.qhist_sum_w2; p[2] = o.qhist_counts; return 3;
+    default: return 0;
+  }
+}
+
+// sart_angular_scan, and with `out` sart_angular_scan_outputs: then every single-mass accumulator the handle has on also
+// gets one row per scan point, in the stage buffer next to the images, copied into the caller's arrays `out` at the end.
+// Without `out` the scan runs the kernels a run without accumulators runs.
+static int angular_scan(sart_handle* h, int n_angles, const double* angles_deg, uint64_t first_ray, uint64_t n_rays_per_angle,
+                        uint64_t seed, double* fluxes, sart_counters_t* counters, double* images, const sart_scan_out_t* out) {
   DeviceGuard dg(h->device);
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
   double *dImg, *dImg2;
   sart_counters_t* dCnt;
+  Accum rows[kAccums];   // bins > 0: the [n_angles] rows of accumulator k, shaped like the handle's
   auto layout = [&](Carve c) {
     c.take(dImg, size_t(n_angles) * plane); c.take(dImg2, size_t(n_angles) * plane); c.take(dCnt, size_t(n_angles));
+    void* unused[5];
+    for (AccumKind k : kAllAccums) {
+      if (!out || !h->accum[k].blob || !scan_out_arrays(*out, k, unused)) continue;
+      rows[k] = Accum{};
+      rows[k].bins = h->accum[k].bins;
+      accum_arrays(k, rows[k], rows[k], size_t(n_angles), [&](auto*& p, auto*&, size_t n) { c.take(p, n); });
+    }
     return c.off;
   };
   const size_t bytes = layout(Carve());
   int rc = ensure_stage(h, bytes);
+  if (rc && out) {
+    cudaGetLastError();   // the failed cudaMalloc must not surface at the next launch
+    return fail(SART_ERR_NOMEM, "sart_angular_scan_outputs: no room for the %zu bytes of the scan points' images and rows", bytes);
+  }
   if (rc) return rc;
   layout(Carve(h->d_stage));
   SART_CUDA(cudaMemsetAsync(h->d_stage, 0, bytes, h->stream));
   // One launch per scan point, queued back to back on the handle's stream: only the by-value parameter block differs
   // (the rotation of the telescope frame), the tables and shell records in HBM are shared, nothing synchronises.
-  fast::FastTables ft = h->ftables;
-  Tables et = h->tables;
-  ft.rad = RadialHist{}; et.rad = RadialHist{};
   for (int i = 0; i < n_angles; ++i) {
+    // The accumulators of scan point i: the handle's, with every array the kernels add into directly moved to row i. The
+    // replicas of the throughput kernels stay the handle's: each fold below clears them for the next point.
+    Accum v[kAccums];
+    for (AccumKind k : kAllAccums) {
+      if (!rows[k].bins) continue;
+      v[k] = h->accum[k];
+      accum_arrays(k, v[k], rows[k], 1, [&](auto*& p, auto* r, size_t n) { p = r + size_t(i) * n; });
+    }
+    v[kBandImages].tput_band.n = v[kBandImages].band.n;   // the band counts are never replicated
+    fast::FastTables ft = h->ftables;
+    Tables et = h->tables;
+    ft.rad = et.rad = v[kRadialHist].rad;
+    ft.spec = v[kSpectra].tput;
+    et.spec = v[kSpectra].spec;
     sart_setup_t s = h->setup;
     s.telescope.telescope_turned_y = angles_deg[i];   // rt:2796
     Params P;
@@ -1549,16 +1592,72 @@ int sart_angular_scan(sart_handle_t* h, int n_angles, const double* angles_deg, 
     }
     const uint64_t first = first_ray + uint64_t(i) * n_rays_per_angle;   // every scan point traces its own rays, like the reference
     double *img = dImg + size_t(i) * plane, *img2 = dImg2 + size_t(i) * plane;
-    if ((rc = trace_image(h, P, F, G, ft, et, first, n_rays_per_angle, seed, img, img2, img, img2, dCnt + i))) return rc;
+    if ((rc = trace_image(h, P, F, G, ft, et, first, n_rays_per_angle, seed, img, img2, img, img2, dCnt + i,
+                          v[kBandImages].tput_band, v[kBandImages].band, v[kQuantityHists].qh)))
+      return rc;
+    if (h->precision >= 1 && (rc = fold_accums(h, v))) return rc;
   }
   std::vector<sart_counters_t> cnt;
   cnt.resize(size_t(n_angles));
   SART_CUDA(cudaMemcpyAsync(cnt.data(), dCnt, cnt.size() * sizeof(sart_counters_t), cudaMemcpyDeviceToHost, h->stream));
   if (images) SART_CUDA(cudaMemcpyAsync(images, dImg, size_t(n_angles) * plane * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  for (AccumKind k : kAllAccums) {
+    if (!rows[k].bins) continue;
+    void* host[5];
+    scan_out_arrays(*out, k, host);
+    void* const* hp = host;
+    cudaError_t e = cudaSuccess;
+    accum_arrays(k, rows[k], rows[k], size_t(n_angles), [&](auto* d, auto*, size_t n) {
+      void* p = *hp++;
+      if (p && e == cudaSuccess) e = cudaMemcpyAsync(p, d, n * sizeof *d, cudaMemcpyDeviceToHost, h->stream);
+    });
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync (scan rows, device to host)");
+  }
   SART_CUDA(cudaStreamSynchronize(h->stream));
   for (int i = 0; i < n_angles; ++i) fluxes[i] = cnt[size_t(i)].sum_w;   // axions.filterIt(it.passed).mapIt(it.weights).sum() rt:2800
   if (counters) std::memcpy(counters, cnt.data(), cnt.size() * sizeof(sart_counters_t));
   return SART_OK;
+}
+
+// The checks both scan entry points make.
+static int check_scan(sart_handle* h, int n_angles, const double* angles_deg, double* fluxes, const char* who) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (n_angles < 1 || !angles_deg || !fluxes) return fail(SART_ERR_ARG, "%s: bad argument", who);
+  if (h->n_masses != 1) return fail(SART_ERR_ARG, "%s: set a single axion mass", who);
+  if (h->sampler == SART_SAMPLER_ALIAS && h->precision != 2)
+    return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2");
+  return SART_OK;
+}
+
+int sart_angular_scan(sart_handle_t* h, int n_angles, const double* angles_deg, uint64_t first_ray,
+                      uint64_t n_rays_per_angle, uint64_t seed, double* fluxes, sart_counters_t* counters, double* images) {
+  const int rc = check_scan(h, n_angles, angles_deg, fluxes, "sart_angular_scan");
+  return rc ? rc : angular_scan(h, n_angles, angles_deg, first_ray, n_rays_per_angle, seed, fluxes, counters, images, nullptr);
+}
+
+int sart_angular_scan_outputs(sart_handle_t* h, int n_angles, const double* angles_deg, uint64_t first_ray,
+                              uint64_t n_rays_per_angle, uint64_t seed, double* fluxes, sart_counters_t* counters,
+                              double* images, const sart_scan_out_t* out) {
+  int rc = check_scan(h, n_angles, angles_deg, fluxes, "sart_angular_scan_outputs");
+  if (rc) return rc;
+  if (h->accum[kMassSpectra].blob)
+    return fail(SART_ERR_CONFIG, "sart_angular_scan_outputs: the per-mass spectra are on; a scan fills single-mass rows only");
+  const sart_scan_out_t none{};
+  if (!out) out = &none;
+  static const char* const names[kAccums] = {"radial histogram", "spectra", "per-mass spectra", "band images",
+                                             "quantity histograms"};
+  bool any = false;
+  for (AccumKind k : kAllAccums) {
+    void* p[5];
+    const int np = scan_out_arrays(*out, k, p);
+    any |= np > 0 && h->accum[k].blob != nullptr;
+    for (int j = 0; j < np && !h->accum[k].blob; ++j)
+      if (p[j]) return fail(SART_ERR_ARG, "sart_angular_scan_outputs: an output array for the %s, which the handle has off", names[k]);
+  }
+  if (!any)
+    return fail(SART_ERR_ARG, "sart_angular_scan_outputs: no radial histogram, spectra, band images or quantity histograms "
+                              "are on (sart_angular_scan scans without them)");
+  return angular_scan(h, n_angles, angles_deg, first_ray, n_rays_per_angle, seed, fluxes, counters, images, out);
 }
 
 int sart_synchronize(sart_handle_t* h) {

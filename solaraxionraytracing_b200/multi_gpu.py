@@ -6,7 +6,8 @@ detector image, the sum-of-squares image and the counters (512 KiB + 512 KiB + 2
 all-reduce over NVLink (NCCL) on the device buffers libsart exposes. The reference's only parallel construct is the
 Weave parallelFor over rays inside one process (src/raytracer.nim:2234-2244).
 
-One process can also drive several GPUs itself (trace_on_devices, angular_scan_on_devices): one RayTracer per device,
+One process can also drive several GPUs itself (trace_on_devices, angular_scan_on_devices, angular_scan_outputs_on_devices):
+one RayTracer per device,
 one NCCL communicator over all of them (sart_comm_init_all), and the same collectives behind the C-ABI, which then take
 every handle of the process in one call.
 """
@@ -20,7 +21,7 @@ import numpy as np
 
 from . import abi
 from ._lib import check, lib
-from .output import BandImages, QuantityHist, Spectra
+from .output import BandImages, QuantityHist, ScanOutputs, Spectra, concat_scan_outputs
 
 
 def shard(n_rays: int, rank: int, world: int, first_ray: int = 0) -> tuple[int, int]:
@@ -274,3 +275,48 @@ def angular_scan_on_devices(fullSetup, devices, angularScanMin: float, angularSc
     if errors:
         raise errors[0]
     return angles, fluxes / fluxes.max(), fluxes
+
+
+def angular_scan_outputs_on_devices(fullSetup, devices, angularScanMin: float, angularScanMax: float,
+                                    numAngularScanPoints: int = 50, nRays: int = 1_000_000, seed: int = 299792458, *,
+                                    precision: int = 2, sampler=None, masses=None, radial_hist: bool = True,
+                                    spectra: bool = False, bands=None, quantity_hists=None, want_images: bool = False,
+                                    warn=None) -> ScanOutputs:
+    """RayTracer.angular_scan_outputs over `devices` in one process, scan points dealt as in angular_scan_on_devices
+    (device k takes the contiguous block shard(points, k, n), scan point i traces the global rays [i*nRays, (i+1)*nRays)).
+    The accumulators `radial_hist`, `spectra` (single-mass), `bands` (band edges) and `quantity_hists` (specs) are switched
+    on every device; the blocks of scan points are put together on the host, so the result is that of one GPU."""
+    angles = np.linspace(angularScanMin, angularScanMax, numAngularScanPoints)
+    tracers, _ = _open_tracers(fullSetup, devices, precision, sampler, masses, warn)
+    parts: list[ScanOutputs | None] = [None] * len(tracers)
+    errors = []
+
+    def scan(rank, t):
+        lo, cnt = shard(numAngularScanPoints, rank, len(tracers))
+        try:
+            if cnt:
+                parts[rank] = t.angular_scan_outputs(angles[lo:lo + cnt], nRays, seed, want_images, first_ray=lo * nRays)
+        except BaseException as e:   # re-raised in the calling thread
+            errors.append(e)
+
+    try:
+        for t in tracers:
+            if radial_hist:
+                t.enable_radial_hist()
+            if spectra:
+                t.enable_spectra()
+            if bands is not None:
+                t.enable_band_images(bands)
+            if quantity_hists:
+                t.enable_quantity_hists(quantity_hists)
+        threads = [threading.Thread(target=scan, args=(k, t)) for k, t in enumerate(tracers)]
+        for th in threads:
+            th.start()
+        for th in threads:
+            th.join()
+    finally:
+        for t in tracers:
+            t.close()
+    if errors:
+        raise errors[0]
+    return concat_scan_outputs([p for p in parts if p is not None])

@@ -293,8 +293,8 @@ def band_suffix(lo: float, hi: float) -> str:
 
 
 def write_band_image_csvs(bands: BandImages, windowYear: int, outpath: str | Path, radii: ContainmentRadii | None = None,
-                          chipXMax: float = 14.0, chipYMax: float = 14.0, precision: int = 17) -> list[Path]:
-    """One write_axion_image_csv file per energy band, `axion_image_{year}_E{lo:g}-{hi:g}keV.csv`, next to the run's
+                          chipXMax: float = 14.0, chipYMax: float = 14.0, precision: int = 17, suffix: str = "") -> list[Path]:
+    """One write_axion_image_csv file per energy band, `axion_image_{year}_E{lo:g}-{hi:g}keV{suffix}.csv`, next to the run's
     image. The radius columns carry `radii`, the containment radii of the whole run: per-band radii are not computed."""
     edges = [float(e) for e in bands.edges]
     if len(edges) != bands.image.shape[0] + 1:
@@ -304,7 +304,7 @@ def write_band_image_csvs(bands: BandImages, windowYear: int, outpath: str | Pat
         raise ValueError("two bands share a file name (their edges agree to 6 significant digits)")
     radii = radii or ContainmentRadii(0.0, 0.0, 0.0, 0.0)
     year = WINDOW_YEAR_NAMES.get(windowYear, str(windowYear))
-    return [write_axion_image_csv(Path(outpath) / f"axion_image_{year}{sfx}.csv", img, radii.rSigma1W, radii.rSigma2W,
+    return [write_axion_image_csv(Path(outpath) / f"axion_image_{year}{sfx}{suffix}.csv", img, radii.rSigma1W, radii.rSigma2W,
                                   chipXMax, chipYMax, precision) for sfx, img in zip(names, bands.image)]
 
 
@@ -400,8 +400,8 @@ QUANTITY_HIST_COLUMNS = ["lower edge", "upper edge", "flux", "flux error", "rays
 
 
 def write_quantity_hist_csvs(hists: list[QuantityHist], windowYear: int, outpath: str | Path,
-                             precision: int = 17) -> list[Path]:
-    """One `axion_hist_{name}_{year}.csv` per histogram next to the image CSV: columns `lower edge`, `upper edge`, `flux`
+                             precision: int = 17, suffix: str = "") -> list[Path]:
+    """One `axion_hist_{name}_{year}{suffix}.csv` per histogram next to the image CSV: columns `lower edge`, `upper edge`, `flux`
     (Σw), `flux error` (√Σw²) and `rays`, one row per entry; the underflow row has the lower edge -inf, the overflow row
     (NaN values included) the upper edge inf."""
     year = WINDOW_YEAR_NAMES.get(windowYear, str(windowYear))
@@ -409,8 +409,75 @@ def write_quantity_hist_csvs(hists: list[QuantityHist], windowYear: int, outpath
     for h in hists:
         lower = np.concatenate(([-np.inf], h.edges))
         upper = np.concatenate((h.edges, [np.inf]))
-        paths.append(_write_columns(Path(outpath) / f"axion_hist_{h.name}_{year}.csv", QUANTITY_HIST_COLUMNS,
+        paths.append(_write_columns(Path(outpath) / f"axion_hist_{h.name}_{year}{suffix}.csv", QUANTITY_HIST_COLUMNS,
                                     [lower, upper, h.sum_w, np.sqrt(h.sum_w2), h.counts], {4}, precision))
+    return paths
+
+
+@dataclass
+class ScanOutputs:
+    """An angular scan with its accumulators (RayTracer.angular_scan_outputs): per scan point the flux, the counters, the
+    image, and a row of every accumulator that was on (None for those that were off)."""
+    angles: np.ndarray                                  # [n] telescope_turned_y [deg]
+    fluxes: np.ndarray                                  # [n] Σw of the passed rays
+    counters: list[dict]                                # [n]
+    images: np.ndarray | None                           # [n, 256, 256] when asked for
+    radial_hists: list[tuple] | None                    # [n] (bin edges, Σw, counts), as RayTracer.read_radial_hist
+    spectra: list[Spectra] | None                       # [n]
+    band_images: list[BandImages] | None                # [n]
+    quantity_hists: list[list[QuantityHist]] | None     # [n] one QuantityHist per spec
+
+
+def concat_scan_outputs(parts: list[ScanOutputs]) -> ScanOutputs:
+    """The scan points of `parts` (consecutive blocks of one scan, e.g. one per GPU) as one ScanOutputs."""
+    def cat(name):
+        vals = [getattr(p, name) for p in parts]
+        if any(v is None for v in vals):
+            return None
+        return np.concatenate(vals) if isinstance(vals[0], np.ndarray) else [x for v in vals for x in v]
+    return ScanOutputs(*(cat(f) for f in ScanOutputs.__dataclass_fields__))
+
+
+def angle_suffix(angle_deg: float) -> str:
+    """File-name suffix of one point of an angular scan: `_angle{a:g}deg`."""
+    return f"_angle{angle_deg:g}deg"
+
+
+RADII_COLUMNS = ["Angle [deg]", "rSigma1", "rSigma2", "rSigma1W", "rSigma2W"]
+
+
+def write_scan_radii_csv(path: str | Path, angles, radii: list[ContainmentRadii], precision: int = 17) -> Path:
+    """The containment radii of every scan point (containment_radii_from_hist of its radial histogram, about the chip
+    centre): columns `Angle [deg]`, rSigma1, rSigma2, rSigma1W, rSigma2W [mm]."""
+    a = np.asarray(angles, dtype=np.float64)
+    if a.size != len(radii):
+        raise ValueError(f"{len(radii)} radii for {a.size} angles")
+    cols = [a] + [np.array([getattr(r, f) for r in radii], dtype=np.float64) for f in RADII_COLUMNS[1:]]
+    return _write_columns(path, RADII_COLUMNS, cols, set(), precision)
+
+
+def write_scan_outputs(scan: ScanOutputs, windowYear: int, outpath: str | Path, chipXMax: float = 14.0,
+                       chipYMax: float = 14.0, precision: int = 17) -> list[Path]:
+    """The files of an angular scan with accumulators: `angular_scan_telescope_y_radii.csv` (write_scan_radii_csv; with the
+    radial histogram on), and for
+    every scan point the spectra, band-image and quantity-histogram files of a fused run with the suffix `_angle{a:g}deg`
+    (angle_suffix). The band images carry that point's own containment radii."""
+    suffixes = [angle_suffix(float(a)) for a in scan.angles]
+    if len(set(suffixes)) != len(suffixes):
+        raise ValueError("two scan points share a file name (their angles agree to 6 significant digits)")
+    paths: list[Path] = []
+    radii = [None] * len(suffixes)
+    if scan.radial_hists is not None:
+        radii = [containment_radii_from_hist(*h) for h in scan.radial_hists]
+        paths.append(write_scan_radii_csv(Path(outpath) / "angular_scan_telescope_y_radii.csv", scan.angles, radii, precision))
+    for i, sfx in enumerate(suffixes):
+        if scan.spectra is not None:
+            paths.extend(write_spectra_csvs(scan.spectra[i], windowYear, outpath, suffix=sfx, precision=precision))
+        if scan.band_images is not None:
+            paths.extend(write_band_image_csvs(scan.band_images[i], windowYear, outpath, radii[i], chipXMax, chipYMax,
+                                               precision, suffix=sfx))
+        if scan.quantity_hists is not None:
+            paths.extend(write_quantity_hist_csvs(scan.quantity_hists[i], windowYear, outpath, precision, suffix=sfx))
     return paths
 
 

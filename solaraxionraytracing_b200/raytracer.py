@@ -15,11 +15,16 @@ import numpy as np
 
 from . import abi, tables as _tables
 from ._lib import SartError, check, lib  # noqa: F401  (re-exported)
-from .output import BandImages, QuantityHist, Spectra, check_quantity_hist_specs, quantity_hist_edges
+from .output import BandImages, QuantityHist, ScanOutputs, Spectra, check_quantity_hist_specs, quantity_hist_edges
 
 
 def _dp(a: np.ndarray):
     return a.ctypes.data_as(abi.c_double_p)
+
+
+def _ptr(a: np.ndarray):
+    """A float64 or uint64 array as the ctypes pointer the C-ABI takes."""
+    return a.ctypes.data_as(abi.c_double_p if a.dtype == np.float64 else C.POINTER(C.c_uint64))
 
 
 def fast_available() -> bool:
@@ -290,12 +295,19 @@ class RayTracer:
         check(lib.sart_enable_radial_hist(self._h, nbins, r_max))
         self._rad = (nbins, r_max)
 
-    def _read_radial(self, read):
+    # Each accumulator's host arrays for `rows` rows (one read, or the scan points of angular_scan_outputs), in the order the
+    # C-ABI takes them, and the function that cuts them into one result per row.
+    def _radial_rows(self, rows: int):
         nbins, r_max = self._rad
-        w = np.empty(nbins)
-        n = np.empty(nbins, dtype=np.uint64)
-        check(read(self._h, _dp(w), n.ctypes.data_as(C.POINTER(C.c_uint64))))
-        return np.linspace(0.0, r_max, nbins + 1), w, n
+        w = np.empty((rows, nbins))
+        n = np.empty((rows, nbins), dtype=np.uint64)
+        edges = np.linspace(0.0, r_max, nbins + 1)
+        return (w, n), lambda: [(edges.copy(), w[k], n[k]) for k in range(rows)]
+
+    def _read_radial(self, read):
+        arrays, split = self._radial_rows(1)
+        check(read(self._h, *map(_ptr, arrays)))
+        return split()[0]
 
     def read_radial_hist(self):
         """(bin edges [nbins + 1], sum of weights [nbins], ray counts [nbins])."""
@@ -305,23 +317,29 @@ class RayTracer:
         """Energy spectrum and per-shell flux of the rays that pass in trace_mc (single axion mass; sart_enable_spectra).
         Switching them on clears them; precision modes 1 and 2 then run their generic kernel variant."""
         check(lib.sart_enable_spectra(self._h, int(bool(on))))
+        self._spectra_on = bool(on)
 
-    def _read_spectra_rows(self, read, rows: int) -> list[Spectra]:
-        """`rows` spectra copied out by `read` (sart_read_spectra / sart_read_mass_spectra), each with the energies of the
-        bins: the tabulated energies, then the X-ray source's (NaN without a source); shells cut to the telescope's."""
+    def _spectra_rows(self, rows: int):
+        """Each Spectra with the energies of the bins: the tabulated energies, then the X-ray source's (NaN without a
+        source); shells cut to the telescope's."""
         en = np.asarray(self.fullSetup.tables.energies if self.fullSetup.tables.energies is not None else [], dtype=np.float64)
         nE1 = en.size + 1
         w, w2 = np.empty((rows, nE1)), np.empty((rows, nE1))
         n = np.empty((rows, nE1), dtype=np.uint64)
         sw = np.empty((rows, abi.MAX_SHELLS))
         sn = np.empty((rows, abi.MAX_SHELLS), dtype=np.uint64)
-        u64 = C.POINTER(C.c_uint64)
-        check(read(self._h, _dp(w), _dp(w2), n.ctypes.data_as(u64), _dp(sw), sn.ctypes.data_as(u64)))
         s = self.fullSetup.expSetup
         src = s.testSource.energy if s.testSource.active else np.nan
         ns = s.telescope.nShells
         energies = np.append(en, src)
-        return [Spectra(energies.copy(), w[k], w2[k], n[k], sw[k, :ns].copy(), sn[k, :ns].copy()) for k in range(rows)]
+        return (w, w2, n, sw, sn), lambda: [Spectra(energies.copy(), w[k], w2[k], n[k], sw[k, :ns].copy(), sn[k, :ns].copy())
+                                            for k in range(rows)]
+
+    def _read_spectra_rows(self, read, rows: int) -> list[Spectra]:
+        """`rows` spectra copied out by `read` (sart_read_spectra / sart_read_mass_spectra)."""
+        arrays, split = self._spectra_rows(rows)
+        check(read(self._h, *map(_ptr, arrays)))
+        return split()
 
     def read_spectra(self) -> Spectra:
         """The spectra accumulated since enable_spectra / reset_image (raises SartError while they are off)."""
@@ -349,14 +367,18 @@ class RayTracer:
         check(lib.sart_enable_band_images(self._h, e.size - 1 if e.size > 1 else -1, _dp(e)))   # one edge: no band, refused
         self._band_edges = e.copy()
 
-    def _read_bands(self, read) -> BandImages:
+    def _band_rows(self, rows: int):
         edges = getattr(self, "_band_edges", None)
         nb = 0 if edges is None else edges.size - 1
-        img = np.empty((nb, abi.IMAGE_BINS, abi.IMAGE_BINS))
+        img = np.empty((rows, nb, abi.IMAGE_BINS, abi.IMAGE_BINS))
         img2 = np.empty_like(img)
-        n = np.empty(nb, dtype=np.uint64)
-        check(read(self._h, _dp(img), _dp(img2), n.ctypes.data_as(C.POINTER(C.c_uint64))))
-        return BandImages(edges.copy(), img, img2, n)
+        n = np.empty((rows, nb), dtype=np.uint64)
+        return (img, img2, n), lambda: [BandImages(edges.copy(), img[k], img2[k], n[k]) for k in range(rows)]
+
+    def _read_bands(self, read) -> BandImages:
+        arrays, split = self._band_rows(1)
+        check(read(self._h, *map(_ptr, arrays)))
+        return split()[0]
 
     def read_band_images(self) -> BandImages:
         """The band images accumulated since enable_band_images / reset_image (raises SartError while they are off)."""
@@ -377,18 +399,29 @@ class RayTracer:
         check(lib.sart_enable_quantity_hists(self._h, len(specs), arr if specs else None))
         self._qhist_specs = specs or None
 
-    def _read_qhists(self, read) -> list[QuantityHist]:
+    def _qhist_rows(self, rows: int):
         specs = getattr(self, "_qhist_specs", None) or []
         n = sum(nb + 2 for _, nb, _, _ in specs)
-        w, w2 = np.empty(n), np.empty(n)
-        c = np.empty(n, dtype=np.uint64)
-        check(read(self._h, _dp(w), _dp(w2), c.ctypes.data_as(C.POINTER(C.c_uint64))))
-        out, off = [], 0
-        for name, nb, lo, hi in specs:
-            sl = slice(off, off + nb + 2)
-            out.append(QuantityHist(name, quantity_hist_edges(nb, lo, hi), w[sl].copy(), w2[sl].copy(), c[sl].copy()))
-            off += nb + 2
-        return out
+        w, w2 = np.empty((rows, n)), np.empty((rows, n))
+        c = np.empty((rows, n), dtype=np.uint64)
+
+        def split():
+            out = []
+            for k in range(rows):
+                row, off = [], 0
+                for name, nb, lo, hi in specs:
+                    sl = slice(off, off + nb + 2)
+                    row.append(QuantityHist(name, quantity_hist_edges(nb, lo, hi), w[k, sl].copy(), w2[k, sl].copy(),
+                                            c[k, sl].copy()))
+                    off += nb + 2
+                out.append(row)
+            return out
+        return (w, w2, c), split
+
+    def _read_qhists(self, read) -> list[QuantityHist]:
+        arrays, split = self._qhist_rows(1)
+        check(read(self._h, *map(_ptr, arrays)))
+        return split()[0]
 
     def read_quantity_hists(self) -> list[QuantityHist]:
         """The quantity histograms accumulated since enable_quantity_hists / reset_image, one output.QuantityHist per spec
@@ -419,6 +452,34 @@ class RayTracer:
         check(lib.sart_angular_scan(self._h, a.size, _dp(a), first_ray, n_rays_per_angle, seed, _dp(fl), cnt,
                                     _dp(img) if want_images else None))
         return fl, [c.as_dict() for c in cnt], img
+
+    def angular_scan_outputs(self, angles_deg, n_rays_per_angle: int, seed: int = 299792458, want_images: bool = False,
+                             first_ray: int = 0) -> ScanOutputs:
+        """sart_angular_scan_outputs: angular_scan, plus for every scan point a row of each accumulator this tracer has on
+        (enable_radial_hist, enable_spectra, enable_band_images, enable_quantity_hists): what a fused run of that point's
+        rays would add to a freshly reset tracer. The tracer's own accumulators, image and counters stay as they are.
+        Raises SartError when none of the four is on."""
+        a = np.ascontiguousarray(angles_deg, dtype=np.float64)
+        n = a.size
+        fl = np.empty(n)
+        cnt = (abi.Counters * n)()
+        img = np.empty((n, abi.IMAGE_BINS, abi.IMAGE_BINS)) if want_images else None
+        on = {"radial": getattr(self, "_rad", (0, 0.0))[0] > 0, "spectra": getattr(self, "_spectra_on", False),
+              "bands": getattr(self, "_band_edges", None) is not None, "qhists": bool(getattr(self, "_qhist_specs", None))}
+        rows = {"radial": self._radial_rows, "spectra": self._spectra_rows, "bands": self._band_rows,
+                "qhists": self._qhist_rows}
+        out = abi.ScanOut()
+        split = {}
+        for kind, fields in abi.SCAN_OUT_FIELDS.items():
+            if on[kind]:
+                arrays, split[kind] = rows[kind](n)
+                for (name, _), arr in zip(fields, arrays):
+                    setattr(out, name, _ptr(arr))
+        check(lib.sart_angular_scan_outputs(self._h, n, _dp(a), first_ray, n_rays_per_angle, seed, _dp(fl), cnt,
+                                            _dp(img) if want_images else None, C.byref(out)))
+        got = {kind: f() for kind, f in split.items()}
+        return ScanOutputs(a.copy(), fl, [c.as_dict() for c in cnt], img, got.get("radial"), got.get("spectra"),
+                           got.get("bands"), got.get("qhists"))
 
     # -- multi-GPU (sart_allreduce): one NCCL all-reduce of image | w^2 image | counters into a separate merged buffer
     @staticmethod
