@@ -359,7 +359,8 @@ int sart_reset_image(sart_handle_t* h);
  * generateResultPlots (rt:2459-2527, which sorts pointdataR of every passed ray): bin = floor(pointdataR * nbins / r_max),
  * the last bin also collects r >= r_max. Filled by sart_trace_mc for a single axion mass, cleared by sart_reset_image;
  * sart_angular_scan leaves it untouched and sart_angular_scan_outputs fills rows of its own.
- * nbins = 0 switches it off (default). sum_w / counts are host arrays [nbins] (either may be NULL). */
+ * nbins = 0 switches it off (default). sum_w / counts are host arrays [nbins] (either may be NULL). Switching it on while
+ * the per-mass radial histograms (sart_enable_mass_radial_hist) are on fails with SART_ERR_CONFIG. */
 int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max);
 int sart_read_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
 /* Optional weighted spectra of the rays that PASS (weight != 0, rt:2220) in sart_trace_mc, single axion mass — the
@@ -368,7 +369,8 @@ int sart_read_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
  * X-ray test source's energy; shell bin j = shellNumber (rt:2198). Accumulated (+=) like the image and cleared by
  * sart_reset_image; filled in every precision mode, by the FP32 kernel and by the FP64 re-trace of its uncertain rays
  * alike, so precision 2 has the counts of precision 0. With spectra on, precision modes 1 and 2 run the generic kernel
- * variant (as with the radial histogram) and sart_trace_mc with more than one axion mass fails with SART_ERR_CONFIG.
+ * variant (as with the radial histogram) and sart_trace_mc with more than one axion mass, or with the per-mass radial
+ * histograms or band images on, fails with SART_ERR_CONFIG.
  * sart_angular_scan, sart_angular_scan_outputs (which fills rows of its own), sart_trace_mc_rays, sart_trace_mc_passed,
  * sart_trace_presampled(_dev) and sart_trace_words leave them untouched. on != 0 synchronises, then (re)allocates and zeroes them; on = 0 switches them off (default).
  * Switching them on while the per-mass spectra (sart_enable_mass_spectra) are on fails with SART_ERR_CONFIG. */
@@ -393,6 +395,38 @@ int sart_enable_mass_spectra(sart_handle_t* h, int on);
  * shell_* [M][SART_MAX_SHELLS]. SART_ERR_ARG when the per-mass spectra are off. */
 int sart_read_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                            double* shell_sum_w, uint64_t* shell_counts);
+/* Per-mass radial histograms and band images of the passed rays of sart_trace_mc: for each of the M axion masses
+ * (sart_set_axion_masses) one row of what sart_enable_radial_hist or sart_enable_band_images with the same arguments gives
+ * a single-mass run, from one traced ray per mass scan, as the per-mass images are. Row m is what sart_trace_mc of the
+ * single mass masses[m], with the single-mass counterpart on, adds to a freshly reset handle: the same radial bin rule,
+ * the band of a ray from its record energy (the X-ray source's included), the same image bin; a ray counts for mass m when
+ * its weight for m is not 0, and a band's count includes the passed rays that land outside the image. Their containment
+ * radii give the 68 % / 95.5 % radii of rt:2459-2527 for every mass.
+ *   Filled in every precision mode, by the FP32 kernel and by the FP64 re-trace of its uncertain rays alike, so precision
+ * 2 has the counts of precision 0 for every mass. Accumulated (+=) like the image; cleared by sart_reset_image and by
+ * sart_set_axion_masses when it changes the number of masses (which also invalidates their merged copies). With either
+ * on, sart_trace_mc runs the mass-scan kernels for every M, M = 1 included, as with the per-mass spectra, which may be on
+ * as well; it fails with SART_ERR_CONFIG with the alias sampler, with the quantity histograms on, or with the single-mass
+ * spectra or band images on (the mass-scan kernels fill only the per-mass forms; sart_enable_mass_spectra gives the
+ * spectra of every mass). sart_angular_scan, sart_trace_mc_rays, sart_trace_mc_passed, sart_trace_presampled(_dev) and
+ * sart_trace_words leave them untouched; sart_angular_scan_outputs refuses them (SART_ERR_CONFIG).
+ *   sart_enable_mass_radial_hist takes the arguments of sart_enable_radial_hist, sart_enable_mass_band_images those of
+ * sart_enable_band_images, with the same checks (SART_ERR_ARG); nbins = 0 / n_bands = 0 switches them off (default).
+ * Switching one on while its single-mass counterpart is on fails with SART_ERR_CONFIG, and so does switching the
+ * counterpart on while it is on. On synchronises, then (re)allocates and zeroes them for SART_MAX_MASSES masses; when the
+ * device has no room, SART_ERR_NOMEM, and the accumulator stays off (the others are left as they were).
+ *   Device memory: the radial histograms 16 bytes per bin and mass for the rows, the same for the merged copy of
+ * sart_allreduce_outputs and 12 for the mass-minor accumulators the throughput kernels add into (28 MB at the default
+ * 16384 bins and SART_MAX_MASSES = 64 without the merged copy); the band images 64 MiB per band each for the rows, the
+ * mass-minor accumulators and the merged copy, about 3 x 64 MiB per band in all (768 MiB at 4 bands). */
+int sart_enable_mass_radial_hist(sart_handle_t* h, int nbins, double r_max);
+/* Synchronises and copies out the rows of the M masses; host arrays, either may be NULL: sum_w, counts [M][nbins].
+ * SART_ERR_ARG when they are off. */
+int sart_read_mass_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
+int sart_enable_mass_band_images(sart_handle_t* h, int n_bands, const double* edges_keV);
+/* Synchronises and copies out the rows of the M masses; host arrays, any may be NULL: image, image_w2
+ * [M][n_bands][256][256], counts [M][n_bands]. SART_ERR_ARG when they are off. */
+int sart_read_mass_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts);
 /* Optional detector images of the passed rays of sart_trace_mc per energy band, single axion mass: band b collects the
  * passed rays whose energy (energiesAx, rt:2197, as a per-ray record reports it: max(0.03 keV, the tabulated energy),
  * rt:470-471; the X-ray source's energy for its rays) lies in [edges_keV[b], edges_keV[b+1]). Each band has Σw and Σw² per
@@ -409,7 +443,8 @@ int sart_read_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energ
  * (re)allocates and zeroes them; n_bands = 0 switches them off (default; edges_keV may then be NULL); anything else is
  * SART_ERR_ARG. Device memory at n_bands bands: 1 MB per band for Σw and Σw², the same again for each of the 8 replicas the
  * throughput kernels add into (a fold after every launch adds them up), and 1 MB per band for the merged copy of
- * sart_allreduce_outputs: 16 + 128 + 16 MB at 16 bands. */
+ * sart_allreduce_outputs: 16 + 128 + 16 MB at 16 bands. Switching them on while the per-mass band images
+ * (sart_enable_mass_band_images) are on fails with SART_ERR_CONFIG. */
 int sart_enable_band_images(sart_handle_t* h, int n_bands, const double* edges_keV);
 /* Synchronises and copies out; host arrays, any may be NULL: image, image_w2 [n_bands][256][256] (the layout of the image),
  * counts [n_bands]. SART_ERR_ARG when the band images are off. */
@@ -469,8 +504,8 @@ void sart_comm_destroy(sart_handle_t* h);   /* also done by sart_destroy */
 int sart_allreduce(sart_handle_t* const* handles, int n);
 int sart_read_merged(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);
 /* Sums the optional accumulators of the fused run over all ranks: the radial histogram, the spectra, the per-mass
- * spectra, the band images, the quantity histograms, whichever are on (the band images with the same edges, the quantity
- * histograms with the same specs on every rank). Each goes into a merged copy per handle; the handles' own accumulators
+ * spectra, the band images, the quantity histograms, the per-mass radial histograms and band images, whichever are on
+ * (the band images with the same edges, the quantity histograms with the same specs on every rank). Each goes into a merged copy per handle; the handles' own accumulators
  * are untouched.
  * Every rank must have the same ones on with the same shapes. This is checked collectively, so a mismatch fails
  * with SART_ERR_CONFIG on every rank instead of hanging. Synchronises the handles' streams.
@@ -478,16 +513,16 @@ int sart_read_merged(sart_handle_t* h, double* image, double* image_w2, sart_cou
  * on one rank's state is decided from those words on every rank alike: a mismatch (SART_ERR_CONFIG), a rank that could not
  * allocate its merged copies (SART_ERR_NOMEM), nothing on anywhere (SART_ERR_ARG). Handles of one call (one process) are
  * compared on the host first (SART_ERR_CONFIG, before any collective). Then one group of all-reduces sums counts as u64
- * and sums as f64, so the counts stay exact; of the per-mass spectra only the rows of the M masses set are summed. These
+ * and sums as f64, so the counts stay exact; of the per-mass accumulators only the rows of the M masses set are summed. These
  * are queued on the handles' streams; the readers synchronise. Same forms as sart_allreduce (&h, 1 per rank, or n handles
  * of sart_comm_init_all); it does not need sart_allreduce and leaves its merged image alone.
  *   The merged copies are allocated at the first call (resized when a shape changes, freed by sart_destroy) and stay
  * readable until the next sart_allreduce_outputs; sart_reset_image leaves them. Switching an accumulator on, off or to
- * another size (and a new number of axion masses, for the per-mass spectra) invalidates its merged copy. */
+ * another size (and a new number of axion masses, for the per-mass accumulators) invalidates its merged copy. */
 int sart_allreduce_outputs(sart_handle_t* const* handles, int n);
 /* The merged copies; same arguments and array shapes as sart_read_radial_hist, sart_read_spectra,
- * sart_read_mass_spectra, sart_read_band_images and sart_read_quantity_hists. Synchronise and copy out; SART_ERR_ARG
- * without a valid merged copy. */
+ * sart_read_mass_spectra, sart_read_band_images, sart_read_quantity_hists, sart_read_mass_radial_hist and
+ * sart_read_mass_band_images. Synchronise and copy out; SART_ERR_ARG without a valid merged copy. */
 int sart_read_merged_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
 int sart_read_merged_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,
                              double* shell_sum_w, uint64_t* shell_counts);
@@ -495,6 +530,8 @@ int sart_read_merged_mass_spectra(sart_handle_t* h, double* energy_sum_w, double
                                   double* shell_sum_w, uint64_t* shell_counts);
 int sart_read_merged_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts);
 int sart_read_merged_quantity_hists(sart_handle_t* h, double* sum_w, double* sum_w2, uint64_t* counts);
+int sart_read_merged_mass_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts);
+int sart_read_merged_mass_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts);
 
 /* Synchronise and copy out. image/image_w2 may be NULL. counters is [M]. */
 int sart_read_image(sart_handle_t* h, double* image, double* image_w2, sart_counters_t* counters);
@@ -519,7 +556,8 @@ int sart_angular_scan(sart_handle_t* h, int n_angles, const double* angles_deg, 
  * images and the ray indices are those of sart_angular_scan; the handle's own accumulators, image and counters are left
  * bit-identical. The arrays of `out` are host arrays, any may be NULL (out itself too), with the scan point as their leading
  * dimension; one for an accumulator that is off is SART_ERR_ARG, and so is a call with none of the four on (use
- * sart_angular_scan). The per-mass spectra on give SART_ERR_CONFIG, more than one axion mass SART_ERR_ARG.
+ * sart_angular_scan). The per-mass spectra, radial histograms or band images on give SART_ERR_CONFIG, more than one axion
+ * mass SART_ERR_ARG.
  *   Device memory: the rows live in the handle's stage buffer next to the per-point images (1 MB per scan point), which
  * keeps its size after the call: the band images take n_angles x n_bands x 1 MB (800 MB for 50 points at 16 bands), the
  * radial histogram 16 bytes per bin and point, the spectra about 36 KB per point at nEnergies = 1500, the quantity

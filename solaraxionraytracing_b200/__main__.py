@@ -4,7 +4,8 @@
   python -m solaraxionraytracing_b200 [--ignoreDetWindow] [--ignoreGasAbs] [--ignoreConvProb] [--ignoreReflection]
       [--xrayTest] [--detectorInstall] [--magnet] [--angularScanMin A --angularScanMax B --numAngularScanPoints N]
       [--noPlots] [--config FILE | --configPath DIR] [--nRays N] [--precision f32|fast|exact] [--writeSpectra]
-      [--energyBands E0,E1,...] [--histogram NAME:NBINS:LO:HI ...] [--device D | --devices 0,1,... | --devices all]
+      [--energyBands E0,E1,...] [--histogram NAME:NBINS:LO:HI ...] [--massScanRadii] [--massScanBands E0,E1,...]
+      [--device D | --devices 0,1,... | --devices all]
 
 Inputs the reference reads from `resources/` and that are not shipped with it (solar_model_dataframe.csv, the two
 reflectivity HDF5 files) are taken from [Resources] when present, else generated: Primakoff emission rates from AGSS09
@@ -42,7 +43,8 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--energyBands", default=None,
                     help="also write one detector image per energy band: comma-separated band edges in keV, e.g. 0.5,2,4,8 "
                          "(2 to 17 values, ascending) writes axion_image_{year}_E0.5-2keV.csv and so on next to the image "
-                         "(an angular scan: one set per scan point, suffixed _angle{a}deg); a single axion mass only")
+                         "(an angular scan: one set per scan point, suffixed _angle{a}deg); a single axion mass only (a mass "
+                         "scan: --massScanBands)")
     ap.add_argument("--histogram", action="append", default=None, metavar="NAME:NBINS:LO:HI",
                     help="also write a weighted histogram of a per-ray record quantity of the passed rays, e.g. "
                          "transMagnet:256:0:1e-20, to axion_hist_{NAME}_{year}.csv next to the image (NBINS regular bins over "
@@ -51,6 +53,15 @@ def build_parser() -> argparse.ArgumentParser:
                          "writes one file per scan point, suffixed _angle{a}deg; a single axion mass only. With an angular "
                          "scan, each of these three switches also writes the containment radii of every scan point to "
                          "angular_scan_telescope_y_radii.csv")
+    ap.add_argument("--massScanRadii", action="store_true",
+                    help="a mass scan (several axion masses) also writes the 68 %% / 95.5 %% containment radii of every mass "
+                         "to mass_scan_radii.csv, from one traced ray per mass scan (a single axion mass: the radii are in "
+                         "the image CSV; see also --energyBands)")
+    ap.add_argument("--massScanBands", default=None, metavar="E0,E1,...",
+                    help="a mass scan also writes one detector image per energy band and mass, "
+                         "axion_image_{year}_E{lo}-{hi}keV_ma{m}eV.csv, with that mass's containment radii in the radius "
+                         "columns, and mass_scan_radii.csv as --massScanRadii; band edges as --energyBands (a single axion "
+                         "mass: --energyBands)")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--devices", default=None,
                     help="trace on several GPUs: a comma-separated list of CUDA ordinals or `all`. A fused run shards the "
@@ -102,6 +113,12 @@ def parse_args(argv=None) -> argparse.Namespace:
             a.energyBands = parse_energy_bands(a.energyBands)
         except ValueError as e:
             ap.error(f"--energyBands: {e}")
+    if a.massScanBands is not None:
+        from .output import parse_energy_bands
+        try:
+            a.massScanBands = parse_energy_bands(a.massScanBands)
+        except ValueError as e:
+            ap.error(f"--massScanBands: {e}")
     if a.histogram is not None:
         from .output import check_quantity_hist_specs, parse_quantity_hist
         try:
@@ -169,10 +186,13 @@ def load_tables(rt, tables, res, setup, device: int, allow_synthetic: bool = Fal
     return tables.TableSet(energies=em.energies, fluxRadiusCDF=rc, diffFluxCDFs=dc, reflectivity=refl, **extra, **det)
 
 
-def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath, bands=None, qhists=None):
+def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath, bands=None, qhists=None, mass_radial=None,
+                        mass_bands=None):
     """The files of a fused run: the image CSV and containment radii (at most one mass), or the per-mass images of a mass
     scan; with `spectra` also the spectra CSVs (one Spectra, or one per mass); with `bands` (output.BandImages, at most one
-    mass) one image CSV per energy band; with `qhists` (output.QuantityHist list, at most one mass) one CSV per histogram."""
+    mass) one image CSV per energy band; with `qhists` (output.QuantityHist list, at most one mass) one CSV per histogram;
+    with `mass_radial` (a mass scan: one radial histogram per mass) mass_scan_radii.csv, and with `mass_bands` (one
+    output.BandImages per mass) one image CSV per band and mass (output.write_mass_scan_outputs)."""
     from . import output
     if len(masses) <= 1:
         radii = output.containment_radii_from_hist(*radial_hist)
@@ -196,6 +216,10 @@ def write_fused_outputs(result, radial_hist, spectra, masses, setup, outpath, ba
         np.save(Path(outpath) / "axion_images_mass_scan.npy", result.image)
         if spectra is not None:
             for p in output.write_mass_spectra_csvs(spectra, masses, setup.detector.windowYear, outpath):
+                print("wrote", p)
+        if mass_radial is not None:
+            for p in output.write_mass_scan_outputs(masses, mass_radial, mass_bands, setup.detector.windowYear, outpath,
+                                                    setup.consts.chipXMax, setup.consts.chipYMax):
                 print("wrote", p)
 
 
@@ -227,7 +251,13 @@ def main(argv=None) -> int:
     setup, res = cfgmod.setup_from_config(cfg_file, flags)
     run = cfgmod.parseRun(cfgmod.load_config(cfg_file))
     if a.energyBands is not None and len(run.mAxion) > 1:
-        build_parser().error("--energyBands: the band images need a single axion mass, and the configuration sets a mass scan")
+        build_parser().error("--energyBands: the band images need a single axion mass, and the configuration sets a mass scan "
+                             "(use --massScanBands)")
+    mass_outputs = a.massScanRadii or a.massScanBands is not None
+    if mass_outputs and (len(run.mAxion) <= 1 or a.angularScanMin != a.angularScanMax):
+        which = "--massScanBands" if a.massScanBands is not None else "--massScanRadii"
+        build_parser().error(f"{which}: needs a mass scan (several axion masses in [Run] mAxion) without an angular scan; a "
+                             "single axion mass writes its radii with the image and its band images with --energyBands")
     if a.histogram is not None and len(run.mAxion) > 1:
         build_parser().error("--histogram: the quantity histograms need a single axion mass, and the configuration sets a mass scan")
     a.nRays = run.nRays if a.nRays is None else a.nRays
@@ -251,12 +281,14 @@ def main(argv=None) -> int:
             try:
                 r = multi_gpu.trace_on_devices(fs, devices, n, a.seed, precision=want, sampler=sampler,
                                                masses=run.mAxion or None, radial_hist=single, spectra=a.writeSpectra,
-                                               bands=a.energyBands, quantity_hists=a.histogram, warn=warn)
+                                               bands=a.energyBands, quantity_hists=a.histogram,
+                                               mass_radial_hist=mass_outputs, mass_bands=a.massScanBands, warn=warn)
             except rt.SartError as e:
                 if "NCCL" in str(e):
                     raise SystemExit(f"raytracer: {e}") from None
                 raise
-            write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath, r.band_images, r.quantity_hists)
+            write_fused_outputs(r.result, r.radial_hist, r.spectra, run.mAxion, setup, outpath, r.band_images, r.quantity_hists,
+                                r.mass_radial_hists, r.mass_band_images)
         elif scan_outputs:
             scan = multi_gpu.angular_scan_outputs_on_devices(fs, devices, a.angularScanMin, a.angularScanMax,
                                                              a.numAngularScanPoints, n, a.seed, precision=want,
@@ -286,6 +318,10 @@ def main(argv=None) -> int:
                 tr.enable_band_images(a.energyBands)
             if a.histogram is not None:
                 tr.enable_quantity_hists(a.histogram)
+            if mass_outputs:
+                tr.enable_mass_radial_hist()
+            if a.massScanBands is not None:
+                tr.enable_mass_band_images(a.massScanBands)
             tr.reset_image()
             tr.trace_mc(n, a.seed)
             result = tr.read_image()
@@ -295,7 +331,8 @@ def main(argv=None) -> int:
             bands = tr.read_band_images() if a.energyBands is not None else None
             qhists = tr.read_quantity_hists() if a.histogram is not None else None
             write_fused_outputs(result, tr.read_radial_hist() if single else None, spectra, run.mAxion, setup, outpath, bands,
-                                qhists)
+                                qhists, tr.read_mass_radial_hist() if mass_outputs else None,
+                                tr.read_mass_band_images() if a.massScanBands is not None else None)
         elif scan_outputs:
             tr.enable_radial_hist()
             if a.writeSpectra:

@@ -229,6 +229,10 @@ SIGNATURES = {
     "sart_enable_mass_spectra": (C.c_int, [H, C.c_int]),
     "sart_read_mass_spectra": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64), c_double_p,
                                          C.POINTER(C.c_uint64)]),
+    "sart_enable_mass_radial_hist": (C.c_int, [H, C.c_int, C.c_double]),
+    "sart_read_mass_radial_hist": (C.c_int, [H, c_double_p, C.POINTER(C.c_uint64)]),
+    "sart_enable_mass_band_images": (C.c_int, [H, C.c_int, c_double_p]),
+    "sart_read_mass_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_enable_band_images": (C.c_int, [H, C.c_int, c_double_p]),
     "sart_read_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_enable_quantity_hists": (C.c_int, [H, C.c_int, C.POINTER(QuantityHistSpec)]),
@@ -253,6 +257,8 @@ SIGNATURES = {
                                                 C.POINTER(C.c_uint64)]),
     "sart_read_merged_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_read_merged_quantity_hists": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
+    "sart_read_merged_mass_radial_hist": (C.c_int, [H, c_double_p, C.POINTER(C.c_uint64)]),
+    "sart_read_merged_mass_band_images": (C.c_int, [H, c_double_p, c_double_p, C.POINTER(C.c_uint64)]),
     "sart_angular_scan": (C.c_int, [H, C.c_int, c_double_p, C.c_uint64, C.c_uint64, C.c_uint64, c_double_p, C.POINTER(Counters),
                                     c_double_p]),
     "sart_angular_scan_outputs": (C.c_int, [H, C.c_int, c_double_p, C.c_uint64, C.c_uint64, C.c_uint64, c_double_p,

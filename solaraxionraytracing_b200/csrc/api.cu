@@ -357,10 +357,18 @@ static int upload_fast(sart_handle* h, const sart_tables_t* t) {
 static size_t carve_accum(AccumKind k, void* base, Accum* a) {
   Carve c(base);
   accum_arrays(k, *a, *a, accum_rows(k, SART_MAX_MASSES), [&](auto*& p, auto*&, size_t n) { c.take(p, n); });
-  if (k == kRadialHist) { a->rad.invStep = double(a->bins) / a->rmax; a->rad.nbins = a->bins; }
+  if (k == kRadialHist || k == kMassRadialHist) { a->rad.invStep = double(a->bins) / a->rmax; a->rad.nbins = a->bins; }
   if (k == kMassSpectra) { a->spec.eRow = uint32_t(a->bins); a->spec.sRow = uint32_t(SART_MAX_SHELLS); }
-  if (k == kBandImages) a->band.nBands = a->bins;
+  if (k == kBandImages || k == kMassBandImages) a->band.nBands = a->bins;
   return c.off;
+}
+
+// A failed allocation of accumulator k: the CUDA error, except that the per-mass radial histograms and band images, which
+// take SART_MAX_MASSES rows (about 3 x 64 MiB per band), report an out-of-memory device as SART_ERR_NOMEM.
+static int accum_alloc_fail(AccumKind k, cudaError_t e, size_t bytes) {
+  if (e == cudaErrorMemoryAllocation && (k == kMassRadialHist || k == kMassBandImages))
+    return fail(SART_ERR_NOMEM, "cudaMalloc (accumulator): no room for %zu bytes on the device", bytes);
+  return cuda_fail(e, "cudaMalloc (accumulator)");
 }
 
 int alloc_accum(AccumKind k, int bins, double rmax, Accum* a) {
@@ -368,7 +376,7 @@ int alloc_accum(AccumKind k, int bins, double rmax, Accum* a) {
   a->bins = bins; a->rmax = rmax;
   const size_t bytes = carve_accum(k, nullptr, a);
   const cudaError_t e = cudaMalloc(&a->blob, bytes);
-  if (e != cudaSuccess) { *a = Accum{}; return cuda_fail(e, "cudaMalloc (accumulator)"); }
+  if (e != cudaSuccess) { *a = Accum{}; return accum_alloc_fail(k, e, bytes); }
   a->bytes = bytes;
   carve_accum(k, a->blob, a);
   return SART_OK;
@@ -381,6 +389,9 @@ int alloc_accum(AccumKind k, int bins, double rmax, Accum* a) {
 // images' replicas (device_params.h: BandImages): w | w2, each bRep x [bins][256][256], and the band of each of the nE1
 // energy bins, which the exact kernels read through the handle's block (a->band) as well; their counts are the handle's. The
 // quantity histograms' replicas of Σw and Σw² (device_params.h: QuantityHists::rw, rw2), each qRep x bins, in a->qh itself.
+// The per-mass radial histograms' mass-minor accumulators (fast_common.cuh: mass_scan_loop): w | 32-bit n, each
+// [bins][SART_MAX_MASSES]. The per-mass band images' mass-minor accumulators: w | w2, each [bins][256][256][SART_MAX_MASSES] |
+// 32-bit n [bins][SART_MAX_MASSES], and the band table as for the band images.
 static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, int bRep, int qRep, void* base, Accum* a) {
   Carve c(base);
   Spectra* r = &a->tput;
@@ -402,6 +413,20 @@ static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, int bRe
     c.take(b.w, size_t(bRep) * len); c.take(b.w2, size_t(bRep) * len); c.take(b.band, size_t(nE1));
     b.repStride = uint32_t(len); b.repMask = uint32_t(bRep - 1);
     a->band.band = b.band;
+  } else if (k == kMassRadialHist) {
+    RadialHist& m = a->tput_rad;
+    m = a->rad;
+    unsigned int* n;
+    c.take(m.w, size_t(a->bins) * SART_MAX_MASSES); c.take(n, size_t(a->bins) * SART_MAX_MASSES);
+    m.n = reinterpret_cast<unsigned long long*>(n);
+  } else if (k == kMassBandImages) {
+    BandImages& b = a->tput_band;
+    b = a->band;
+    const size_t len = size_t(a->bins) * SART_IMAGE_BINS * SART_IMAGE_BINS * SART_MAX_MASSES;
+    unsigned int* n;
+    c.take(b.w, len); c.take(b.w2, len); c.take(n, size_t(a->bins) * SART_MAX_MASSES); c.take(b.band, size_t(nE1));
+    b.n = reinterpret_cast<unsigned long long*>(n);
+    a->band.band = b.band;
   } else if (k == kQuantityHists) {
     QuantityHists& q = a->qh;
     c.take(q.rw, size_t(qRep) * size_t(a->bins)); c.take(q.rw2, size_t(qRep) * size_t(a->bins));
@@ -410,11 +435,11 @@ static size_t carve_throughput(AccumKind k, int nE1, int eRep, int sRep, int bRe
   return c.off;
 }
 
-// The band images' table of the energy bins from bin `from` on (sart_enable_band_images; device_params.h: BandImages): the band
-// of the energy a per-ray record reports, max(0.03 keV, energies[i]) for tabulated energy i (rt:470-471) and the X-ray
-// source's energy for bin nEnergies.
-static int put_band_table(sart_handle* h, int from) {
-  const Accum& a = h->accum[kBandImages];
+// The (per-mass) band images' table of the energy bins from bin `from` on (sart_enable_band_images,
+// sart_enable_mass_band_images; device_params.h: BandImages): the band of the energy a per-ray record reports,
+// max(0.03 keV, energies[i]) for tabulated energy i (rt:470-471) and the X-ray source's energy for bin nEnergies.
+static int put_band_table(sart_handle* h, AccumKind k, int from) {
+  const Accum& a = h->accum[k];
   const int nE = h->params.nEnergies;
   auto band_of = [&](double E) {
     for (int b = 0; b < a.bins; ++b)
@@ -481,13 +506,16 @@ static int new_accum(sart_handle* h, AccumKind k, int bins, double rmax, const d
   const int qRep = std::min(pow2("SART_QHIST_REPLICAS", 8), 64);
   const int nE1 = h->params.nEnergies + 1;
   const size_t tputBytes = carve_throughput(k, nE1, eRep, sRep, bRep, qRep, nullptr, &a);
-  if (tputBytes) SART_CUDA(cudaMalloc(&a.tput_blob, tputBytes));
+  if (tputBytes) {
+    const cudaError_t e = cudaMalloc(&a.tput_blob, tputBytes);
+    if (e != cudaSuccess) { a.tput_blob = nullptr; return accum_alloc_fail(k, e, tputBytes); }
+  }
   SART_CUDA(cudaMemsetAsync(a.blob, 0, a.bytes, h->stream));
   if (tputBytes) SART_CUDA(cudaMemsetAsync(a.tput_blob, 0, tputBytes, h->stream));
   SART_CUDA(cudaStreamSynchronize(h->stream));
   carve_throughput(k, nE1, eRep, sRep, bRep, qRep, a.tput_blob, &a);
   if (k == kRadialHist) h->tables.rad = h->ftables.rad = a.rad;
-  return k == kBandImages ? put_band_table(h, 0) : SART_OK;
+  return k == kBandImages || k == kMassBandImages ? put_band_table(h, k, 0) : SART_OK;
 }
 
 // What every sart_enable_* does after its own checks: synchronises, switches accumulator k off, and with bins > 0 on again,
@@ -498,7 +526,10 @@ static int set_accum(sart_handle* h, AccumKind k, int bins, double rmax = 0.0, c
   SART_CUDA(cudaStreamSynchronize(h->stream));
   free_accum(h, k);
   const int rc = bins > 0 ? new_accum(h, k, bins, rmax, edges, n_q, qspecs) : SART_OK;
-  if (rc) free_accum(h, k);
+  if (rc) {
+    free_accum(h, k);
+    cudaGetLastError();   // a failed cudaMalloc must not surface at the next launch
+  }
   return rc;
 }
 
@@ -526,9 +557,11 @@ int read_accum(sart_handle* h, AccumKind k, bool merged, std::initializer_list<v
 static int ensure_image(sart_handle* h, int nMasses) {
   const size_t len = size_t(nMasses) * SART_IMAGE_BINS * SART_IMAGE_BINS;
   if (h->d_image && h->image_masses == nMasses) return SART_OK;
-  const int rc = clear_accum(h, kMassSpectra);   // a new mass list: the per-mass rows of the old one are meaningless
-  if (rc) return rc;
-  h->merged_accum[kMassSpectra].valid = 0;
+  for (AccumKind k : kAllAccums) {   // a new mass list: the per-mass rows of the old one are meaningless
+    if (!per_mass(k)) continue;
+    if (const int rc = clear_accum(h, k)) return rc;
+    h->merged_accum[k].valid = 0;
+  }
   cudaFree(h->d_image); cudaFree(h->d_counters);   // d_image_w2 points into d_image's block
   h->d_image = nullptr; h->d_image_w2 = nullptr; h->d_counters = nullptr; h->image_masses = 0; h->merged_valid = 0;
   SART_CUDA(cudaMalloc(&h->d_image, merged_words(nMasses) * sizeof(double)));
@@ -847,8 +880,9 @@ int sart_update_setup(sart_handle_t* h, const sart_setup_t* setup) {
     return fail(rc, "sart_update_setup failed, previous setup kept: %s", msg);
   }
   // the band of the X-ray source's energy bin, like its reflectivity row (upload_fast)
-  if (h->accum[kBandImages].blob && old.testSource.energy != setup->testSource.energy && (rc = put_band_table(h, h->params.nEnergies)))
-    return rc;
+  for (AccumKind k : {kBandImages, kMassBandImages})
+    if (h->accum[k].blob && old.testSource.energy != setup->testSource.energy && (rc = put_band_table(h, k, h->params.nEnergies)))
+      return rc;
   if (h->n_masses == 1 && h->masses_default) {
     h->masses[0] = setup->consts.mAxion;
     SART_CUDA(cudaMemcpyAsync(h->d_masses, h->masses, sizeof(double), cudaMemcpyHostToDevice, h->stream));
@@ -1295,26 +1329,39 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
   if (h->sampler == SART_SAMPLER_ALIAS && (h->precision != 2 || h->n_masses > 1))
     return fail(SART_ERR_CONFIG, "the alias sampler needs precision mode 2 and a single axion mass");
   const Accum &spec = h->accum[kSpectra], &mspec = h->accum[kMassSpectra];
+  const Accum &mrad = h->accum[kMassRadialHist], &mbands = h->accum[kMassBandImages];
+  const bool massRows = mrad.blob || mbands.blob;
+  const bool perMass = mspec.blob || massRows;   // the per-mass accumulators run the mass-scan kernels for every M
   if (spec.blob && h->n_masses > 1) return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass");
+  if (spec.blob && massRows)   // the mass-scan kernels fill the per-mass spectra, not these
+    return fail(SART_ERR_CONFIG, "sart_trace_mc: the spectra need a single axion mass and the per-mass radial histograms "
+                                 "and band images off (use sart_enable_mass_spectra)");
   if (mspec.blob && h->sampler == SART_SAMPLER_ALIAS)
     return fail(SART_ERR_CONFIG, "sart_trace_mc: the per-mass spectra run the mass-scan kernels, which need the inverse-CDF sampler");
+  if (massRows && h->sampler == SART_SAMPLER_ALIAS)
+    return fail(SART_ERR_CONFIG, "sart_trace_mc: the per-mass radial histograms and band images run the mass-scan kernels, "
+                                 "which need the inverse-CDF sampler");
   const Accum& bands = h->accum[kBandImages];
-  if (bands.blob && (h->n_masses > 1 || mspec.blob))
-    return fail(SART_ERR_CONFIG, "sart_trace_mc: the band images need a single axion mass and the per-mass spectra off");
+  if (bands.blob && (h->n_masses > 1 || perMass))
+    return fail(SART_ERR_CONFIG, "sart_trace_mc: the band images need a single axion mass and the per-mass spectra, radial "
+                                 "histograms and band images off");
   const Accum& qhists = h->accum[kQuantityHists];
-  if (qhists.blob && (h->n_masses > 1 || mspec.blob))
-    return fail(SART_ERR_CONFIG, "sart_trace_mc: the quantity histograms need a single axion mass and the per-mass spectra off");
+  if (qhists.blob && (h->n_masses > 1 || perMass))
+    return fail(SART_ERR_CONFIG, "sart_trace_mc: the quantity histograms need a single axion mass and the per-mass spectra, "
+                                 "radial histograms and band images off");
   const size_t plane = size_t(SART_IMAGE_BINS) * SART_IMAGE_BINS;
   int rc = SART_OK;
-  // A mass scan, or any run with the per-mass spectra on (one contract for every mass list, M = 1 included): the exact
-  // kernels add the spectra into the handle's rows directly, the throughput kernels into mass-minor accumulators that
-  // k_fold_mass_spectra adds up after every launch.
-  if (h->n_masses > 1 || mspec.blob) {
+  // A mass scan, or any run with a per-mass accumulator on (one contract for every mass list, M = 1 included): the exact
+  // kernels add the per-mass spectra, radial histograms and band images into the handle's rows directly, the throughput
+  // kernels into mass-minor accumulators that k_fold_mass_spectra, k_fold_mass_hist and k_fold_mass_acc add up after every
+  // launch.
+  if (h->n_masses > 1 || perMass) {
     Tables et = h->tables;
     et.spec = mspec.spec;   // or off
+    const MassRows rows{mrad.rad, mbands.band}, acc{mrad.tput_rad, mbands.tput_band};   // or off
     if (h->precision == 0) {
       SART_CUDA(launch_mc_image_exact(h->params, et, h->n_masses, h->d_masses, first_ray, n_rays, seed, h->d_image,
-                                      h->d_image_w2, h->d_counters, h->sm_count, h->stream));
+                                      h->d_image_w2, h->d_counters, h->sm_count, h->stream, {}, {}, rows));
       return SART_OK;
     }
     const size_t accLen = plane * SART_MAX_MASSES;
@@ -1324,31 +1371,43 @@ int sart_trace_mc(sart_handle_t* h, uint64_t first_ray, uint64_t n_rays, uint64_
     }
     fast::FastTables ft = h->ftables;
     ft.spec = mspec.tput;   // or off
-    // the spectra's 32-bit counts are folded after every launch of at most kMaxRaysPerLaunch rays
-    auto fold_spectra = [&]() { return mspec.blob ? launch_fold_mass_spectra(mspec.tput, h->n_masses, mspec.bins, mspec.spec, h->stream)
-                                                  : cudaSuccess; };
+    // the 32-bit counts of the per-mass accumulators are folded after every launch of at most kMaxRaysPerLaunch rays
+    auto fold_spectra = [&]() {
+      cudaError_t e = cudaSuccess;
+      if (mspec.blob) e = launch_fold_mass_spectra(mspec.tput, h->n_masses, mspec.bins, mspec.spec, h->stream);
+      if (e == cudaSuccess && mrad.blob)
+        e = launch_fold_mass_hist(acc.rad.w, reinterpret_cast<unsigned int*>(acc.rad.n), h->n_masses, mrad.bins, mrad.rad.w,
+                                  mrad.rad.n, h->stream);
+      if (e == cudaSuccess && mbands.blob)
+        e = launch_fold_mass_hist(nullptr, reinterpret_cast<unsigned int*>(acc.band.n), h->n_masses, mbands.bins, nullptr,
+                                  mbands.band.n, h->stream);
+      if (e == cudaSuccess && mbands.blob)
+        e = launch_fold_mass_acc(acc.band.w, acc.band.w2, h->n_masses, size_t(mbands.bins) * plane, mbands.band.w, mbands.band.w2,
+                                 h->stream);
+      return e;
+    };
     if (h->precision == 2) {
       rc = f32_then_retrace(h, n_rays, true,   // the alias sampler was refused above
           [&](uint64_t done, uint64_t m, const fast::RetraceQueue& q) {
             ft.rq = q;
             const cudaError_t e = launch_mc_image_f32_masses(h->fparams, h->geo32, ft, h->n_masses, h->d_masses, first_ray + done,
                                                              m, seed, h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters,
-                                                             h->sm_count, h->stream);
+                                                             h->sm_count, h->stream, acc);
             return e != cudaSuccess ? e : fold_spectra();
           },
           [&](uint64_t done, uint64_t, const fast::RetraceQueue& q) {
             return launch_retrace_mc_image(h->params, et, h->n_masses, h->d_masses, first_ray + done, seed, q, h->d_image,
-                                           h->d_image_w2, h->d_counters, h->sm_count, h->stream);
+                                           h->d_image_w2, h->d_counters, h->sm_count, h->stream, {}, {}, rows);
           });
       if (rc) return rc;
-    } else if (!mspec.blob) {
+    } else if (!perMass) {
       SART_CUDA(launch_mc_image_fast_masses(h->fparams, ft, h->n_masses, h->d_masses, first_ray, n_rays, seed,
                                             h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream));
     } else {
       for (uint64_t done = 0; done < n_rays; done += fast::kMaxRaysPerLaunch) {
         const uint64_t m = std::min<uint64_t>(n_rays - done, fast::kMaxRaysPerLaunch);
         SART_CUDA(launch_mc_image_fast_masses(h->fparams, ft, h->n_masses, h->d_masses, first_ray + done, m, seed,
-                                              h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream));
+                                              h->d_mass_acc, h->d_mass_acc + accLen, h->d_counters, h->sm_count, h->stream, acc));
         SART_CUDA(fold_spectra());
       }
     }
@@ -1388,6 +1447,45 @@ int sart_reset_image(sart_handle_t* h) {
   return SART_OK;
 }
 
+// The argument checks of sart_enable_band_images and sart_enable_mass_band_images.
+static int check_band_edges(int n_bands, const double* edges_keV, const char* who) {
+  if (n_bands < 0 || n_bands > SART_MAX_BANDS || (n_bands > 0 && !edges_keV))
+    return fail(SART_ERR_ARG, "%s: need 1..%d bands and their edges, or 0 (off)", who, SART_MAX_BANDS);
+  for (int b = 0; n_bands > 0 && b <= n_bands; ++b)
+    if (!std::isfinite(edges_keV[b]) || edges_keV[b] < 0.0 || (b > 0 && !(edges_keV[b] > edges_keV[b - 1])))
+      return fail(SART_ERR_ARG, "%s: the band edges must be finite, >= 0 and strictly ascending", who);
+  return SART_OK;
+}
+
+int sart_enable_mass_radial_hist(sart_handle_t* h, int nbins, double r_max) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (nbins < 0 || nbins > (1 << 24) || (nbins > 0 && !(r_max > 0.0)))
+    return fail(SART_ERR_ARG, "sart_enable_mass_radial_hist: bad argument");
+  if (nbins > 0 && h->accum[kRadialHist].blob)
+    return fail(SART_ERR_CONFIG, "sart_enable_mass_radial_hist: the single-mass radial histogram is on (sart_enable_radial_hist); "
+                                 "switch it off first");
+  return set_accum(h, kMassRadialHist, nbins, r_max);
+}
+
+int sart_read_mass_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts) {
+  return read_accum(h, kMassRadialHist, false, {sum_w, counts},
+                    "sart_read_mass_radial_hist: no per-mass radial histograms enabled (sart_enable_mass_radial_hist)");
+}
+
+int sart_enable_mass_band_images(sart_handle_t* h, int n_bands, const double* edges_keV) {
+  if (!h) return fail(SART_ERR_ARG, "handle is NULL");
+  if (int rc = check_band_edges(n_bands, edges_keV, "sart_enable_mass_band_images")) return rc;
+  if (n_bands > 0 && h->accum[kBandImages].blob)
+    return fail(SART_ERR_CONFIG, "sart_enable_mass_band_images: the single-mass band images are on (sart_enable_band_images); "
+                                 "switch them off first");
+  return set_accum(h, kMassBandImages, n_bands, 0.0, edges_keV);
+}
+
+int sart_read_mass_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts) {
+  return read_accum(h, kMassBandImages, false, {image, image_w2, counts},
+                    "sart_read_mass_band_images: no per-mass band images enabled (sart_enable_mass_band_images)");
+}
+
 int sart_enable_mass_spectra(sart_handle_t* h, int on) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
   if (on && h->accum[kSpectra].blob)
@@ -1416,11 +1514,10 @@ int sart_read_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum
 
 int sart_enable_band_images(sart_handle_t* h, int n_bands, const double* edges_keV) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
-  if (n_bands < 0 || n_bands > SART_MAX_BANDS || (n_bands > 0 && !edges_keV))
-    return fail(SART_ERR_ARG, "sart_enable_band_images: need 1..%d bands and their edges, or 0 (off)", SART_MAX_BANDS);
-  for (int b = 0; n_bands > 0 && b <= n_bands; ++b)
-    if (!std::isfinite(edges_keV[b]) || edges_keV[b] < 0.0 || (b > 0 && !(edges_keV[b] > edges_keV[b - 1])))
-      return fail(SART_ERR_ARG, "sart_enable_band_images: the band edges must be finite, >= 0 and strictly ascending");
+  if (int rc = check_band_edges(n_bands, edges_keV, "sart_enable_band_images")) return rc;
+  if (n_bands > 0 && h->accum[kMassBandImages].blob)
+    return fail(SART_ERR_CONFIG, "sart_enable_band_images: the per-mass band images are on (sart_enable_mass_band_images); "
+                                 "switch them off first");
   return set_accum(h, kBandImages, n_bands, 0.0, edges_keV);
 }
 
@@ -1457,6 +1554,9 @@ int sart_read_quantity_hists(sart_handle_t* h, double* sum_w, double* sum_w2, ui
 int sart_enable_radial_hist(sart_handle_t* h, int nbins, double r_max) {
   if (!h) return fail(SART_ERR_ARG, "handle is NULL");
   if (nbins < 0 || nbins > (1 << 24) || (nbins > 0 && !(r_max > 0.0))) return fail(SART_ERR_ARG, "sart_enable_radial_hist: bad argument");
+  if (nbins > 0 && h->accum[kMassRadialHist].blob)
+    return fail(SART_ERR_CONFIG, "sart_enable_radial_hist: the per-mass radial histograms are on (sart_enable_mass_radial_hist); "
+                                 "switch them off first");
   return set_accum(h, kRadialHist, nbins, r_max);
 }
 
@@ -1603,7 +1703,7 @@ static int angular_scan(sart_handle* h, int n_angles, const double* angles_deg, 
   if (images) SART_CUDA(cudaMemcpyAsync(images, dImg, size_t(n_angles) * plane * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   for (AccumKind k : kAllAccums) {
     if (!rows[k].bins) continue;
-    void* host[5];
+    void* host[5] = {};
     scan_out_arrays(*out, k, host);
     void* const* hp = host;
     cudaError_t e = cudaSuccess;
@@ -1642,10 +1742,13 @@ int sart_angular_scan_outputs(sart_handle_t* h, int n_angles, const double* angl
   if (rc) return rc;
   if (h->accum[kMassSpectra].blob)
     return fail(SART_ERR_CONFIG, "sart_angular_scan_outputs: the per-mass spectra are on; a scan fills single-mass rows only");
+  if (h->accum[kMassRadialHist].blob || h->accum[kMassBandImages].blob)
+    return fail(SART_ERR_CONFIG, "sart_angular_scan_outputs: the per-mass radial histograms or band images are on; a scan fills "
+                                 "single-mass rows only");
   const sart_scan_out_t none{};
   if (!out) out = &none;
   static const char* const names[kAccums] = {"radial histogram", "spectra", "per-mass spectra", "band images",
-                                             "quantity histograms"};
+                                             "quantity histograms", "per-mass radial histograms", "per-mass band images"};
   bool any = false;
   for (AccumKind k : kAllAccums) {
     void* p[5];

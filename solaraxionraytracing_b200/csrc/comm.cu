@@ -101,9 +101,13 @@ static_assert(2 * kDescWords <= kDescCapacity, "the descriptor travels in sart_h
 
 static void describe_outputs(const sart_handle* h, long long d[kDescWords]) {
   for (AccumKind k : kAllAccums) d[k] = h->accum[k].bins;
-  std::memcpy(&d[kDescRadMax], &h->accum[kRadialHist].rmax, sizeof(long long));
+  // a handle has at most one of the single-mass and the per-mass radial histogram on, and at most one of the band images:
+  // the r_max and edge words are those of the one that is on (its bins word tells which)
+  const AccumKind rad = h->accum[kMassRadialHist].blob ? kMassRadialHist : kRadialHist;
+  const AccumKind band = h->accum[kMassBandImages].blob ? kMassBandImages : kBandImages;
+  std::memcpy(&d[kDescRadMax], &h->accum[rad].rmax, sizeof(long long));
   d[kDescMasses] = h->n_masses;
-  std::memcpy(&d[kDescEdges], h->accum[kBandImages].edges, (SART_MAX_BANDS + 1) * sizeof(long long));
+  std::memcpy(&d[kDescEdges], h->accum[band].edges, (SART_MAX_BANDS + 1) * sizeof(long long));
   const Accum& q = h->accum[kQuantityHists];
   for (int j = 0; j < SART_N_QUANTITIES; ++j) {
     uint64_t lo = 0, hi = 0;
@@ -273,7 +277,8 @@ int sart_allreduce_outputs(sart_handle_t* const* handles, int n) {
     for (int k = 0; k < kDescErr; ++k)
       if (desc[size_t(i) * 2 * kDescWords + k] != desc[k])
         return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: handles 0 and %d differ in their radial histogram, spectra, "
-                                     "per-mass spectra, band images, quantity histograms or number of axion masses", i);
+                                     "per-mass spectra, band images, quantity histograms, per-mass radial histograms, "
+                                     "per-mass band images or number of axion masses", i);
   auto desc_dev = [](sart_handle* h) { return h->d_desc; };
   for (int i = 0; i < n; ++i) {
     sart_handle* h = handles[i];
@@ -316,15 +321,18 @@ int sart_allreduce_outputs(sart_handle_t* const* handles, int n) {
   const long long* neg_lo = &red[kDescWords];
   if (hi[kDescErr]) return fail(SART_ERR_NOMEM, "sart_allreduce_outputs: a rank could not allocate its merged copies");
   static const char* const what[kDescEdges] = {"radial histogram bins", "spectra bins", "per-mass spectra bins",
-                                               "number of energy bands", "quantity histogram entries", "radial histogram r_max",
-                                               "number of axion masses"};
+                                               "number of energy bands", "quantity histogram entries",
+                                               "per-mass radial histogram bins", "number of per-mass energy bands",
+                                               "radial histogram r_max", "number of axion masses"};
   for (int k = 0; k < kDescErr; ++k)
     if (hi[k] != -neg_lo[k])
       return fail(SART_ERR_CONFIG, "sart_allreduce_outputs: the ranks differ in their %s",
                   k < kDescEdges ? what[k] : (k < kDescQSpec ? "energy band edges" : "quantity histogram specs"));
-  if (!hi[kRadialHist] && !hi[kSpectra] && !hi[kMassSpectra] && !hi[kBandImages] && !hi[kQuantityHists])
+  bool any = false;
+  for (AccumKind k : kAllAccums) any |= hi[k] != 0;
+  if (!any)
     return fail(SART_ERR_ARG, "sart_allreduce_outputs: no radial histogram, spectra or per-mass spectra enabled, and no band "
-                              "images or quantity histograms");
+                              "images, quantity histograms, per-mass radial histograms or per-mass band images");
   // the payload: counts as u64, sums as f64, of the per-mass rows only those of the M masses set, every all-reduce of every
   // handle in one group
   r = api->GroupStart();
@@ -365,6 +373,16 @@ int sart_read_merged_band_images(sart_handle_t* h, double* image, double* image_
 int sart_read_merged_quantity_hists(sart_handle_t* h, double* sum_w, double* sum_w2, uint64_t* counts) {
   return read_accum(h, kQuantityHists, true, {sum_w, sum_w2, counts},
                     "sart_read_merged_quantity_hists: no merged quantity histograms (call sart_allreduce_outputs first)");
+}
+
+int sart_read_merged_mass_radial_hist(sart_handle_t* h, double* sum_w, uint64_t* counts) {
+  return read_accum(h, kMassRadialHist, true, {sum_w, counts},
+                    "sart_read_merged_mass_radial_hist: no merged per-mass radial histograms (call sart_allreduce_outputs first)");
+}
+
+int sart_read_merged_mass_band_images(sart_handle_t* h, double* image, double* image_w2, uint64_t* counts) {
+  return read_accum(h, kMassBandImages, true, {image, image_w2, counts},
+                    "sart_read_merged_mass_band_images: no merged per-mass band images (call sart_allreduce_outputs first)");
 }
 
 int sart_read_merged_mass_spectra(sart_handle_t* h, double* energy_sum_w, double* energy_sum_w2, uint64_t* energy_counts,

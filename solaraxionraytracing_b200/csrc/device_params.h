@@ -134,6 +134,40 @@ __device__ __forceinline__ void band_add(const BandImages& b, int eIdx, int bin,
 }
 #endif
 
+// Optional per-mass radial histograms and band images of a mass scan (sart_enable_mass_radial_hist,
+// sart_enable_mass_band_images): the shapes of RadialHist and BandImages, rad.w / band.w == nullptr: off. The exact kernels get
+// the handle's rows, mass m's radial bins from m * rad.nbins on, its band planes from m * band.nBands * 256 * 256 and its band
+// counts from m * band.nBands (mass_rows_add). The mass-scan kernels of the throughput pipelines get
+// mass-minor accumulators in the same struct (fast_common.cuh: mass_scan_loop). Passed to the kernels that fill them as a
+// parameter of its own.
+struct MassRows {
+  RadialHist rad;
+  BandImages band;
+};
+
+#if defined(__CUDACC__)
+// A passed ray of mass m into row m of the handle's per-mass radial histograms and band images (the exact kernels): the
+// radial bin rule of rad_add, the band and image bin of band_add.
+__device__ __forceinline__ void mass_rows_add(const MassRows& R, int m, double r, int eIdx, int bin, double w) {
+  if (R.rad.w) {
+    int b = int(r * R.rad.invStep);
+    b = b < 0 ? 0 : (b > R.rad.nbins - 1 ? R.rad.nbins - 1 : b);
+    const size_t at = size_t(m) * size_t(R.rad.nbins) + size_t(b);
+    atomicAdd(R.rad.w + at, w);
+    atomicAdd(R.rad.n + at, 1ull);
+  }
+  if (!R.band.w) return;
+  const unsigned k = __ldg(R.band.band + eIdx);
+  if (k == kNoBand) return;
+  const uint32_t row = uint32_t(m) * uint32_t(R.band.nBands) + k;
+  atomicAdd(R.band.n + row, 1ull);
+  if (bin < 0) return;
+  const size_t at = size_t(row) * (SART_IMAGE_BINS * SART_IMAGE_BINS) + size_t(bin);
+  atomicAdd(R.band.w + at, w);
+  atomicAdd(R.band.w2 + at, w * w);
+}
+#endif
+
 // Optional weighted histograms of per-ray record quantities of the passed rays (sart_enable_quantity_hists): histogram j
 // (quantity[j], a SART_Q_*) has nbins[j] + 2 entries from entry off[j] on — underflow, the regular bins, overflow — of
 // `entries` in all. w / w2 / n: Σw, Σw² and the count per entry, the handle's arrays (the exact kernels add into them per

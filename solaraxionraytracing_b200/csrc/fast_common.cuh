@@ -593,8 +593,17 @@ __device__ __forceinline__ void mass_spec_add(const Spectra& a, int m, int eBin,
 // kPer = masses per lane (1, 2 or SART_MAX_MASSES / 32): the launcher picks the smallest that holds nMasses, because the
 // per-mass sums are 15 registers per mass and lane (with 4 masses per lane the FP32 kernel spilled: 80 registers, 112 bytes).
 // kSpectra: the passed ray-masses also go to the per-mass spectra `spec` (mass_spec_add); false compiles them out.
-template <int kPer, bool kSpectra, class Trace>
-__device__ __forceinline__ void mass_scan_loop(const FastParams& P, const RadialHist& rad, const Spectra& spec,
+// kRows: the passed ray-masses also go to the per-mass radial histograms and band images R that are on (device_params.h:
+// MassRows; here mass-minor accumulators like the image's: Σw [bin][SART_MAX_MASSES] and a 32-bit count of the same shape
+// for the radial histograms, Σw and Σw² [band][256 * 256][SART_MAX_MASSES] and a 32-bit count [band][SART_MAX_MASSES] for
+// the band images, which k_fold_mass_acc / k_fold_mass_hist add into the handle's rows after every launch of at most
+// kMaxRaysPerLaunch rays). The tracing lane resolves its ray's radial bin and band, so that two integers go through the
+// broadcast. The band counts are
+// a few hundred addresses that every passed ray-mass of the grid would add to, so a block counts them in shared memory and
+// adds them into the accumulators once, at its end (measured on B200, config 4, 4 bands: with the counts in global memory
+// the band images cost 5.98x the plain scan).
+template <int kPer, bool kSpectra, bool kRows = false, class Trace>
+__device__ __forceinline__ void mass_scan_loop(const FastParams& P, const RadialHist& rad, const Spectra& spec, const MassRows& R,
                                                const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays,
                                                double* __restrict__ image, double* __restrict__ imageW2,
                                                sart_counters_t* __restrict__ counters, WarpCounters* wc, Trace trace) {
@@ -612,6 +621,13 @@ __device__ __forceinline__ void mass_scan_loop(const FastParams& P, const Radial
     nPassed[k] = nZero[k] = nTill[k] = 0u;
   }
   unsigned int nIter = 0;
+  unsigned int* bandN = nullptr;   // kRows: the block's band counts [band][SART_MAX_MASSES]
+  if constexpr (kRows) {
+    __shared__ unsigned int n[SART_MAX_BANDS * SART_MAX_MASSES];
+    for (int i = threadIdx.x; i < SART_MAX_BANDS * SART_MAX_MASSES; i += blockDim.x) n[i] = 0u;
+    __syncthreads();
+    bandN = n;
+  }
   const uint64_t stride = uint64_t(gridDim.x) * blockDim.x;
   for (uint64_t b = uint64_t(blockIdx.x) * blockDim.x + (threadIdx.x & ~31); b < nRays; b += stride) {   // warp-uniform
     const uint64_t i = b + lane;
@@ -626,6 +642,14 @@ __device__ __forceinline__ void mass_scan_loop(const FastParams& P, const Radial
       else if (r.windowMiss) atomicAdd(&wc[warp].n_exit[SART_EXIT_WINDOW_APERTURE], 1u);
       if (r.clamped) atomicAdd(&wc[warp].n_clamped, 1u);
     }
+    int radBin = 0, band = kNoBand;   // kRows: this lane's ray's radial bin and band
+    if (kRows && valid && r.code < 0) {
+      if (R.rad.w) {
+        radBin = int(r.r * R.rad.invStep);
+        radBin = radBin < 0 ? 0 : (radBin > R.rad.nbins - 1 ? R.rad.nbins - 1 : radBin);
+      }
+      if (R.band.w) band = __ldg(R.band.band + r.eIdx);
+    }
     unsigned alive = __ballot_sync(kFull, valid && r.code < 0);
     while (alive) {
       const int src = __ffs(alive) - 1;
@@ -639,6 +663,7 @@ __device__ __forceinline__ void mass_scan_loop(const FastParams& P, const Radial
       const int bin = __shfl_sync(kFull, r.bin, src);
       const bool miss = __shfl_sync(kFull, int(r.windowMiss), src) != 0;
       const int eBin = kSpectra ? __shfl_sync(kFull, r.eIdx, src) : 0, shell = kSpectra ? __shfl_sync(kFull, r.shell, src) : 0;
+      const int rBin = kRows ? __shfl_sync(kFull, radBin, src) : 0, bBand = kRows ? __shfl_sync(kFull, band, src) : int(kNoBand);
 #pragma unroll
       for (int k = 0; k < kPer; ++k) {
         const int m = lane + 32 * k;
@@ -658,6 +683,20 @@ __device__ __forceinline__ void mass_scan_loop(const FastParams& P, const Radial
           }
           if (m == 0 && rad.w) rad_add(rad, rr, w);   // the radial histogram follows the first mass, as in the exact kernel
           if (kSpectra) mass_spec_add(spec, m, eBin, shell, w);
+          if (kRows && R.rad.w) {
+            const uint32_t at = uint32_t(rBin) * SART_MAX_MASSES + uint32_t(m);
+            atomicAdd(R.rad.w + at, w);
+            atomicAdd(reinterpret_cast<unsigned int*>(R.rad.n) + at, 1u);
+          }
+          if (kRows && bBand != int(kNoBand)) {
+            atomicAdd(bandN + (uint32_t(bBand) * SART_MAX_MASSES + uint32_t(m)), 1u);
+            if (bin >= 0) {
+              const uint32_t at = (uint32_t(bBand) * uint32_t(SART_IMAGE_BINS * SART_IMAGE_BINS) + uint32_t(bin)) * SART_MAX_MASSES +
+                                  uint32_t(m);
+              atomicAdd(R.band.w + at, w);
+              atomicAdd(R.band.w2 + at, w * w);
+            }
+          }
         } else {
           ++nZero[k];
         }
@@ -686,6 +725,11 @@ __device__ __forceinline__ void mass_scan_loop(const FastParams& P, const Radial
     addu(&c->n_unresolved, wc[warp].n_unresolved);
     atomicAdd(&c->sum_w, sumW[k]); atomicAdd(&c->sum_w2, sumW2[k]);
     atomicAdd(&c->sum_x, sumX[k]); atomicAdd(&c->sum_y, sumY[k]); atomicAdd(&c->sum_r, sumR[k]);
+  }
+  if constexpr (kRows) {
+    __syncthreads();
+    for (int i = threadIdx.x; i < R.band.nBands * SART_MAX_MASSES; i += blockDim.x)
+      if (bandN[i]) atomicAdd(reinterpret_cast<unsigned int*>(R.band.n) + i, bandN[i]);
   }
 }
 

@@ -65,12 +65,12 @@ cudaError_t launch_mc_rays_exact(const Params& P, const Tables& T, double mAxion
 cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                   uint64_t nRays, uint64_t seed, double* image, double* imageW2,
                                   sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands = {},
-                                  const QuantityHists& qh = {});
+                                  const QuantityHists& qh = {}, const MassRows& rows = {});
 // re-trace of the uncertain rays of an FP32 launch (fast_params.h: RetraceQueue) by the exact pipeline
 cudaError_t launch_retrace_mc_image(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                     uint64_t seed, const fast::RetraceQueue& q, double* image, double* imageW2,
                                     sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands = {},
-                                    const QuantityHists& qh = {});
+                                    const QuantityHists& qh = {}, const MassRows& rows = {});
 cudaError_t launch_retrace_mc_rays(const Params& P, const Tables& T, double mAxion, uint64_t first, size_t n, uint64_t seed,
                                    const uint32_t* words, const fast::RetraceQueue& q, const sart_ray_out_t& out, int smCount,
                                    cudaStream_t s);
@@ -86,6 +86,9 @@ cudaError_t launch_retrace_presampled(const Params& P, const Tables& T, double m
 cudaError_t launch_build_cdfs(int nR, int nE, const double* radii, const double* energies, const double* emRates,
                               double* rowTotals, double* cdfs, double* radiusCDF, cudaStream_t s);
 
+// rows: the per-mass radial histograms and band images of a mass scan (device_params.h: MassRows; off by default), the
+// handle's rows for the exact launchers, mass-minor accumulators for the mass-scan launchers, which then run the kernel
+// variants that fill them.
 // ---- "fast" pipeline (kernels_fast.cu)
 // bands: the band images (device_params.h: BandImages; w == nullptr: off), in modes 1 and 2 their replicas, which
 // launch_fold_replicas adds up after the launch; with them on, the launchers run the kernel variants that fill them.
@@ -99,7 +102,7 @@ cudaError_t launch_mc_image_fast(const fast::FastParams& P, const fast::FastTabl
 cudaError_t launch_mc_image_fast_masses(const fast::FastParams& P, const fast::FastTables& T, int nMasses,
                                         const double* dMasses, uint64_t first, uint64_t nRays, uint64_t seed,
                                         double* image, double* imageW2, sart_counters_t* counters, int smCount,
-                                        cudaStream_t s);
+                                        cudaStream_t s, const MassRows& rows = {});
 cudaError_t launch_mc_rays_fast(const fast::FastParams& P, const fast::FastTables& T, double mAxion, uint64_t first,
                                 uint64_t nRays, uint64_t seed, const sart_ray_out_t& o, int smCount, cudaStream_t s);
 cudaError_t launch_emission_rates(int nR, int nE, const double* dTemp, const double* dRho, const double* dFrac,
@@ -112,7 +115,8 @@ cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G,
                                 const BandImages& bands = {}, const QuantityHists& qh = {});
 cudaError_t launch_mc_image_f32_masses(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T,
                                        int nMasses, const double* dMasses, uint64_t first, uint64_t nRays, uint64_t seed,
-                                       double* acc, double* accW2, sart_counters_t* counters, int smCount, cudaStream_t s);
+                                       double* acc, double* accW2, sart_counters_t* counters, int smCount, cudaStream_t s,
+                                       const MassRows& rows = {});
 cudaError_t launch_presampled_f32(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T, double mAxion,
                                   size_t n, const double* origin, const double* exitxy, const double* energy,
                                   const sart_ray_out_t& o, int smCount, cudaStream_t s);
@@ -126,6 +130,8 @@ cudaError_t launch_fold_spectra(const Spectra& rep, int nE1, const Spectra& dst,
 cudaError_t launch_fold_mass_acc(double* acc, double* acc2, int nMasses, size_t plane, double* image, double* imageW2,
                                  cudaStream_t s);
 cudaError_t launch_fold_mass_spectra(const Spectra& acc, int nMasses, int nE1, const Spectra& dst, cudaStream_t s);
+cudaError_t launch_fold_mass_hist(double* accW, unsigned int* accN, int nMasses, int bins, double* dstW,
+                                  unsigned long long* dstN, cudaStream_t s);
 cudaError_t launch_heatmap(int rows, int cols, double start_x, double step_x, double start_y, double step_y, size_t n,
                            const double* X, const double* Y, const double* W, double norm, double* result,
                            unsigned long long* nBad, cudaStream_t s);

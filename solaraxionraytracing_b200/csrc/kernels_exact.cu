@@ -209,12 +209,14 @@ struct MassCounters {
 };
 
 // One ray of the fused run: sample, trace, weight for every axion mass, histogram (rt:1736-2221 + 818-842). kBands: the
-// passed rays of the first mass also go to the band images B (sart_enable_band_images); false compiles them out.
-template <bool kBands>
+// passed rays of the first mass also go to the band images B (sart_enable_band_images); false compiles them out. kRows: the
+// passed rays of every mass also go to its row of the per-mass radial histograms and band images R that are on
+// (sart_enable_mass_radial_hist / _band_images); false compiles them out.
+template <bool kBands, bool kRows = false>
 __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, int nMasses, const double* __restrict__ masses,
                                              uint64_t seed, uint64_t ray, double* __restrict__ image,
                                              double* __restrict__ imageW2, const BandImages& B, BlockCounters* bc,
-                                             MassCounters* mc, ThreadSums& ts) {
+                                             MassCounters* mc, ThreadSums& ts, const MassRows& R = MassRows{}) {
   const double step = (P.chipCX * 2.0 - 0.0) / double(SART_IMAGE_BINS);  // (stop - start)/rows rt:828-830
   const double stepY = (P.chipCY * 2.0 - 0.0) / double(SART_IMAGE_BINS);
   V3 O, E;
@@ -279,6 +281,10 @@ __device__ __forceinline__ void mc_image_ray(const Params& P, const Tables& T, i
     if (kBands && m == 0) {
       const bool inImage = cx >= 0.0 && cx < double(SART_IMAGE_BINS) && cy >= 0.0 && cy < double(SART_IMAGE_BINS);
       band_add(B, g.eIdx >= 0 ? g.eIdx : P.nEnergies, inImage ? int(cy) * SART_IMAGE_BINS + int(cx) : -1, f.w);
+    }
+    if (kRows) {
+      const bool inImage = cx >= 0.0 && cx < double(SART_IMAGE_BINS) && cy >= 0.0 && cy < double(SART_IMAGE_BINS);
+      mass_rows_add(R, m, f.r, g.eIdx >= 0 ? g.eIdx : P.nEnergies, inImage ? int(cy) * SART_IMAGE_BINS + int(cx) : -1, f.w);
     }
   }
 }
@@ -385,12 +391,12 @@ __device__ __forceinline__ void mc_image_ray_qh(const Params& P, const Tables& T
 #define SART_EXACT_MINBLOCKS 6   // 85 registers instead of 108: 24 instead of 16 warps per SM for this latency-bound kernel (+5 %; 8 is slower)
 #endif
 // `list` != nullptr: trace the rays first + list[j], j < min(*listCount, listCap), instead of first + [0, nRays).
-template <bool kBands>
+template <bool kBands, bool kRows = false>
 __device__ __forceinline__ void mc_image(const Params& P, const Tables& T, int nMasses, const double* __restrict__ masses,
                                          uint64_t first, uint64_t nRays, uint64_t seed, const uint32_t* __restrict__ list,
                                          const uint32_t* __restrict__ listCount, uint32_t listCap, double* __restrict__ image,
                                          double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
-                                         const BandImages& B) {
+                                         const BandImages& B, const MassRows& R = MassRows{}) {
   extern __shared__ unsigned char smem_raw[];
   BlockCounters* bc = reinterpret_cast<BlockCounters*>(smem_raw);
   MassCounters* mc = reinterpret_cast<MassCounters*>(smem_raw + sizeof(BlockCounters));
@@ -411,7 +417,7 @@ __device__ __forceinline__ void mc_image(const Params& P, const Tables& T, int n
   for (uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < total; i += stride) {
     const uint64_t ray = first + (listMode ? uint64_t(list[i]) : i);
     if (!listMode) ++ts.n_rays;
-    mc_image_ray<kBands>(P, T, nMasses, masses, seed, ray, image, imageW2, B, bc, mc, ts);
+    mc_image_ray<kBands, kRows>(P, T, nMasses, masses, seed, ray, image, imageW2, B, bc, mc, ts, R);
   }
   if (listMode && blockIdx.x == 0 && threadIdx.x == 0)
     for (int m = 0; m < nMasses; ++m) atomicAdd(reinterpret_cast<unsigned long long*>(&counters[m].n_retraced), (unsigned long long)total);
@@ -472,6 +478,16 @@ k_trace_mc_image_bands(const __grid_constant__ Params P, const __grid_constant__
                        double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
                        const __grid_constant__ BandImages B) {
   mc_image<true>(P, T, nMasses, masses, first, nRays, seed, list, listCount, listCap, image, imageW2, counters, B);
+}
+// The same with the per-mass radial histograms and band images R, which every mass fills in its own row (mass scans).
+__global__ void __launch_bounds__(128, SART_EXACT_MINBLOCKS)
+k_trace_mc_image_mass_rows(const __grid_constant__ Params P, const __grid_constant__ Tables T, int nMasses,
+                           const double* __restrict__ masses, uint64_t first, uint64_t nRays, uint64_t seed,
+                           const uint32_t* __restrict__ list, const uint32_t* __restrict__ listCount, uint32_t listCap,
+                           double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                           const __grid_constant__ MassRows R) {
+  mc_image<false, true>(P, T, nMasses, masses, first, nRays, seed, list, listCount, listCap, image, imageW2, counters,
+                        BandImages{}, R);
 }
 // The same with the quantity histograms Q, and the band images B when B.w != nullptr (single mass); a copy of mc_image for the
 // reason of mc_image_ray_qh.
@@ -625,11 +641,18 @@ cudaError_t launch_mc_rays_exact(const Params& P, const Tables& T, double mAxion
 cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                   uint64_t nRays, uint64_t seed, double* image, double* imageW2,
                                   sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands,
-                                  const QuantityHists& qh) {
+                                  const QuantityHists& qh, const MassRows& rows) {
   if (nRays == 0) return cudaSuccess;
   const int block = 128;
   const size_t smem = sizeof(BlockCounters) + size_t(nMasses) * sizeof(MassCounters);
   unsigned grid = 0;   // one resident wave; the grid-stride loop covers the rest
+  if (rows.rad.w || rows.band.w) {
+    const cudaError_t e = grid_size(k_trace_mc_image_mass_rows, block, smem, nRays, smCount, 0, &grid);
+    if (e != cudaSuccess) return e;
+    k_trace_mc_image_mass_rows<<<grid, block, smem, s>>>(P, T, nMasses, masses, first, nRays, seed, nullptr, nullptr, 0u, image,
+                                                         imageW2, counters, rows);
+    return cudaGetLastError();
+  }
   const cudaError_t e = qh.w      ? grid_size(k_trace_mc_image_qhists, block, smem, nRays, smCount, 0, &grid)
                         : bands.w ? grid_size(k_trace_mc_image_bands, block, smem, nRays, smCount, 0, &grid)
                                   : grid_size(k_trace_mc_image, block, smem, nRays, smCount, 0, &grid);
@@ -650,10 +673,17 @@ cudaError_t launch_mc_image_exact(const Params& P, const Tables& T, int nMasses,
 cudaError_t launch_retrace_mc_image(const Params& P, const Tables& T, int nMasses, const double* masses, uint64_t first,
                                     uint64_t seed, const fast::RetraceQueue& q, double* image, double* imageW2,
                                     sart_counters_t* counters, int smCount, cudaStream_t s, const BandImages& bands,
-                                    const QuantityHists& qh) {
+                                    const QuantityHists& qh, const MassRows& rows) {
   const int block = 128;
   const size_t smem = sizeof(BlockCounters) + size_t(nMasses) * sizeof(MassCounters);
   int perSM = 0;
+  if (rows.rad.w || rows.band.w) {
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image_mass_rows, block, smem);
+    if (e != cudaSuccess) return e;
+    k_trace_mc_image_mass_rows<<<unsigned(smCount * (perSM < 1 ? 1 : perSM)), block, smem, s>>>(
+        P, T, nMasses, masses, first, 0, seed, q.list, q.count, q.cap, image, imageW2, counters, rows);
+    return cudaGetLastError();
+  }
   cudaError_t e = qh.w      ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image_qhists, block, smem)
                   : bands.w ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image_bands, block, smem)
                             : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_trace_mc_image, block, smem);

@@ -426,11 +426,11 @@ k_trace_mc_f32_compact_qhists(const __grid_constant__ FastParams P, const __grid
   qhist_flush<kQH == 1>(QH, qs);
 }
 // ---- axion-mass scan with FP32 tracing (the per-mass weighting is fast_common.cuh's mass_scan_loop) --------------
-template <bool kWolter, bool kMargins, int kPer, bool kSpectra>
+template <bool kWolter, bool kMargins, int kPer, bool kSpectra, bool kRows = false>
 __device__ __forceinline__ void f32_masses(const FastParams& P, const Geo32& G, const FastTables& T,
                                            const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays,
                                            const PhiloxKeys& K, double* __restrict__ image, double* __restrict__ imageW2,
-                                           sart_counters_t* __restrict__ counters) {
+                                           sart_counters_t* __restrict__ counters, const MassRows& R = MassRows{}) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem32 S;
   unsigned char* tail;
@@ -439,7 +439,7 @@ __device__ __forceinline__ void f32_masses(const FastParams& P, const Geo32& G, 
   smem_fill32(P, T, S);
   for (int i = threadIdx.x; i < kWarpsM * int(sizeof(WarpCounters) / 4); i += kBlockM) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
   __syncthreads();
-  mass_scan_loop<kPer, kSpectra>(P, T.rad, T.spec, masses, nMasses, first, nRays, image, imageW2, counters, wc,
+  mass_scan_loop<kPer, kSpectra, kRows>(P, T.rad, T.spec, R, masses, nMasses, first, nRays, image, imageW2, counters, wc,
                  [&](uint64_t ray, uint32_t id, RayResult& r) {
     RecordSink<false> sink{r, 0.0, T.rq, true};
     Head32 hd;
@@ -467,6 +467,17 @@ k_trace_mc_f32_masses_spectra(const __grid_constant__ FastParams P, const __grid
                               uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image,
                               double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
   f32_masses<kWolter, kMargins, kPer, true>(P, G, T, masses, nMasses, first, nRays, K, image, imageW2, counters);
+}
+// The same with the per-mass radial histograms and band images R (sart_enable_mass_radial_hist / _band_images; their
+// mass-minor accumulators, see mass_scan_loop), and with the per-mass spectra as well (kSpectra).
+template <bool kWolter, bool kMargins, int kPer, bool kSpectra>
+__global__ void __launch_bounds__(kBlockM, SART_F32_MINBLOCKS_M)
+k_trace_mc_f32_masses_rows(const __grid_constant__ FastParams P, const __grid_constant__ Geo32 G,
+                           const __grid_constant__ FastTables T, const double* __restrict__ masses, int nMasses,
+                           uint64_t first, uint64_t nRays, const __grid_constant__ PhiloxKeys K, double* __restrict__ image,
+                           double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                           const __grid_constant__ MassRows R) {
+  f32_masses<kWolter, kMargins, kPer, kSpectra, true>(P, G, T, masses, nMasses, first, nRays, K, image, imageW2, counters, R);
 }
 
 }  // namespace fast
@@ -539,26 +550,43 @@ cudaError_t launch_mc_image_f32(const fast::FastParams& P, const fast::Geo32& G,
 
 cudaError_t launch_mc_image_f32_masses(const fast::FastParams& P, const fast::Geo32& G, const fast::FastTables& T,
                                        int nMasses, const double* dMasses, uint64_t first, uint64_t nRays, uint64_t seed,
-                                       double* acc, double* accW2, sart_counters_t* counters, int smCount, cudaStream_t s) {
+                                       double* acc, double* accW2, sart_counters_t* counters, int smCount, cudaStream_t s,
+                                       const MassRows& rows) {
   if (nRays == 0) return cudaSuccess;
   const LaunchVariant v = launch_variant(P, T);
   const size_t smem = fast::smem_bytes32(P, fast::kWarpsM);
+  auto run = [&](auto kern, auto... extra) {
+    cudaError_t e = fast::set_smem(kern, smem);
+    if (e != cudaSuccess) return e;
+    unsigned grid = 0;
+    if ((e = grid_size(kern, fast::kBlockM, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
+    kern<<<grid, fast::kBlockM, smem, s>>>(P, G, T, dMasses, nMasses, first, nRays, philox_round_keys(seed), acc, accW2, counters,
+                                           extra...);
+    return cudaGetLastError();
+  };
   using Kern = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, const double*, int, uint64_t, uint64_t, PhiloxKeys, double*,
                         double*, sart_counters_t*);
   constexpr int kAll = SART_MAX_MASSES / 32;
+  const int per = nMasses <= 32 ? 0 : (nMasses <= 64 ? 1 : 2);
   // [spectra][wolter][margins][masses per lane]; spectra: T.spec holds the per-mass spectra accumulators
 #define SART_ROW(K, W, M) {fast::K<W, M, 1>, fast::K<W, M, 2>, fast::K<W, M, kAll>}
 #define SART_KERN(K) {{SART_ROW(K, false, false), SART_ROW(K, false, true)}, {SART_ROW(K, true, false), SART_ROW(K, true, true)}}
+  if (rows.rad.w || rows.band.w) {
+    using KernR = void (*)(fast::FastParams, fast::Geo32, fast::FastTables, const double*, int, uint64_t, uint64_t, PhiloxKeys,
+                           double*, double*, sart_counters_t*, MassRows);
+    // [spectra][wolter][margins][masses per lane]
+#define SART_ROW_S(W, M, S) {fast::k_trace_mc_f32_masses_rows<W, M, 1, S>, fast::k_trace_mc_f32_masses_rows<W, M, 2, S>, \
+                             fast::k_trace_mc_f32_masses_rows<W, M, kAll, S>}
+#define SART_KERN_S(S) {{SART_ROW_S(false, false, S), SART_ROW_S(false, true, S)}, {SART_ROW_S(true, false, S), SART_ROW_S(true, true, S)}}
+    static const KernR table[2][2][2][3] = {SART_KERN_S(false), SART_KERN_S(true)};
+#undef SART_KERN_S
+#undef SART_ROW_S
+    return run(table[T.spec.eW ? 1 : 0][v.wolter ? 1 : 0][v.margins ? 1 : 0][per], rows);
+  }
   static const Kern table[2][2][2][3] = {SART_KERN(k_trace_mc_f32_masses), SART_KERN(k_trace_mc_f32_masses_spectra)};
 #undef SART_KERN
 #undef SART_ROW
-  const Kern kern = table[T.spec.eW ? 1 : 0][v.wolter ? 1 : 0][v.margins ? 1 : 0][nMasses <= 32 ? 0 : (nMasses <= 64 ? 1 : 2)];
-  cudaError_t e = fast::set_smem(kern, smem);
-  if (e != cudaSuccess) return e;
-  unsigned grid = 0;
-  if ((e = grid_size(kern, fast::kBlockM, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
-  kern<<<grid, fast::kBlockM, smem, s>>>(P, G, T, dMasses, nMasses, first, nRays, philox_round_keys(seed), acc, accW2, counters);
-  return cudaGetLastError();
+  return run(table[T.spec.eW ? 1 : 0][v.wolter ? 1 : 0][v.margins ? 1 : 0][per]);
 }
 
 #endif  // SART_NO_LAUNCHERS

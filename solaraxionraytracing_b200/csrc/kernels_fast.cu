@@ -830,10 +830,11 @@ k_trace_mc_fast_compact_qhists(const __grid_constant__ FastParams P, const __gri
 // Rays are traced once (lanes = rays); each ray that reaches the weight stage is then broadcast through the warp and
 // weighted for all M masses at once with lanes = masses (mass lane + 32 k), so the per-mass sums live in registers of
 // the lane that owns the mass and need no reduction, and the per-mass image planes are hit by distinct lanes.
-template <bool kWolter, bool kSpectra>
+template <bool kWolter, bool kSpectra, bool kRows = false>
 __device__ __forceinline__ void fast_masses(const FastParams& P, const FastTables& T, const double* __restrict__ masses,
                                             int nMasses, uint64_t first, uint64_t nRays, uint64_t seed, double* __restrict__ image,
-                                            double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
+                                            double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                                            const MassRows& R = MassRows{}) {
   extern __shared__ __align__(16) unsigned char smem[];
   Smem S;
   unsigned char* tail;
@@ -843,7 +844,7 @@ __device__ __forceinline__ void fast_masses(const FastParams& P, const FastTable
   for (int i = threadIdx.x; i < kWarps * int(sizeof(WarpCounters) / 4); i += kBlock) reinterpret_cast<unsigned int*>(wc)[i] = 0u;
   __syncthreads();
 
-  mass_scan_loop<SART_MAX_MASSES / 32, kSpectra>(P, T.rad, T.spec, masses, nMasses, first, nRays, image, imageW2, counters, wc,
+  mass_scan_loop<SART_MAX_MASSES / 32, kSpectra, kRows>(P, T.rad, T.spec, R, masses, nMasses, first, nRays, image, imageW2, counters, wc,
                  [&](uint64_t ray, uint32_t, RayResult& r) { trace_one<kWolter, false>(P, T, S, seed, ray, 0.0, r); return false; });
 }
 template <bool kWolter>
@@ -860,6 +861,16 @@ k_trace_mc_fast_masses_spectra(const __grid_constant__ FastParams P, const __gri
                                const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays, uint64_t seed,
                                double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters) {
   fast_masses<kWolter, true>(P, T, masses, nMasses, first, nRays, seed, image, imageW2, counters);
+}
+// The same with the per-mass radial histograms and band images R (sart_enable_mass_radial_hist / _band_images; their
+// mass-minor accumulators, see mass_scan_loop), and with the per-mass spectra as well (kSpectra).
+template <bool kWolter, bool kSpectra>
+__global__ void __launch_bounds__(kBlock, 2)
+k_trace_mc_fast_masses_rows(const __grid_constant__ FastParams P, const __grid_constant__ FastTables T,
+                            const double* __restrict__ masses, int nMasses, uint64_t first, uint64_t nRays, uint64_t seed,
+                            double* __restrict__ image, double* __restrict__ imageW2, sart_counters_t* __restrict__ counters,
+                            const __grid_constant__ MassRows R) {
+  fast_masses<kWolter, kSpectra, true>(P, T, masses, nMasses, first, nRays, seed, image, imageW2, counters, R);
 }
 
 // ---- per-ray records (traceAxionWrapper in fast mode) ----------------------------------------------------------
@@ -929,18 +940,24 @@ cudaError_t launch_mc_image_fast(const fast::FastParams& P, const fast::FastTabl
 cudaError_t launch_mc_image_fast_masses(const fast::FastParams& P, const fast::FastTables& T, int nMasses,
                                         const double* dMasses, uint64_t first, uint64_t nRays, uint64_t seed,
                                         double* image, double* imageW2, sart_counters_t* counters, int smCount,
-                                        cudaStream_t s) {
+                                        cudaStream_t s, const MassRows& rows) {
   if (nRays == 0) return cudaSuccess;
   const size_t smem = fast::smem_bytes(P);
   const bool wolter = launch_variant(P, T).wolter;
-  auto kern = T.spec.eW ? (wolter ? fast::k_trace_mc_fast_masses_spectra<true> : fast::k_trace_mc_fast_masses_spectra<false>)
-                        : (wolter ? fast::k_trace_mc_fast_masses<true> : fast::k_trace_mc_fast_masses<false>);
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-  if (e != cudaSuccess) return e;
-  unsigned grid = 0;
-  if ((e = grid_size(kern, fast::kBlock, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
-  kern<<<grid, fast::kBlock, smem, s>>>(P, T, dMasses, nMasses, first, nRays, seed, image, imageW2, counters);
-  return cudaGetLastError();
+  auto run = [&](auto kern, auto... extra) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return e;
+    unsigned grid = 0;
+    if ((e = grid_size(kern, fast::kBlock, smem, nRays, smCount, 0, &grid)) != cudaSuccess) return e;
+    kern<<<grid, fast::kBlock, smem, s>>>(P, T, dMasses, nMasses, first, nRays, seed, image, imageW2, counters, extra...);
+    return cudaGetLastError();
+  };
+  if (rows.rad.w || rows.band.w)
+    return run(T.spec.eW ? (wolter ? fast::k_trace_mc_fast_masses_rows<true, true> : fast::k_trace_mc_fast_masses_rows<false, true>)
+                         : (wolter ? fast::k_trace_mc_fast_masses_rows<true, false> : fast::k_trace_mc_fast_masses_rows<false, false>),
+               rows);
+  return run(T.spec.eW ? (wolter ? fast::k_trace_mc_fast_masses_spectra<true> : fast::k_trace_mc_fast_masses_spectra<false>)
+                       : (wolter ? fast::k_trace_mc_fast_masses<true> : fast::k_trace_mc_fast_masses<false>));
 }
 
 cudaError_t launch_mc_rays_fast(const fast::FastParams& P, const fast::FastTables& T, double mAxion, uint64_t first,

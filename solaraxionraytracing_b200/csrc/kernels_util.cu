@@ -124,6 +124,32 @@ cudaError_t launch_fold_mass_spectra(const Spectra& acc, int nMasses, int nE1, c
   return cudaGetLastError();
 }
 
+// Mass scan with per-mass radial histograms or band images: adds the mass-minor accumulators of a launch (fast_common.cuh:
+// mass_scan_loop; Σw [bins][SART_MAX_MASSES], accW == nullptr: counts only, and 32-bit counts of the same shape) to the
+// rows [mass][bins] of the handle's arrays and clears them. One thread per accumulator element. The band images' planes go
+// through k_fold_mass_acc.
+__global__ void __launch_bounds__(256) k_fold_mass_hist(double* __restrict__ accW, unsigned int* __restrict__ accN, int nMasses,
+                                                        int bins, double* __restrict__ dstW, unsigned long long* __restrict__ dstN) {
+  const size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;   // = bin * SART_MAX_MASSES + mass
+  if (i >= size_t(bins) * SART_MAX_MASSES) return;
+  const unsigned int n = accN[i];
+  if (n == 0u) return;   // no passed ray in this bin: its sum is zero as well
+  accN[i] = 0u;
+  const int m = int(i % SART_MAX_MASSES);
+  const size_t o = size_t(m) * size_t(bins) + i / SART_MAX_MASSES;
+  if (m < nMasses) dstN[o] += n;
+  if (!accW) return;
+  const double a = accW[i];
+  accW[i] = 0.0;
+  if (m < nMasses) dstW[o] += a;
+}
+cudaError_t launch_fold_mass_hist(double* accW, unsigned int* accN, int nMasses, int bins, double* dstW,
+                                  unsigned long long* dstN, cudaStream_t s) {
+  const size_t n = size_t(bins) * SART_MAX_MASSES;
+  k_fold_mass_hist<<<unsigned((n + 255) / 256), 256, 0, s>>>(accW, accN, nMasses, bins, dstW, dstN);
+  return cudaGetLastError();
+}
+
 template <typename T, int kChains>
 __global__ void __launch_bounds__(256) k_fma_peak(T* out, T a, T b, int iters) {
   T acc[kChains];

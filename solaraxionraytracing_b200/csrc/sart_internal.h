@@ -67,39 +67,46 @@ struct Carve {
 };
 
 // The optional accumulators of the passed rays, each switched on and off by its own entry point: the radial histogram
-// (sart_enable_radial_hist), the spectra (sart_enable_spectra), the per-mass spectra (sart_enable_mass_spectra) and the
-// band images (sart_enable_band_images) and the quantity histograms (sart_enable_quantity_hists).
-enum AccumKind { kRadialHist, kSpectra, kMassSpectra, kBandImages, kQuantityHists, kAccums };
-constexpr AccumKind kAllAccums[kAccums] = {kRadialHist, kSpectra, kMassSpectra, kBandImages, kQuantityHists};
+// (sart_enable_radial_hist), the spectra (sart_enable_spectra), the per-mass spectra (sart_enable_mass_spectra), the
+// band images (sart_enable_band_images), the quantity histograms (sart_enable_quantity_hists), the per-mass radial
+// histograms (sart_enable_mass_radial_hist) and the per-mass band images (sart_enable_mass_band_images).
+enum AccumKind { kRadialHist, kSpectra, kMassSpectra, kBandImages, kQuantityHists, kMassRadialHist, kMassBandImages, kAccums };
+constexpr AccumKind kAllAccums[kAccums] = {kRadialHist, kSpectra, kMassSpectra, kBandImages, kQuantityHists, kMassRadialHist,
+                                           kMassBandImages};
+// The per-mass accumulators: one row per axion mass, filled by the mass-scan kernels.
+constexpr bool per_mass(AccumKind k) { return k == kMassSpectra || k == kMassRadialHist || k == kMassBandImages; }
 
 // One block of an accumulator: the handle's own (sart_handle::accum) or its merged copy (sart_handle::merged_accum), both
 // one allocation laid out by the same code (api.cu: alloc_accum). blob == nullptr: off (and bins == 0).
 struct Accum {
   void* blob = nullptr;
   size_t bytes = 0;
-  int bins = 0;         // radial histogram: its bins; (per-mass) spectra: energy bins per row, nEnergies + 1; band images: bands;
-                        // quantity histograms: their entries, Σ(nbins + 2)
-  double rmax = 0.0;    // radial histogram: its range
-  double edges[SART_MAX_BANDS + 1] = {};   // band images: the bins + 1 band edges [keV]
+  int bins = 0;         // (per-mass) radial histogram: its bins per row; (per-mass) spectra: energy bins per row, nEnergies + 1;
+                        // (per-mass) band images: bands per row; quantity histograms: their entries, Σ(nbins + 2)
+  double rmax = 0.0;    // (per-mass) radial histogram: its range
+  double edges[SART_MAX_BANDS + 1] = {};   // (per-mass) band images: the bins + 1 band edges [keV]
   int n_qhists = 0;                        // quantity histograms: their specs, in the caller's order
   sart_quantity_hist_t qspecs[SART_N_QUANTITIES] = {};
-  RadialHist rad{};     // radial histogram: w, n
+  RadialHist rad{};     // (per-mass) radial histogram: w, n [bins], per mass one such row
   Spectra spec{};       // (per-mass) spectra: eW, eW2, eN, sW, sN; the per-mass spectra have one row per mass (eRow, sRow)
-  BandImages band{};    // band images: w, w2 [bins][256][256], n [bins]; the handle's block also its energy -> band table
+  BandImages band{};    // (per-mass) band images: w, w2 [bins][256][256], n [bins], per mass one such row; the handle's
+                        // block also its energy -> band table
   QuantityHists qh{};   // quantity histograms: w, w2, n [bins]; the handle's block also the specs and the replicas rw, rw2
   int valid = 0;        // merged copy: it holds the sums of the last sart_allreduce_outputs for the masses set
   // The handle's own block only: the buffers the throughput kernels add into instead (api.cu: carve_throughput), which the
   // fold after every launch adds into the arrays above and clears. The spectra's replicas, the per-mass spectra's
-  // mass-minor accumulators, the band images' replicas (tput_band, which also holds the energy -> band table); the radial
-  // histogram has none, the quantity histograms keep theirs in qh.
+  // mass-minor accumulators, the band images' replicas (tput_band, which also holds the energy -> band table), the
+  // per-mass radial histograms' and band images' mass-minor accumulators (tput_rad, tput_band); the radial histogram has
+  // none, the quantity histograms keep theirs in qh.
   void* tput_blob = nullptr;
   Spectra tput{};
   BandImages tput_band{};
+  RadialHist tput_rad{};
 };
 
-// Rows of accumulator k for nMasses axion masses: one per mass for the per-mass spectra (allocated for SART_MAX_MASSES,
+// Rows of accumulator k for nMasses axion masses: one per mass for the per-mass accumulators (allocated for SART_MAX_MASSES,
 // read and merged for the masses set), one for the others.
-inline size_t accum_rows(AccumKind k, int nMasses) { return k == kMassSpectra ? size_t(nMasses) : 1; }
+inline size_t accum_rows(AccumKind k, int nMasses) { return per_mass(k) ? size_t(nMasses) : 1; }
 
 // The arrays of an accumulator: f(a.array, b.array, count) for every device array of a pair of blocks of kind k (a block
 // and itself, or a handle's block and its merged copy) in layout order, `count` elements for `rows` rows of a.bins bins.
@@ -107,11 +114,11 @@ inline size_t accum_rows(AccumKind k, int nMasses) { return k == kMassSpectra ? 
 template <class A, class B, class F>
 inline void accum_arrays(AccumKind k, A& a, B& b, size_t rows, F&& f) {
   const size_t e = rows * size_t(a.bins), s = rows * SART_MAX_SHELLS;
-  if (k == kRadialHist) {
+  if (k == kRadialHist || k == kMassRadialHist) {
     f(a.rad.w, b.rad.w, e); f(a.rad.n, b.rad.n, e);
     return;
   }
-  if (k == kBandImages) {
+  if (k == kBandImages || k == kMassBandImages) {
     const size_t p = e * SART_IMAGE_BINS * SART_IMAGE_BINS;
     f(a.band.w, b.band.w, p); f(a.band.w2, b.band.w2, p); f(a.band.n, b.band.n, e);
     return;
@@ -127,7 +134,7 @@ inline void accum_arrays(AccumKind k, A& a, B& b, size_t rows, F&& f) {
 // api.cu: a block of accumulator k with `bins` bins (rmax: the radial histogram's range), allocated and carved but not
 // cleared. On failure `a` stays empty and the error is recorded.
 int alloc_accum(AccumKind k, int bins, double rmax, Accum* a);
-// api.cu: the reader behind sart_read_radial_hist / _spectra / _mass_spectra and their sart_read_merged_* twins. Copies the
+// api.cu: the reader behind sart_read_radial_hist / _spectra / _mass_spectra / ... and their sart_read_merged_* twins. Copies the
 // rows in use of accumulator k, the handle's own block or its merged copy, into the caller's arrays `host`, one per array
 // in the order of accum_arrays (NULL: skipped), and synchronises. `off`: the error while there is nothing to read.
 int read_accum(sart_handle* h, AccumKind k, bool merged, std::initializer_list<void*> host, const char* off);

@@ -160,8 +160,8 @@ def allreduce(tracers):
 
 
 def allreduce_outputs(tracers):
-    """sart_allreduce_outputs over every tracer of comm_init_all: the radial histogram and the (per-mass) spectra that are
-    on, into each one's read_merged_radial_hist / read_merged_spectra / read_merged_mass_spectra. Synchronises."""
+    """sart_allreduce_outputs over every tracer of comm_init_all: the accumulators that are on (radial histogram, spectra,
+    band images, quantity histograms and their per-mass forms), into each one's read_merged_* readers. Synchronises."""
     check(lib.sart_allreduce_outputs(_handles(tracers), len(tracers)))
 
 
@@ -174,6 +174,8 @@ class DevicesResult:
     precision: int                           # the precision mode the run took
     band_images: BandImages | None = None    # the band images of `bands` (RayTracer.read_band_images)
     quantity_hists: list[QuantityHist] | None = None   # the histograms of `quantity_hists` (RayTracer.read_quantity_hists)
+    mass_radial_hists: list[tuple] | None = None        # per mass, as RayTracer.read_mass_radial_hist
+    mass_band_images: list[BandImages] | None = None    # per mass, the band images of `mass_bands`
 
 
 def _open_tracers(fullSetup, devices, precision: int, sampler, masses, warn):
@@ -202,14 +204,15 @@ def _open_tracers(fullSetup, devices, precision: int, sampler, masses, warn):
 
 def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, precision: int = 2, sampler=None,
                      masses=None, radial_hist: bool = False, spectra: bool = False, bands=None, quantity_hists=None,
-                     warn=None) -> DevicesResult:
+                     mass_radial_hist: bool = False, mass_bands=None, warn=None) -> DevicesResult:
     """The fused run of `nRays` rays over `devices`, one process: device k traces shard(nRays, k, n) of the global rays,
     so the result is that of one GPU tracing all of them, up to the order of the floating-point sums. The shards run
     concurrently (trace_mc only queues work); then sart_allreduce and, with `radial_hist` or `spectra`,
     sart_allreduce_outputs merge them. `spectra` means the single-mass spectra for at most one axion mass and the per-mass
     spectra for a mass scan. `bands`: the edges of the band images (RayTracer.enable_band_images; at most one axion
     mass). `quantity_hists`: the specs of the quantity histograms (RayTracer.enable_quantity_hists; at most one axion mass).
-    `warn` receives the precision fall-back messages (see raytracer.set_fastest_precision)."""
+    `mass_radial_hist` / `mass_bands` (band edges): the per-mass radial histograms and band images
+    (RayTracer.enable_mass_radial_hist / enable_mass_band_images) of a mass scan. `warn` receives the precision fall-back messages (see raytracer.set_fastest_precision)."""
     tracers, mode = _open_tracers(fullSetup, devices, precision, sampler, masses, warn)
     try:
         scan = masses is not None and len(masses) > 1
@@ -222,6 +225,10 @@ def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, p
                 t.enable_band_images(bands)
             if quantity_hists:
                 t.enable_quantity_hists(quantity_hists)
+            if mass_radial_hist:
+                t.enable_mass_radial_hist()
+            if mass_bands is not None:
+                t.enable_mass_band_images(mass_bands)
             t.reset_image()
         comm_init_all(tracers)
         for rank, t in enumerate(tracers):
@@ -229,7 +236,7 @@ def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, p
             if count:
                 t.trace_mc(count, seed, first_ray=first)
         allreduce(tracers)
-        if radial_hist or spectra or bands is not None or quantity_hists:
+        if radial_hist or spectra or bands is not None or quantity_hists or mass_radial_hist or mass_bands is not None:
             allreduce_outputs(tracers)
         t0 = tracers[0]
         merged_spectra = None
@@ -237,7 +244,9 @@ def trace_on_devices(fullSetup, devices, nRays: int, seed: int = 299792458, *, p
             merged_spectra = t0.read_merged_mass_spectra() if scan else t0.read_merged_spectra()
         return DevicesResult(t0.read_merged(), t0.read_merged_radial_hist() if radial_hist else None, merged_spectra, mode,
                              t0.read_merged_band_images() if bands is not None else None,
-                             t0.read_merged_quantity_hists() if quantity_hists else None)
+                             t0.read_merged_quantity_hists() if quantity_hists else None,
+                             t0.read_merged_mass_radial_hist() if mass_radial_hist else None,
+                             t0.read_merged_mass_band_images() if mass_bands is not None else None)
     finally:
         for t in tracers:
             t.close()

@@ -444,16 +444,19 @@ def angle_suffix(angle_deg: float) -> str:
 
 
 RADII_COLUMNS = ["Angle [deg]", "rSigma1", "rSigma2", "rSigma1W", "rSigma2W"]
+MASS_COLUMN = "mAxion [eV]"   # first column of mass_scan_radii.csv
 
 
-def write_scan_radii_csv(path: str | Path, angles, radii: list[ContainmentRadii], precision: int = 17) -> Path:
+def write_scan_radii_csv(path: str | Path, angles, radii: list[ContainmentRadii], precision: int = 17,
+                         first_column: str = RADII_COLUMNS[0]) -> Path:
     """The containment radii of every scan point (containment_radii_from_hist of its radial histogram, about the chip
-    centre): columns `Angle [deg]`, rSigma1, rSigma2, rSigma1W, rSigma2W [mm]."""
+    centre): columns `first_column` (the scan variable: `Angle [deg]` of an angular scan, MASS_COLUMN of a mass scan), then
+    rSigma1, rSigma2, rSigma1W, rSigma2W [mm]."""
     a = np.asarray(angles, dtype=np.float64)
     if a.size != len(radii):
-        raise ValueError(f"{len(radii)} radii for {a.size} angles")
+        raise ValueError(f"{len(radii)} radii for {a.size} scan points")
     cols = [a] + [np.array([getattr(r, f) for r in radii], dtype=np.float64) for f in RADII_COLUMNS[1:]]
-    return _write_columns(path, RADII_COLUMNS, cols, set(), precision)
+    return _write_columns(path, [first_column] + RADII_COLUMNS[1:], cols, set(), precision)
 
 
 def write_scan_outputs(scan: ScanOutputs, windowYear: int, outpath: str | Path, chipXMax: float = 14.0,
@@ -492,3 +495,26 @@ def generateResultPlots(result, windowYear: int, outpath: str | Path, suffix: st
     year = WINDOW_YEAR_NAMES.get(windowYear, str(windowYear))
     return write_axion_image_csv(Path(outpath) / f"axion_image_{year}{suffix}.csv", result.image[0], radii.rSigma1W,
                                  radii.rSigma2W, chipXMax, chipYMax, precision)
+
+
+def write_mass_scan_outputs(masses, radial_hists: list[tuple], band_images: list[BandImages] | None, windowYear: int,
+                            outpath: str | Path, chipXMax: float = 14.0, chipYMax: float = 14.0,
+                            precision: int = 17) -> list[Path]:
+    """The per-mass radii and band images of a mass scan (RayTracer.read_mass_radial_hist / read_mass_band_images):
+    `mass_scan_radii.csv` (write_scan_radii_csv with the masses in column MASS_COLUMN), and with `band_images` for every
+    mass the write_band_image_csvs files `axion_image_{year}_E{lo:g}-{hi:g}keV_ma{m:.6g}eV.csv`, whose radius columns
+    carry that mass's containment radii."""
+    masses = [float(m) for m in masses]
+    if len(radial_hists) != len(masses) or (band_images is not None and len(band_images) != len(masses)):
+        raise ValueError(f"{len(radial_hists)} radial histograms and "
+                         f"{'no' if band_images is None else len(band_images)} band images for {len(masses)} masses")
+    suffixes = [mass_suffix(m) for m in masses]
+    if len(set(suffixes)) != len(suffixes):
+        raise ValueError("two masses of the scan share a file name (they agree to 6 significant digits)")
+    radii = [containment_radii_from_hist(*h) for h in radial_hists]
+    paths = [write_scan_radii_csv(Path(outpath) / "mass_scan_radii.csv", masses, radii, precision, MASS_COLUMN)]
+    for k, sfx in enumerate(suffixes):
+        if band_images is not None:
+            paths.extend(write_band_image_csvs(band_images[k], windowYear, outpath, radii[k], chipXMax, chipYMax, precision,
+                                               suffix=sfx))
+    return paths

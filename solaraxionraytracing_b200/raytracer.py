@@ -287,18 +287,22 @@ class RayTracer:
     def reset_image(self):
         check(lib.sart_reset_image(self._h))
 
-    def enable_radial_hist(self, nbins: int = 16384, r_max: float | None = None):
-        """Radial histogram of the passed rays (for the containment radii); r_max defaults to the chip diagonal / 2."""
+    def _default_r_max(self, r_max: float | None) -> float:
         if r_max is None:
             c = self.fullSetup.expSetup.consts
             r_max = 0.5 * float(np.hypot(c.chipXMax, c.chipYMax)) * 1.0001
+        return r_max
+
+    def enable_radial_hist(self, nbins: int = 16384, r_max: float | None = None):
+        """Radial histogram of the passed rays (for the containment radii); r_max defaults to the chip diagonal / 2."""
+        r_max = self._default_r_max(r_max)
         check(lib.sart_enable_radial_hist(self._h, nbins, r_max))
         self._rad = (nbins, r_max)
 
-    # Each accumulator's host arrays for `rows` rows (one read, or the scan points of angular_scan_outputs), in the order the
-    # C-ABI takes them, and the function that cuts them into one result per row.
-    def _radial_rows(self, rows: int):
-        nbins, r_max = self._rad
+    # Each accumulator's host arrays for `rows` rows (one read, the masses of a mass scan, or the scan points of
+    # angular_scan_outputs), in the order the C-ABI takes them, and the function that cuts them into one result per row.
+    def _radial_rows(self, rows: int, shape=None):
+        nbins, r_max = shape or self._rad
         w = np.empty((rows, nbins))
         n = np.empty((rows, nbins), dtype=np.uint64)
         edges = np.linspace(0.0, r_max, nbins + 1)
@@ -312,6 +316,30 @@ class RayTracer:
     def read_radial_hist(self):
         """(bin edges [nbins + 1], sum of weights [nbins], ray counts [nbins])."""
         return self._read_radial(lib.sart_read_radial_hist)
+
+    def enable_mass_radial_hist(self, nbins: int = 16384, r_max: float | None = None):
+        """Radial histogram of the rays that pass in trace_mc for every axion mass of set_axion_masses
+        (sart_enable_mass_radial_hist), binned like enable_radial_hist, from the one traced ray per mass scan; nbins = 0
+        switches them off. Switching them on clears them; trace_mc then runs the mass-scan kernels for any number of masses.
+        Not together with enable_radial_hist or the alias sampler."""
+        r_max = self._default_r_max(r_max)
+        check(lib.sart_enable_mass_radial_hist(self._h, nbins, r_max))
+        self._mass_rad = (nbins, r_max)
+
+    def _read_mass_radial(self, read):
+        arrays, split = self._radial_rows(self.n_masses, getattr(self, "_mass_rad", (0, 1.0)))
+        check(read(self._h, *map(_ptr, arrays)))
+        return split()
+
+    def read_mass_radial_hist(self) -> list[tuple]:
+        """One (bin edges, sum of weights, ray counts) per axion mass, in the order of set_axion_masses, accumulated since
+        enable_mass_radial_hist / reset_image (raises SartError while they are off); each ready for
+        output.containment_radii_from_hist."""
+        return self._read_mass_radial(lib.sart_read_mass_radial_hist)
+
+    def read_merged_mass_radial_hist(self) -> list[tuple]:
+        """read_mass_radial_hist of the last allreduce_outputs (raises SartError without one)."""
+        return self._read_mass_radial(lib.sart_read_merged_mass_radial_hist)
 
     def enable_spectra(self, on: bool = True):
         """Energy spectrum and per-shell flux of the rays that pass in trace_mc (single axion mass; sart_enable_spectra).
@@ -367,8 +395,8 @@ class RayTracer:
         check(lib.sart_enable_band_images(self._h, e.size - 1 if e.size > 1 else -1, _dp(e)))   # one edge: no band, refused
         self._band_edges = e.copy()
 
-    def _band_rows(self, rows: int):
-        edges = getattr(self, "_band_edges", None)
+    def _band_rows(self, rows: int, edges=False):
+        edges = getattr(self, "_band_edges", None) if edges is False else edges
         nb = 0 if edges is None else edges.size - 1
         img = np.empty((rows, nb, abi.IMAGE_BINS, abi.IMAGE_BINS))
         img2 = np.empty_like(img)
@@ -387,6 +415,33 @@ class RayTracer:
     def read_merged_band_images(self) -> BandImages:
         """read_band_images of the last allreduce_outputs (raises SartError without one)."""
         return self._read_bands(lib.sart_read_merged_band_images)
+
+    def enable_mass_band_images(self, edges_keV=None):
+        """Band images (as enable_band_images) of the rays that pass in trace_mc for every axion mass of set_axion_masses
+        (sart_enable_mass_band_images), from the one traced ray per mass scan; None switches them off. Switching them on
+        clears them; trace_mc then runs the mass-scan kernels for any number of masses. Not together with
+        enable_band_images or the alias sampler. Device memory: about 3 x 64 MiB per band."""
+        if edges_keV is None:
+            check(lib.sart_enable_mass_band_images(self._h, 0, None))
+            self._mass_band_edges = None
+            return
+        e = np.ascontiguousarray(edges_keV, dtype=np.float64)
+        check(lib.sart_enable_mass_band_images(self._h, e.size - 1 if e.size > 1 else -1, _dp(e)))   # one edge: refused
+        self._mass_band_edges = e.copy()
+
+    def _read_mass_bands(self, read) -> list[BandImages]:
+        arrays, split = self._band_rows(self.n_masses, getattr(self, "_mass_band_edges", None))
+        check(read(self._h, *map(_ptr, arrays)))
+        return split()
+
+    def read_mass_band_images(self) -> list[BandImages]:
+        """One BandImages per axion mass, in the order of set_axion_masses, accumulated since enable_mass_band_images /
+        reset_image (raises SartError while they are off)."""
+        return self._read_mass_bands(lib.sart_read_mass_band_images)
+
+    def read_merged_mass_band_images(self) -> list[BandImages]:
+        """read_mass_band_images of the last allreduce_outputs (raises SartError without one)."""
+        return self._read_mass_bands(lib.sart_read_merged_mass_band_images)
 
     def enable_quantity_hists(self, specs=None):
         """Weighted histograms of per-ray record quantities of the rays that pass in trace_mc (single axion mass;
